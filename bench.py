@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the PPO hot path (BASELINE.json metric: PPO env-steps/s and update samples/s).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c1|c4]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c1|c4] [--dump-outputs DIR]
 
 A "step" is one PPO update: rollout of n_steps x n_envs transitions on the GPU-resident synthetic 18-dim env
 (policy step + env + VecNormalize per env step, then GAE) followed by noptepochs x nminibatches train steps.
@@ -12,6 +12,9 @@ envs; per-minibatch gradients are allreduced with NCCL.
 
 --impl reference times the CPU restatement of the reference (oracle/, OpenMP over all host cores) on the same
 config — TensorFlow 1.14/Eigen are not installable, see DESIGN.md.
+
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy (see dump_outputs), so that two builds
+can be compared output for output: every input is seeded, the same arguments give the same inputs.
 """
 import argparse
 import json
@@ -26,6 +29,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree, which may be read-only
 
 WORKLOADS = {
     # name: (n_envs per GPU, n_steps, h1, h2, nminibatches, noptepochs, description)
@@ -193,6 +197,30 @@ class ClockSampler:
                 "samples": len(sm), "power_w_max": max(pw) if pw else None}
 
 
+DUMP_MAX_ROWS = 262144  # all of C3's rollout; 168 B per transition over the eight buffers keeps a dump under 64 MB
+
+
+def dump_outputs(core, c, out_dir):
+    """What a caller of the timed path holds after its last update, one DIR/<name>.npy each: the weights and the Adam state
+    (params, adam_m, adam_v, beta1_power, beta2_power), the VecNormalize statistics (vecnorm_*, counts in float64) and the
+    rollout buffers of that update (rollout_*, rows as ppo_rollout_get lays them out).  Rollouts of more than DUMP_MAX_ROWS
+    transitions are cut to the same seeded sample of rows in every run, whose indices go to rollout_rows.npy."""
+    import numpy as np
+    out = {name: c.get_tensor(name) for name in ("params", "adam_m", "adam_v", "beta1_power", "beta2_power")}
+    for k, v in c.vecnorm_stats().items():
+        out["vecnorm_" + k] = np.asarray(v, np.float64) if k.endswith("count") else v
+    rows = None
+    if c.n_batch > DUMP_MAX_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(c.n_batch, DUMP_MAX_ROWS, replace=False))
+        out["rollout_rows"] = rows.astype(np.float64)
+    for name in core.BUFFER_WIDTH:
+        buf = c.rollout_get(name)
+        out["rollout_" + name] = buf if rows is None else buf[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -265,6 +293,8 @@ def run_ours(args):
     t_wall1 = time.perf_counter()
     t_wall = t_wall1 - t_wall0
     ctr = c.counters()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(core, c, args.dump_outputs)  # before anything below moves the core's state on
     clocks = None
     if rank == 0:
         clocks = sampler.window(t_wall0, t_wall1)
@@ -517,9 +547,14 @@ def c5_microbench(hbm_peak):
 
 
 def main():
+    def positive(s):
+        if int(s) < 1:
+            raise argparse.ArgumentTypeError("must be at least 1")
+        return int(s)
+
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=positive, default=50, help="timed PPO updates")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS))
@@ -528,7 +563,10 @@ def main():
     ap.add_argument("--no-microbench", dest="microbench", action="store_false")
     ap.add_argument("--no-parity", dest="parity", action="store_false")
     ap.add_argument("--no-c4", dest="c4", action="store_false")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

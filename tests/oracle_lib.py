@@ -8,6 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -50,10 +51,13 @@ class LearnerDesc(C.Structure):
                 ("env_kind", C.c_int), ("threads", C.c_int)]
 
 
-def build(fast: bool = False) -> str:
-    target = "fast" if fast else "exact"
-    subprocess.run(["make", "-s", "-C", ORACLE_DIR, target], check=True)
-    return os.path.join(ORACLE_DIR, "_native/libppo_oracle_fast.so" if fast else "libppo_oracle.so")
+def build(fast: bool = False, native_dir: str = None) -> str:
+    """Path of the oracle library: the exact build in oracle/, or the -march=native fast build compiled into `native_dir`."""
+    if not fast:
+        subprocess.run(["make", "-s", "-C", ORACLE_DIR, "exact"], check=True)
+        return os.path.join(ORACLE_DIR, "libppo_oracle.so")
+    subprocess.run(["make", "-s", "-C", ORACLE_DIR, "fast", f"NATIVE_DIR={native_dir}"], check=True)
+    return os.path.join(native_dir, "libppo_oracle_fast.so")
 
 
 _libs = {}
@@ -62,8 +66,13 @@ _libs = {}
 def load(fast: bool = False):
     if fast in _libs:
         return _libs[fast]
-    path = build(fast)
-    lib = C.CDLL(path)
+    if fast:
+        # built for the host that runs it, outside the tree (bench.py must work from a read-only checkout); the directory
+        # can go once the library is mapped
+        with tempfile.TemporaryDirectory(prefix="ppo_oracle_fast_") as d:
+            lib = C.CDLL(build(True, d))
+    else:
+        lib = C.CDLL(build())
     vp = C.c_void_p
     lib.oracle_param_offset.argtypes = [C.POINTER(Dims), C.c_int]
     lib.oracle_param_offset.restype = C.c_int

@@ -10,8 +10,6 @@ import pytest
 from ppo_cpp_b200 import _lib, core
 from ppo_cpp_b200.meta_graph import TENSOR_ORDER, parse_meta_txt, write_meta_txt
 
-REF_GRAPH = "/root/reference/resources/ppo_cl/graphs/ppo_cpp_[4_5]_lr_0.0004_cr_0.1610_ent_0.0007.meta.txt"
-
 
 def test_library_exports_every_declared_symbol():
     lib = _lib.load()
@@ -44,19 +42,6 @@ def test_host_rand_matches_live_libc():
     libc.rand.restype = C.c_int
     libc.srand(987654321)
     assert core.host_rand(987654321, 5000).tolist() == [libc.rand() for _ in range(5000)]
-
-
-@pytest.mark.skipif(not os.path.exists(REF_GRAPH), reason="reference tree not present (GPU box)")
-def test_meta_parse_reference_graph(init_weights, kat):
-    info, params = core.meta_parse(REF_GRAPH)
-    c = kat["consts"]
-    assert (info.obs_dim, info.act_dim, info.hidden1, info.hidden2) == (18, 18, 4, 5)
-    assert (info.n_params_trainable, info.n_params_total) == (334, 442)
-    assert info.ent_coef == np.float32(c["ent_coef"]) and info.vf_coef == 0.5 and info.max_grad_norm == 0.5
-    assert info.adam_beta1 == np.float32(0.9) and info.adam_beta2 == np.float32(0.999) and info.adam_epsilon == np.float32(1e-5)
-    assert np.array_equal(params, init_weights[1])
-    py = parse_meta_txt(REF_GRAPH)
-    assert np.array_equal(py.flat_params(), params)
 
 
 def test_meta_parse_written_graph(tmp_path):
