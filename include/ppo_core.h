@@ -87,10 +87,23 @@ typedef struct {
  * n_params_total initial values in core order (see ppo_core_tensor_name). */
 int ppo_meta_parse(const char *meta_txt_path, ppo_meta_info *info, float *params_out, size_t params_capacity);
 
+/* Value-function loss of Stable-Baselines' PPO2 (SURVEY §3.5), fixed by `cliprange_vf` when the graph was exported:
+ *   SHARED    vc = old_v + clip(v - old_v, -cliprange, cliprange)        (cliprange_vf None: the shipped graph)
+ *   NONE      vc = v, no clipping                                         (cliprange_vf < 0: the original PPO loss)
+ *   SEPARATE  vc = old_v + clip(v - old_v, -cliprange_vf, cliprange_vf)   (cliprange_vf >= 0: placeholder loss/clip_range_vf_ph)
+ * vf_loss = 0.5 * mean(max((v - R)^2, (vc - R)^2)) in every mode. */
+typedef enum { PPO_VF_CLIP_SHARED = 0, PPO_VF_CLIP_NONE = 1, PPO_VF_CLIP_SEPARATE = 2 } ppo_vf_clip;
+/* the ppo_vf_clip of a graph file, read from the data flow of its loss sub-graph (a file without one, as written by
+ * meta_graph.write_meta_txt without vf_clip, is SHARED); PPO_ERR_UNSUPPORTED if the value loss is of no known form */
+int ppo_meta_vf_clip(const char *meta_txt_path);
+
 int ppo_core_create(const ppo_core_desc *desc, ppo_core **out);
 void ppo_core_destroy(ppo_core *core);
-/* load initial weights from the graph file; its shapes must match the desc (ppo2.hpp:90-105 reset()) */
+/* load initial weights from the graph file; its shapes must match the desc (ppo2.hpp:90-105 reset()); sets the core's ppo_vf_clip */
 int ppo_core_load_meta_txt(ppo_core *core, const char *meta_txt_path);
+/* the value loss of a graph-less core (default SHARED); ppo_core_load_meta_txt sets it from the graph */
+int ppo_core_set_vf_clip(ppo_core *core, int mode);
+int ppo_core_vf_clip(ppo_core *core); /* the core's ppo_vf_clip, or a negative ppo_status */
 /* Stable-Baselines' orthogonal init for graph-less configs (synthetic benchmarks with [64,64], [256,256]) */
 int ppo_core_init_orthogonal(ppo_core *core, uint64_t seed);
 /* TF Saver V2 bundle written by PPO2::save (ppo2.hpp:107-131): `<prefix>.data-00000-of-00001` holds the 15
@@ -191,6 +204,11 @@ int ppo_host_random_shuffle(unsigned seed, int n, int epochs, int *perms_out);  
 /* one whole update over the current rollout: noptepochs x nminibatches train steps with the
  * reference's permutation semantics; mean_losses[5] = pg, vf, entropy, approxkl, clipfrac (ppo2.hpp:335) */
 int ppo_train_update(ppo_core *core, float lr, float cliprange, float *mean_losses);
+/* ... with the value clip range of a SEPARATE graph (>= 0; ignored in the other modes).  The calls without _vf fail with
+ * PPO_ERR_INVALID on a SEPARATE core, as TensorFlow does on the unfed loss/clip_range_vf_ph.  lr, cliprange and
+ * cliprange_vf live in device memory, written on the core's stream before each call's work: the captured update graphs
+ * are replayed, not rebuilt, when they change from update to update (schedules, ppo2.hpp:264-335) */
+int ppo_train_update_vf(ppo_core *core, float lr, float cliprange, float cliprange_vf, float *mean_losses);
 /* finer grain for parity tests: set this epoch's permutation (perm.indices, n_batch ints) and run minibatch k;
  * losses[5] of that step; grads (may be NULL) = the unclipped gradient, n_params_trainable floats */
 int ppo_train_set_permutation(ppo_core *core, const int *perm, int n);
@@ -200,10 +218,14 @@ int ppo_train_set_permutation(ppo_core *core, const int *perm, int n);
  * (they depend on the rand() stream only) and this call returns PPO_ERR_INVALID. */
 int ppo_train_get_permutation(ppo_core *core, int epoch, int *out, int n);
 int ppo_train_minibatch(ppo_core *core, int k, float lr, float cliprange, float *losses, float *grads);
+int ppo_train_minibatch_vf(ppo_core *core, int k, float lr, float cliprange, float cliprange_vf, float *losses, float *grads);
 /* standalone pieces on caller data (host pointers): advantage normalisation (ppo2.hpp:401-406) and loss+grad */
 int ppo_advnorm(ppo_core *core, const float *returns, const float *values, int n, float *advs);
 int ppo_loss_grad(ppo_core *core, const float *obs, const float *actions, const float *advs, const float *returns,
                   const float *old_neglogp, const float *old_values, int B, float cliprange, float *grads, float *losses);
+int ppo_loss_grad_vf(ppo_core *core, const float *obs, const float *actions, const float *advs, const float *returns,
+                     const float *old_neglogp, const float *old_values, int B, float cliprange, float cliprange_vf, float *grads,
+                     float *losses);
 /* rollout + update on the synthetic env; env-steps/s accounting is the caller's (ppo2.hpp:337-341) */
 int ppo_learn_update_synthetic(ppo_core *core, float lr, float cliprange, float *mean_losses);
 
@@ -231,6 +253,8 @@ typedef struct {
     uint64_t h2d_bytes, d2h_bytes;
 } ppo_counters;
 int ppo_core_counters(ppo_core *core, ppo_counters *out, int reset);
+/* CUDA graphs captured and instantiated since create (rollout, permutations, update / epochs) */
+int ppo_core_graph_builds(ppo_core *core, uint64_t *out);
 /* which kernel family the core selected for this MLP shape: "which" = "train" | "policy";
  * returns e.g. "train_umma_kernel (tcgen05, bf16x3 split)", "train_fused_kernel (fp32 FFMA, weights in smem)",
  * "train_tile_kernel (fp32 FFMA, generic)"; NULL on bad arguments */

@@ -16,6 +16,7 @@ LIB_PATH = os.environ.get("PPO_CORE_LIB") or os.path.join(HERE, "libppo_core.so"
 HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "ppo_core.h")
 
 PPO_HOST, PPO_DEVICE = 0, 1
+PPO_VF_CLIP_SHARED, PPO_VF_CLIP_NONE, PPO_VF_CLIP_SEPARATE = 0, 1, 2
 PPO_COMM_ID_BYTES = 128
 PPO_IPC_HANDLE_BYTES = 64
 ABI_VERSION = 1
@@ -75,9 +76,12 @@ def load():
         "ppo_abi_version": ([], C.c_int),
         "ppo_core_desc_default": ([C.POINTER(CoreDesc)], C.c_int),
         "ppo_meta_parse": ([C.c_char_p, C.POINTER(MetaInfo), fp, C.c_size_t], C.c_int),
+        "ppo_meta_vf_clip": ([C.c_char_p], C.c_int),
         "ppo_core_create": ([C.POINTER(CoreDesc), C.POINTER(core)], C.c_int),
         "ppo_core_destroy": ([core], None),
         "ppo_core_load_meta_txt": ([core, C.c_char_p], C.c_int),
+        "ppo_core_set_vf_clip": ([core, C.c_int], C.c_int),
+        "ppo_core_vf_clip": ([core], C.c_int),
         "ppo_core_init_orthogonal": ([core, C.c_uint64], C.c_int),
         "ppo_core_load_checkpoint_data": ([core, C.c_char_p], C.c_int),
         "ppo_core_save_checkpoint_data": ([core, C.c_char_p], C.c_int),
@@ -115,11 +119,14 @@ def load():
         "ppo_host_srand_rand": ([C.c_uint, C.c_int, ip], C.c_int),
         "ppo_host_random_shuffle": ([C.c_uint, C.c_int, C.c_int, ip], C.c_int),
         "ppo_train_update": ([core, C.c_float, C.c_float, fp], C.c_int),
+        "ppo_train_update_vf": ([core, C.c_float, C.c_float, C.c_float, fp], C.c_int),
         "ppo_train_set_permutation": ([core, ip, C.c_int], C.c_int),
         "ppo_train_get_permutation": ([core, C.c_int, ip, C.c_int], C.c_int),
         "ppo_train_minibatch": ([core, C.c_int, C.c_float, C.c_float, fp, fp], C.c_int),
+        "ppo_train_minibatch_vf": ([core, C.c_int, C.c_float, C.c_float, C.c_float, fp, fp], C.c_int),
         "ppo_advnorm": ([core, fp, fp, C.c_int, fp], C.c_int),
         "ppo_loss_grad": ([core, fp, fp, fp, fp, fp, fp, C.c_int, C.c_float, fp, fp], C.c_int),
+        "ppo_loss_grad_vf": ([core, fp, fp, fp, fp, fp, fp, C.c_int, C.c_float, C.c_float, fp, fp], C.c_int),
         "ppo_learn_update_synthetic": ([core, C.c_float, C.c_float, fp], C.c_int),
         "ppo_comm_get_unique_id": ([C.c_char_p], C.c_int),
         "ppo_comm_init": ([core, C.c_char_p, C.c_int, C.c_int], C.c_int),
@@ -128,6 +135,7 @@ def load():
         "ppo_comm_error": ([core], C.c_int),
         "ppo_comm_set_p2p": ([core, C.c_int], C.c_int),
         "ppo_core_counters": ([core, C.POINTER(Counters), C.c_int], C.c_int),
+        "ppo_core_graph_builds": ([core, C.POINTER(C.c_uint64)], C.c_int),
         "ppo_core_kernel_family": ([core, C.c_char_p], C.c_char_p),
         "ppo_profile_kernel": ([core, C.c_char_p, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_int)], C.c_int),
     }

@@ -15,6 +15,9 @@ from . import _lib
 from ._lib import PPO_DEVICE, PPO_HOST, CoreDesc, Counters, MetaInfo
 
 LOSS_NAMES = ("pg_loss", "vf_loss", "entropy", "approxkl", "clipfrac")
+# the value losses of ppo_vf_clip (include/ppo_core.h), by the names write_meta_txt(vf_clip=...) takes
+VF_CLIP_MODES = {"shared": _lib.PPO_VF_CLIP_SHARED, "none": _lib.PPO_VF_CLIP_NONE, "separate": _lib.PPO_VF_CLIP_SEPARATE}
+VF_CLIP_NAMES = {v: k for k, v in VF_CLIP_MODES.items()}
 BUFFER_WIDTH = {"obs": None, "returns": 1, "dones": 1, "actions": None, "values": 1, "neglogpacs": 1,
                 "true_rewards": 1, "unnormalized_rewards": 1}
 
@@ -51,6 +54,15 @@ def meta_parse(path: str):
     params = np.zeros(info.n_params_total, np.float32)
     _check(lib, lib.ppo_meta_parse(path.encode(), C.byref(info), params.ctypes.data, params.size))
     return info, params
+
+
+def meta_vf_clip(path: str) -> str:
+    """Which value loss the graph file builds: "shared", "none" or "separate" (read by the C parser)."""
+    lib = _lib.load()
+    r = lib.ppo_meta_vf_clip(path.encode())
+    if r < 0:
+        _check(lib, r)
+    return VF_CLIP_NAMES[r]
 
 
 def host_rand(seed: int, count: int) -> np.ndarray:
@@ -107,6 +119,26 @@ class PPOCore:
     # ---- weights
     def load_meta_txt(self, path):
         _check(self.lib, self.lib.ppo_core_load_meta_txt(self._h, path.encode()))
+
+    @property
+    def vf_clip(self) -> str:
+        """The core's value loss: "shared" (the policy clip range), "none" (no clipping) or "separate" (cliprange_vf)."""
+        r = self.lib.ppo_core_vf_clip(self._h)
+        if r < 0:
+            _check(self.lib, r)
+        return VF_CLIP_NAMES[r]
+
+    @vf_clip.setter
+    def vf_clip(self, mode: str):
+        if mode not in VF_CLIP_MODES:
+            raise ValueError(f"vf_clip must be one of {sorted(VF_CLIP_MODES)}, not {mode!r}")
+        _check(self.lib, self.lib.ppo_core_set_vf_clip(self._h, VF_CLIP_MODES[mode]))
+
+    def graph_builds(self) -> int:
+        """CUDA graphs captured and instantiated since the core was created."""
+        n = C.c_uint64()
+        _check(self.lib, self.lib.ppo_core_graph_builds(self._h, C.byref(n)))
+        return n.value
 
     def init_orthogonal(self, seed=0):
         _check(self.lib, self.lib.ppo_core_init_orthogonal(self._h, seed))
@@ -292,9 +324,12 @@ class PPOCore:
     def shuffle_seed(self, seed):
         _check(self.lib, self.lib.ppo_shuffle_seed(self._h, seed))
 
-    def train_update(self, lr, cliprange, want_losses=True):
+    def train_update(self, lr, cliprange, want_losses=True, cliprange_vf=None):
         out = np.zeros(5, np.float32) if want_losses else None
-        _check(self.lib, self.lib.ppo_train_update(self._h, lr, cliprange, _addr(out)))
+        if cliprange_vf is None:
+            _check(self.lib, self.lib.ppo_train_update(self._h, lr, cliprange, _addr(out)))
+        else:
+            _check(self.lib, self.lib.ppo_train_update_vf(self._h, lr, cliprange, cliprange_vf, _addr(out)))
         return out
 
     def train_set_permutation(self, perm):
@@ -306,9 +341,12 @@ class PPOCore:
         _check(self.lib, self.lib.ppo_train_get_permutation(self._h, epoch, out.ctypes.data, out.size))
         return out
 
-    def train_minibatch(self, k, lr, cliprange):
+    def train_minibatch(self, k, lr, cliprange, cliprange_vf=None):
         losses, grads = np.zeros(5, np.float32), np.zeros(self.P, np.float32)
-        _check(self.lib, self.lib.ppo_train_minibatch(self._h, k, lr, cliprange, _addr(losses), _addr(grads)))
+        if cliprange_vf is None:
+            _check(self.lib, self.lib.ppo_train_minibatch(self._h, k, lr, cliprange, _addr(losses), _addr(grads)))
+        else:
+            _check(self.lib, self.lib.ppo_train_minibatch_vf(self._h, k, lr, cliprange, cliprange_vf, _addr(losses), _addr(grads)))
         return losses, grads
 
     def advnorm(self, returns, values):
@@ -317,12 +355,15 @@ class PPOCore:
         _check(self.lib, self.lib.ppo_advnorm(self._h, _addr(r), _addr(v), r.size, _addr(out)))
         return out
 
-    def loss_grad(self, obs, actions, advs, returns, old_neglogp, old_values, cliprange):
+    def loss_grad(self, obs, actions, advs, returns, old_neglogp, old_values, cliprange, cliprange_vf=None):
         o, a = _f32(obs), _f32(actions)
         ad, r, on, ov = _f32(advs).ravel(), _f32(returns).ravel(), _f32(old_neglogp).ravel(), _f32(old_values).ravel()
         grads, losses = np.zeros(self.P, np.float32), np.zeros(5, np.float32)
-        _check(self.lib, self.lib.ppo_loss_grad(self._h, _addr(o), _addr(a), _addr(ad), _addr(r), _addr(on), _addr(ov), o.shape[0],
-                                                cliprange, _addr(grads), _addr(losses)))
+        args = (self._h, _addr(o), _addr(a), _addr(ad), _addr(r), _addr(on), _addr(ov), o.shape[0], cliprange)
+        if cliprange_vf is None:
+            _check(self.lib, self.lib.ppo_loss_grad(*args, _addr(grads), _addr(losses)))
+        else:
+            _check(self.lib, self.lib.ppo_loss_grad_vf(*args, cliprange_vf, _addr(grads), _addr(losses)))
         return grads, losses
 
     def learn_update_synthetic(self, lr, cliprange, want_losses=True):

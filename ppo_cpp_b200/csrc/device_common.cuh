@@ -28,6 +28,36 @@ struct NetDims {
 // columns appended to every per-CTA partial gradient slab: loss sums
 enum { L_PG = 0, L_VF = 1, L_ENT = 2, L_KL = 3, L_CLIP = 4, L_PAD = 8 };
 
+// Per-update scalars of one core in device memory.  Written on the core's stream before each update (a one-thread
+// kernel, so the host never waits); the train kernels and the Adam steps read them there, so the captured update
+// graphs do not depend on their values and a learning-rate / clip-range schedule replays the same graphs.
+struct UpdateScalars {
+    float lr, cliprange, cliprange_vf, pad;
+};
+
+// Value-function loss of Stable-Baselines' PPO2 (ppo_vf_clip in ppo_core.h); uniform per launch
+enum { VF_CLIP_SHARED = 0, VF_CLIP_NONE = 1, VF_CLIP_SEPARATE = 2 };
+
+__host__ __device__ __forceinline__ float vf_clip_range(int mode, float cliprange, float cliprange_vf) {
+    return mode == VF_CLIP_SEPARATE ? cliprange_vf : cliprange;
+}
+
+// One sample's value loss (GRAPH:10213-10400): returns max(l1, l2) with l1 = (v - R)^2, l2 = (vc - R)^2,
+// vc = old_v + clip(v - old_v, -range, range), and sets dv = dL/dv = vf_coef * 0.5/B * d max(l1, l2)/dv.
+// TF's tie rules: Maximum's gradient goes to l1 on l1 >= l2, clip_by_value's passes on -range <= v - old_v <= range.
+// VF_CLIP_NONE is vc = v exactly (not an infinite range: old_v + (v - old_v) is not v in fp32, and the tie would
+// then fall on either branch by rounding), so l2 == l1 and the tie takes the unclipped branch.
+__device__ __forceinline__ float value_loss_term(int mode, float range, float v, float oldv, float R, float vf_coef, float invB, float& dv) {
+    const bool none = mode == VF_CLIP_NONE;
+    const float dvo = v - oldv;
+    const float vc = none ? v : oldv + fmaxf(fminf(dvo, range), -range);
+    const float l1 = (v - R) * (v - R), l2 = (vc - R) * (vc - R);
+    const bool tk = l1 >= l2;
+    const bool inr = none || ((dvo <= range) && (dvo >= -range));
+    dv = vf_coef * 0.5f * invB * (tk ? 2.f * (v - R) : (inr ? 2.f * (vc - R) : 0.f));
+    return tk ? l1 : l2;
+}
+
 // 0.5*log(2*pi), 0.5*log(2*pi*e) as the fp32 constants baked in the graph (GRAPH:6103-6672, 10021-10180)
 #define PPO_HALF_LOG_2PI 0.9189385175704956f
 #define PPO_HALF_LOG_2PIE 1.4189385175704956f

@@ -831,7 +831,8 @@ struct AdamArgs {
     const float* grad;         // [PS] summed over CTAs (and ranks); columns P.. hold the loss sums
     const double* sq_partial;  // [nblk]
     int nblk, P;
-    float lr, beta1, beta2, eps, clip_norm;
+    const UpdateScalars* sc;  // lr of this update (device)
+    float beta1, beta2, eps, clip_norm;
     const float* bpow_in;  // [2] beta1_power, beta2_power
     float* bpow_out;       // [2]
     float invB, inv_world;
@@ -842,6 +843,7 @@ struct AdamArgs {
 __global__ void adam_kernel(const AdamArgs a) {
     __shared__ float s_scale;
     __shared__ double s_ss[256];
+    const float lr = a.sc->lr;
     {  // sum of the per-block partials in a fixed order: strided per thread, then a tree (every block does the same)
         double t = 0.0;
         for (int b = threadIdx.x; b < a.nblk; b += blockDim.x) t += a.sq_partial[b];
@@ -875,7 +877,7 @@ __global__ void adam_kernel(const AdamArgs a) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.P) return;
     const float b1p = a.bpow_in[0], b2p = a.bpow_in[1];
-    const float alpha = __fdiv_rn(__fmul_rn(a.lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
+    const float alpha = __fdiv_rn(__fmul_rn(lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
     const float g = __fmul_rn(a.grad[i], s_scale);
     float m = a.m[i], v = a.v[i];
     m = __fadd_rn(m, __fmul_rn(__fsub_rn(g, m), __fsub_rn(1.0f, a.beta1)));
@@ -1020,6 +1022,7 @@ __device__ __forceinline__ void reduce_adam_device(const ReduceAdamArgs& r, int 
     float am = mine ? __ldcg(a.m + c) : 0.f;
     float av = mine ? __ldcg(a.v + c) : 0.f;
     const float ap = mine ? __ldcg(a.params + c) : 0.f;
+    const float lr = a.sc->lr;  // (ahead of the exchange as well: after it, its latency would add to every minibatch)
     RA_PROF();
     const bool ll = r.sq_ll != nullptr;  // (nblk <= 256)
     if (ll) {
@@ -1082,7 +1085,7 @@ __device__ __forceinline__ void reduce_adam_device(const ReduceAdamArgs& r, int 
         loss_row[4] = L[L_CLIP] * a.invB;
     }
     if (mine) {
-        const float alpha = __fdiv_rn(__fmul_rn(a.lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
+        const float alpha = __fdiv_rn(__fmul_rn(lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
         const float g = __fmul_rn(gsum[0], s_scale);
         am = __fadd_rn(am, __fmul_rn(__fsub_rn(g, am), __fsub_rn(1.0f, a.beta1)));
         av = __fadd_rn(av, __fmul_rn(__fsub_rn(__fmul_rn(g, g), av), __fsub_rn(1.0f, a.beta2)));
@@ -1127,6 +1130,7 @@ __global__ void __launch_bounds__(256) grad_reduce_adam_big_kernel(const ReduceA
     const int world = r.mbox.world;
     const unsigned seq = world > 1 ? (*r.mbox_seq + 1u) : 0u;
     const float b1p = a.bpow_in[0], b2p = a.bpow_in[1];
+    const float lr = a.sc->lr;
     double q = 0.0;
     for (int chunk0 = blk; chunk0 < nchunks; chunk0 += 4 * nblk) {  // pass A, four chunks per trip: their loads are in flight together
         float acc[4] = {0.f, 0.f, 0.f, 0.f};
@@ -1214,7 +1218,7 @@ __global__ void __launch_bounds__(256) grad_reduce_adam_big_kernel(const ReduceA
         a.loss_row[4] = L[L_CLIP] * a.invB;
     }
     if (rg == 0) {  // pass C, four chunks per trip: the sixteen loads of a trip are in flight together
-        const float alpha = __fdiv_rn(__fmul_rn(a.lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
+        const float alpha = __fdiv_rn(__fmul_rn(lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
         for (int chunk0 = blk; chunk0 < nchunks; chunk0 += 4 * nblk) {
             float gg[4], mm[4], vv[4], pp[4];
 #pragma unroll

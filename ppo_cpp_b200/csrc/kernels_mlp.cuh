@@ -329,7 +329,9 @@ struct TrainArgs {
     const float* adv_direct;                    // already-normalised advantages per slot (ppo_loss_grad), or NULL
     int slot0, count;                           // this rank processes slots [slot0, slot0+count)
     float invB;                                 // 1 / (global minibatch size)
-    float cliprange, ent_coef, vf_coef;
+    const UpdateScalars* sc;                    // cliprange, cliprange_vf of this update (device)
+    int vf_mode;                                // VF_CLIP_*
+    float ent_coef, vf_coef;
     float* partial;  // [gridDim.x][PS]
     int PS;
     long long* prof;  // optional [2][32] phase timestamps of CTA 0 of each tower (U family, PPO_UMMA_PROF=1)
@@ -362,7 +364,8 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
     const int tid = threadIdx.x;
     float* my = a.partial + (size_t)blockIdx.x * a.PS;
     const int ntiles = (a.count + TM - 1) / TM;
-    const float lo = 1.f - a.cliprange, hi = 1.f + a.cliprange;
+    const float cr = a.sc->cliprange, vr = vf_clip_range(a.vf_mode, cr, a.sc->cliprange_vf);
+    const float lo = 1.f - cr, hi = 1.f + cr;
     float l_pg = 0.f, l_vf = 0.f, l_kl = 0.f, l_cf = 0.f;
     bool acc = false;
 
@@ -419,7 +422,7 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
                 l_pg += take1 ? pg1 : pg2;
                 const float dn = nlp - oldn;
                 l_kl += dn * dn;
-                l_cf += (fabsf(ratio - 1.f) > a.cliprange) ? 1.f : 0.f;
+                l_cf += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
                 g_nlp = take1 ? (adv * ratio) * a.invB : 0.f;
             }
             for (int j = 0; j < d.A; ++j) {
@@ -454,14 +457,7 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
             const int m = tid;
             float dv = 0.f;
             if (m < nv) {
-                const float v = MU[m], oldv = s_oldv[m], R = s_ret[m];
-                const float dvo = v - oldv;
-                const float vc = oldv + fmaxf(fminf(dvo, a.cliprange), -a.cliprange);  // GRAPH:10213-10305
-                const float l1 = (v - R) * (v - R), l2 = (vc - R) * (vc - R);
-                const bool take1 = l1 >= l2;  // ties -> unclipped (GRAPH:14975-15142)
-                l_vf += take1 ? l1 : l2;
-                const bool inr = (dvo <= a.cliprange) && (dvo >= -a.cliprange);
-                dv = a.vf_coef * 0.5f * a.invB * (take1 ? 2.f * (v - R) : (inr ? 2.f * (vc - R) : 0.f));
+                l_vf += value_loss_term(a.vf_mode, vr, MU[m], s_oldv[m], s_ret[m], a.vf_coef, a.invB, dv);  // GRAPH:10213-10305, 14975-15142
             }
             MU[m] = dv;
         }

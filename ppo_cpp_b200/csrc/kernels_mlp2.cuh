@@ -261,7 +261,8 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
     float* D1 = smem + L.d1[tw];
     float* my = a.partial + (size_t)blockIdx.x * a.PS;
     const int ntiles = (a.count + TM - 1) / TM;
-    const float lo = 1.f - a.cliprange, hi = 1.f + a.cliprange;
+    const float cr = a.sc->cliprange, vr = vf_clip_range(a.vf_mode, cr, a.sc->cliprange_vf);
+    const float lo = 1.f - cr, hi = 1.f + cr;
 
     stage_weights<NTH>(sW, a.params, d.P);
     // rows of ones behind every activation matrix (bias gradients fall out of the dW GEMM)
@@ -354,16 +355,10 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
                     l_pg += take1 ? pg1 : pg2;
                     const float dn = nlp - oldn;
                     l_kl += dn * dn;
-                    l_cf += (fabsf(ratio - 1.f) > a.cliprange) ? 1.f : 0.f;
-                    // value loss (GRAPH:10213-10400)
-                    const float v = Vs[m], oldv = s_oldv[m], R = s_ret[m];
-                    const float dvo = v - oldv;
-                    const float vc = oldv + fmaxf(fminf(dvo, a.cliprange), -a.cliprange);
-                    const float l1 = (v - R) * (v - R), l2 = (vc - R) * (vc - R);
-                    const bool tk = l1 >= l2;
-                    l_vf += tk ? l1 : l2;
-                    const bool inr = (dvo <= a.cliprange) && (dvo >= -a.cliprange);
-                    Vs[m] = a.vf_coef * 0.5f * a.invB * (tk ? 2.f * (v - R) : (inr ? 2.f * (vc - R) : 0.f));
+                    l_cf += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
+                    float dv;
+                    l_vf += value_loss_term(a.vf_mode, vr, Vs[m], s_oldv[m], s_ret[m], a.vf_coef, a.invB, dv);  // GRAPH:10213-10400
+                    Vs[m] = dv;
                 }
             } else if (jg == 0) {
                 Vs[m] = 0.f;

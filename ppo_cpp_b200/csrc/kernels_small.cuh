@@ -70,7 +70,7 @@ struct SmallAcc {
 // One warp tile (32 samples, one per lane): forward, loss, backward; the per-parameter contributions summed over the warp into acc
 template <int O, int A, int H1, int H2>
 __device__ __forceinline__ void small_warp_tile(const TrainArgs& a, const float* __restrict__ sW, int slot, bool valid, const float2* mbstats,
-                                                const float (&sd)[A], const float (&isd)[A], float sum_ls, float lo, float hi,
+                                                const float (&sd)[A], const float (&isd)[A], float sum_ls,
                                                 SmallAcc<Dims<O, A, H1, H2>::GROUPS>& acc, float* tile, int lane) {
     using D = Dims<O, A, H1, H2>;
     float (&accg)[D::GROUPS] = acc.accg;
@@ -153,6 +153,8 @@ __device__ __forceinline__ void small_warp_tile(const TrainArgs& a, const float*
             }
             float g_nlp = 0.f;
             if (valid) {
+                // the clip ranges are loaded where they are used: kept live across the loop they cost the epoch kernel spills
+                const float cr = a.sc->cliprange, lo = 1.f - cr, hi = 1.f + cr;
                 const float nlp = (0.5f * ss + PPO_HALF_LOG_2PI * (float)A) + sum_ls;
                 const float ratio = expf(oldn - nlp);                          // GRAPH:10423-10447
                 const float pg1 = -adv * ratio;
@@ -162,15 +164,9 @@ __device__ __forceinline__ void small_warp_tile(const TrainArgs& a, const float*
                 l_pg += take1 ? pg1 : pg2;
                 const float dn = nlp - oldn;
                 l_kl += dn * dn;
-                l_cf += (fabsf(ratio - 1.f) > a.cliprange) ? 1.f : 0.f;
-                // value loss (GRAPH:10213-10400)
-                const float dvo = v - oldv;
-                const float vc = oldv + fmaxf(fminf(dvo, a.cliprange), -a.cliprange);
-                const float l1 = (v - R) * (v - R), l2 = (vc - R) * (vc - R);
-                const bool tk = l1 >= l2;  // ties -> unclipped branch
-                l_vf += tk ? l1 : l2;
-                const bool inr = (dvo <= a.cliprange) && (dvo >= -a.cliprange);
-                dv = a.vf_coef * 0.5f * a.invB * (tk ? 2.f * (v - R) : (inr ? 2.f * (vc - R) : 0.f));
+                l_cf += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
+                const float vr = vf_clip_range(a.vf_mode, cr, a.sc->cliprange_vf);
+                l_vf += value_loss_term(a.vf_mode, vr, v, oldv, R, a.vf_coef, a.invB, dv);  // GRAPH:10213-10400
             }
 #pragma unroll
             for (int j = 0; j < A; ++j) {
@@ -247,7 +243,6 @@ __global__ void __launch_bounds__(NTH) train_small_kernel(const TrainArgs a) {
         isd[j] = 1.f / sd[j];
         sum_ls += ls;
     }
-    const float lo = 1.f - a.cliprange, hi = 1.f + a.cliprange;
     SmallAcc<D::GROUPS> acc;
     acc.clear();
 
@@ -255,7 +250,7 @@ __global__ void __launch_bounds__(NTH) train_small_kernel(const TrainArgs a) {
     for (int wt = blockIdx.x * (NTH / 32) + warp; wt < nwarp_tiles; wt += gridDim.x * (NTH / 32)) {
         const int slot = a.slot0 + wt * 32 + lane;
         const bool valid = wt * 32 + lane < a.count;
-        small_warp_tile<O, A, H1, H2>(a, sW, slot, valid, a.mbstats, sd, isd, sum_ls, lo, hi, acc, s_tile[warp], lane);
+        small_warp_tile<O, A, H1, H2>(a, sW, slot, valid, a.mbstats, sd, isd, sum_ls, acc, s_tile[warp], lane);
     }
     float (&accg)[D::GROUPS] = acc.accg;
     const float l_pg = acc.l_pg, l_vf = acc.l_vf, l_kl = acc.l_kl, l_cf = acc.l_cf;
@@ -450,7 +445,6 @@ __global__ void __launch_bounds__(NTH) train_small_epoch_kernel(const TrainArgs 
         sV[i] = __ldcg(ad.v + i);
     }
     float b1p = ad.bpow_in[0], b2p = ad.bpow_in[1];
-    const float lo = 1.f - a.cliprange, hi = 1.f + a.cliprange;
     const int nwarp_tiles = (a.count + 31) / 32;
     __syncthreads();
     for (int mb = 0; mb < ep.M; ++mb) {
@@ -468,7 +462,7 @@ __global__ void __launch_bounds__(NTH) train_small_epoch_kernel(const TrainArgs 
         for (int wt = warp; wt < nwarp_tiles; wt += NTH / 32) {
             const int slot = mb * ep.B + a.slot0 + wt * 32 + lane;
             const bool valid = wt * 32 + lane < a.count;
-            small_warp_tile<O, A, H1, H2>(a, sW, slot, valid, ep.mbstats + mb, sd, isd, sum_ls, lo, hi, acc, s_tile[warp], lane);
+            small_warp_tile<O, A, H1, H2>(a, sW, slot, valid, ep.mbstats + mb, sd, isd, sum_ls, acc, s_tile[warp], lane);
         }
         // ---- combine the warps in a fixed order (as train_small_kernel), gradient of parameter i in thread i % NTH
 #pragma unroll
@@ -524,7 +518,7 @@ __global__ void __launch_bounds__(NTH) train_small_epoch_kernel(const TrainArgs 
         }
         __syncthreads();  // thread 0 has read logstd before it moves
         // ---- TF ApplyAdam (epsilon outside the sqrt), in place in shared memory
-        const float alpha = __fdiv_rn(__fmul_rn(ad.lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
+        const float alpha = __fdiv_rn(__fmul_rn(ad.sc->lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
 #pragma unroll
         for (int u = 0; u < PT; ++u) {
             const int i = tid + u * NTH;

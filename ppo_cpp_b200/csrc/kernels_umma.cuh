@@ -539,7 +539,8 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
     const uint32_t id_v8 = make_idesc(64, 8, 1, 0);       // H2_lo^T x dv_hi
     const uint32_t id_s16 = make_idesc(128, 16, 1, 0);    // column sums: MN-major [A_hi ; A_lo] x K-major ones
 
-    const float lo = 1.f - a.cliprange, hi = 1.f + a.cliprange;
+    const float cr = a.sc->cliprange, vr = vf_clip_range(a.vf_mode, cr, a.sc->cliprange_vf);
+    const float lo = 1.f - cr, hi = 1.f + cr;
     // the backward tensors (which carry the 1/B of the batch mean) are stored times a power of two so that they are O(1) as
     // fp16 operands (see the header); exponents are chosen per minibatch when the weights are staged
     int invB_exp;
@@ -871,7 +872,7 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
                         l_0 += take1 ? pg1 : pg2;
                         const float dn = nlp - oldn;
                         l_1 += dn * dn;
-                        l_2 += (fabsf(ratio - 1.f) > a.cliprange) ? 1.f : 0.f;
+                        l_2 += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
                     }
                 }
                 if (half == 0) {
@@ -914,13 +915,7 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
                 float dv = 0.f;
                 if (valid) {
                     const float v = (f32[F32_PV + row] + f32[F32_PV + TM + row]) + f32[F32_MISC + 0];
-                    const float dvo = v - c_oldv;
-                    const float vc = c_oldv + fmaxf(fminf(dvo, a.cliprange), -a.cliprange);
-                    const float l1 = (v - c_ret) * (v - c_ret), l2 = (vc - c_ret) * (vc - c_ret);
-                    const bool tk = l1 >= l2;  // ties -> unclipped branch
-                    l_0 += tk ? l1 : l2;
-                    const bool inr = (dvo <= a.cliprange) && (dvo >= -a.cliprange);
-                    dv = a.vf_coef * 0.5f * a.invB * (tk ? 2.f * (v - c_ret) : (inr ? 2.f * (vc - c_ret) : 0.f));
+                    l_0 += value_loss_term(a.vf_mode, vr, v, c_oldv, c_ret, a.vf_coef, a.invB, dv);
                     l_dbv += dv;
                     dv *= S_b;  // as an operand: times S
                 }

@@ -389,7 +389,7 @@ __global__ void __launch_bounds__(GEMM_NTH, 1) wgemm_kernel(const GemmArgs g) {
                     if (k.tower == 0) {
                         float l_pg = 0.f, l_kl = 0.f, l_cf = 0.f;
                         if (valid) {
-                            const float lo = 1.f - a.cliprange, hi = 1.f + a.cliprange;
+                            const float cr = a.sc->cliprange, lo = 1.f - cr, hi = 1.f + cr;
                             float z[A], isd[A];
                             float ss = 0.f, sl = 0.f;
 #pragma unroll
@@ -408,7 +408,7 @@ __global__ void __launch_bounds__(GEMM_NTH, 1) wgemm_kernel(const GemmArgs g) {
                             l_pg = take1 ? pg1 : pg2;
                             const float dn = nlp - oldn;
                             l_kl = dn * dn;
-                            l_cf = (fabsf(ratio - 1.f) > a.cliprange) ? 1.f : 0.f;
+                            l_cf = (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
                             const float g_nlp = take1 ? (adv * ratio) * a.invB : 0.f;
 #pragma unroll
                             for (int j = 0; j < A; ++j) {
@@ -435,13 +435,8 @@ __global__ void __launch_bounds__(GEMM_NTH, 1) wgemm_kernel(const GemmArgs g) {
                         float dv = 0.f, l_vf = 0.f;
                         if (valid) {
                             const float vv = fmaf(mu[0], u_hd, __ldg(P + d.off[T_VF_B]));
-                            const float dvo = vv - oldv;
-                            const float vc = oldv + fmaxf(fminf(dvo, a.cliprange), -a.cliprange);
-                            const float l1 = (vv - ret) * (vv - ret), l2 = (vc - ret) * (vc - ret);
-                            const bool tk = l1 >= l2;  // ties -> unclipped branch
-                            l_vf = tk ? l1 : l2;
-                            const bool inr = (dvo <= a.cliprange) && (dvo >= -a.cliprange);
-                            dv = a.vf_coef * 0.5f * a.invB * (tk ? 2.f * (vv - ret) : (inr ? 2.f * (vc - ret) : 0.f));
+                            const float vr = vf_clip_range(a.vf_mode, a.sc->cliprange, a.sc->cliprange_vf);
+                            l_vf = value_loss_term(a.vf_mode, vr, vv, oldv, ret, a.vf_coef, a.invB, dv);
                         }
                         v[0] = dv * S_b;
                         const float t0 = warp_sum(dv), t2 = warp_sum(l_vf);

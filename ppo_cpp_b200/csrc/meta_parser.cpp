@@ -188,6 +188,64 @@ bool const_tensor(const Msg& node, MetaTensor& t) {
     return true;
 }
 
+using NodeMap = std::map<std::string, const Msg*>;
+
+// data inputs of a node ("name:0" -> "name"; control inputs "^name" skipped)
+std::vector<std::string> node_inputs(const Msg& node) {
+    std::vector<std::string> in;
+    for (const auto& f : node.fields) {
+        if (f.key != "input" || f.scalar.empty() || f.scalar[0] == '^') continue;
+        const size_t colon = f.scalar.find(':');
+        in.push_back(colon == std::string::npos ? f.scalar : f.scalar.substr(0, colon));
+    }
+    return in;
+}
+
+// Stable-Baselines' PPO2 builds vf_loss = 0.5 * mean(max(square(vpred - R), square(vpred_clipped - R))) with
+//   vpred_clipped = vpred                                                      (cliprange_vf < 0: no clipping)
+//   vpred_clipped = old_vpred_ph + clip_by_value(vpred - old_vpred_ph, -b, b)  (b = loss/clip_range_ph or loss/clip_range_vf_ph)
+// Classified by following the data flow from the second operand of loss/Maximum back through its Square and Sub.
+int classify_vf_clip(const NodeMap& nodes, std::string& err) {
+    auto node = [&](const std::string& name, const char* op) -> const Msg* {
+        auto it = nodes.find(name);
+        return it != nodes.end() && it->second->str("op") == op ? it->second : nullptr;
+    };
+    auto sub_of_square = [&](const std::string& sq, std::vector<std::string>& ins) -> bool {
+        const Msg* s = node(sq, "Square");
+        if (!s || node_inputs(*s).size() != 1) return false;
+        const Msg* d = node(node_inputs(*s)[0], "Sub");
+        if (!d) return false;
+        ins = node_inputs(*d);
+        return ins.size() == 2;
+    };
+    if (nodes.find("loss/Maximum") == nodes.end()) return 0;  // no loss sub-graph (files of write_meta_txt): the shipped graph's form
+    const Msg* mx = node("loss/Maximum", "Maximum");
+    const std::vector<std::string> mi = mx ? node_inputs(*mx) : std::vector<std::string>();
+    std::vector<std::string> s1, s2;
+    if (mi.size() != 2 || !sub_of_square(mi[0], s1) || !sub_of_square(mi[1], s2) || s1[1] != s2[1]) {
+        err = "loss/Maximum is not max(square(vpred - R), square(vpred_clipped - R))";
+        return -1;
+    }
+    if (s2[0] == s1[0]) return 1;  // vpred_clipped is vpred itself
+    const Msg* add = node(s2[0], "Add");
+    std::vector<std::string> ai = add ? node_inputs(*add) : std::vector<std::string>();
+    if (ai.size() == 2 && ai[1] == "loss/old_vpred_ph") std::swap(ai[0], ai[1]);
+    const Msg* clip = ai.size() == 2 && ai[0] == "loss/old_vpred_ph" ? node(ai[1], "Maximum") : nullptr;  // clip_by_value = max(min(x, b), -b)
+    const std::vector<std::string> ci = clip ? node_inputs(*clip) : std::vector<std::string>();
+    const Msg* mn = ci.size() == 2 ? node(ci[0], "Minimum") : nullptr;
+    const Msg* neg = ci.size() == 2 ? node(ci[1], "Neg") : nullptr;
+    const std::vector<std::string> ni = mn ? node_inputs(*mn) : std::vector<std::string>();
+    const std::vector<std::string> gi = neg ? node_inputs(*neg) : std::vector<std::string>();
+    if (ni.size() != 2 || gi.size() != 1 || ni[1] != gi[0]) {
+        err = "the clipped value " + s2[0] + " is neither vpred nor old_vpred_ph + clip_by_value(..., -b, b)";
+        return -1;
+    }
+    if (ni[1] == "loss/clip_range_ph") return 0;
+    if (ni[1] == "loss/clip_range_vf_ph") return 2;
+    err = "the value clip bound " + ni[1] + " is neither loss/clip_range_ph nor loss/clip_range_vf_ph";
+    return -1;
+}
+
 }  // namespace
 
 std::string parse_meta_txt(const std::string& path, MetaGraph& out) {
@@ -201,9 +259,10 @@ std::string parse_meta_txt(const std::string& path, MetaGraph& out) {
     if (!ps.parse_msg(root, true)) return "cannot parse " + path + ": " + (ps.err.empty() ? "unbalanced braces" : ps.err);
     const Msg* graph = root.sub("graph_def");
     if (!graph) return "no graph_def in " + path;
-    std::map<std::string, const Msg*> nodes;
+    NodeMap nodes;
     for (const auto& f : graph->fields)
         if (f.key == "node" && f.msg) nodes[f.msg->str("name")] = f.msg.get();
+    out.vf_clip = classify_vf_clip(nodes, out.vf_clip_error);
 
     for (int i = 0; i < kNumTensors; ++i) {
         const std::string name = kTensorNames[i];

@@ -1,6 +1,7 @@
 // Minimal reader for TensorFlow-1.14 text-proto MetaGraphDef files (.meta.txt).
 // Replaces SessionCreator::load_graph (reference ppo2/session_creator.hpp:23-57): the graph is read,
-// never executed.  Extracts variable shapes, initial values and the constants the graph bakes in.
+// never executed.  Extracts variable shapes, initial values, the constants the graph bakes in and which value loss
+// the graph builds.
 #pragma once
 #include <map>
 #include <string>
@@ -16,6 +17,10 @@ struct MetaTensor {
 struct MetaGraph {
     int obs_dim = 0, act_dim = 0, hidden1 = 0, hidden2 = 0;
     float ent_coef = 0, vf_coef = 0, clip_norm = 0, beta1 = 0, beta2 = 0, adam_eps = 0;
+    // value loss of the graph (ppo_vf_clip: 0 shared clip range, 1 no clipping, 2 own range loss/clip_range_vf_ph), or -1
+    // when the loss sub-graph is there but matches none of them (vf_clip_error says why)
+    int vf_clip = 0;
+    std::string vf_clip_error;
     std::map<std::string, MetaTensor> tensors;  // the 15 model/* variables with their initial values
 };
 

@@ -7,9 +7,11 @@
 #include <chrono>
 #include <cmath>
 #include <fstream>
+#include <functional>
 #include <iostream>
 #include <memory>
 #include <sstream>
+#include <stdexcept>
 #include <string>
 #include <vector>
 
@@ -62,6 +64,14 @@ public:
         shuffle_seed_ = shuffle_seed;
         noise_seed_ = noise_seed;
         if (core_) reset();
+    }
+    // Stable-Baselines' schedules (an addition over the reference, whose PPO2 takes constants): each is evaluated once per
+    // update at frac = 1 - (update - 1) / n_updates, as ppo2.py does; the constructor's floats are the constant schedules.
+    // An empty function keeps that constant.
+    void set_schedules(std::function<float(float)> lr, std::function<float(float)> cr, std::function<float(float)> cr_vf) {
+        lr_schedule_ = std::move(lr);
+        cr_schedule_ = std::move(cr);
+        cr_vf_schedule_ = std::move(cr_vf);
     }
     // graph-less construction for sizes the reference ships no graph for (orthogonal init as Stable-Baselines)
     void reset_without_graph(int hidden1, int hidden2, uint64_t init_seed) {
@@ -191,7 +201,17 @@ public:
             assert(false);
             return;
         }
-        if (cliprange_vf >= 0.f) std::cout << "cliprange_vf is ignored: the graph clips the value with cliprange (SURVEY 3.5)" << std::endl;
+        // the value loss is fixed by the graph (SURVEY 3.5): only a graph with loss/clip_range_vf_ph takes cliprange_vf
+        const bool separate = ppo_core_vf_clip(core_.get()) == PPO_VF_CLIP_SEPARATE;
+        if (separate && !cr_vf_schedule_ && cliprange_vf < 0.f) {
+            std::cerr << "the graph clips the value with its own range (loss/clip_range_vf_ph): cliprange_vf must be >= 0, got " << cliprange_vf << std::endl;
+            throw std::runtime_error("PPO2::learn: the graph needs cliprange_vf >= 0");
+        }
+        if (!separate && cliprange_vf >= 0.f) {
+            std::cout << (ppo_core_vf_clip(core_.get()) == PPO_VF_CLIP_NONE ? "cliprange_vf is ignored: the graph does not clip the value"
+                                                                            : "cliprange_vf is ignored: the graph clips the value with cliprange (SURVEY 3.5)")
+                      << std::endl;
+        }
         _init_num_timesteps();
         Runner runner{env, *act_model, n_steps, gamma, lam};
         std::vector<float> episode_reward(n_envs, 0.f);
@@ -206,7 +226,12 @@ public:
             runner.run(false);
             num_timesteps += n_batch;
             float loss_vals[5];
-            ppo_check(ppo_train_update(core_.get(), learning_rate, cliprange, loss_vals), "train");
+            const float frac = 1.0f - (static_cast<float>(update) - 1.0f) / static_cast<float>(n_updates);
+            const float lr_now = lr_schedule_ ? lr_schedule_(frac) : learning_rate;
+            const float cr_now = cr_schedule_ ? cr_schedule_(frac) : cliprange;
+            const float cr_vf_now = cr_vf_schedule_ ? cr_vf_schedule_(frac) : cliprange_vf;
+            if (separate) ppo_check(ppo_train_update_vf(core_.get(), lr_now, cr_now, cr_vf_now, loss_vals), "train");
+            else ppo_check(ppo_train_update(core_.get(), lr_now, cr_now, loss_vals), "train");
             auto t_now = std::chrono::system_clock::now();
             auto duration = std::chrono::duration_cast<std::chrono::microseconds>(t_now - t_start).count();
             last_fps = static_cast<long>(static_cast<double>(n_batch) * 1e6 / static_cast<double>(duration > 0 ? duration : 1));
@@ -265,6 +290,7 @@ private:
     int noptepochs;
     float cliprange;
     float cliprange_vf;
+    std::function<float(float)> lr_schedule_, cr_schedule_, cr_vf_schedule_;
     std::string tensorboard_log;
     int n_batch = 0;
     unsigned shuffle_seed_ = 1;

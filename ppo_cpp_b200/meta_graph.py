@@ -5,7 +5,8 @@ this framework has no TensorFlow, so the graph file is only *read*: hidden sizes
 ``VariableV2`` shapes of ``model/{pi,vf}_fc{k}/w``, the initial weights from the ``Const``
 ``tensor_content`` of ``model/*/Initializer/*`` and the constants that the graph bakes in
 (entropy coefficient ``loss/mul_4/y``, value coefficient ``loss/mul_5/y``, clip norm
-``loss/clip_by_global_norm/mul/x``, Adam ``ppo2/_train/{beta1,beta2,epsilon}``).
+``loss/clip_by_global_norm/mul/x``, Adam ``ppo2/_train/{beta1,beta2,epsilon}``) and which value loss the
+graph builds (``vf_clip``, see ``classify_vf_clip``).
 
 This is the Python twin of ``csrc/meta_parser.cpp`` (the one the product path uses); tests check that
 both agree on the reference fixture.  No protobuf dependency: a 60-line recursive text-proto reader.
@@ -105,6 +106,7 @@ class MetaInfo:
     beta2: float
     adam_eps: float
     tf_version: str = ""
+    vf_clip: str = "shared"
     shapes: Dict[str, Tuple[int, ...]] = field(default_factory=dict)
 
     def flat_params(self, include_q: bool = True) -> np.ndarray:
@@ -131,6 +133,57 @@ def _tensor_value(node: dict) -> np.ndarray:
     else:  # all-zero tensors carry neither field
         arr = np.zeros(count, dtype=np.float32)
     return arr.reshape(dims) if dims else arr.reshape(())
+
+
+def _inputs(node: dict) -> List[str]:
+    """Data inputs of a node ("name:0" -> "name"; control inputs "^name" skipped)."""
+    return [i.decode().split(":")[0] for i in node.get("input", []) if not i.startswith(b"^")]
+
+
+def classify_vf_clip(nodes: Dict[str, dict]) -> str:
+    """The value loss of Stable-Baselines' PPO2, vf_loss = 0.5 * mean(max(square(vpred - R), square(vpred_clipped - R))):
+    "none" (vpred_clipped is vpred), "shared" / "separate" (old_vpred_ph + clip_by_value(vpred - old_vpred_ph, -b, b) with
+    b = loss/clip_range_ph / loss/clip_range_vf_ph), from the data flow behind the second operand of loss/Maximum.  A graph
+    without loss/Maximum is "shared" (the shipped graph's form); any other shape raises ValueError.  Twin of
+    classify_vf_clip in csrc/meta_parser.cpp."""
+    def node(name, op):
+        n = nodes.get(name)
+        return n if n is not None and n["op"][0] == op.encode() else None
+
+    def sub_of_square(sq):
+        s = node(sq, "Square")
+        if s is None or len(_inputs(s)) != 1:
+            return None
+        d = node(_inputs(s)[0], "Sub")
+        return _inputs(d) if d is not None and len(_inputs(d)) == 2 else None
+
+    if "loss/Maximum" not in nodes:
+        return "shared"
+    mx = node("loss/Maximum", "Maximum")
+    mi = _inputs(mx) if mx is not None else []
+    s1 = sub_of_square(mi[0]) if len(mi) == 2 else None
+    s2 = sub_of_square(mi[1]) if len(mi) == 2 else None
+    if s1 is None or s2 is None or s1[1] != s2[1]:
+        raise ValueError("loss/Maximum is not max(square(vpred - R), square(vpred_clipped - R))")
+    if s2[0] == s1[0]:
+        return "none"
+    add = node(s2[0], "Add")
+    ai = _inputs(add) if add is not None else []
+    if len(ai) == 2 and ai[1] == "loss/old_vpred_ph":
+        ai = [ai[1], ai[0]]
+    clip = node(ai[1], "Maximum") if len(ai) == 2 and ai[0] == "loss/old_vpred_ph" else None  # clip_by_value = max(min(x, b), -b)
+    ci = _inputs(clip) if clip is not None else []
+    mn = node(ci[0], "Minimum") if len(ci) == 2 else None
+    neg = node(ci[1], "Neg") if len(ci) == 2 else None
+    ni = _inputs(mn) if mn is not None else []
+    gi = _inputs(neg) if neg is not None else []
+    if len(ni) != 2 or len(gi) != 1 or ni[1] != gi[0]:
+        raise ValueError(f"the clipped value {s2[0]} is neither vpred nor old_vpred_ph + clip_by_value(..., -b, b)")
+    if ni[1] == "loss/clip_range_ph":
+        return "shared"
+    if ni[1] == "loss/clip_range_vf_ph":
+        return "separate"
+    raise ValueError(f"the value clip bound {ni[1]} is neither loss/clip_range_ph nor loss/clip_range_vf_ph")
 
 
 def parse_meta_txt(path: str) -> MetaInfo:
@@ -178,6 +231,7 @@ def parse_meta_txt(path: str) -> MetaInfo:
         beta2=scalar("ppo2/_train/beta2"),
         adam_eps=scalar("ppo2/_train/epsilon"),
         tf_version=ver,
+        vf_clip=classify_vf_clip(nodes),
         shapes=shapes,
     )
 
@@ -236,11 +290,17 @@ def _escape(b: bytes) -> str:
 
 
 def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 0.0, vf_coef: float = 0.5,
-                   clip_norm: float = 0.5, beta1: float = 0.9, beta2: float = 0.999, adam_eps: float = 1e-5) -> None:
+                   clip_norm: float = 0.5, beta1: float = 0.9, beta2: float = 0.999, adam_eps: float = 1e-5,
+                   vf_clip: str | None = None) -> None:
     """Write a minimal .meta.txt (variables + initialisers + baked constants) that both readers accept.
 
     The reference's graphs come from a Stable-Baselines/TensorFlow export script that is not part of the
-    repo; this writer lets a user produce a graph file for other hidden sizes without TensorFlow."""
+    repo; this writer lets a user produce a graph file for other hidden sizes without TensorFlow.
+    vf_clip = "shared" | "none" | "separate" adds the value-loss nodes that tell the readers which value loss the
+    graph builds (Stable-Baselines' cliprange_vf None / < 0 / >= 0), named as Stable-Baselines names them;
+    without it the file has no loss sub-graph and reads as "shared"."""
+    if vf_clip not in (None, "shared", "none", "separate"):
+        raise ValueError(f"vf_clip must be None, 'shared', 'none' or 'separate', not {vf_clip!r}")
     def dims(shape, ind):
         return "".join(f"{ind}dim {{\n{ind}  size: {d}\n{ind}}}\n" for d in shape)
 
@@ -265,9 +325,37 @@ def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 
         arr = np.asarray(tensors[name], np.float32)
         parts.append(const_node(f"{name}/Initializer/initial_value", arr))
         parts.append(var_node(name, arr.shape))
+    if vf_clip is not None:
+        parts.append(_vf_loss_nodes(vf_clip))
     for name, val in (("loss/mul_4/y", ent_coef), ("loss/mul_5/y", vf_coef), ("loss/clip_by_global_norm/mul/x", clip_norm),
                       ("ppo2/_train/beta1", beta1), ("ppo2/_train/beta2", beta2), ("ppo2/_train/epsilon", adam_eps)):
         parts.append(const_node(name, np.float32(val)))
     parts.append("}\n")
     with open(path, "w", encoding="latin-1") as f:
         f.write("".join(parts))
+
+
+def _vf_loss_nodes(vf_clip: str) -> str:
+    """The nodes of Stable-Baselines' value loss that classify_vf_clip reads (ops and data inputs only)."""
+    def op(name, kind, *inputs):
+        ins = "".join(f'    input: "{i}"\n' for i in inputs)
+        return f'  node {{\n    name: "{name}"\n    op: "{kind}"\n{ins}  }}\n'
+
+    v = "train_model/strided_slice"  # train_model.value_flat = vf[:, 0]
+    nodes = [op("loss/rewards_ph", "Placeholder"), op("loss/old_vpred_ph", "Placeholder"), op("loss/clip_range_ph", "Placeholder"),
+             op(v, "StridedSlice", "train_model/vf/add")]
+    vc = v
+    if vf_clip != "none":
+        bound = "loss/clip_range_ph"
+        if vf_clip == "separate":
+            bound = "loss/clip_range_vf_ph"
+            nodes.append(op(bound, "Placeholder"))
+        nodes += [op("loss/sub", "Sub", v, "loss/old_vpred_ph"), op("loss/Neg", "Neg", bound),
+                  op("loss/clip_by_value/Minimum", "Minimum", "loss/sub", bound),
+                  op("loss/clip_by_value", "Maximum", "loss/clip_by_value/Minimum", "loss/Neg"),
+                  op("loss/add", "Add", "loss/old_vpred_ph", "loss/clip_by_value")]
+        vc = "loss/add"
+    nodes += [op("loss/sub_1", "Sub", v, "loss/rewards_ph"), op("loss/Square_1", "Square", "loss/sub_1"),
+              op("loss/sub_2", "Sub", vc, "loss/rewards_ph"), op("loss/Square_2", "Square", "loss/sub_2"),
+              op("loss/Maximum", "Maximum", "loss/Square_1", "loss/Square_2")]
+    return "".join(nodes)
