@@ -97,13 +97,27 @@ typedef enum { PPO_VF_CLIP_SHARED = 0, PPO_VF_CLIP_NONE = 1, PPO_VF_CLIP_SEPARAT
  * meta_graph.write_meta_txt without vf_clip, is SHARED); PPO_ERR_UNSUPPORTED if the value loss is of no known form */
 int ppo_meta_vf_clip(const char *meta_txt_path);
 
+/* Hidden-layer activation of the MLP (Stable-Baselines' policy_kwargs act_fun: tf.tanh, the default, or tf.nn.relu), the
+ * same for both hidden layers of both towers.  ReLU's gradient is TensorFlow's ReluGrad: a unit whose pre-activation is
+ * exactly 0 gets none. */
+typedef enum { PPO_ACT_TANH = 0, PPO_ACT_RELU = 1 } ppo_activation;
+/* the ppo_activation of a graph file, read from the data flow into each layer that reads a hidden layer (a file without
+ * forward nodes, as written by meta_graph.write_meta_txt without activation, is TANH); PPO_ERR_UNSUPPORTED for any other
+ * activation, mixed activations, or a deeper / shared-trunk net_arch.  ppo_meta_parse fails the same way. */
+int ppo_meta_activation(const char *meta_txt_path);
+
 int ppo_core_create(const ppo_core_desc *desc, ppo_core **out);
 void ppo_core_destroy(ppo_core *core);
-/* load initial weights from the graph file; its shapes must match the desc (ppo2.hpp:90-105 reset()); sets the core's ppo_vf_clip */
+/* load initial weights from the graph file; its shapes must match the desc (ppo2.hpp:90-105 reset()); sets the core's
+ * ppo_vf_clip and ppo_activation */
 int ppo_core_load_meta_txt(ppo_core *core, const char *meta_txt_path);
 /* the value loss of a graph-less core (default SHARED); ppo_core_load_meta_txt sets it from the graph */
 int ppo_core_set_vf_clip(ppo_core *core, int mode);
 int ppo_core_vf_clip(ppo_core *core); /* the core's ppo_vf_clip, or a negative ppo_status */
+/* the hidden-layer activation of a graph-less core (default TANH); ppo_core_load_meta_txt sets it from the graph.  A change
+ * drops the captured CUDA graphs (they are re-captured on their next use). */
+int ppo_core_set_activation(ppo_core *core, int act);
+int ppo_core_activation(ppo_core *core); /* the core's ppo_activation, or a negative ppo_status */
 /* Stable-Baselines' orthogonal init for graph-less configs (synthetic benchmarks with [64,64], [256,256]) */
 int ppo_core_init_orthogonal(ppo_core *core, uint64_t seed);
 /* TF Saver V2 bundle written by PPO2::save (ppo2.hpp:107-131): `<prefix>.data-00000-of-00001` holds the 15

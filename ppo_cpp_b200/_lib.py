@@ -17,6 +17,7 @@ HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "ppo_core.h")
 
 PPO_HOST, PPO_DEVICE = 0, 1
 PPO_VF_CLIP_SHARED, PPO_VF_CLIP_NONE, PPO_VF_CLIP_SEPARATE = 0, 1, 2
+PPO_ACT_TANH, PPO_ACT_RELU = 0, 1
 PPO_COMM_ID_BYTES = 128
 PPO_IPC_HANDLE_BYTES = 64
 ABI_VERSION = 1
@@ -77,11 +78,14 @@ def load():
         "ppo_core_desc_default": ([C.POINTER(CoreDesc)], C.c_int),
         "ppo_meta_parse": ([C.c_char_p, C.POINTER(MetaInfo), fp, C.c_size_t], C.c_int),
         "ppo_meta_vf_clip": ([C.c_char_p], C.c_int),
+        "ppo_meta_activation": ([C.c_char_p], C.c_int),
         "ppo_core_create": ([C.POINTER(CoreDesc), C.POINTER(core)], C.c_int),
         "ppo_core_destroy": ([core], None),
         "ppo_core_load_meta_txt": ([core, C.c_char_p], C.c_int),
         "ppo_core_set_vf_clip": ([core, C.c_int], C.c_int),
         "ppo_core_vf_clip": ([core], C.c_int),
+        "ppo_core_set_activation": ([core, C.c_int], C.c_int),
+        "ppo_core_activation": ([core], C.c_int),
         "ppo_core_init_orthogonal": ([core, C.c_uint64], C.c_int),
         "ppo_core_load_checkpoint_data": ([core, C.c_char_p], C.c_int),
         "ppo_core_save_checkpoint_data": ([core, C.c_char_p], C.c_int),

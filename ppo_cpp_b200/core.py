@@ -18,6 +18,9 @@ LOSS_NAMES = ("pg_loss", "vf_loss", "entropy", "approxkl", "clipfrac")
 # the value losses of ppo_vf_clip (include/ppo_core.h), by the names write_meta_txt(vf_clip=...) takes
 VF_CLIP_MODES = {"shared": _lib.PPO_VF_CLIP_SHARED, "none": _lib.PPO_VF_CLIP_NONE, "separate": _lib.PPO_VF_CLIP_SEPARATE}
 VF_CLIP_NAMES = {v: k for k, v in VF_CLIP_MODES.items()}
+# the hidden-layer activations of ppo_activation, by the names write_meta_txt(activation=...) takes
+ACTIVATIONS = {"tanh": _lib.PPO_ACT_TANH, "relu": _lib.PPO_ACT_RELU}
+ACTIVATION_NAMES = {v: k for k, v in ACTIVATIONS.items()}
 BUFFER_WIDTH = {"obs": None, "returns": 1, "dones": 1, "actions": None, "values": 1, "neglogpacs": 1,
                 "true_rewards": 1, "unnormalized_rewards": 1}
 
@@ -65,6 +68,15 @@ def meta_vf_clip(path: str) -> str:
     return VF_CLIP_NAMES[r]
 
 
+def meta_activation(path: str) -> str:
+    """The hidden-layer activation of the graph file's forward pass: "tanh" or "relu" (read by the C parser)."""
+    lib = _lib.load()
+    r = lib.ppo_meta_activation(path.encode())
+    if r < 0:
+        _check(lib, r)
+    return ACTIVATION_NAMES[r]
+
+
 def host_rand(seed: int, count: int) -> np.ndarray:
     lib = _lib.load()
     out = np.zeros(count, np.int32)
@@ -87,8 +99,10 @@ def comm_unique_id() -> bytes:
 
 
 class PPOCore:
-    def __init__(self, **kw):
+    def __init__(self, activation: str = "tanh", **kw):
         self.lib = _lib.load()
+        if activation not in ACTIVATIONS:
+            raise ValueError(f"activation must be one of {sorted(ACTIVATIONS)}, not {activation!r}")
         d = CoreDesc()
         _check(self.lib, self.lib.ppo_core_desc_default(C.byref(d)))
         for k, v in kw.items():
@@ -104,6 +118,8 @@ class PPOCore:
         self.n_batch_global = self.n_batch * max(1, d.world_size)
         self.P = self.tensor_size("params_trainable")
         self.Pq = self.tensor_size("params")
+        if activation != "tanh":
+            self.activation = activation
 
     def close(self):
         if self._h:
@@ -133,6 +149,20 @@ class PPOCore:
         if mode not in VF_CLIP_MODES:
             raise ValueError(f"vf_clip must be one of {sorted(VF_CLIP_MODES)}, not {mode!r}")
         _check(self.lib, self.lib.ppo_core_set_vf_clip(self._h, VF_CLIP_MODES[mode]))
+
+    @property
+    def activation(self) -> str:
+        """The core's hidden-layer activation: "tanh" or "relu"."""
+        r = self.lib.ppo_core_activation(self._h)
+        if r < 0:
+            _check(self.lib, r)
+        return ACTIVATION_NAMES[r]
+
+    @activation.setter
+    def activation(self, act: str):
+        if act not in ACTIVATIONS:
+            raise ValueError(f"activation must be one of {sorted(ACTIVATIONS)}, not {act!r}")
+        _check(self.lib, self.lib.ppo_core_set_activation(self._h, ACTIVATIONS[act]))
 
     def graph_builds(self) -> int:
         """CUDA graphs captured and instantiated since the core was created."""

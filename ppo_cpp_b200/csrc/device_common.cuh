@@ -58,6 +58,24 @@ __device__ __forceinline__ float value_loss_term(int mode, float range, float v,
     return tk ? l1 : l2;
 }
 
+// Hidden-layer activation of the MLP (ppo_activation in ppo_core.h); uniform per core, a template parameter of every kernel
+// that evaluates it, so each activation compiles to its own code.  The derivative is taken from the OUTPUT h, as a factor:
+// TanhGrad (1 - h^2) and ReluGrad (h > 0: a unit whose pre-activation is exactly 0 gets no gradient, as TF's
+// gradients * (features > 0)).
+enum { ACT_TANH = 0, ACT_RELU = 1, ACT_NONE = 2 };  // ACT_NONE: the linear heads of the tile forward helpers
+
+template <int ACT>
+__device__ __forceinline__ float act_fwd(float x) {
+    if (ACT == ACT_NONE) return x;
+    if (ACT == ACT_RELU) return x < 0.f ? 0.f : x;
+    return tanhf(x);
+}
+template <int ACT>
+__device__ __forceinline__ float act_dfac(float h) {
+    if (ACT == ACT_RELU) return h > 0.f ? 1.f : 0.f;
+    return 1.f - h * h;
+}
+
 // 0.5*log(2*pi), 0.5*log(2*pi*e) as the fp32 constants baked in the graph (GRAPH:6103-6672, 10021-10180)
 #define PPO_HALF_LOG_2PI 0.9189385175704956f
 #define PPO_HALF_LOG_2PIE 1.4189385175704956f

@@ -13,8 +13,8 @@ namespace ppo {
 
 constexpr int NT = 256;  // threads per CTA for the tile kernels
 
-// Cs[n][m] = act( sum_k As[k][m] * W[k][n] + b[n] )      As: [K][TM] smem, W: [K][N] global, Cs: [N][TM] smem
-template <int TM, bool kTanh>
+// Cs[n][m] = act( sum_k As[k][m] * W[k][n] + b[n] )      As: [K][TM] smem, W: [K][N] global, Cs: [N][TM] smem; act = FA (ACT_NONE: linear)
+template <int TM, int FA>
 __device__ __forceinline__ void tile_fwd(const float* __restrict__ As, int K, const float* __restrict__ W,
                                          const float* __restrict__ b, int N, float* __restrict__ Cs) {
     constexpr int MG = TM / 4, NGS = NT / MG;
@@ -59,15 +59,15 @@ __device__ __forceinline__ void tile_fwd(const float* __restrict__ As, int K, co
                 const float bb = __ldg(b + n + i);
                 float4 o;
                 o.x = acc[i][0] + bb; o.y = acc[i][1] + bb; o.z = acc[i][2] + bb; o.w = acc[i][3] + bb;
-                if (kTanh) { o.x = tanhf(o.x); o.y = tanhf(o.y); o.z = tanhf(o.z); o.w = tanhf(o.w); }
+                if (FA != ACT_NONE) { o.x = act_fwd<FA>(o.x); o.y = act_fwd<FA>(o.y); o.z = act_fwd<FA>(o.z); o.w = act_fwd<FA>(o.w); }
                 *reinterpret_cast<float4*>(Cs + (n + i) * TM + mg * 4) = o;
             }
         }
     }
 }
 
-// Ds[k][m] = ( sum_n W[k][n] * Ys[n][m] ) * (1 - Hs[k][m]^2)        (dY·Wᵀ then TanhGrad; GRAPH:20925-23699)
-template <int TM>
+// Ds[k][m] = ( sum_n W[k][n] * Ys[n][m] ) * act'(Hs[k][m])        (dY·Wᵀ then TanhGrad / ReluGrad; GRAPH:20925-23699)
+template <int TM, int ACT>
 __device__ __forceinline__ void tile_bwd_dx(const float* __restrict__ Ys, int N, const float* __restrict__ W, int K,
                                             const float* __restrict__ Hs, float* __restrict__ Ds) {
     constexpr int MG = TM / 4, KGS = NT / MG;
@@ -121,10 +121,10 @@ __device__ __forceinline__ void tile_bwd_dx(const float* __restrict__ Ys, int N,
             if (k + i < K) {
                 const float4 h = *reinterpret_cast<const float4*>(Hs + (k + i) * TM + mg * 4);
                 float4 o;
-                o.x = acc[i][0] * (1.f - h.x * h.x);
-                o.y = acc[i][1] * (1.f - h.y * h.y);
-                o.z = acc[i][2] * (1.f - h.z * h.z);
-                o.w = acc[i][3] * (1.f - h.w * h.w);
+                o.x = acc[i][0] * act_dfac<ACT>(h.x);
+                o.y = acc[i][1] * act_dfac<ACT>(h.y);
+                o.z = acc[i][2] * act_dfac<ACT>(h.z);
+                o.w = acc[i][3] * act_dfac<ACT>(h.w);
                 *reinterpret_cast<float4*>(Ds + (k + i) * TM + mg * 4) = o;
             }
         }
@@ -229,7 +229,7 @@ __host__ __device__ inline size_t policy_smem_floats(const NetDims& d) {
     return (size_t)(d.O + d.H1 + d.H2 + d.A + 1) * TM + (size_t)d.A * (TM + 1);
 }
 
-template <int TM>
+template <int TM, int ACT>
 __global__ void __launch_bounds__(NT) policy_tile_kernel(const PolicyArgs a) {
     extern __shared__ __align__(16) float smem[];
     const NetDims& d = a.d;
@@ -252,19 +252,19 @@ __global__ void __launch_bounds__(NT) policy_tile_kernel(const PolicyArgs a) {
         }
         __syncthreads();
         if (a.mode != 1) {
-            tile_fwd<TM, true>(Xs, d.O, p + d.off[T_PI_FC0_W], p + d.off[T_PI_FC0_B], d.H1, H1s);
+            tile_fwd<TM, ACT>(Xs, d.O, p + d.off[T_PI_FC0_W], p + d.off[T_PI_FC0_B], d.H1, H1s);
             __syncthreads();
-            tile_fwd<TM, true>(H1s, d.H1, p + d.off[T_PI_FC1_W], p + d.off[T_PI_FC1_B], d.H2, H2s);
+            tile_fwd<TM, ACT>(H1s, d.H1, p + d.off[T_PI_FC1_W], p + d.off[T_PI_FC1_B], d.H2, H2s);
             __syncthreads();
-            tile_fwd<TM, false>(H2s, d.H2, p + d.off[T_PI_W], p + d.off[T_PI_B], d.A, MU);
+            tile_fwd<TM, ACT_NONE>(H2s, d.H2, p + d.off[T_PI_W], p + d.off[T_PI_B], d.A, MU);
             __syncthreads();
         }
         if (a.mode != 2) {
-            tile_fwd<TM, true>(Xs, d.O, p + d.off[T_VF_FC0_W], p + d.off[T_VF_FC0_B], d.H1, H1s);
+            tile_fwd<TM, ACT>(Xs, d.O, p + d.off[T_VF_FC0_W], p + d.off[T_VF_FC0_B], d.H1, H1s);
             __syncthreads();
-            tile_fwd<TM, true>(H1s, d.H1, p + d.off[T_VF_FC1_W], p + d.off[T_VF_FC1_B], d.H2, H2s);
+            tile_fwd<TM, ACT>(H1s, d.H1, p + d.off[T_VF_FC1_W], p + d.off[T_VF_FC1_B], d.H2, H2s);
             __syncthreads();
-            tile_fwd<TM, false>(H2s, d.H2, p + d.off[T_VF_W], p + d.off[T_VF_B], 1, Vs);
+            tile_fwd<TM, ACT_NONE>(H2s, d.H2, p + d.off[T_VF_W], p + d.off[T_VF_B], 1, Vs);
             __syncthreads();
         }
         if (tid < nv) {
@@ -342,7 +342,7 @@ __host__ __device__ inline size_t train_smem_floats(const NetDims& d) {
     return (size_t)(d.O + 2 * d.A + 2 * d.H1 + 2 * d.H2) * TM + 5 * (size_t)TM + 64;
 }
 
-template <int TM>
+template <int TM, int ACT>
 __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
     extern __shared__ __align__(16) float smem[];
     const NetDims& d = a.d;
@@ -395,11 +395,11 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
         __syncthreads();
 
         // ---------------- pi tower ----------------
-        tile_fwd<TM, true>(Xs, d.O, p + d.off[T_PI_FC0_W], p + d.off[T_PI_FC0_B], d.H1, H1s);
+        tile_fwd<TM, ACT>(Xs, d.O, p + d.off[T_PI_FC0_W], p + d.off[T_PI_FC0_B], d.H1, H1s);
         __syncthreads();
-        tile_fwd<TM, true>(H1s, d.H1, p + d.off[T_PI_FC1_W], p + d.off[T_PI_FC1_B], d.H2, H2s);
+        tile_fwd<TM, ACT>(H1s, d.H1, p + d.off[T_PI_FC1_W], p + d.off[T_PI_FC1_B], d.H2, H2s);
         __syncthreads();
-        tile_fwd<TM, false>(H2s, d.H2, p + d.off[T_PI_W], p + d.off[T_PI_B], d.A, MU);
+        tile_fwd<TM, ACT_NONE>(H2s, d.H2, p + d.off[T_PI_W], p + d.off[T_PI_B], d.A, MU);
         __syncthreads();
         if (tid < TM) {
             const int m = tid;
@@ -436,22 +436,22 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
         tile_dw<TM>(H2s, d.H2, MU, d.A, my + d.off[T_PI_W], acc);
         tile_rowsum<TM>(MU, d.A, my + d.off[T_PI_B], acc);
         tile_rowsum<TM>(Ac, d.A, my + d.off[T_LOGSTD], acc);
-        tile_bwd_dx<TM>(MU, d.A, p + d.off[T_PI_W], d.H2, H2s, D2);
+        tile_bwd_dx<TM, ACT>(MU, d.A, p + d.off[T_PI_W], d.H2, H2s, D2);
         __syncthreads();
         tile_dw<TM>(H1s, d.H1, D2, d.H2, my + d.off[T_PI_FC1_W], acc);
         tile_rowsum<TM>(D2, d.H2, my + d.off[T_PI_FC1_B], acc);
-        tile_bwd_dx<TM>(D2, d.H2, p + d.off[T_PI_FC1_W], d.H1, H1s, D1);
+        tile_bwd_dx<TM, ACT>(D2, d.H2, p + d.off[T_PI_FC1_W], d.H1, H1s, D1);
         __syncthreads();
         tile_dw<TM>(Xs, d.O, D1, d.H1, my + d.off[T_PI_FC0_W], acc);
         tile_rowsum<TM>(D1, d.H1, my + d.off[T_PI_FC0_B], acc);
         __syncthreads();
 
         // ---------------- value tower ----------------
-        tile_fwd<TM, true>(Xs, d.O, p + d.off[T_VF_FC0_W], p + d.off[T_VF_FC0_B], d.H1, H1s);
+        tile_fwd<TM, ACT>(Xs, d.O, p + d.off[T_VF_FC0_W], p + d.off[T_VF_FC0_B], d.H1, H1s);
         __syncthreads();
-        tile_fwd<TM, true>(H1s, d.H1, p + d.off[T_VF_FC1_W], p + d.off[T_VF_FC1_B], d.H2, H2s);
+        tile_fwd<TM, ACT>(H1s, d.H1, p + d.off[T_VF_FC1_W], p + d.off[T_VF_FC1_B], d.H2, H2s);
         __syncthreads();
-        tile_fwd<TM, false>(H2s, d.H2, p + d.off[T_VF_W], p + d.off[T_VF_B], 1, MU);
+        tile_fwd<TM, ACT_NONE>(H2s, d.H2, p + d.off[T_VF_W], p + d.off[T_VF_B], 1, MU);
         __syncthreads();
         if (tid < TM) {
             const int m = tid;
@@ -464,11 +464,11 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
         __syncthreads();
         tile_dw<TM>(H2s, d.H2, MU, 1, my + d.off[T_VF_W], acc);
         tile_rowsum<TM>(MU, 1, my + d.off[T_VF_B], acc);
-        tile_bwd_dx<TM>(MU, 1, p + d.off[T_VF_W], d.H2, H2s, D2);
+        tile_bwd_dx<TM, ACT>(MU, 1, p + d.off[T_VF_W], d.H2, H2s, D2);
         __syncthreads();
         tile_dw<TM>(H1s, d.H1, D2, d.H2, my + d.off[T_VF_FC1_W], acc);
         tile_rowsum<TM>(D2, d.H2, my + d.off[T_VF_FC1_B], acc);
-        tile_bwd_dx<TM>(D2, d.H2, p + d.off[T_VF_FC1_W], d.H1, H1s, D1);
+        tile_bwd_dx<TM, ACT>(D2, d.H2, p + d.off[T_VF_FC1_W], d.H1, H1s, D1);
         __syncthreads();
         tile_dw<TM>(Xs, d.O, D1, d.H1, my + d.off[T_VF_FC0_W], acc);
         tile_rowsum<TM>(D1, d.H1, my + d.off[T_VF_FC0_B], acc);

@@ -18,7 +18,7 @@ struct Sub {
 };
 
 // Cs[n][m] = act( sum_k As[k][m] * W[k][n] + b[n] ), W/b in shared memory
-template <int TM, bool kTanh>
+template <int TM, int FA>
 __device__ __forceinline__ void f_fwd(const float* __restrict__ As, int K, const float* __restrict__ W,
                                       const float* __restrict__ b, int N, float* __restrict__ Cs, Sub s) {
     constexpr int MG = TM / 4;
@@ -63,15 +63,15 @@ __device__ __forceinline__ void f_fwd(const float* __restrict__ As, int K, const
                 const float bb = b[n + i];
                 float4 o;
                 o.x = acc[i][0] + bb; o.y = acc[i][1] + bb; o.z = acc[i][2] + bb; o.w = acc[i][3] + bb;
-                if (kTanh) { o.x = tanhf(o.x); o.y = tanhf(o.y); o.z = tanhf(o.z); o.w = tanhf(o.w); }
+                if (FA != ACT_NONE) { o.x = act_fwd<FA>(o.x); o.y = act_fwd<FA>(o.y); o.z = act_fwd<FA>(o.z); o.w = act_fwd<FA>(o.w); }
                 *reinterpret_cast<float4*>(Cs + (n + i) * TM + mg * 4) = o;
             }
         }
     }
 }
 
-// Ds[k][m] = ( sum_n W[k][n] * Ys[n][m] ) * (1 - Hs[k][m]^2), W in shared memory
-template <int TM>
+// Ds[k][m] = ( sum_n W[k][n] * Ys[n][m] ) * act'(Hs[k][m]), W in shared memory
+template <int TM, int ACT>
 __device__ __forceinline__ void f_bwd_dx(const float* __restrict__ Ys, int N, const float* __restrict__ W, int K,
                                          const float* __restrict__ Hs, float* __restrict__ Ds, Sub s) {
     constexpr int MG = TM / 4;
@@ -127,10 +127,10 @@ __device__ __forceinline__ void f_bwd_dx(const float* __restrict__ Ys, int N, co
             if (k + i < K) {
                 const float4 h = *reinterpret_cast<const float4*>(Hs + (k + i) * TM + mg * 4);
                 float4 o;
-                o.x = acc[i][0] * (1.f - h.x * h.x);
-                o.y = acc[i][1] * (1.f - h.y * h.y);
-                o.z = acc[i][2] * (1.f - h.z * h.z);
-                o.w = acc[i][3] * (1.f - h.w * h.w);
+                o.x = acc[i][0] * act_dfac<ACT>(h.x);
+                o.y = acc[i][1] * act_dfac<ACT>(h.y);
+                o.z = acc[i][2] * act_dfac<ACT>(h.z);
+                o.w = acc[i][3] * act_dfac<ACT>(h.w);
                 *reinterpret_cast<float4*>(Ds + (k + i) * TM + mg * 4) = o;
             }
         }
@@ -232,7 +232,7 @@ __device__ __forceinline__ void stage_weights(float* sW, const float* __restrict
 }
 
 // ------------------------------------------------------------------------------------------------ train
-template <int TM, int NTH>
+template <int TM, int NTH, int ACT>
 __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) {
     extern __shared__ __align__(16) float smem[];
     const NetDims& d = a.d;
@@ -318,12 +318,12 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
         }
 
         // ---- forward, both towers at once
-        f_fwd<TM, true>(Xs, d.O, sW + d.off[tw ? T_VF_FC0_W : T_PI_FC0_W], sW + d.off[tw ? T_VF_FC0_B : T_PI_FC0_B], d.H1, H1, half);
+        f_fwd<TM, ACT>(Xs, d.O, sW + d.off[tw ? T_VF_FC0_W : T_PI_FC0_W], sW + d.off[tw ? T_VF_FC0_B : T_PI_FC0_B], d.H1, H1, half);
         __syncthreads();
-        f_fwd<TM, true>(H1, d.H1, sW + d.off[tw ? T_VF_FC1_W : T_PI_FC1_W], sW + d.off[tw ? T_VF_FC1_B : T_PI_FC1_B], d.H2, H2, half);
+        f_fwd<TM, ACT>(H1, d.H1, sW + d.off[tw ? T_VF_FC1_W : T_PI_FC1_W], sW + d.off[tw ? T_VF_FC1_B : T_PI_FC1_B], d.H2, H2, half);
         __syncthreads();
-        if (tw == 0) f_fwd<TM, false>(H2, d.H2, sW + d.off[T_PI_W], sW + d.off[T_PI_B], d.A, MU, half);
-        else f_fwd<TM, false>(H2, d.H2, sW + d.off[T_VF_W], sW + d.off[T_VF_B], 1, Vs, half);
+        if (tw == 0) f_fwd<TM, ACT_NONE>(H2, d.H2, sW + d.off[T_PI_W], sW + d.off[T_PI_B], d.A, MU, half);
+        else f_fwd<TM, ACT_NONE>(H2, d.H2, sW + d.off[T_VF_W], sW + d.off[T_VF_B], 1, Vs, half);
         __syncthreads();
 
         // ---- loss stage.  Thread (m, jg) handles actions j = jg, jg + JG, ... of sample m.
@@ -374,10 +374,10 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
 
         // ---- backward: heads
         if (tw == 0) {
-            f_bwd_dx<TM>(MU, d.A, sW + d.off[T_PI_W], d.H2, H2, D2, half);
+            f_bwd_dx<TM, ACT>(MU, d.A, sW + d.off[T_PI_W], d.H2, H2, D2, half);
             f_dw<TM>(H2, d.H2, MU, d.A, my + d.off[T_PI_W], my + d.off[T_PI_B], acc, half);
         } else {
-            f_bwd_dx<TM>(Vs, 1, sW + d.off[T_VF_W], d.H2, H2, D2, half);
+            f_bwd_dx<TM, ACT>(Vs, 1, sW + d.off[T_VF_W], d.H2, H2, D2, half);
             f_dw<TM>(H2, d.H2, Vs, 1, my + d.off[T_VF_W], my + d.off[T_VF_B], acc, half);
             // logstd gradient = row sums of Ac: ones-row trick with K = 0 (As = the ones row of Xs)
             f_dw<TM>(Xs + d.O * TM, 0, Ac, d.A, my + d.off[T_LOGSTD], my + d.off[T_LOGSTD], acc, half);
@@ -385,7 +385,7 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
         __syncthreads();
         // ---- backward: hidden layer 1
         f_dw<TM>(H1, d.H1, D2, d.H2, my + d.off[tw ? T_VF_FC1_W : T_PI_FC1_W], my + d.off[tw ? T_VF_FC1_B : T_PI_FC1_B], acc, half);
-        f_bwd_dx<TM>(D2, d.H2, sW + d.off[tw ? T_VF_FC1_W : T_PI_FC1_W], d.H1, H1, D1, half);
+        f_bwd_dx<TM, ACT>(D2, d.H2, sW + d.off[tw ? T_VF_FC1_W : T_PI_FC1_W], d.H1, H1, D1, half);
         __syncthreads();
         // ---- backward: hidden layer 0
         f_dw<TM>(Xs, d.O, D1, d.H1, my + d.off[tw ? T_VF_FC0_W : T_PI_FC0_W], my + d.off[tw ? T_VF_FC0_B : T_PI_FC0_B], acc, half);
@@ -420,7 +420,7 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
 }
 
 // ------------------------------------------------------------------------------------------------ policy
-template <int TM, int NTH>
+template <int TM, int NTH, int ACT>
 __global__ void __launch_bounds__(NTH) policy_fused_kernel(const PolicyArgs a) {
     extern __shared__ __align__(16) float smem[];
     const NetDims& d = a.d;
@@ -455,13 +455,13 @@ __global__ void __launch_bounds__(NTH) policy_fused_kernel(const PolicyArgs a) {
         }
         __syncthreads();
         if ((tw == 0 && do_pi) || (tw == 1 && do_v))
-            f_fwd<TM, true>(Xs, d.O, sW + d.off[tw ? T_VF_FC0_W : T_PI_FC0_W], sW + d.off[tw ? T_VF_FC0_B : T_PI_FC0_B], d.H1, H1, half);
+            f_fwd<TM, ACT>(Xs, d.O, sW + d.off[tw ? T_VF_FC0_W : T_PI_FC0_W], sW + d.off[tw ? T_VF_FC0_B : T_PI_FC0_B], d.H1, H1, half);
         __syncthreads();
         if ((tw == 0 && do_pi) || (tw == 1 && do_v))
-            f_fwd<TM, true>(H1, d.H1, sW + d.off[tw ? T_VF_FC1_W : T_PI_FC1_W], sW + d.off[tw ? T_VF_FC1_B : T_PI_FC1_B], d.H2, H2, half);
+            f_fwd<TM, ACT>(H1, d.H1, sW + d.off[tw ? T_VF_FC1_W : T_PI_FC1_W], sW + d.off[tw ? T_VF_FC1_B : T_PI_FC1_B], d.H2, H2, half);
         __syncthreads();
-        if (tw == 0 && do_pi) f_fwd<TM, false>(H2, d.H2, sW + d.off[T_PI_W], sW + d.off[T_PI_B], d.A, MU, half);
-        if (tw == 1 && do_v) f_fwd<TM, false>(H2, d.H2, sW + d.off[T_VF_W], sW + d.off[T_VF_B], 1, Vs, half);
+        if (tw == 0 && do_pi) f_fwd<TM, ACT_NONE>(H2, d.H2, sW + d.off[T_PI_W], sW + d.off[T_PI_B], d.A, MU, half);
+        if (tw == 1 && do_v) f_fwd<TM, ACT_NONE>(H2, d.H2, sW + d.off[T_VF_W], sW + d.off[T_VF_B], 1, Vs, half);
         __syncthreads();
         if (tid < nv) {
             const int m = tid, row = r0 + m;

@@ -114,7 +114,7 @@ struct RLayout {
 // Forward pass of ONE env by one warp with the layer widths known at compile time (the reference's [4,5] net and the [64,64] default):
 // lane l owns output units l, l + 32, ... of [pi tower | V tower]; fully unrolled, so the loads of a chain are issued ahead of its fmaf
 // sequence (k ascending, as f_fwd).  With run-time widths the same loops took ~70 cycles per k-step.
-template <int O, int H1, int H2, int A, int TM>
+template <int O, int H1, int H2, int A, int TM, int ACT>
 __device__ __forceinline__ void solo_forward(const float* __restrict__ sW, const NetDims& d, const float* __restrict__ OBS, float* H1p, float* H1v,
                                              float* H2p, float* H2v, float* MU, float* Vs, int lane) {
 #pragma unroll
@@ -127,7 +127,7 @@ __device__ __forceinline__ void solo_forward(const float* __restrict__ sW, const
             float acc = 0.f;
 #pragma unroll
             for (int k = 0; k < O; ++k) acc = fmaf(w[k * H1], OBS[k * TM], acc);
-            (vt ? H1v : H1p)[n * TM] = tanhf(acc + sW[d.off[vt ? T_VF_FC0_B : T_PI_FC0_B] + n]);
+            (vt ? H1v : H1p)[n * TM] = act_fwd<ACT>(acc + sW[d.off[vt ? T_VF_FC0_B : T_PI_FC0_B] + n]);
         }
     }
     __syncwarp();
@@ -142,7 +142,7 @@ __device__ __forceinline__ void solo_forward(const float* __restrict__ sW, const
             float acc = 0.f;
 #pragma unroll
             for (int k = 0; k < H1; ++k) acc = fmaf(w[k * H2], hin[k * TM], acc);
-            (vt ? H2v : H2p)[n * TM] = tanhf(acc + sW[d.off[vt ? T_VF_FC1_B : T_PI_FC1_B] + n]);
+            (vt ? H2v : H2p)[n * TM] = act_fwd<ACT>(acc + sW[d.off[vt ? T_VF_FC1_B : T_PI_FC1_B] + n]);
         }
     }
     __syncwarp();
@@ -161,6 +161,7 @@ __device__ __forceinline__ void solo_forward(const float* __restrict__ sW, const
     __syncwarp();
 }
 
+template <int ACT>
 __global__ void __launch_bounds__(R_NTH) rollout_persistent_kernel(const RolloutArgs a) {
     extern __shared__ __align__(16) float smem[];
     const NetDims& d = a.d;
@@ -303,9 +304,9 @@ __global__ void __launch_bounds__(R_NTH) rollout_persistent_kernel(const Rollout
                     for (int k = lane; k < O; k += 32) a.obs_store[(size_t)t * O + k] = OBS[k * TM];
                     // -- MlpPolicy::step, both towers: lane per output unit, k ascending as f_fwd
                     if (O == 18 && A == 18 && nH1 == 4 && nH2 == 5) {
-                        solo_forward<18, 4, 5, 18, TM>(sW, d, OBS, H1p, H1v, H2p, H2v, MU, Vs, lane);
+                        solo_forward<18, 4, 5, 18, TM, ACT>(sW, d, OBS, H1p, H1v, H2p, H2v, MU, Vs, lane);
                     } else if (O == 18 && A == 18 && nH1 == 64 && nH2 == 64) {
-                        solo_forward<18, 64, 64, 18, TM>(sW, d, OBS, H1p, H1v, H2p, H2v, MU, Vs, lane);
+                        solo_forward<18, 64, 64, 18, TM, ACT>(sW, d, OBS, H1p, H1v, H2p, H2v, MU, Vs, lane);
                     } else {
                     for (int o = lane; o < 2 * nH1; o += 32) {
                         const bool vt = o >= nH1;
@@ -314,7 +315,7 @@ __global__ void __launch_bounds__(R_NTH) rollout_persistent_kernel(const Rollout
                         float acc = 0.f;
 #pragma unroll 6
                         for (int k = 0; k < O; ++k) acc = fmaf(w[k * nH1], OBS[k * TM], acc);
-                        (vt ? H1v : H1p)[n * TM] = tanhf(acc + (vt ? B0v : B0p)[n]);
+                        (vt ? H1v : H1p)[n * TM] = act_fwd<ACT>(acc + (vt ? B0v : B0p)[n]);
                     }
                     __syncwarp();
                     for (int o = lane; o < 2 * nH2; o += 32) {
@@ -325,7 +326,7 @@ __global__ void __launch_bounds__(R_NTH) rollout_persistent_kernel(const Rollout
                         float acc = 0.f;
 #pragma unroll 4
                         for (int k = 0; k < nH1; ++k) acc = fmaf(w[k * nH2], hin[k * TM], acc);
-                        (vt ? H2v : H2p)[n * TM] = tanhf(acc + (vt ? B1v : B1p)[n]);
+                        (vt ? H2v : H2p)[n * TM] = act_fwd<ACT>(acc + (vt ? B1v : B1p)[n]);
                     }
                     __syncwarp();
                     for (int o = lane; o < A + 1; o += 32) {
@@ -584,12 +585,12 @@ __global__ void __launch_bounds__(R_NTH) rollout_persistent_kernel(const Rollout
                 }
             }
             // -- MlpPolicy::step: both towers in the same phase
-            f_fwd<TM, true>(Xs, O, sW + d.off[tw ? T_VF_FC0_W : T_PI_FC0_W], sW + d.off[tw ? T_VF_FC0_B : T_PI_FC0_B], d.H1, H1, half);
+            f_fwd<TM, ACT>(Xs, O, sW + d.off[tw ? T_VF_FC0_W : T_PI_FC0_W], sW + d.off[tw ? T_VF_FC0_B : T_PI_FC0_B], d.H1, H1, half);
             __syncthreads();
-            f_fwd<TM, true>(H1, d.H1, sW + d.off[tw ? T_VF_FC1_W : T_PI_FC1_W], sW + d.off[tw ? T_VF_FC1_B : T_PI_FC1_B], d.H2, H2, half);
+            f_fwd<TM, ACT>(H1, d.H1, sW + d.off[tw ? T_VF_FC1_W : T_PI_FC1_W], sW + d.off[tw ? T_VF_FC1_B : T_PI_FC1_B], d.H2, H2, half);
             __syncthreads();
-            if (tw == 0) f_fwd<TM, false>(H2, d.H2, sW + d.off[T_PI_W], sW + d.off[T_PI_B], A, MU, half);
-            else f_fwd<TM, false>(H2, d.H2, sW + d.off[T_VF_W], sW + d.off[T_VF_B], 1, Vs, half);
+            if (tw == 0) f_fwd<TM, ACT_NONE>(H2, d.H2, sW + d.off[T_PI_W], sW + d.off[T_PI_B], A, MU, half);
+            else f_fwd<TM, ACT_NONE>(H2, d.H2, sW + d.off[T_VF_W], sW + d.off[T_VF_B], 1, Vs, half);
             __syncthreads();
             R_PROF();  // forward done
             // -- Gaussian sample (GRAPH:5894-6019): thread (m, blk) draws 4 actions
@@ -878,11 +879,11 @@ __global__ void __launch_bounds__(R_NTH) rollout_persistent_kernel(const Rollout
     for (int tl = 0; tl < my_tiles; ++tl) {
         const int r0 = (tile0 + tl) * TM, nv = min(TM, a.n - r0);
         float* Xs = OBS + tl * O * TM;
-        if (tw == 1) f_fwd<TM, true>(Xs, O, sW + d.off[T_VF_FC0_W], sW + d.off[T_VF_FC0_B], d.H1, H1, half);
+        if (tw == 1) f_fwd<TM, ACT>(Xs, O, sW + d.off[T_VF_FC0_W], sW + d.off[T_VF_FC0_B], d.H1, H1, half);
         __syncthreads();
-        if (tw == 1) f_fwd<TM, true>(H1, d.H1, sW + d.off[T_VF_FC1_W], sW + d.off[T_VF_FC1_B], d.H2, H2, half);
+        if (tw == 1) f_fwd<TM, ACT>(H1, d.H1, sW + d.off[T_VF_FC1_W], sW + d.off[T_VF_FC1_B], d.H2, H2, half);
         __syncthreads();
-        if (tw == 1) f_fwd<TM, false>(H2, d.H2, sW + d.off[T_VF_W], sW + d.off[T_VF_B], 1, Vs, half);
+        if (tw == 1) f_fwd<TM, ACT_NONE>(H2, d.H2, sW + d.off[T_VF_W], sW + d.off[T_VF_B], 1, Vs, half);
         __syncthreads();
         if (tid < nv) LASTV[tl * TM + tid] = Vs[tid];
         for (int e = tid; e < nv * D; e += NTH) {

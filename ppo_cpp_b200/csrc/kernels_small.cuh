@@ -68,7 +68,7 @@ struct SmallAcc {
 };
 
 // One warp tile (32 samples, one per lane): forward, loss, backward; the per-parameter contributions summed over the warp into acc
-template <int O, int A, int H1, int H2>
+template <int O, int A, int H1, int H2, int ACT>
 __device__ __forceinline__ void small_warp_tile(const TrainArgs& a, const float* __restrict__ sW, int slot, bool valid, const float2* mbstats,
                                                 const float (&sd)[A], const float (&isd)[A], float sum_ls,
                                                 SmallAcc<Dims<O, A, H1, H2>::GROUPS>& acc, float* tile, int lane) {
@@ -117,8 +117,8 @@ __device__ __forceinline__ void small_warp_tile(const TrainArgs& a, const float*
                 sp = fmaf(x[k], sW[D::PI0W + k * H1 + n], sp);
                 sv = fmaf(x[k], sW[D::VF0W + k * H1 + n], sv);
             }
-            h1[n] = tanhf(sp + sW[D::PI0B + n]);
-            g1[n] = tanhf(sv + sW[D::VF0B + n]);
+            h1[n] = act_fwd<ACT>(sp + sW[D::PI0B + n]);
+            g1[n] = act_fwd<ACT>(sv + sW[D::VF0B + n]);
         }
 #pragma unroll
         for (int n = 0; n < H2; ++n) {
@@ -128,8 +128,8 @@ __device__ __forceinline__ void small_warp_tile(const TrainArgs& a, const float*
                 sp = fmaf(h1[k], sW[D::PI1W + k * H2 + n], sp);
                 sv = fmaf(g1[k], sW[D::VF1W + k * H2 + n], sv);
             }
-            h2[n] = tanhf(sp + sW[D::PI1B + n]);
-            g2[n] = tanhf(sv + sW[D::VF1B + n]);
+            h2[n] = act_fwd<ACT>(sp + sW[D::PI1B + n]);
+            g2[n] = act_fwd<ACT>(sv + sW[D::VF1B + n]);
         }
         float v = 0.f;
 #pragma unroll
@@ -174,15 +174,15 @@ __device__ __forceinline__ void small_warp_tile(const TrainArgs& a, const float*
                 dls[j] = g_nlp * (1.f - z[j] * z[j]);
             }
         }
-        // ---- backward through the towers (TanhGrad(y, dy) = dy * (1 - y^2))
+        // ---- backward through the towers (TanhGrad(y, dy) = dy * (1 - y^2), ReluGrad = dy * (y > 0))
         float dp2[H2], dg2[H2], dp1[H1], dg1[H1];
 #pragma unroll
         for (int k = 0; k < H2; ++k) {
             float s = 0.f;
 #pragma unroll
             for (int j = 0; j < A; ++j) s = fmaf(dmu[j], sW[D::PIW + k * A + j], s);
-            dp2[k] = s * (1.f - h2[k] * h2[k]);
-            dg2[k] = dv * sW[D::VFW + k] * (1.f - g2[k] * g2[k]);
+            dp2[k] = s * act_dfac<ACT>(h2[k]);
+            dg2[k] = dv * sW[D::VFW + k] * act_dfac<ACT>(g2[k]);
         }
 #pragma unroll
         for (int k = 0; k < H1; ++k) {
@@ -192,8 +192,8 @@ __device__ __forceinline__ void small_warp_tile(const TrainArgs& a, const float*
                 sp = fmaf(dp2[n], sW[D::PI1W + k * H2 + n], sp);
                 sv = fmaf(dg2[n], sW[D::VF1W + k * H2 + n], sv);
             }
-            dp1[k] = sp * (1.f - h1[k] * h1[k]);
-            dg1[k] = sv * (1.f - g1[k] * g1[k]);
+            dp1[k] = sp * act_dfac<ACT>(h1[k]);
+            dg1[k] = sv * act_dfac<ACT>(g1[k]);
         }
         // ---- per-sample gradient contributions, 32 parameters at a time, summed over the warp's 32 samples
 #pragma unroll
@@ -223,7 +223,7 @@ __device__ __forceinline__ void small_warp_tile(const TrainArgs& a, const float*
     }
 }
 
-template <int O, int A, int H1, int H2>
+template <int O, int A, int H1, int H2, int ACT>
 __global__ void __launch_bounds__(NTH) train_small_kernel(const TrainArgs a) {
     using D = Dims<O, A, H1, H2>;
     static_assert(O % 2 == 0 && A % 2 == 0, "rows are read as float2");
@@ -250,7 +250,7 @@ __global__ void __launch_bounds__(NTH) train_small_kernel(const TrainArgs a) {
     for (int wt = blockIdx.x * (NTH / 32) + warp; wt < nwarp_tiles; wt += gridDim.x * (NTH / 32)) {
         const int slot = a.slot0 + wt * 32 + lane;
         const bool valid = wt * 32 + lane < a.count;
-        small_warp_tile<O, A, H1, H2>(a, sW, slot, valid, a.mbstats, sd, isd, sum_ls, acc, s_tile[warp], lane);
+        small_warp_tile<O, A, H1, H2, ACT>(a, sW, slot, valid, a.mbstats, sd, isd, sum_ls, acc, s_tile[warp], lane);
     }
     float (&accg)[D::GROUPS] = acc.accg;
     const float l_pg = acc.l_pg, l_vf = acc.l_vf, l_kl = acc.l_kl, l_cf = acc.l_cf;
@@ -291,11 +291,11 @@ __global__ void __launch_bounds__(NTH) train_small_kernel(const TrainArgs a) {
 
 // Policy step of the S family (MlpPolicy::step / value / deterministic action, policies.hpp:33-77): one THREAD per env, parameters in
 // shared memory (LDS.128 broadcasts), the env's observation row in registers, the same accumulation order as the tile kernels
-// (k ascending from 0, bias added last, tanhf) so that actions / values / neglogp are bit-identical to every other forward path.
+// (k ascending from 0, bias added last, act_fwd) so that actions / values / neglogp are bit-identical to every other forward path.
 // Observation rows come in and action rows go out through a shared-memory tile, so global accesses are contiguous per warp.
 // (policy_tile_kernel, which served this net before, spends 12 M warp instructions on 65 536 envs: 4x4 register tiles over layers
 // that are 4 and 5 wide leave most threads of a phase idle — 37 us per step against 7; profiles/r2_small_kernels_ncu.txt.)
-template <int O, int A, int H1, int H2>
+template <int O, int A, int H1, int H2, int ACT>
 __global__ void __launch_bounds__(NTH) policy_small_kernel(const PolicyArgs a) {
     using D = Dims<O, A, H1, H2>;
     constexpr int XL = O + 1 + ((O + 1) % 2 == 0 ? 1 : 0);  // odd row strides: a lane reading its own row hits its own bank
@@ -332,14 +332,14 @@ __global__ void __launch_bounds__(NTH) policy_small_kernel(const PolicyArgs a) {
                     float s = 0.f;
 #pragma unroll
                     for (int k = 0; k < O; ++k) s = fmaf(sW[D::PI0W + k * H1 + n], x[k], s);
-                    h1[n] = tanhf(s + sW[D::PI0B + n]);
+                    h1[n] = act_fwd<ACT>(s + sW[D::PI0B + n]);
                 }
 #pragma unroll
                 for (int n = 0; n < H2; ++n) {
                     float s = 0.f;
 #pragma unroll
                     for (int k = 0; k < H1; ++k) s = fmaf(sW[D::PI1W + k * H2 + n], h1[k], s);
-                    h2[n] = tanhf(s + sW[D::PI1B + n]);
+                    h2[n] = act_fwd<ACT>(s + sW[D::PI1B + n]);
                 }
 #pragma unroll
                 for (int j = 0; j < A; ++j) {
@@ -356,14 +356,14 @@ __global__ void __launch_bounds__(NTH) policy_small_kernel(const PolicyArgs a) {
                     float s = 0.f;
 #pragma unroll
                     for (int k = 0; k < O; ++k) s = fmaf(sW[D::VF0W + k * H1 + n], x[k], s);
-                    g1[n] = tanhf(s + sW[D::VF0B + n]);
+                    g1[n] = act_fwd<ACT>(s + sW[D::VF0B + n]);
                 }
 #pragma unroll
                 for (int n = 0; n < H2; ++n) {
                     float s = 0.f;
 #pragma unroll
                     for (int k = 0; k < H1; ++k) s = fmaf(sW[D::VF1W + k * H2 + n], g1[k], s);
-                    g2[n] = tanhf(s + sW[D::VF1B + n]);
+                    g2[n] = act_fwd<ACT>(s + sW[D::VF1B + n]);
                 }
                 float v = 0.f;
 #pragma unroll
@@ -428,7 +428,7 @@ struct SmallEpochArgs {
     float* loss_rows;        // [M][5]
     AdamArgs adam;           // canonical params / m / v, lr, betas, eps, clip_norm, beta powers in / out, invB, gnorm_out
 };
-template <int O, int A, int H1, int H2>
+template <int O, int A, int H1, int H2, int ACT>
 __global__ void __launch_bounds__(NTH) train_small_epoch_kernel(const TrainArgs a, const SmallEpochArgs ep) {
     using D = Dims<O, A, H1, H2>;
     constexpr int PP = (D::P + 3 + 4) & ~3;
@@ -462,7 +462,7 @@ __global__ void __launch_bounds__(NTH) train_small_epoch_kernel(const TrainArgs 
         for (int wt = warp; wt < nwarp_tiles; wt += NTH / 32) {
             const int slot = mb * ep.B + a.slot0 + wt * 32 + lane;
             const bool valid = wt * 32 + lane < a.count;
-            small_warp_tile<O, A, H1, H2>(a, sW, slot, valid, ep.mbstats + mb, sd, isd, sum_ls, acc, s_tile[warp], lane);
+            small_warp_tile<O, A, H1, H2, ACT>(a, sW, slot, valid, ep.mbstats + mb, sd, isd, sum_ls, acc, s_tile[warp], lane);
         }
         // ---- combine the warps in a fixed order (as train_small_kernel), gradient of parameter i in thread i % NTH
 #pragma unroll

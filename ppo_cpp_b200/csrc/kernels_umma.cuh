@@ -12,7 +12,7 @@
 //     products hi*hi, hi*lo, lo*hi (the dropped lo*lo is < 2^-22 relative).  Round 1 used three bf16 pieces and six
 //     products: twice the tensor-pipe time and 1.5x the shared-memory traffic for the same accuracy.  fp16 has a 5-bit
 //     exponent, so the operands must be O(1): observations are clipped to +-10 by VecNormalize, activations are tanh
-//     outputs, weights are O(1), and the BACKWARD tensors (which carry the 1/B of the batch mean, ~1e-4) are scaled by
+//     outputs (ReLU outputs get their own scale, see PW_H_RELU), weights are O(1), and the BACKWARD tensors (which carry the 1/B of the batch mean, ~1e-4) are scaled by
 //     a power of two S with S/B in [1/16, 1/8) — exact in fp32 — and the weight gradients are multiplied by 1/S when
 //     they leave TMEM.  |x| * S/B > 65504 (a per-sample dL/dmu beyond ~5e5 / B) would overflow to inf and surface as a
 //     non-finite global norm (NaN update, as the graph's IsFinite select does for any non-finite gradient).
@@ -49,7 +49,12 @@ namespace umma {
 // Operand blocks sit high in fp16's range (an fp16 lo piece below 2^-14 is subnormal: values whose hi piece is below ~0.25
 // would lose relative accuracy): weights max in [2^8, 2^9), activations and the ones block times 2^8, observations times 2^5
 // (|obs| <= clip_obs = 10), back-propagated tensors times S and renormalised by 2^-8 after every product with a weight block.
-constexpr int PW_W = 8, PW_H = 8, PW_X = 5;
+// ReLU activations are unbounded, so their blocks (and the ones block with them) hold H * 2^PW_H_RELU = H itself: exact as
+// two pieces for H >= 2^-3, an absolute error <= 2^-25 below that, and H up to fp16's 65504.  A larger activation becomes
+// inf and surfaces as a non-finite global norm (a NaN update), as an overflowing backward tensor does.
+constexpr int PW_W = 8, PW_H = 8, PW_X = 5, PW_H_RELU = 0;
+template <int ACT>
+constexpr int pw_h() { return ACT == ACT_RELU ? PW_H_RELU : PW_H; }
 constexpr int TM = 128;   // samples per tile
 constexpr int NTH = 256;  // threads per CTA
 constexpr int HID = 64;   // hidden width handled by this family
@@ -301,6 +306,11 @@ __device__ __forceinline__ float tanh_epi(float x) {
     const float small = fmaf(x * x2, fmaf(x2, 0.13333333f, -0.33333333f), x);
     return fabsf(x) < 0.0625f ? small : big;
 }
+template <int ACT>
+__device__ __forceinline__ float act_epi(float x) {
+    if (ACT == ACT_RELU) return act_fwd<ACT_RELU>(x);
+    return tanh_epi(x);
+}
 // x0, x1 -> two packed fp16 pairs hi, lo with x = hi + lo (x0 in the low half = lower address)
 __device__ __forceinline__ void split_pair(float x0, float x1, uint32_t& p0, uint32_t& p1) {
     const __half2 h = __floats2half2_rn(x0, x1);
@@ -408,7 +418,7 @@ struct EpochArgs {
 // minibatch.  (A barrier-free variant — every cross-CTA hand-over an LL word polled by its consumer — was built and measured
 // in round 2: 7.22 ms per C3 update against 6.97 ms; each dependent global hop costs ~0.8 us either way and the LL slabs
 // double the bytes of the largest exchange.  profiles/r2_u_family_ll_experiment.txt; not kept.)
-template <int O, int A, int MODE>
+template <int O, int A, int MODE, int ACT>
 __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, const EpochArgs ep) {
     constexpr bool PERSIST = MODE != 0;
     static_assert(O % 2 == 0 && O >= 2 && O <= 30 && A % 2 == 0 && A >= 2 && A <= 32, "unsupported obs/act width");
@@ -490,11 +500,12 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
     }
     // constant operand blocks: the V tower's dv rows (row 0 is rewritten per tile, rows 1..7 stay zero) and the ones block
-    // (row 0 of each 8-row group = 2^PW_H = 256.0 = fp16 0x5C00, the scale of the activation blocks; rows 1..7 = 0)
+    // (row 0 of each 8-row group = 2^PW_H = 256.0 = fp16 0x5C00, the scale of the activation blocks; rows 1..7 = 0;
+    // ReLU: 2^PW_H_RELU = 1.0 = fp16 0x3C00)
     if (tower != 0)
         for (int i = tid; i < (int)ROW16_BLOCK / 16; i += NTH) reinterpret_cast<uint4*>(smem + OFF_WP)[i] = make_uint4(0, 0, 0, 0);
     if (tid < (int)ROW16_BLOCK / 16) {  // per 64-sample half: 128 chunks of 16 B, the first 8 are row 0
-        const uint32_t v = ((tid & 127) < 8) ? 0x5C005C00u : 0u;
+        const uint32_t v = ((tid & 127) < 8) ? (ACT == ACT_RELU ? 0x3C003C00u : 0x5C005C00u) : 0u;
         reinterpret_cast<uint4*>(smem + OFF_ONES)[tid] = make_uint4(v, v, v, v);
     }
     // persistent state: grid barrier generation, mailbox sequence number, Adam's beta powers (every CTA tracks them)
@@ -730,13 +741,14 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
         }
         UMMA_PROF();  // weight blocks written
         // epilogue factors of this minibatch (exact powers of two)
-        const float u_w0 = pow2f(-k_w0 - PW_X), u_w1 = pow2f(-k_w1 - PW_H), u_hd = pow2f(-k_hd - PW_H);
+        constexpr int PWH = pw_h<ACT>();
+        const float u_w0 = pow2f(-k_w0 - PW_X), u_w1 = pow2f(-k_w1 - PWH), u_hd = pow2f(-k_hd - PWH);
         const float s_hd_v = pow2f(k_hd - PW_W);                 // V tower: dP2 = dv * (wv 2^kh) (1 - g2^2), kh = k_hd - PW_W
         const float S_b = pow2f(n_s);                            // backward tensors are stored times S_b
         constexpr float RENORM = 1.0f / (float)(1 << PW_W);      // after a product with a weight block (W * 2^(kh + PW_W))
-        constexpr float H_SCALE = (float)(1 << PW_H);            // activation blocks hold H * 2^PW_H
-        const float un_hd = pow2f(-n_s - PW_H);                               // dWpi, column sums (ones = 2^PW_H), dWv
-        const float un_w1 = pow2f(-n_s - (k_hd - PW_W) - PW_H);                // dW1, db1
+        constexpr float H_SCALE = (float)(1 << PWH);             // activation blocks hold H * 2^PWH
+        const float un_hd = pow2f(-n_s - PWH);                                // dWpi, column sums (ones = 2^PWH), dWv
+        const float un_w1 = pow2f(-n_s - (k_hd - PW_W) - PWH);                 // dW1, db1
         const float un_w0 = pow2f(-n_s - (k_hd - PW_W) - (k_w1 - PW_W) - PW_X);  // dW0' (bias column: the ones of X' are 2^PW_X)
         xin.store(sY, gr, gh);
         fence_async_smem();
@@ -774,7 +786,7 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
             float v[16];
             tmem_ld16_sum(tlane + ACC_WORK + 32 * half + 16 * hh, tlane + ACC_WORK_C + 32 * half + 16 * hh, v);
 #pragma unroll
-            for (int j = 0; j < 16; ++j) h1r[16 * hh + j] = tanh_epi(v[j] * u_w0);
+            for (int j = 0; j < 16; ++j) h1r[16 * hh + j] = act_epi<ACT>(v[j] * u_w0);
         }
         store_row32(sH1, row, half, h1r, H_SCALE);
         fence_async_smem();
@@ -810,7 +822,7 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
 #pragma unroll
                 for (int j = 0; j < 16; ++j) {
                     const int jj = 16 * hh + j;
-                    h2r[jj] = tanh_epi(fmaf(v[j], u_w1, f32[F32_B1 + 32 * half + jj]));
+                    h2r[jj] = act_epi<ACT>(fmaf(v[j], u_w1, f32[F32_B1 + 32 * half + jj]));
                     pv = fmaf(h2r[jj], f32[F32_WV + 32 * half + jj], pv);
                 }
             }
@@ -907,7 +919,7 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
             float v[32];
             tmem_ld32_sum(tlane + ACC_WORK + 32 * half, tlane + ACC_WORK_C + 32 * half, v);
 #pragma unroll
-            for (int j = 0; j < 32; ++j) v[j] *= (1.f - h2r[j] * h2r[j]) * RENORM;
+            for (int j = 0; j < 32; ++j) v[j] *= act_dfac<ACT>(h2r[j]) * RENORM;
             store_row32(sD2, row, half, v);  // dP2 (its own block: the dWpi GEMM may still be reading H2)
         } else {
             // ---- V head (GRAPH:10213-10400): value, clipped value loss and dL/dv on the CUDA cores
@@ -939,7 +951,7 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
             const float dvr = f32[F32_DV + row];
             float v[32];
 #pragma unroll
-            for (int j = 0; j < 32; ++j) v[j] = dvr * (f32[F32_WV + 32 * half + j] * s_hd_v) * (1.f - h2r[j] * h2r[j]);
+            for (int j = 0; j < 32; ++j) v[j] = dvr * (f32[F32_WV + 32 * half + j] * s_hd_v) * act_dfac<ACT>(h2r[j]);
             UMMA_PROF();
             store_row32(sD2, row, half, v);  // dP2
         }
@@ -970,7 +982,7 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
             float v[32];
             tmem_ld32_sum(tlane + ACC_WORK + 32 * half, tlane + ACC_WORK_C + 32 * half, v);
 #pragma unroll
-            for (int j = 0; j < 32; ++j) v[j] *= (1.f - h1r[j] * h1r[j]) * RENORM;
+            for (int j = 0; j < 32; ++j) v[j] *= act_dfac<ACT>(h1r[j]) * RENORM;
             store_row32(sD1, row, half, v);  // dP1
         }
         fence_async_smem();

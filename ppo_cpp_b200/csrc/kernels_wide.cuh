@@ -54,7 +54,10 @@ enum { SC_S_W0 = 0, SC_U_W0, SC_S_W1, SC_U_W1, SC_S_HD, SC_U_HD, SC_S_B, SC_UN_H
 //   weights  max in [2^8, 2^9)   activations H * 2^8   observations X' * 2^5 (|obs| <= clip_obs = 10)
 //   back-propagated tensors times S (pi: S / (B sigma_min) in (4, 16], V: S / B in [32, 64)), renormalised by 2^-8 after
 //   every product with a weight image.  fp16 overflows at 65504: headroom of 2^6 .. 2^7 over the typical magnitude.
-constexpr int PW_W = 8, PW_H = 8, PW_X = 5;
+// ReLU activations are unbounded: their images hold H * 2^PW_H_RELU = H (umma::pw_h), exact as two pieces for H >= 2^-3,
+// an absolute error <= 2^-25 below that, H up to 65504; beyond it inf, a non-finite global norm and a NaN update.
+constexpr int PW_W = 8, PW_X = 5;
+using umma::pw_h;
 constexpr uint32_t EPI_STAGE = 4096;  // per epilogue warp: 32 rows x 128 B of an image block, staged for a bulk store
 constexpr uint32_t GEMM_SMEM = NSTAGE * STAGE + 128 + 8 * EPI_STAGE + 1024;  // + barriers + epilogue staging + alignment slack
 constexpr int COLPART = 64;        // floats per tile written by the loss kernel
@@ -88,7 +91,7 @@ struct Geom {
 
 enum { MODE_FWD = 0, MODE_BWD = 1, MODE_DW = 2 };
 enum { DW_W1 = 0, DW_HEAD = 1, DW_W0 = 2 };
-enum { EPI_STORE = 0, EPI_ACT = 1, EPI_DACT = 2, EPI_LOSS = 3 };  // fp32 result | tanh(acc + b) -> image | acc * (1 - H^2) -> image (+ column sums) | heads -> losses -> dY image
+enum { EPI_STORE = 0, EPI_ACT = 1, EPI_DACT = 2, EPI_LOSS = 3 };  // fp32 result | act(acc + b) -> image | acc * act'(H) -> image (+ column sums) | heads -> losses -> dY image
 
 struct DwProb {
     const uint8_t* A; size_t a_tower, a_tile, a_piece;  // M side: image whose features become the rows of the result
@@ -111,7 +114,7 @@ struct GemmArgs {
     uint8_t* img_out;
     size_t img_tower, img_tile, img_piece;
     float* colsum; int cap;                   // EPI_DACT: [tower][tile * 4 + lane quarter][H] partial column sums, or NULL
-    float* gbuf;                              // 1 - H^2 as fp32, [tower][tile][column][128 rows]: written by EPI_ACT, read by EPI_DACT
+    float* gbuf;                              // act'(H) (1 - H^2 / H > 0) as fp32, [tower][tile][column][128 rows]: written by EPI_ACT, read by EPI_DACT
     TrainArgs ta;                             // EPI_LOSS: the minibatch (gather list, rollout buffers, advantage statistics)
     uint8_t* dY; size_t dy_tower, dy_tile;    // EPI_LOSS: head gradients image [tower][tile][piece][16 KB]
     float* colloss;                           // EPI_LOSS: [tile * 4 + lane quarter][COLPART] per-warp sums
@@ -191,6 +194,7 @@ __device__ __forceinline__ Task decode_task(const GemmArgs& g, int t) {
     return k;
 }
 
+template <int ACT>
 __global__ void __launch_bounds__(GEMM_NTH, 1) wgemm_kernel(const GemmArgs g) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -445,7 +449,7 @@ __global__ void __launch_bounds__(GEMM_NTH, 1) wgemm_kernel(const GemmArgs g) {
                     out_base = g.dY + k.tower * g.dy_tower + (size_t)k.m * g.dy_tile + (size_t)q * EPI_STAGE;
                     out_piece = BLK16;
                 } else {
-                // ---- H = tanh(acc + b) or dP = acc * (1 - H^2), 64 columns = column block cb of the layer
+                // ---- H = act(acc + b) or dP = acc * act'(H), 64 columns = column block cb of the layer
                 const int col0 = k.n * g.n_tile + 64 * half;
                 const size_t boff = k.tower * g.img_tower + (size_t)k.m * g.img_tile + (size_t)(col0 >> 6) * BLK16 + (size_t)q * EPI_STAGE;
                 float* gp = g.gbuf + (((size_t)k.tower * g.cap + k.m) * g.H + col0) * TM + row;
@@ -467,11 +471,11 @@ __global__ void __launch_bounds__(GEMM_NTH, 1) wgemm_kernel(const GemmArgs g) {
                     const float u_w = __ldg(g.sc + k.tower * SC_STRIDE + g.sc_fwd);  // the weight image is W * 2^k
 #pragma unroll
                     for (int i = 0; i < 64; ++i) {
-                        v[i] = tanhf(ob >= 0 ? fmaf(v[i], u_w, __ldg(g.P + ob + col0 + i)) : v[i] * u_w);
-                        if (g.gbuf) gp[(size_t)i * TM] = 1.f - v[i] * v[i];  // kept for the backward pass (training only)
-                        v[i] *= (float)(1 << PW_H);                          // the image holds H * 2^PW_H
+                        v[i] = act_fwd<ACT>(ob >= 0 ? fmaf(v[i], u_w, __ldg(g.P + ob + col0 + i)) : v[i] * u_w);
+                        if (g.gbuf) gp[(size_t)i * TM] = act_dfac<ACT>(v[i]);  // kept for the backward pass (training only)
+                        v[i] *= (float)(1 << pw_h<ACT>());                    // the image holds H * 2^pw_h
                     }
-                } else {  // TanhGrad (GRAPH:20925-23699)
+                } else {  // TanhGrad / ReluGrad (GRAPH:20925-23699)
 #pragma unroll
                     for (int i = 0; i < 64; ++i) v[i] *= gr[i] * (1.0f / (float)(1 << PW_W));  // renormalised: the weight image was W * 2^(k + PW_W)
                     if (g.colsum) {  // bias gradient: column sums over this warp's 32 rows
@@ -647,6 +651,7 @@ __device__ __forceinline__ int pow2_to_unit(float m) {
 }
 
 // fp32 parameters -> weight images.  One thread per 16-byte chunk.
+template <int ACT>
 __global__ void wide_prep_weights_kernel(const float* __restrict__ P, const NetDims d, const WideBufs w, float invB) {
     const Geom& G = w.G;
     const int nb = G.nb, H = G.H;
@@ -670,6 +675,7 @@ __global__ void wide_prep_weights_kernel(const float* __restrict__ P, const NetD
         const int n_s = t == 0 ? (-e_b + k_sig + 4) : (-e_b + 6);   // pi: S * invB / sigma_min in (4, 16]; V: S * invB in [32, 64)
         // the backward chain renormalises by 2^-PW_W after each weight image, so dP2 carries S * 2^kh, dP1 S * 2^(kh + k1)
         const int kh = k_hd - PW_W, k1 = k_w1 - PW_W;
+        constexpr int PW_H = pw_h<ACT>();  // activation images hold H * 2^PW_H
         float* r = s_sc[t];
         r[SC_S_W0] = ldexpf(1.f, k_w0); r[SC_U_W0] = ldexpf(1.f, -k_w0 - PW_X);   // layer 0: acc = (X' 2^PW_X)(W0' 2^k)
         r[SC_S_W1] = ldexpf(1.f, k_w1); r[SC_U_W1] = ldexpf(1.f, -k_w1 - PW_H);   // layer 1: acc = (H1 2^PW_H)(W1 2^k)

@@ -246,6 +246,94 @@ int classify_vf_clip(const NodeMap& nodes, std::string& err) {
     return -1;
 }
 
+// Stable-Baselines' MlpPolicy builds every hidden layer as act(matmul(x, w) + b) (policies.py mlp_extractor / a2c/utils.py
+// linear), with act the policy's act_fun.  The activation is classified by following the data flow into the layer that reads
+// it: for each (hidden layer L, reader N) pair, every forward MatMul (in the model/ or train_model/ scope, neither operand
+// transposed) whose weight operand is the read of model/N/w must take a Tanh or Relu of Add(MatMul(., read of model/L/w),
+// read of model/L/b), and every pair has such a reader in both scopes.  The gradient sub-graph's MatMuls (under
+// loss/gradients/, dY * W^T with transpose_b, X^T * dY with transpose_a) also read the weights and are not readers.  Node
+// names of the activations are not relied on (model/Tanh, model/Tanh_1, ... in construction order).  Returns ACT_TANH (0)
+// or ACT_RELU (1); a file with no forward nodes (files of write_meta_txt) is tanh; -1 with err naming the node otherwise.
+int classify_activation(const NodeMap& nodes, std::string& err) {
+    for (const char* v : {"model/pi_fc2/w", "model/vf_fc2/w", "model/shared_fc0/w"})
+        if (nodes.count(v)) {
+            err = std::string("variable ") + v + ": only two hidden layers per tower, without a shared trunk, are supported";
+            return -1;
+        }
+    auto op_of = [&](const std::string& name) -> std::string {
+        auto it = nodes.find(name);
+        return it == nodes.end() ? std::string() : it->second->str("op");
+    };
+    auto is_read_of = [&](const std::string& name, const std::string& var) -> bool {
+        auto it = nodes.find(name);
+        if (it == nodes.end() || it->second->str("op") != "Identity") return false;
+        const std::vector<std::string> in = node_inputs(*it->second);
+        return in.size() == 1 && in[0] == var;
+    };
+    auto attr_true = [](const Msg& node, const char* key) -> bool {
+        const Msg* v = attr_value(node, key);
+        return v && v->str("b") == "true";
+    };
+    // 0: model/, 1: train_model/, -1: neither or not a plain x * W product
+    auto forward_scope = [&](const std::string& name, const Msg& node) -> int {
+        if (node.str("op") != "MatMul" || attr_true(node, "transpose_a") || attr_true(node, "transpose_b")) return -1;
+        if (name.compare(0, 6, "model/") == 0) return 0;
+        if (name.compare(0, 12, "train_model/") == 0) return 1;
+        return -1;
+    };
+    static const char* const kPairs[4][2] = {{"pi_fc0", "pi_fc1"}, {"pi_fc1", "pi"}, {"vf_fc0", "vf_fc1"}, {"vf_fc1", "vf"}};
+    std::string first_op, first_node;
+    int found = 0, per_scope[4][2] = {};
+    for (int pi = 0; pi < 4; ++pi) {
+        const std::string L = kPairs[pi][0], N = kPairs[pi][1];
+        for (const auto& kv : nodes) {
+            const Msg& mm = *kv.second;
+            const int scope = forward_scope(kv.first, mm);
+            if (scope < 0) continue;
+            const std::vector<std::string> mi = node_inputs(mm);
+            if (mi.size() != 2 || !is_read_of(mi[1], "model/" + N + "/w")) continue;
+            ++found;
+            ++per_scope[pi][scope];
+            const std::string act = mi[0], aop = op_of(act);
+            if (aop != "Tanh" && aop != "Relu") {
+                err = "node " + kv.first + " reads " + act + " (op " + (aop.empty() ? std::string("missing") : aop) +
+                      "), not a Tanh or Relu of layer " + L;
+                return -1;
+            }
+            const std::vector<std::string> ai = node_inputs(*nodes.at(act));
+            const std::string add = ai.size() == 1 ? ai[0] : std::string(), addop = op_of(add);
+            std::vector<std::string> di;
+            if (addop == "Add" || addop == "AddV2" || addop == "BiasAdd") di = node_inputs(*nodes.at(add));
+            bool ok = false;
+            for (int s = 0; s < 2 && di.size() == 2; ++s) {
+                const std::string &m = di[s], &b = di[1 - s];
+                if (op_of(m) != "MatMul" || forward_scope(m, *nodes.at(m)) < 0 || !is_read_of(b, "model/" + L + "/b")) continue;
+                const std::vector<std::string> li = node_inputs(*nodes.at(m));
+                ok = li.size() == 2 && is_read_of(li[1], "model/" + L + "/w");
+            }
+            if (!ok) {
+                err = "activation node " + act + " (read by " + kv.first + ") is not act(matmul(x, model/" + L + "/w) + model/" + L + "/b)";
+                return -1;
+            }
+            if (first_op.empty()) {
+                first_op = aop;
+                first_node = act;
+            } else if (aop != first_op) {
+                err = "the graph mixes activations: " + first_node + " is " + first_op + ", " + act + " is " + aop;
+                return -1;
+            }
+        }
+    }
+    if (found == 0) return 0;
+    for (int pi = 0; pi < 4; ++pi)
+        for (int scope = 0; scope < 2; ++scope)
+            if (per_scope[pi][scope] == 0) {
+                err = std::string("no forward MatMul under ") + (scope ? "train_model/" : "model/") + " reads model/" + kPairs[pi][1] + "/w";
+                return -1;
+            }
+    return first_op == "Relu" ? 1 : 0;
+}
+
 }  // namespace
 
 std::string parse_meta_txt(const std::string& path, MetaGraph& out) {
@@ -263,6 +351,7 @@ std::string parse_meta_txt(const std::string& path, MetaGraph& out) {
     for (const auto& f : graph->fields)
         if (f.key == "node" && f.msg) nodes[f.msg->str("name")] = f.msg.get();
     out.vf_clip = classify_vf_clip(nodes, out.vf_clip_error);
+    out.activation = classify_activation(nodes, out.activation_error);
 
     for (int i = 0; i < kNumTensors; ++i) {
         const std::string name = kTensorNames[i];

@@ -1,7 +1,7 @@
 // Minimal reader for TensorFlow-1.14 text-proto MetaGraphDef files (.meta.txt).
 // Replaces SessionCreator::load_graph (reference ppo2/session_creator.hpp:23-57): the graph is read,
 // never executed.  Extracts variable shapes, initial values, the constants the graph bakes in and which value loss
-// the graph builds.
+// the graph builds and the hidden-layer activation of its forward pass.
 #pragma once
 #include <map>
 #include <string>
@@ -21,6 +21,10 @@ struct MetaGraph {
     // when the loss sub-graph is there but matches none of them (vf_clip_error says why)
     int vf_clip = 0;
     std::string vf_clip_error;
+    // hidden-layer activation (ppo_activation: 0 tanh, 1 relu), or -1 when the forward pass is not two tanh or two relu
+    // hidden layers per tower (activation_error says why)
+    int activation = 0;
+    std::string activation_error;
     std::map<std::string, MetaTensor> tensors;  // the 15 model/* variables with their initial values
 };
 

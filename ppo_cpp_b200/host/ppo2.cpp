@@ -33,7 +33,7 @@ const std::map<std::string, std::string> kValueFlags = {
     {"--reset_noise_scale", "rns"}, {"--reset_noise", "rns"}, {"--rns", "rns"}, {"--rn", "rns"}, {"--duration", "duration"}, {"--du", "duration"},
     {"-j", "threads"}, {"--jobs", "threads"}, {"--threads", "threads"}, {"--n_threads", "threads"}, {"--num_threads", "threads"}, {"--nt", "threads"},
     {"-f", "fps"}, {"--framerate", "fps"}, {"--fps", "fps"}, {"--env", "env"}, {"--seed", "seed"}, {"--hidden", "hidden"},
-    {"--cliprange_vf", "cliprange_vf"}, {"--clip_range_vf", "cliprange_vf"}};
+    {"--cliprange_vf", "cliprange_vf"}, {"--clip_range_vf", "cliprange_vf"}, {"--activation", "activation"}};
 const std::map<std::string, std::string> kBoolFlags = {
     {"--closed_loop", "cl"}, {"--closed-loop", "cl"}, {"--cl", "cl"}, {"-v", "verbose"}, {"--verbose", "verbose"}, {"-r", "resume"},
     {"--resume", "resume"}, {"--bullet", "bullet"}, {"--use_bullet", "bullet"}, {"--bullet_solver", "bullet"}, {"-h", "help"}, {"--help", "help"}};
@@ -86,7 +86,8 @@ int main(int argc, char** argv) {
                      "  --saves, --epochs --num_epochs, --batch_steps --n_steps, --rns, --cl, -v, -r --resume, --bullet,\n"
                      "  --duration, -j --threads, -f --fps   (as in the reference's ppo2.cpp:93-128)\n"
                      "  --env synthetic|mock, --seed N, --hidden H1,H2,\n"
-                     "  --cliprange_vf (-1: the graph's value loss decides; >= 0 for a graph with loss/clip_range_vf_ph)\n";
+                     "  --cliprange_vf (-1: the graph's value loss decides; >= 0 for a graph with loss/clip_range_vf_ph),\n"
+                     "  --activation tanh|relu (graph-less runs; with a graph it must name the graph's own activation)\n";
         return 0;
     }
     const std::string save_path = get(a, "dir", "./exp/ppo_cpp"), graph_path = get(a, "graph", "");
@@ -98,6 +99,20 @@ int main(int argc, char** argv) {
     const int threads = std::stoi(get(a, "threads", "1"));
     const double duration = std::stod(get(a, "duration", "5."));
     const std::string env_kind = get(a, "env", "synthetic");
+    const std::string act_name = get(a, "activation", "");
+    if (!act_name.empty() && act_name != "tanh" && act_name != "relu") {
+        std::cerr << "--activation must be tanh or relu, not " << act_name << std::endl;
+        return 1;
+    }
+    const int act = act_name == "relu" ? PPO_ACT_RELU : PPO_ACT_TANH;
+    if (!act_name.empty() && !graph_path.empty()) {
+        const int graph_act = ppo_meta_activation(graph_path.c_str());
+        if (graph_act >= 0 && graph_act != act) {
+            std::cerr << "--activation " << act_name << " contradicts the graph " << graph_path << ", whose hidden layers are "
+                      << (graph_act == PPO_ACT_RELU ? "relu" : "tanh") << std::endl;
+            return 1;
+        }
+    }
 
     unsigned seed_val;
     if (a.values.count("seed")) {
@@ -136,9 +151,15 @@ int main(int argc, char** argv) {
     if (graph_path.empty() && !has_load) {
         int h1 = 64, h2 = 64;
         if (a.values.count("hidden")) sscanf(a.values["hidden"].c_str(), "%d,%d", &h1, &h2);
-        algorithm.reset_without_graph(h1, h2, seed_val);
+        algorithm.reset_without_graph(h1, h2, seed_val, act);
     }
-    if (has_load) algorithm.load(a.values["path"]);
+    if (has_load) {
+        algorithm.load(a.values["path"]);
+        if (!act_name.empty() && algorithm.activation() != act) {
+            std::cerr << "--activation " << act_name << " contradicts the checkpoint " << a.values["path"] << std::endl;
+            return 1;
+        }
+    }
 
     if (training) {
         mkdir_p(tb_path);

@@ -73,13 +73,16 @@ public:
         cr_schedule_ = std::move(cr);
         cr_vf_schedule_ = std::move(cr_vf);
     }
-    // graph-less construction for sizes the reference ships no graph for (orthogonal init as Stable-Baselines)
-    void reset_without_graph(int hidden1, int hidden2, uint64_t init_seed) {
+    // graph-less construction for sizes the reference ships no graph for (orthogonal init as Stable-Baselines);
+    // activation is a ppo_activation (a graph-built model follows its graph's)
+    void reset_without_graph(int hidden1, int hidden2, uint64_t init_seed, int activation = PPO_ACT_TANH) {
         hidden_override_[0] = hidden1;
         hidden_override_[1] = hidden2;
         init_seed_ = init_seed;
+        activation_ = activation;
         reset();
     }
+    int activation() const { return activation_; }
 
     void reset() {
         n_batch = n_envs * n_steps;
@@ -114,8 +117,10 @@ public:
         if (from_graph) {
             // the graph's baked ent_coef / vf_coef / clip norm / Adam constants win over the constructor's (SURVEY §3.5)
             ppo_check(ppo_core_load_meta_txt(core_.get(), model_filename.c_str()), "graph load");
+            activation_ = ppo_core_activation(core_.get());
         } else {
             ppo_check(ppo_core_init_orthogonal(core_.get(), init_seed_), "orthogonal init");
+            ppo_check(ppo_core_set_activation(core_.get(), activation_), "activation");
         }
         ppo_check(ppo_shuffle_seed(core_.get(), shuffle_seed_), "shuffle seed");
         if (normalize) normalize->attach_core(core_);
@@ -138,6 +143,7 @@ public:
         if (hidden_override_[0] > 0) {
             json["hidden1"] = hidden_override_[0];
             json["hidden2"] = hidden_override_[1];
+            if (activation_ == PPO_ACT_RELU) json["activation"] = "relu";  // absent: tanh
         }
         std::ofstream myfile(save_path + ".json");
         if (myfile.is_open()) {
@@ -182,6 +188,9 @@ public:
             }
             hidden_override_[0] = json["hidden1"].get<int>();
             hidden_override_[1] = json["hidden2"].get<int>();
+            const std::string act = json.contains("activation") ? json["activation"].get<std::string>() : std::string("tanh");
+            if (act != "tanh" && act != "relu") throw std::runtime_error("checkpoint " + save_path + ".json: unknown activation " + act);
+            activation_ = act == "relu" ? PPO_ACT_RELU : PPO_ACT_TANH;
         }
         reset();
         env.deserialize(json);  // after reset(): the statistics live in the (new) core
@@ -297,6 +306,7 @@ private:
     uint64_t noise_seed_ = 0;
     int hidden_override_[2] = {0, 0};
     uint64_t init_seed_ = 0;
+    int activation_ = PPO_ACT_TANH;  // ppo_activation of the core (graph-less: chosen; otherwise the graph's)
     CorePtr core_;
     std::unique_ptr<MlpPolicy> act_model;
 };

@@ -107,6 +107,7 @@ class MetaInfo:
     adam_eps: float
     tf_version: str = ""
     vf_clip: str = "shared"
+    activation: str = "tanh"
     shapes: Dict[str, Tuple[int, ...]] = field(default_factory=dict)
 
     def flat_params(self, include_q: bool = True) -> np.ndarray:
@@ -186,6 +187,84 @@ def classify_vf_clip(nodes: Dict[str, dict]) -> str:
     raise ValueError(f"the value clip bound {ni[1]} is neither loss/clip_range_ph nor loss/clip_range_vf_ph")
 
 
+_ACT_PAIRS = (("pi_fc0", "pi_fc1"), ("pi_fc1", "pi"), ("vf_fc0", "vf_fc1"), ("vf_fc1", "vf"))
+
+
+def classify_activation(nodes: Dict[str, dict]) -> str:
+    """The hidden-layer activation of Stable-Baselines' MlpPolicy, act(matmul(x, w) + b) with act = act_fun: for each
+    (hidden layer L, reader N) pair, every forward MatMul (in the model/ or train_model/ scope, neither operand transposed;
+    the gradient sub-graph's MatMuls also read the weights) whose weight operand is the read of model/N/w must take a Tanh
+    or Relu of Add(MatMul(., read of model/L/w), read of model/L/b), and every pair has such a reader in both scopes.
+    "tanh" / "relu" when all agree; a graph without forward nodes is "tanh"; anything else (another activation, mixed
+    activations, a deeper or shared-trunk net_arch) raises ValueError.  Twin of classify_activation in csrc/meta_parser.cpp."""
+    for v in ("model/pi_fc2/w", "model/vf_fc2/w", "model/shared_fc0/w"):
+        if v in nodes:
+            raise ValueError(f"variable {v}: only two hidden layers per tower, without a shared trunk, are supported")
+
+    def op_of(name):
+        n = nodes.get(name)
+        return n["op"][0].decode() if n is not None else ""
+
+    def is_read_of(name, var):
+        return op_of(name) == "Identity" and _inputs(nodes[name]) == [var]
+
+    def attr_true(node, key):
+        v = _attr(node, key)
+        return v is not None and v.get("b", ["false"])[0] == "true"
+
+    def forward_scope(name):
+        """0: model/, 1: train_model/, -1: neither or not a plain x * W product."""
+        n = nodes.get(name)
+        if n is None or op_of(name) != "MatMul" or attr_true(n, "transpose_a") or attr_true(n, "transpose_b"):
+            return -1
+        return 0 if name.startswith("model/") else 1 if name.startswith("train_model/") else -1
+
+    first = None
+    found = 0
+    per_scope = [[0, 0] for _ in _ACT_PAIRS]
+    for pi, (L, N) in enumerate(_ACT_PAIRS):
+        for name in sorted(nodes):
+            scope = forward_scope(name)
+            if scope < 0:
+                continue
+            mi = _inputs(nodes[name])
+            if len(mi) != 2 or not is_read_of(mi[1], f"model/{N}/w"):
+                continue
+            found += 1
+            per_scope[pi][scope] += 1
+            act, aop = mi[0], op_of(mi[0])
+            if aop not in ("Tanh", "Relu"):
+                raise ValueError(f"node {name} reads {act} (op {aop or 'missing'}), not a Tanh or Relu of layer {L}")
+            ai = _inputs(nodes[act])
+            add = ai[0] if len(ai) == 1 else ""
+            di = _inputs(nodes[add]) if op_of(add) in ("Add", "AddV2", "BiasAdd") else []
+            ok = False
+            for s in range(2 if len(di) == 2 else 0):
+                m, b = di[s], di[1 - s]
+                if forward_scope(m) < 0 or not is_read_of(b, f"model/{L}/b"):
+                    continue
+                li = _inputs(nodes[m])
+                ok = len(li) == 2 and is_read_of(li[1], f"model/{L}/w")
+            if not ok:
+                raise ValueError(f"activation node {act} (read by {name}) is not act(matmul(x, model/{L}/w) + model/{L}/b)")
+            if first is None:
+                first = (aop, act)
+            elif aop != first[0]:
+                raise ValueError(f"the graph mixes activations: {first[1]} is {first[0]}, {act} is {aop}")
+    if found == 0:
+        return "tanh"
+    for (L, N), counts in zip(_ACT_PAIRS, per_scope):
+        for scope, n in zip(("model/", "train_model/"), counts):
+            if n == 0:
+                raise ValueError(f"no forward MatMul under {scope} reads model/{N}/w")
+    return "relu" if first[0] == "Relu" else "tanh"
+
+
+def meta_activation(path: str) -> str:
+    """The hidden-layer activation of a graph file ("tanh" / "relu"), read by this module's parser."""
+    return parse_meta_txt(path).activation
+
+
 def parse_meta_txt(path: str) -> MetaInfo:
     with open(path, "r", encoding="latin-1") as f:
         text = f.read()
@@ -232,6 +311,7 @@ def parse_meta_txt(path: str) -> MetaInfo:
         adam_eps=scalar("ppo2/_train/epsilon"),
         tf_version=ver,
         vf_clip=classify_vf_clip(nodes),
+        activation=classify_activation(nodes),
         shapes=shapes,
     )
 
@@ -291,16 +371,20 @@ def _escape(b: bytes) -> str:
 
 def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 0.0, vf_coef: float = 0.5,
                    clip_norm: float = 0.5, beta1: float = 0.9, beta2: float = 0.999, adam_eps: float = 1e-5,
-                   vf_clip: str | None = None) -> None:
+                   vf_clip: str | None = None, activation: str | None = None) -> None:
     """Write a minimal .meta.txt (variables + initialisers + baked constants) that both readers accept.
 
     The reference's graphs come from a Stable-Baselines/TensorFlow export script that is not part of the
     repo; this writer lets a user produce a graph file for other hidden sizes without TensorFlow.
     vf_clip = "shared" | "none" | "separate" adds the value-loss nodes that tell the readers which value loss the
     graph builds (Stable-Baselines' cliprange_vf None / < 0 / >= 0), named as Stable-Baselines names them;
-    without it the file has no loss sub-graph and reads as "shared"."""
+    without it the file has no loss sub-graph and reads as "shared".
+    activation = "tanh" | "relu" adds the forward nodes that tell the readers the hidden-layer activation (Stable-Baselines'
+    act_fun), under model/ and train_model/ as Stable-Baselines names them; without it the file has none and reads as "tanh"."""
     if vf_clip not in (None, "shared", "none", "separate"):
         raise ValueError(f"vf_clip must be None, 'shared', 'none' or 'separate', not {vf_clip!r}")
+    if activation not in (None, "tanh", "relu"):
+        raise ValueError(f"activation must be None, 'tanh' or 'relu', not {activation!r}")
     def dims(shape, ind):
         return "".join(f"{ind}dim {{\n{ind}  size: {d}\n{ind}}}\n" for d in shape)
 
@@ -325,6 +409,8 @@ def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 
         arr = np.asarray(tensors[name], np.float32)
         parts.append(const_node(f"{name}/Initializer/initial_value", arr))
         parts.append(var_node(name, arr.shape))
+    if activation is not None:
+        parts.append(_forward_nodes(activation))
     if vf_clip is not None:
         parts.append(_vf_loss_nodes(vf_clip))
     for name, val in (("loss/mul_4/y", ent_coef), ("loss/mul_5/y", vf_coef), ("loss/clip_by_global_norm/mul/x", clip_norm),
@@ -333,6 +419,40 @@ def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 
     parts.append("}\n")
     with open(path, "w", encoding="latin-1") as f:
         f.write("".join(parts))
+
+
+def _op_node(name, kind, *inputs):
+    ins = "".join(f'    input: "{i}"\n' for i in inputs)
+    return f'  node {{\n    name: "{name}"\n    op: "{kind}"\n{ins}  }}\n'
+
+
+def _forward_nodes(activation: str) -> str:
+    """The forward pass of Stable-Baselines' MlpPolicy that classify_activation reads (ops and data inputs only): the
+    variables' reads, then per scope (the act model, and train_model that reuses its variables) the hidden layers in
+    mlp_extractor's order (pi_fc0, vf_fc0, pi_fc1, vf_fc1: activations Tanh, Tanh_1, ... or Relu, Relu_1, ...) and the heads."""
+    kind = {"tanh": "Tanh", "relu": "Relu"}[activation]
+    layers = ("pi_fc0", "pi_fc1", "vf_fc0", "vf_fc1", "vf", "pi")
+    nodes = []
+    for layer in layers:
+        for v in ("w", "b"):
+            nodes.append(_op_node(f"model/{layer}/{v}/read", "Identity", f"model/{layer}/{v}"))
+    for scope in ("model", "train_model"):
+        x = f"{scope}/flatten/Reshape"
+        latent = {"pi": x, "vf": x}
+        k = 0
+        for idx in (0, 1):
+            for tower in ("pi", "vf"):
+                layer = f"{tower}_fc{idx}"
+                act = f"{scope}/{kind}" + (f"_{k}" if k else "")
+                k += 1
+                nodes += [_op_node(f"{scope}/{layer}/MatMul", "MatMul", latent[tower], f"model/{layer}/w/read"),
+                          _op_node(f"{scope}/{layer}/add", "Add", f"{scope}/{layer}/MatMul", f"model/{layer}/b/read"),
+                          _op_node(act, kind, f"{scope}/{layer}/add")]
+                latent[tower] = act
+        for head, tower in (("vf", "vf"), ("pi", "pi")):
+            nodes += [_op_node(f"{scope}/{head}/MatMul", "MatMul", latent[tower], f"model/{head}/w/read"),
+                      _op_node(f"{scope}/{head}/add", "Add", f"{scope}/{head}/MatMul", f"model/{head}/b/read")]
+    return "".join(nodes)
 
 
 def _vf_loss_nodes(vf_clip: str) -> str:
