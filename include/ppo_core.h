@@ -106,10 +106,27 @@ typedef enum { PPO_ACT_TANH = 0, PPO_ACT_RELU = 1 } ppo_activation;
  * activation, mixed activations, or a deeper / shared-trunk net_arch.  ppo_meta_parse fails the same way. */
 int ppo_meta_activation(const char *meta_txt_path);
 
-int ppo_core_create(const ppo_core_desc *desc, ppo_core **out);
+/* Action space of the policy head (Stable-Baselines' probability distribution of the env's action space):
+ *   BOX       DiagGaussianProbabilityDistribution: mean = model/pi, std = exp(model/pi/logstd); actions are act_dim floats
+ *   DISCRETE  CategoricalProbabilityDistribution over act_dim = n logits (model/pi, no logstd): an action is ONE index
+ *             0 .. n-1, stored as fp32 wherever actions are passed (action width 1); it is sampled as
+ *             argmax_j (l_j - log(-log(u_j))) with u uniform in [0, 1), and ppo_policy_step's eps holds those n uniforms per env.
+ *             ppo_meta_parse counts 14 tensors (no logstd); checkpoints hold them in sorted-name order.
+ *             The S / U / W kernel families, the persistent rollout and the synthetic env are continuous-only: a DISCRETE core
+ *             runs the F or T family, and the synthetic-env entry points return PPO_ERR_UNSUPPORTED. */
+typedef enum { PPO_ACTION_BOX = 0, PPO_ACTION_DISCRETE = 1 } ppo_action_space;
+/* the ppo_action_space of a graph file: BOX with model/pi/logstd, DISCRETE without it.  When the file has PPO2's placeholder
+ * loss/action_ph it must agree (float [?, n] for BOX, int32 / int64 [?] for DISCRETE), otherwise PPO_ERR_UNSUPPORTED naming the
+ * node; ppo_meta_parse fails the same way. */
+int ppo_meta_action_space(const char *meta_txt_path);
+
+int ppo_core_create(const ppo_core_desc *desc, ppo_core **out); /* ppo_core_create_ex(desc, PPO_ACTION_BOX, out) */
+/* a core whose policy head is of the given ppo_action_space (fixed for the core's lifetime) */
+int ppo_core_create_ex(const ppo_core_desc *desc, int action_space, ppo_core **out);
+int ppo_core_action_space(ppo_core *core); /* the core's ppo_action_space, or a negative ppo_status */
 void ppo_core_destroy(ppo_core *core);
-/* load initial weights from the graph file; its shapes must match the desc (ppo2.hpp:90-105 reset()); sets the core's
- * ppo_vf_clip and ppo_activation */
+/* load initial weights from the graph file; its shapes and its ppo_action_space must match the core's (ppo2.hpp:90-105 reset());
+ * sets the core's ppo_vf_clip and ppo_activation */
 int ppo_core_load_meta_txt(ppo_core *core, const char *meta_txt_path);
 /* the value loss of a graph-less core (default SHARED); ppo_core_load_meta_txt sets it from the graph */
 int ppo_core_set_vf_clip(ppo_core *core, int mode);
@@ -129,6 +146,9 @@ int ppo_core_save_checkpoint_data(ppo_core *core, const char *prefix);
 /* the `.index` alone, for a `.data` payload held by the caller (the 15 tensors of an MLP [hidden1, hidden2] policy in ascending name
  * order, n_floats values); no device needed.  Byte-identical to TensorFlow 1.14's BundleWriter on the reference's shipped checkpoint. */
 int ppo_checkpoint_write_index(const char *prefix, int obs_dim, int act_dim, int hidden1, int hidden2, const float *data, size_t n_floats);
+/* ... for either head: PPO_ACTION_DISCRETE leaves model/pi/logstd out (14 tensors) */
+int ppo_checkpoint_write_index_ex(const char *prefix, int action_space, int obs_dim, int act_dim, int hidden1, int hidden2,
+                                  const float *data, size_t n_floats);
 
 /* tensors by TF variable name: "model/pi_fc0/w" ... "model/q/b"; Adam slots "<name>/Adam", "<name>/Adam_1";
  * "beta1_power", "beta2_power"; "params" = the whole flat vector (n_params_total). Host buffers. */

@@ -18,6 +18,7 @@ HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "ppo_core.h")
 PPO_HOST, PPO_DEVICE = 0, 1
 PPO_VF_CLIP_SHARED, PPO_VF_CLIP_NONE, PPO_VF_CLIP_SEPARATE = 0, 1, 2
 PPO_ACT_TANH, PPO_ACT_RELU = 0, 1
+PPO_ACTION_BOX, PPO_ACTION_DISCRETE = 0, 1
 PPO_COMM_ID_BYTES = 128
 PPO_IPC_HANDLE_BYTES = 64
 ABI_VERSION = 1
@@ -79,7 +80,10 @@ def load():
         "ppo_meta_parse": ([C.c_char_p, C.POINTER(MetaInfo), fp, C.c_size_t], C.c_int),
         "ppo_meta_vf_clip": ([C.c_char_p], C.c_int),
         "ppo_meta_activation": ([C.c_char_p], C.c_int),
+        "ppo_meta_action_space": ([C.c_char_p], C.c_int),
         "ppo_core_create": ([C.POINTER(CoreDesc), C.POINTER(core)], C.c_int),
+        "ppo_core_create_ex": ([C.POINTER(CoreDesc), C.c_int, C.POINTER(core)], C.c_int),
+        "ppo_core_action_space": ([core], C.c_int),
         "ppo_core_destroy": ([core], None),
         "ppo_core_load_meta_txt": ([core, C.c_char_p], C.c_int),
         "ppo_core_set_vf_clip": ([core, C.c_int], C.c_int),
@@ -90,6 +94,7 @@ def load():
         "ppo_core_load_checkpoint_data": ([core, C.c_char_p], C.c_int),
         "ppo_core_save_checkpoint_data": ([core, C.c_char_p], C.c_int),
         "ppo_checkpoint_write_index": ([C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.c_size_t], C.c_int),
+        "ppo_checkpoint_write_index_ex": ([C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.c_size_t], C.c_int),
         "ppo_core_num_tensors": ([], C.c_int),
         "ppo_core_tensor_name": ([C.c_int], C.c_char_p),
         "ppo_core_tensor_size": ([core, C.c_char_p], C.c_int),

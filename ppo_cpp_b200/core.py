@@ -21,6 +21,9 @@ VF_CLIP_NAMES = {v: k for k, v in VF_CLIP_MODES.items()}
 # the hidden-layer activations of ppo_activation, by the names write_meta_txt(activation=...) takes
 ACTIVATIONS = {"tanh": _lib.PPO_ACT_TANH, "relu": _lib.PPO_ACT_RELU}
 ACTIVATION_NAMES = {v: k for k, v in ACTIVATIONS.items()}
+# the policy heads of ppo_action_space, by the names write_meta_txt(action_space=...) takes
+ACTION_SPACES = {"box": _lib.PPO_ACTION_BOX, "discrete": _lib.PPO_ACTION_DISCRETE}
+ACTION_SPACE_NAMES = {v: k for k, v in ACTION_SPACES.items()}
 BUFFER_WIDTH = {"obs": None, "returns": 1, "dones": 1, "actions": None, "values": 1, "neglogpacs": 1,
                 "true_rewards": 1, "unnormalized_rewards": 1}
 
@@ -77,6 +80,16 @@ def meta_activation(path: str) -> str:
     return ACTIVATION_NAMES[r]
 
 
+def meta_action_space(path: str) -> str:
+    """The action space of the graph file's policy head: "box" (Gaussian, model/pi/logstd) or "discrete" (categorical, read by the
+    C parser)."""
+    lib = _lib.load()
+    r = lib.ppo_meta_action_space(path.encode())
+    if r < 0:
+        _check(lib, r)
+    return ACTION_SPACE_NAMES[r]
+
+
 def host_rand(seed: int, count: int) -> np.ndarray:
     lib = _lib.load()
     out = np.zeros(count, np.int32)
@@ -99,10 +112,12 @@ def comm_unique_id() -> bytes:
 
 
 class PPOCore:
-    def __init__(self, activation: str = "tanh", **kw):
+    def __init__(self, activation: str = "tanh", action_space: str = "box", **kw):
         self.lib = _lib.load()
         if activation not in ACTIVATIONS:
             raise ValueError(f"activation must be one of {sorted(ACTIVATIONS)}, not {activation!r}")
+        if action_space not in ACTION_SPACES:
+            raise ValueError(f"action_space must be one of {sorted(ACTION_SPACES)}, not {action_space!r}")
         d = CoreDesc()
         _check(self.lib, self.lib.ppo_core_desc_default(C.byref(d)))
         for k, v in kw.items():
@@ -111,8 +126,13 @@ class PPOCore:
             setattr(d, k, v)
         self.desc = d
         self._h = C.c_void_p()
-        _check(self.lib, self.lib.ppo_core_create(C.byref(d), C.byref(self._h)))
+        if action_space == "box":
+            _check(self.lib, self.lib.ppo_core_create(C.byref(d), C.byref(self._h)))
+        else:
+            _check(self.lib, self.lib.ppo_core_create_ex(C.byref(d), ACTION_SPACES[action_space], C.byref(self._h)))
         self.O, self.A = d.obs_dim, d.act_dim
+        # floats of one stored action: the action vector (Box), or the index of a categorical head (Discrete)
+        self.AW = 1 if action_space == "discrete" else d.act_dim
         self.n_envs, self.n_steps = d.n_envs, d.n_steps
         self.n_batch = d.n_envs * d.n_steps
         self.n_batch_global = self.n_batch * max(1, d.world_size)
@@ -164,6 +184,14 @@ class PPOCore:
             raise ValueError(f"activation must be one of {sorted(ACTIVATIONS)}, not {act!r}")
         _check(self.lib, self.lib.ppo_core_set_activation(self._h, ACTIVATIONS[act]))
 
+    @property
+    def action_space(self) -> str:
+        """The core's policy head: "box" (Gaussian) or "discrete" (categorical over act_dim logits)."""
+        r = self.lib.ppo_core_action_space(self._h)
+        if r < 0:
+            _check(self.lib, r)
+        return ACTION_SPACE_NAMES[r]
+
     def graph_builds(self) -> int:
         """CUDA graphs captured and instantiated since the core was created."""
         n = C.c_uint64()
@@ -211,7 +239,7 @@ class PPOCore:
         obs = _f32(obs)
         n = obs.shape[0]
         e = None if eps is None else _f32(eps)
-        act, val, nlp = np.zeros((n, self.A), np.float32), np.zeros(n, np.float32), np.zeros(n, np.float32)
+        act, val, nlp = np.zeros((n, self.AW), np.float32), np.zeros(n, np.float32), np.zeros(n, np.float32)
         _check(self.lib, self.lib.ppo_policy_step(self._h, _addr(obs), n, _addr(e), _addr(act), _addr(val), _addr(nlp), PPO_HOST))
         return act, val, nlp
 
@@ -223,7 +251,7 @@ class PPOCore:
 
     def policy_mean(self, obs):
         obs = _f32(obs)
-        act = np.zeros((obs.shape[0], self.A), np.float32)
+        act = np.zeros((obs.shape[0], self.AW), np.float32)
         _check(self.lib, self.lib.ppo_policy_mean(self._h, _addr(obs), obs.shape[0], _addr(act), PPO_HOST))
         return act
 
@@ -296,7 +324,7 @@ class PPOCore:
         _check(self.lib, self.lib.ppo_runner_reset(self._h, _addr(raw), PPO_HOST))
 
     def runner_act(self, t, out: Optional[np.ndarray] = None):
-        act = out if out is not None else np.zeros((self.n_envs, self.A), np.float32)
+        act = out if out is not None else np.zeros((self.n_envs, self.AW), np.float32)
         _check(self.lib, self.lib.ppo_runner_act(self._h, t, _addr(act), PPO_HOST))
         return act
 
@@ -314,14 +342,14 @@ class PPOCore:
                                                             _addr(actions_out) if actions_out is not None else None))
 
     def runner_rollout_host(self, step_fn):
-        """ppo_runner_rollout_host with a Python env: step_fn(t, actions[n_envs, A]) -> (raw_obs, raw_rew, done) or None to abort."""
+        """ppo_runner_rollout_host with a Python env: step_fn(t, actions[n_envs, AW]) -> (raw_obs, raw_rew, done) or None to abort."""
         n = self.n_envs
         keep = {}
         fpp = C.POINTER(C.POINTER(C.c_float))
 
         @C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_float), fpp, fpp, fpp)
         def cb(_user, t, actions, po, pr, pd):
-            act = np.ctypeslib.as_array(actions, (n, self.A))
+            act = np.ctypeslib.as_array(actions, (n, self.AW))
             out = step_fn(t, act)
             if out is None:
                 return 1
@@ -331,7 +359,7 @@ class PPOCore:
             pd[0] = keep["d"].ctypes.data_as(C.POINTER(C.c_float))
             return 0
 
-        actions = np.zeros((n, self.A), np.float32)
+        actions = np.zeros((n, self.AW), np.float32)
         _check(self.lib, self.lib.ppo_runner_rollout_host(self._h, C.cast(cb, C.c_void_p), None, _addr(actions)))
 
     def synth_env_reset(self):
@@ -341,7 +369,7 @@ class PPOCore:
         _check(self.lib, self.lib.ppo_rollout_synthetic(self._h))
 
     def rollout_get(self, name):
-        w = BUFFER_WIDTH[name] or (self.O if name == "obs" else self.A)
+        w = BUFFER_WIDTH[name] or (self.O if name == "obs" else self.AW)
         out = np.zeros((self.n_batch, w), np.float32)
         _check(self.lib, self.lib.ppo_rollout_get(self._h, name.encode(), _addr(out), out.size))
         return out

@@ -146,21 +146,25 @@ std::string bundle_index_image(const std::vector<std::string>& names, const std:
     return file + footer;
 }
 
-// The 15 model tensors of an MLP [h1, h2] policy in checkpoint (ascending name) order with their TF shapes.
-void model_bundle_layout(int obs_dim, int act_dim, int h1, int h2, std::vector<std::string>& names, std::vector<std::vector<int64_t>>& shapes) {
+// The 15 model tensors of an MLP [h1, h2] policy in checkpoint (ascending name) order with their TF shapes; 14 without
+// model/pi/logstd for a categorical head (Discrete action space).
+void model_bundle_layout(int obs_dim, int act_dim, int h1, int h2, bool discrete, std::vector<std::string>& names,
+                         std::vector<std::vector<int64_t>>& shapes) {
     const int64_t O = obs_dim, A = act_dim, H1 = h1, H2 = h2;
     names = {"model/pi/b", "model/pi/logstd", "model/pi/w", "model/pi_fc0/b", "model/pi_fc0/w", "model/pi_fc1/b", "model/pi_fc1/w", "model/q/b",
              "model/q/w", "model/vf/b", "model/vf/w", "model/vf_fc0/b", "model/vf_fc0/w", "model/vf_fc1/b", "model/vf_fc1/w"};
     shapes = {{A}, {1, A}, {H2, A}, {H1}, {O, H1}, {H2}, {H1, H2}, {A}, {H2, A}, {1}, {H2, 1}, {H1}, {O, H1}, {H2}, {H1, H2}};
+    if (discrete) {
+        names.erase(names.begin() + 1);
+        shapes.erase(shapes.begin() + 1);
+    }
 }
 
-}  // namespace ppo
-
-extern "C" int ppo_checkpoint_write_index(const char* prefix, int obs_dim, int act_dim, int hidden1, int hidden2, const float* data, size_t n_floats) {
+int write_index(const char* prefix, int obs_dim, int act_dim, int hidden1, int hidden2, bool discrete, const float* data, size_t n_floats) {
     if (!prefix || !data || obs_dim < 1 || act_dim < 1 || hidden1 < 1 || hidden2 < 1) return -1;  // PPO_ERR_INVALID
     std::vector<std::string> names;
     std::vector<std::vector<int64_t>> shapes;
-    ppo::model_bundle_layout(obs_dim, act_dim, hidden1, hidden2, names, shapes);
+    model_bundle_layout(obs_dim, act_dim, hidden1, hidden2, discrete, names, shapes);
     size_t total = 0;
     for (const auto& s : shapes) {
         size_t c = 1;
@@ -175,4 +179,15 @@ extern "C" int ppo_checkpoint_write_index(const char* prefix, int obs_dim, int a
     const size_t put = fwrite(image.data(), 1, image.size(), f);
     fclose(f);
     return put == image.size() ? 0 : -3;
+}
+
+}  // namespace ppo
+
+extern "C" int ppo_checkpoint_write_index(const char* prefix, int obs_dim, int act_dim, int hidden1, int hidden2, const float* data, size_t n_floats) {
+    return ppo::write_index(prefix, obs_dim, act_dim, hidden1, hidden2, false, data, n_floats);
+}
+extern "C" int ppo_checkpoint_write_index_ex(const char* prefix, int action_space, int obs_dim, int act_dim, int hidden1, int hidden2,
+                                             const float* data, size_t n_floats) {
+    if (action_space != 0 && action_space != 1) return -1;  // PPO_ERR_INVALID
+    return ppo::write_index(prefix, obs_dim, act_dim, hidden1, hidden2, action_space == 1, data, n_floats);
 }

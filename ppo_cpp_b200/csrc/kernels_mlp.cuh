@@ -229,7 +229,7 @@ __host__ __device__ inline size_t policy_smem_floats(const NetDims& d) {
     return (size_t)(d.O + d.H1 + d.H2 + d.A + 1) * TM + (size_t)d.A * (TM + 1);
 }
 
-template <int TM, int ACT>
+template <int TM, int ACT, int HEAD>
 __global__ void __launch_bounds__(NT) policy_tile_kernel(const PolicyArgs a) {
     extern __shared__ __align__(16) float smem[];
     const NetDims& d = a.d;
@@ -274,7 +274,19 @@ __global__ void __launch_bounds__(NT) policy_tile_kernel(const PolicyArgs a) {
                 if (a.value) a.value[row] = v;
                 if (a.val_store) a.val_store[row] = v;
             }
-            if (a.mode == 0) {
+            if (HEAD == HEAD_DISCRETE && a.mode != 1) {  // the index as fp32, one column; eps: [n][A] uniforms when given
+                const float* l = MU + m;
+                const int j = a.mode == 0 ? cat_sample(l, TM, d.A, a.eps ? a.eps + (size_t)row * d.A : nullptr, a.seed,
+                                                       a.env_id0 + (uint32_t)row, a.eps ? 0u : *a.step_ctr)
+                                          : cat_argmax(l, TM, d.A);
+                if (a.action) a.action[row] = (float)j;
+                if (a.act_store) a.act_store[row] = (float)j;
+                if (a.mode == 0) {
+                    const float nl = cat_neglogp(l, TM, d.A, j);
+                    if (a.neglogp) a.neglogp[row] = nl;
+                    if (a.nlp_store) a.nlp_store[row] = nl;
+                }
+            } else if (a.mode == 0) {
                 const float* logstd = p + d.off[T_LOGSTD];
                 const uint32_t step = a.eps ? 0u : *a.step_ctr;
                 float ss = 0.f, sl = 0.f;
@@ -307,7 +319,7 @@ __global__ void __launch_bounds__(NT) policy_tile_kernel(const PolicyArgs a) {
             if (a.dones_store) a.dones_store[row] = a.dones_in[row];
         }
         __syncthreads();
-        if (a.mode != 1) {
+        if (HEAD == HEAD_BOX && a.mode != 1) {  // a categorical head stored its index above
             for (int e = tid; e < nv * d.A; e += NT) {
                 const int m = e / d.A, j = e - m * d.A;
                 const float act = Ac[j * (TM + 1) + m];
@@ -342,7 +354,7 @@ __host__ __device__ inline size_t train_smem_floats(const NetDims& d) {
     return (size_t)(d.O + 2 * d.A + 2 * d.H1 + 2 * d.H2) * TM + 5 * (size_t)TM + 64;
 }
 
-template <int TM, int ACT>
+template <int TM, int ACT, int HEAD>
 __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
     extern __shared__ __align__(16) float smem[];
     const NetDims& d = a.d;
@@ -366,7 +378,7 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
     const int ntiles = (a.count + TM - 1) / TM;
     const float cr = a.sc->cliprange, vr = vf_clip_range(a.vf_mode, cr, a.sc->cliprange_vf);
     const float lo = 1.f - cr, hi = 1.f + cr;
-    float l_pg = 0.f, l_vf = 0.f, l_kl = 0.f, l_cf = 0.f;
+    float l_pg = 0.f, l_vf = 0.f, l_kl = 0.f, l_cf = 0.f, l_ent = 0.f;
     bool acc = false;
 
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
@@ -391,7 +403,7 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
         }
         __syncthreads();
         tile_load_rows<TM>(a.obs, d.O, s_row, nv, Xs);
-        tile_load_rows<TM>(a.act, d.A, s_row, nv, Ac);
+        tile_load_rows<TM>(a.act, HEAD == HEAD_DISCRETE ? 1 : d.A, s_row, nv, Ac);
         __syncthreads();
 
         // ---------------- pi tower ----------------
@@ -401,7 +413,30 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
         __syncthreads();
         tile_fwd<TM, ACT_NONE>(H2s, d.H2, p + d.off[T_PI_W], p + d.off[T_PI_B], d.A, MU);
         __syncthreads();
-        if (tid < TM) {
+        if (HEAD == HEAD_DISCRETE && tid < TM) {  // a thread per sample over the A logits; MU becomes dL/dlogits
+            const int m = tid;
+            float* l = MU + m;
+            if (m < nv) {
+                const int ai = (int)Ac[m];
+                float mx;
+                const float z = cat_partition(l, TM, d.A, mx);
+                const float nlp = logf(z) - (l[ai * TM] - mx);
+                const float H = cat_entropy(l, TM, d.A, mx, z);
+                const float adv = s_adv[m], oldn = s_oldn[m];
+                const float ratio = expf(oldn - nlp);
+                const float pg1 = -adv * ratio;
+                const float pg2 = -adv * fmaxf(fminf(ratio, hi), lo);
+                const bool take1 = pg1 >= pg2;
+                l_pg += take1 ? pg1 : pg2;
+                const float dn = nlp - oldn;
+                l_kl += dn * dn;
+                l_cf += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
+                l_ent += H * (a.invB * a.sc->world);
+                cat_dlogits(l, TM, d.A, ai, mx, z, H, take1 ? (adv * ratio) * a.invB : 0.f, a.ent_coef * a.invB);
+            } else {
+                for (int j = 0; j < d.A; ++j) l[j * TM] = 0.f;
+            }
+        } else if (tid < TM) {
             const int m = tid;
             const float* logstd = p + d.off[T_LOGSTD];
             float g_nlp = 0.f;
@@ -435,7 +470,7 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
         __syncthreads();
         tile_dw<TM>(H2s, d.H2, MU, d.A, my + d.off[T_PI_W], acc);
         tile_rowsum<TM>(MU, d.A, my + d.off[T_PI_B], acc);
-        tile_rowsum<TM>(Ac, d.A, my + d.off[T_LOGSTD], acc);
+        if (HEAD == HEAD_BOX) tile_rowsum<TM>(Ac, d.A, my + d.off[T_LOGSTD], acc);
         tile_bwd_dx<TM, ACT>(MU, d.A, p + d.off[T_PI_W], d.H2, H2s, D2);
         __syncthreads();
         tile_dw<TM>(H1s, d.H1, D2, d.H2, my + d.off[T_PI_FC1_W], acc);
@@ -477,23 +512,29 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
     }
 
     // loss sums of this CTA -> columns P.. of its slab (threads >= TM hold zeros)
-    float v4[4] = {l_pg, l_vf, l_kl, l_cf};
+    constexpr int NL = HEAD == HEAD_DISCRETE ? 5 : 4;
+    float v4[NL];
+    v4[0] = l_pg; v4[1] = l_vf; v4[2] = l_kl; v4[3] = l_cf;
+    if (HEAD == HEAD_DISCRETE) v4[NL - 1] = l_ent;
 #pragma unroll
-    for (int q = 0; q < 4; ++q) v4[q] = warp_sum(v4[q]);
+    for (int q = 0; q < NL; ++q) v4[q] = warp_sum(v4[q]);
     if ((tid & 31) == 0) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q) s_red[(tid >> 5) * 4 + q] = v4[q];
+        for (int q = 0; q < NL; ++q) s_red[(tid >> 5) * NL + q] = v4[q];
     }
     __syncthreads();
     if (tid == 0) {
-        float t[4] = {0.f, 0.f, 0.f, 0.f};
+        float t[NL];
+        for (int q = 0; q < NL; ++q) t[q] = 0.f;
         for (int w = 0; w < NT / 32; ++w)
-            for (int q = 0; q < 4; ++q) t[q] += s_red[w * 4 + q];
+            for (int q = 0; q < NL; ++q) t[q] += s_red[w * NL + q];
         float* L = my + d.P;
         L[L_PG] = t[0]; L[L_VF] = t[1]; L[L_KL] = t[2]; L[L_CLIP] = t[3];
-        // entropy = sum_j(logstd_j + 0.5*log(2*pi*e)) with the pre-update weights (GRAPH:10021-10180)
         float ent = 0.f;
-        if (blockIdx.x == 0) {
+        if (HEAD == HEAD_DISCRETE) {
+            ent = t[NL - 1];  // sum of H / B (x world, see UpdateScalars) over this CTA's samples
+        } else if (blockIdx.x == 0) {
+            // entropy = sum_j(logstd_j + 0.5*log(2*pi*e)) with the pre-update weights (GRAPH:10021-10180)
             const float* logstd = p + d.off[T_LOGSTD];
             for (int j = 0; j < d.A; ++j) ent += __ldg(logstd + j) + PPO_HALF_LOG_2PIE;
         }
@@ -502,7 +543,7 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
     }
     // loss = pg_loss - entropy*ent_coef + vf_loss*vf_coef: d(-ent_coef*entropy)/dlogstd_j = -ent_coef, added once
     // (a.ent_coef is already divided by the number of ranks whose slabs get summed)
-    if (blockIdx.x == 0 && tid < d.A) my[d.off[T_LOGSTD] + tid] -= a.ent_coef;  // same thread wrote it in tile_rowsum
+    if (HEAD == HEAD_BOX && blockIdx.x == 0 && tid < d.A) my[d.off[T_LOGSTD] + tid] -= a.ent_coef;  // same thread wrote it in tile_rowsum
 }
 
 }  // namespace ppo

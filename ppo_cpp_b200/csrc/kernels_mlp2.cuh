@@ -232,7 +232,7 @@ __device__ __forceinline__ void stage_weights(float* sW, const float* __restrict
 }
 
 // ------------------------------------------------------------------------------------------------ train
-template <int TM, int NTH, int ACT>
+template <int TM, int NTH, int ACT, int HEAD>
 __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) {
     extern __shared__ __align__(16) float smem[];
     const NetDims& d = a.d;
@@ -273,7 +273,7 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
             smem[L.h2[t] + d.H2 * TM + m] = 1.f;
         }
     }
-    float l_pg = 0.f, l_vf = 0.f, l_kl = 0.f, l_cf = 0.f;
+    float l_pg = 0.f, l_vf = 0.f, l_kl = 0.f, l_cf = 0.f, l_ent = 0.f;
     bool acc = false;
     bool first = true;
 
@@ -302,16 +302,17 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
             const int m = e / d.O, k = e - m * d.O;
             Xs[k * TM + m] = (m < nv) ? __ldg(a.obs + (size_t)s_row[m] * d.O + k) : 0.f;
         }
-        for (int e = tid; e < TM * d.A; e += NTH) {
-            const int m = e / d.A, j = e - m * d.A;
-            Ac[j * TM + m] = (m < nv) ? __ldg(a.act + (size_t)s_row[m] * d.A + j) : 0.f;
+        const int AW = HEAD == HEAD_DISCRETE ? 1 : d.A;  // stored action width
+        for (int e = tid; e < TM * AW; e += NTH) {
+            const int m = e / AW, j = e - m * AW;
+            Ac[j * TM + m] = (m < nv) ? __ldg(a.act + (size_t)s_row[m] * AW + j) : 0.f;
         }
         if (first) {
             cp_async_wait_all();
             first = false;
         }
         __syncthreads();
-        if (tid < d.A && tile == (int)blockIdx.x) {
+        if (HEAD == HEAD_BOX && tid < d.A && tile == (int)blockIdx.x) {
             const float ls = sW[d.off[T_LOGSTD] + tid];
             s_sd[tid] = expf(ls);
             s_sd[d.A + tid] = ls;
@@ -329,6 +330,35 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
         // ---- loss stage.  Thread (m, jg) handles actions j = jg, jg + JG, ... of sample m.
         constexpr int JG = (NTH / TM) < 8 ? (NTH / TM) : 8;
         const int m = tid % TM, jg = tid / TM;
+        if (HEAD == HEAD_DISCRETE) {  // a thread per sample over the A logits; MU becomes dL/dlogits, Vs dL/dv
+            if (jg == 0) {
+                float* l = MU + m;
+                if (m < nv) {
+                    const int ai = (int)Ac[m];
+                    float mx;
+                    const float z = cat_partition(l, TM, d.A, mx);
+                    const float nlp = logf(z) - (l[ai * TM] - mx);
+                    const float H = cat_entropy(l, TM, d.A, mx, z);
+                    const float adv = s_adv[m], oldn = s_oldn[m];
+                    const float ratio = expf(oldn - nlp);
+                    const float pg1 = -adv * ratio;
+                    const float pg2 = -adv * fmaxf(fminf(ratio, hi), lo);
+                    const bool take1 = pg1 >= pg2;
+                    l_pg += take1 ? pg1 : pg2;
+                    const float dn = nlp - oldn;
+                    l_kl += dn * dn;
+                    l_cf += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
+                    l_ent += H * (a.invB * a.sc->world);
+                    cat_dlogits(l, TM, d.A, ai, mx, z, H, take1 ? (adv * ratio) * a.invB : 0.f, a.ent_coef * a.invB);
+                    float dv;
+                    l_vf += value_loss_term(a.vf_mode, vr, Vs[m], s_oldv[m], s_ret[m], a.vf_coef, a.invB, dv);
+                    Vs[m] = dv;
+                } else {
+                    for (int j = 0; j < d.A; ++j) l[j * TM] = 0.f;
+                    Vs[m] = 0.f;
+                }
+            }
+        } else {
         if (jg < JG) {
             float ss = 0.f;
             for (int j = jg; j < d.A; j += JG) {
@@ -370,6 +400,7 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
                 MU[j * TM + m] = g_nlp * (-z / sd);      // dL/dmu
             }
         }
+        }
         __syncthreads();
 
         // ---- backward: heads
@@ -380,7 +411,7 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
             f_bwd_dx<TM, ACT>(Vs, 1, sW + d.off[T_VF_W], d.H2, H2, D2, half);
             f_dw<TM>(H2, d.H2, Vs, 1, my + d.off[T_VF_W], my + d.off[T_VF_B], acc, half);
             // logstd gradient = row sums of Ac: ones-row trick with K = 0 (As = the ones row of Xs)
-            f_dw<TM>(Xs + d.O * TM, 0, Ac, d.A, my + d.off[T_LOGSTD], my + d.off[T_LOGSTD], acc, half);
+            if (HEAD == HEAD_BOX) f_dw<TM>(Xs + d.O * TM, 0, Ac, d.A, my + d.off[T_LOGSTD], my + d.off[T_LOGSTD], acc, half);
         }
         __syncthreads();
         // ---- backward: hidden layer 1
@@ -394,33 +425,38 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
     }
     if (first) cp_async_wait_all();
 
-    float v4[4] = {l_pg, l_vf, l_kl, l_cf};
+    constexpr int NL = HEAD == HEAD_DISCRETE ? 5 : 4;
+    float v4[NL];
+    v4[0] = l_pg; v4[1] = l_vf; v4[2] = l_kl; v4[3] = l_cf;
+    if (HEAD == HEAD_DISCRETE) v4[NL - 1] = l_ent;
 #pragma unroll
-    for (int q = 0; q < 4; ++q) v4[q] = warp_sum(v4[q]);
+    for (int q = 0; q < NL; ++q) v4[q] = warp_sum(v4[q]);
     if ((tid & 31) == 0) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q) s_red[(tid >> 5) * 4 + q] = v4[q];
+        for (int q = 0; q < NL; ++q) s_red[(tid >> 5) * NL + q] = v4[q];
     }
     __syncthreads();
     if (tid == 0) {
-        float t[4] = {0.f, 0.f, 0.f, 0.f};
+        float t[NL];
+        for (int q = 0; q < NL; ++q) t[q] = 0.f;
         for (int w = 0; w < NTH / 32; ++w)
-            for (int q = 0; q < 4; ++q) t[q] += s_red[w * 4 + q];
+            for (int q = 0; q < NL; ++q) t[q] += s_red[w * NL + q];
         float* Lp = my + d.P;
         Lp[L_PG] = t[0]; Lp[L_VF] = t[1]; Lp[L_KL] = t[2]; Lp[L_CLIP] = t[3];
         float ent = 0.f;
-        if (blockIdx.x == 0)
+        if (HEAD == HEAD_DISCRETE) ent = t[NL - 1];  // sum of H / B (x world, see UpdateScalars) over this CTA's samples
+        else if (blockIdx.x == 0)
             for (int j = 0; j < d.A; ++j) ent += sW[d.off[T_LOGSTD] + j] + PPO_HALF_LOG_2PIE;  // GRAPH:10021-10180
         Lp[L_ENT] = ent;
         Lp[5] = 0.f; Lp[6] = 0.f; Lp[7] = 0.f;
     }
     __syncthreads();
     // d(-ent_coef*entropy)/dlogstd_j = -ent_coef, once (a.ent_coef is pre-divided by the number of ranks)
-    if (blockIdx.x == 0 && tid < d.A) my[d.off[T_LOGSTD] + tid] -= a.ent_coef;
+    if (HEAD == HEAD_BOX && blockIdx.x == 0 && tid < d.A) my[d.off[T_LOGSTD] + tid] -= a.ent_coef;
 }
 
 // ------------------------------------------------------------------------------------------------ policy
-template <int TM, int NTH, int ACT>
+template <int TM, int NTH, int ACT, int HEAD>
 __global__ void __launch_bounds__(NTH) policy_fused_kernel(const PolicyArgs a) {
     extern __shared__ __align__(16) float smem[];
     const NetDims& d = a.d;
@@ -470,7 +506,19 @@ __global__ void __launch_bounds__(NTH) policy_fused_kernel(const PolicyArgs a) {
                 if (a.value) a.value[row] = v;
                 if (a.val_store) a.val_store[row] = v;
             }
-            if (a.mode == 0) {
+            if (HEAD == HEAD_DISCRETE && a.mode != 1) {  // the index as fp32, one column; eps: [n][A] uniforms when given
+                const float* l = MU + m;
+                const int j = a.mode == 0 ? cat_sample(l, TM, d.A, a.eps ? a.eps + (size_t)row * d.A : nullptr, a.seed,
+                                                       a.env_id0 + (uint32_t)row, a.eps ? 0u : *a.step_ctr)
+                                          : cat_argmax(l, TM, d.A);
+                if (a.action) a.action[row] = (float)j;
+                if (a.act_store) a.act_store[row] = (float)j;
+                if (a.mode == 0) {
+                    const float nl = cat_neglogp(l, TM, d.A, j);
+                    if (a.neglogp) a.neglogp[row] = nl;
+                    if (a.nlp_store) a.nlp_store[row] = nl;
+                }
+            } else if (a.mode == 0) {
                 const float* logstd = sW + d.off[T_LOGSTD];
                 const uint32_t step = a.eps ? 0u : *a.step_ctr;
                 float ss = 0.f, sl = 0.f;
@@ -502,7 +550,7 @@ __global__ void __launch_bounds__(NTH) policy_fused_kernel(const PolicyArgs a) {
             if (a.dones_store) a.dones_store[row] = a.dones_in[row];
         }
         __syncthreads();
-        if (do_pi) {
+        if (HEAD == HEAD_BOX && do_pi) {  // a categorical head stored its index above
             for (int e = tid; e < nv * d.A; e += NTH) {
                 const int m = e / d.A, j = e - m * d.A;
                 const float act = Ac[j * (TM + 1) + m];

@@ -334,6 +334,27 @@ int classify_activation(const NodeMap& nodes, std::string& err) {
     return first_op == "Relu" ? 1 : 0;
 }
 
+// Stable-Baselines' policy head follows the action space: a Box gets DiagGaussianProbabilityDistribution (model/pi/w, model/pi/b
+// and model/pi/logstd), a Discrete(n) gets CategoricalProbabilityDistribution (n logits from model/pi/w, model/pi/b, no logstd).
+// PPO2's action placeholder loss/action_ph (pdtype.sample_placeholder([None])), when the file has it, must agree: float [?, n]
+// for Box, int32 / int64 [?] for Discrete.  Returns 0 (Box) or 1 (Discrete); -1 with err naming the node otherwise.
+int classify_action_space(const NodeMap& nodes, int n, std::string& err) {
+    const bool box = nodes.count("model/pi/logstd") != 0;
+    auto it = nodes.find("loss/action_ph");
+    if (it == nodes.end()) return box ? 0 : 1;
+    const Msg* dt = attr_value(*it->second, "dtype");
+    const std::string dtype = dt ? dt->str("type") : std::string();
+    const Msg* shp = attr_value(*it->second, "shape");
+    const std::vector<int> dims = shape_dims(shp ? shp->sub("shape") : nullptr);
+    const bool ok = box ? (dtype == "DT_FLOAT" && dims.size() == 2 && dims[1] == n)
+                        : ((dtype == "DT_INT32" || dtype == "DT_INT64") && dims.size() == 1);
+    if (ok) return box ? 0 : 1;
+    err = "node loss/action_ph (" + (dtype.empty() ? std::string("no dtype") : dtype) + ", rank " + std::to_string(dims.size()) + ") contradicts the " +
+          (box ? "Gaussian head (model/pi/logstd present): a Box space needs a float [?, " + std::to_string(n) + "] placeholder"
+               : "categorical head (no model/pi/logstd): a Discrete space needs an int32 / int64 [?] placeholder");
+    return -1;
+}
+
 }  // namespace
 
 std::string parse_meta_txt(const std::string& path, MetaGraph& out) {
@@ -356,6 +377,7 @@ std::string parse_meta_txt(const std::string& path, MetaGraph& out) {
     for (int i = 0; i < kNumTensors; ++i) {
         const std::string name = kTensorNames[i];
         auto it = nodes.find(name);
+        if (i == kLogstdTensor && it == nodes.end()) continue;  // categorical head
         if (it == nodes.end() || it->second->str("op") != "VariableV2") return "graph has no variable " + name;
         const Msg* shp = attr_value(*it->second, "shape");
         MetaTensor t;
@@ -398,6 +420,7 @@ std::string parse_meta_txt(const std::string& path, MetaGraph& out) {
     out.hidden1 = w0[1];
     out.hidden2 = w1[1];
     out.act_dim = wp[1];
+    out.action_space = classify_action_space(nodes, out.act_dim, out.action_space_error);
     return std::string();
 }
 

@@ -25,7 +25,11 @@ struct MetaGraph {
     // hidden layers per tower (activation_error says why)
     int activation = 0;
     std::string activation_error;
-    std::map<std::string, MetaTensor> tensors;  // the 15 model/* variables with their initial values
+    // action space of the policy head (ppo_action_space: 0 Box, a Gaussian with model/pi/logstd; 1 Discrete, a categorical
+    // without it), or -1 when loss/action_ph contradicts the head (action_space_error says why)
+    int action_space = 0;
+    std::string action_space_error;
+    std::map<std::string, MetaTensor> tensors;  // the model/* variables with their initial values (14 without logstd)
 };
 
 // Returns empty string on success, otherwise the error message.
@@ -36,5 +40,6 @@ std::string parse_meta_txt(const std::string& path, MetaGraph& out);
 extern const char* const kTensorNames[15];
 constexpr int kNumTrainableTensors = 13;
 constexpr int kNumTensors = 15;
+constexpr int kLogstdTensor = 12;  // "model/pi/logstd": absent in a graph with a categorical head
 
 }  // namespace ppo

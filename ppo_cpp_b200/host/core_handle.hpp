@@ -26,9 +26,9 @@ struct CoreDeleter {
 };
 using CorePtr = std::shared_ptr<ppo_core>;
 
-inline CorePtr make_core(const ppo_core_desc& desc) {
+inline CorePtr make_core(const ppo_core_desc& desc, int action_space = PPO_ACTION_BOX) {
     ppo_core* raw = nullptr;
-    ppo_check(ppo_core_create(&desc, &raw), "ppo_core_create");
+    ppo_check(ppo_core_create_ex(&desc, action_space, &raw), "ppo_core_create");
     return CorePtr(raw, CoreDeleter());
 }
 

@@ -43,4 +43,8 @@ public:
     }
 };
 
+// columns of an action matrix: get_action_space_size() for a continuous env; one (the index, as a float) for a discrete env,
+// whose get_action_space_size() is the number of choices (Stable-Baselines' Discrete(n))
+inline int action_width(Env& env) { return env.get_action_space() == Env::SPACE_DISCRETE() ? 1 : env.get_action_space_size(); }
+
 #endif

@@ -1,6 +1,6 @@
 // CLI with the reference's flags (ppo2.cpp:93-128) driving the B200 core.  Envs: the DART hexapod cannot be
 // built here (SURVEY §2 row 12); `--env synthetic` (default) is the host-side stand-in with the same shapes,
-// `--env mock` is the reference's EnvMock.  New flags: --env, --seed (commented out in the reference,
+// `--env mock` is the reference's EnvMock, `--env bandit` a Discrete(4) contextual bandit for the categorical head.  New flags: --env, --seed (commented out in the reference,
 // ppo2.cpp:130-131), --hidden H1,H2 (graph-less orthogonal init when no --graph is given).
 #include <chrono>
 #include <cstdlib>
@@ -12,6 +12,7 @@
 #include <string>
 #include <vector>
 
+#include "env_bandit.hpp"
 #include "env_mock.hpp"
 #include "env_normalize.hpp"
 #include "env_synthetic.hpp"
@@ -85,7 +86,7 @@ int main(int argc, char** argv) {
                      "  -d --dir, -g --graph --graph_path, -p --path, --id, -s --steps, -l --lr, -e --ent, -c --cr,\n"
                      "  --saves, --epochs --num_epochs, --batch_steps --n_steps, --rns, --cl, -v, -r --resume, --bullet,\n"
                      "  --duration, -j --threads, -f --fps   (as in the reference's ppo2.cpp:93-128)\n"
-                     "  --env synthetic|mock, --seed N, --hidden H1,H2,\n"
+                     "  --env synthetic|mock|bandit (bandit: a Discrete(4) contextual bandit), --seed N, --hidden H1,H2,\n"
                      "  --cliprange_vf (-1: the graph's value loss decides; >= 0 for a graph with loss/clip_range_vf_ph),\n"
                      "  --activation tanh|relu (graph-less runs; with a graph it must name the graph's own activation)\n";
         return 0;
@@ -129,6 +130,7 @@ int main(int argc, char** argv) {
     std::vector<std::shared_ptr<Env>> envs;
     auto make_env = [&](int i) -> std::shared_ptr<Env> {
         if (env_kind == "mock") return std::make_shared<EnvMock>(1.0);
+        if (env_kind == "bandit") return std::make_shared<BanditEnv>(static_cast<uint64_t>(seed_val) ^ 0x1234ull, static_cast<uint32_t>(i));
         return std::make_shared<SyntheticEnv>(static_cast<uint64_t>(seed_val) ^ 0x1234ull, static_cast<uint32_t>(i));
     };
     if (threads > 1) {
@@ -136,6 +138,8 @@ int main(int argc, char** argv) {
         wrapped_env = std::make_unique<VecEnv>(envs);
     } else if (env_kind == "mock") {
         wrapped_env = std::make_unique<EnvMock>(1.0);
+    } else if (env_kind == "bandit") {
+        wrapped_env = std::make_unique<BanditEnv>(static_cast<uint64_t>(seed_val) ^ 0x1234ull, 0);
     } else {
         wrapped_env = std::make_unique<SyntheticEnv>(static_cast<uint64_t>(seed_val) ^ 0x1234ull, 0);
     }

@@ -101,10 +101,24 @@ public:
         } else {
             d.norm_obs = 0; d.norm_reward = 0; d.training = 0;
         }
+        // a Discrete env gets a categorical head over its get_action_space_size() choices; action_space is the env's, or the
+        // sidecar's after load()
+        if (action_space != Env::SPACE_CONTINOUS() && action_space != Env::SPACE_DISCRETE())
+            throw std::runtime_error("PPO2: unsupported action space " + action_space);
+        if (action_space != env.get_action_space())
+            throw std::runtime_error("PPO2: the model's action space " + action_space + " is not the env's " + env.get_action_space());
+        const int space = action_space == Env::SPACE_DISCRETE() ? PPO_ACTION_DISCRETE : PPO_ACTION_BOX;
         const bool from_graph = hidden_override_[0] == 0;
         if (from_graph) {
             ppo_meta_info info;
             ppo_check(ppo_meta_parse(model_filename.c_str(), &info, nullptr, 0), "graph load");
+            const int graph_space = ppo_meta_action_space(model_filename.c_str());
+            ppo_check(graph_space < 0 ? graph_space : PPO_OK, "graph load");
+            if (graph_space != space) {
+                std::cout << "the graph's policy head does not match the env's " << action_space << " action space" << std::endl;
+                throw std::runtime_error("PPO2: graph " + model_filename + " has a " + (graph_space == PPO_ACTION_DISCRETE ? "discrete" : "continuous") +
+                                         " policy head, the env a " + action_space + " action space");
+            }
             if (info.obs_dim != d.obs_dim || info.act_dim != d.act_dim) {
                 std::cout << "graph input/output widths do not match the environment" << std::endl;
                 assert(false);
@@ -113,7 +127,7 @@ public:
         } else {
             d.hidden1 = hidden_override_[0]; d.hidden2 = hidden_override_[1];
         }
-        core_ = make_core(d);
+        core_ = make_core(d, space);
         if (from_graph) {
             // the graph's baked ent_coef / vf_coef / clip norm / Adam constants win over the constructor's (SURVEY §3.5)
             ppo_check(ppo_core_load_meta_txt(core_.get(), model_filename.c_str()), "graph load");
@@ -124,7 +138,7 @@ public:
         }
         ppo_check(ppo_shuffle_seed(core_.get(), shuffle_seed_), "shuffle seed");
         if (normalize) normalize->attach_core(core_);
-        act_model = std::make_unique<MlpPolicy>(core_, d.act_dim);
+        act_model = std::make_unique<MlpPolicy>(core_, action_width(env));
     }
 
     void save(std::string save_path, int save_id = -1) {
@@ -200,7 +214,7 @@ public:
 
     Mat eval(const Mat& obs) const {
         Mat actions = act_model->get_deterministic_action(obs);
-        assert(actions.rows() == obs.rows() && actions.cols() == env.get_action_space_size());
+        assert(actions.rows() == obs.rows() && actions.cols() == action_width(env));
         return actions;
     }
 

@@ -34,7 +34,7 @@ public:
     MiniBatch run(bool fetch_all = true) {
         ppo_core* core = model.core().get();
         Env& stepper = normalize ? normalize->inner() : env;
-        Mat actions(num_envs, env.get_action_space_size());
+        Mat actions(num_envs, action_width(env));
         for (int step = 0; step < n_steps; ++step) {
             ppo_check(ppo_runner_act(core, step, actions.data(), PPO_HOST), "Runner::run act");
             const std::vector<Mat>& r = stepper.step(actions);  // env handles action clipping (runner.hpp:112)
@@ -46,7 +46,7 @@ public:
         MiniBatch mb{};
         if (fetch_all) {
             mb.obs = fetch("obs", env.get_observation_space_size());
-            mb.actions = fetch("actions", env.get_action_space_size());
+            mb.actions = fetch("actions", action_width(env));
             mb.returns = fetch("returns", 1);
             mb.dones = fetch("dones", 1);
             mb.values = fetch("values", 1);

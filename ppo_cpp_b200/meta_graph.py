@@ -29,6 +29,7 @@ TENSOR_ORDER = [
     "model/q/w", "model/q/b",
 ]
 N_TRAINABLE_TENSORS = 13
+LOGSTD = "model/pi/logstd"  # absent with a categorical head (Discrete action space): 14 tensors, 12 trainable
 
 _TOKEN = re.compile(r'\s*(?:([A-Za-z_][A-Za-z0-9_]*)|([{}:])|("(?:[^"\\]|\\.)*")|([-+0-9.eE]+[A-Za-z]*|-?inf|nan))')
 
@@ -108,11 +109,12 @@ class MetaInfo:
     tf_version: str = ""
     vf_clip: str = "shared"
     activation: str = "tanh"
+    action_space: str = "box"
     shapes: Dict[str, Tuple[int, ...]] = field(default_factory=dict)
 
     def flat_params(self, include_q: bool = True) -> np.ndarray:
         names = TENSOR_ORDER if include_q else TENSOR_ORDER[:N_TRAINABLE_TENSORS]
-        return np.concatenate([self.tensors[n].ravel() for n in names]).astype(np.float32)
+        return np.concatenate([self.tensors[n].ravel() for n in names if n in self.tensors]).astype(np.float32)
 
 
 def _attr(node: dict, key: str) -> dict | None:
@@ -260,6 +262,33 @@ def classify_activation(nodes: Dict[str, dict]) -> str:
     return "relu" if first[0] == "Relu" else "tanh"
 
 
+def classify_action_space(nodes: Dict[str, dict], n: int) -> str:
+    """The action space of Stable-Baselines' policy head: "box" (DiagGaussianProbabilityDistribution, with model/pi/logstd) or
+    "discrete" (CategoricalProbabilityDistribution over the n logits of model/pi, no logstd).  PPO2's action placeholder
+    loss/action_ph, when the graph has it, must agree: float [?, n] for "box", int32 / int64 [?] for "discrete"; otherwise
+    ValueError naming the node.  Twin of classify_action_space in csrc/meta_parser.cpp."""
+    box = LOGSTD in nodes
+    ph = nodes.get("loss/action_ph")
+    if ph is None:
+        return "box" if box else "discrete"
+    dt = _attr(ph, "dtype")
+    dtype = dt["type"][0] if dt is not None and "type" in dt else ""
+    shp = _attr(ph, "shape")
+    dims = [int(d["size"][0]) for d in shp["shape"][0].get("dim", [])] if shp is not None and "shape" in shp else []
+    if box and dtype == "DT_FLOAT" and len(dims) == 2 and dims[1] == n:
+        return "box"
+    if not box and dtype in ("DT_INT32", "DT_INT64") and len(dims) == 1:
+        return "discrete"
+    head = (f"Gaussian head (model/pi/logstd present): a Box space needs a float [?, {n}] placeholder" if box else
+            "categorical head (no model/pi/logstd): a Discrete space needs an int32 / int64 [?] placeholder")
+    raise ValueError(f"node loss/action_ph ({dtype or 'no dtype'}, rank {len(dims)}) contradicts the {head}")
+
+
+def meta_action_space(path: str) -> str:
+    """The action space of a graph file's policy head ("box" / "discrete"), read by this module's parser."""
+    return parse_meta_txt(path).action_space
+
+
 def meta_activation(path: str) -> str:
     """The hidden-layer activation of a graph file ("tanh" / "relu"), read by this module's parser."""
     return parse_meta_txt(path).activation
@@ -275,6 +304,8 @@ def parse_meta_txt(path: str) -> MetaInfo:
     shapes: Dict[str, Tuple[int, ...]] = {}
     tensors: Dict[str, np.ndarray] = {}
     for name in TENSOR_ORDER:
+        if name == LOGSTD and name not in nodes:  # categorical head
+            continue
         var = nodes[name]
         assert var["op"][0] == b"VariableV2", name
         shp = _attr(var, "shape")["shape"][0]
@@ -312,6 +343,7 @@ def parse_meta_txt(path: str) -> MetaInfo:
         tf_version=ver,
         vf_clip=classify_vf_clip(nodes),
         activation=classify_activation(nodes),
+        action_space=classify_action_space(nodes, shapes["model/pi/w"][1]),
         shapes=shapes,
     )
 
@@ -322,9 +354,12 @@ CKPT_ORDER = sorted(TENSOR_ORDER)
 
 
 def read_checkpoint_data(data_path: str, shapes: Dict[str, Tuple[int, ...]]) -> Dict[str, np.ndarray]:
+    """The tensors of `shapes` (15, or 14 without logstd for a categorical head) from a Saver V2 .data file."""
     raw = np.fromfile(data_path, dtype="<f4")
     out, off = {}, 0
     for name in CKPT_ORDER:
+        if name not in shapes:
+            continue
         n = int(np.prod(shapes[name]))
         out[name] = raw[off:off + n].reshape(shapes[name]).copy()
         off += n
@@ -333,8 +368,11 @@ def read_checkpoint_data(data_path: str, shapes: Dict[str, Tuple[int, ...]]) -> 
     return out
 
 
-def param_layout(obs_dim: int, act_dim: int, h1: int, h2: int) -> Dict[str, Tuple[int, Tuple[int, ...]]]:
-    """Offsets (in floats) of every tensor inside the flat parameter vector used by the core."""
+def param_layout(obs_dim: int, act_dim: int, h1: int, h2: int, action_space: str = "box") -> Dict[str, Tuple[int, Tuple[int, ...]]]:
+    """Offsets (in floats) of every tensor inside the flat parameter vector used by the core.  A categorical head
+    (action_space "discrete", act_dim logits) has no logstd; the other tensors keep their order."""
+    if action_space not in ("box", "discrete"):
+        raise ValueError(f"action_space must be 'box' or 'discrete', not {action_space!r}")
     shp = {
         "model/pi_fc0/w": (obs_dim, h1), "model/pi_fc0/b": (h1,),
         "model/vf_fc0/w": (obs_dim, h1), "model/vf_fc0/b": (h1,),
@@ -347,6 +385,8 @@ def param_layout(obs_dim: int, act_dim: int, h1: int, h2: int) -> Dict[str, Tupl
     }
     out, off = {}, 0
     for name in TENSOR_ORDER:
+        if name == LOGSTD and action_space == "discrete":
+            continue
         out[name] = (off, shp[name])
         off += int(np.prod(shp[name]))
     out["__total__"] = (off, ())
@@ -371,7 +411,7 @@ def _escape(b: bytes) -> str:
 
 def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 0.0, vf_coef: float = 0.5,
                    clip_norm: float = 0.5, beta1: float = 0.9, beta2: float = 0.999, adam_eps: float = 1e-5,
-                   vf_clip: str | None = None, activation: str | None = None) -> None:
+                   vf_clip: str | None = None, activation: str | None = None, action_space: str | None = None) -> None:
     """Write a minimal .meta.txt (variables + initialisers + baked constants) that both readers accept.
 
     The reference's graphs come from a Stable-Baselines/TensorFlow export script that is not part of the
@@ -380,11 +420,16 @@ def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 
     graph builds (Stable-Baselines' cliprange_vf None / < 0 / >= 0), named as Stable-Baselines names them;
     without it the file has no loss sub-graph and reads as "shared".
     activation = "tanh" | "relu" adds the forward nodes that tell the readers the hidden-layer activation (Stable-Baselines'
-    act_fun), under model/ and train_model/ as Stable-Baselines names them; without it the file has none and reads as "tanh"."""
+    act_fun), under model/ and train_model/ as Stable-Baselines names them; without it the file has none and reads as "tanh".
+    action_space = "box" | "discrete" adds PPO2's action placeholder loss/action_ph (float [?, n] / int64 [?]); "discrete" also
+    leaves model/pi/logstd out (a categorical head over the n columns of model/pi/w; `tensors` need not hold logstd).  Without it
+    the file has no placeholder and a logstd, and reads as "box"."""
     if vf_clip not in (None, "shared", "none", "separate"):
         raise ValueError(f"vf_clip must be None, 'shared', 'none' or 'separate', not {vf_clip!r}")
     if activation not in (None, "tanh", "relu"):
         raise ValueError(f"activation must be None, 'tanh' or 'relu', not {activation!r}")
+    if action_space not in (None, "box", "discrete"):
+        raise ValueError(f"action_space must be None, 'box' or 'discrete', not {action_space!r}")
     def dims(shape, ind):
         return "".join(f"{ind}dim {{\n{ind}  size: {d}\n{ind}}}\n" for d in shape)
 
@@ -406,9 +451,14 @@ def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 
 
     parts = ['meta_info_def {\n  tensorflow_version: "1.14.0"\n}\ngraph_def {\n']
     for name in TENSOR_ORDER:
+        if name == LOGSTD and action_space == "discrete":
+            continue
         arr = np.asarray(tensors[name], np.float32)
         parts.append(const_node(f"{name}/Initializer/initial_value", arr))
         parts.append(var_node(name, arr.shape))
+    if action_space is not None:
+        n = np.asarray(tensors["model/pi/w"]).shape[1]
+        parts.append(_action_placeholder("DT_INT64", (-1,)) if action_space == "discrete" else _action_placeholder("DT_FLOAT", (-1, n)))
     if activation is not None:
         parts.append(_forward_nodes(activation))
     if vf_clip is not None:
@@ -419,6 +469,13 @@ def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 
     parts.append("}\n")
     with open(path, "w", encoding="latin-1") as f:
         f.write("".join(parts))
+
+
+def _action_placeholder(dtype: str, shape) -> str:
+    """PPO2's loss/action_ph (train_model.pdtype.sample_placeholder([None])) with its dtype and shape attributes."""
+    dims = "".join(f"          dim {{\n            size: {d}\n          }}\n" for d in shape)
+    return (f'  node {{\n    name: "loss/action_ph"\n    op: "Placeholder"\n    attr {{\n      key: "dtype"\n      value {{\n        type: {dtype}\n      }}\n    }}\n'
+            f'    attr {{\n      key: "shape"\n      value {{\n        shape {{\n{dims}        }}\n      }}\n    }}\n  }}\n')
 
 
 def _op_node(name, kind, *inputs):
