@@ -66,6 +66,21 @@ __device__ __forceinline__ float value_loss_term(int mode, float range, float v,
     return tk ? l1 : l2;
 }
 
+// One sample's clipped surrogate (GRAPH:10423-10447, 12609-12776): pg = max(-adv r, -adv clip(r, 1 - cr, 1 + cr)) with
+// r = exp(oldneglogp - neglogp), its approxkl (dn^2) and clipfrac terms, and g_nlp = dL/dneglogp = adv r / B on the unclipped
+// branch, 0 on the clipped one.  clip_by_value = max(min(x, hi), lo); ties go to the unclipped branch.
+struct PgTerm {
+    float pg, kl, cf, g_nlp;
+};
+__device__ __forceinline__ PgTerm pg_term(float adv, float oldn, float nlp, float cr, float invB) {
+    const float ratio = expf(oldn - nlp);
+    const float pg1 = -adv * ratio;
+    const float pg2 = -adv * fmaxf(fminf(ratio, 1.f + cr), 1.f - cr);
+    const bool take1 = pg1 >= pg2;
+    const float dn = nlp - oldn;
+    return {take1 ? pg1 : pg2, dn * dn, (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f, take1 ? (adv * ratio) * invB : 0.f};
+}
+
 // Hidden-layer activation of the MLP (ppo_activation in ppo_core.h); uniform per core, a template parameter of every kernel
 // that evaluates it, so each activation compiles to its own code.  The derivative is taken from the OUTPUT h, as a factor:
 // TanhGrad (1 - h^2) and ReluGrad (h > 0: a unit whose pre-activation is exactly 0 gets no gradient, as TF's
@@ -87,6 +102,28 @@ __device__ __forceinline__ float act_dfac(float h) {
 // 0.5*log(2*pi), 0.5*log(2*pi*e) as the fp32 constants baked in the graph (GRAPH:6103-6672, 10021-10180)
 #define PPO_HALF_LOG_2PI 0.9189385175704956f
 #define PPO_HALF_LOG_2PIE 1.4189385175704956f
+
+// Diagonal Gaussian neglogp = 0.5*sum(z^2) + 0.5*log(2pi)*float(A) + sum(logstd) from the finished sums ss = sum(z^2),
+// sl = sum(logstd).  Two roundings: the train kernels' form may contract (GRAPH:9428-9997); the policy step's is
+// _rn throughout (GRAPH:6103-6672), as are its sample and z^2 (gauss_sample).
+__device__ __forceinline__ float gauss_neglogp(float ss, float sl, int A) { return (0.5f * ss + PPO_HALF_LOG_2PI * (float)A) + sl; }
+__device__ __forceinline__ float gauss_neglogp_rn(float ss, float sl, int A) {
+    return __fadd_rn(__fadd_rn(__fmul_rn(0.5f, ss), __fmul_rn(PPO_HALF_LOG_2PI, (float)A)), sl);
+}
+// act = mu + sd * e (GRAPH:5992-6019); z2 = ((act - mu) / sd)^2
+__device__ __forceinline__ float gauss_sample(float mu, float sd, float e, float& z2) {
+    const float act = __fadd_rn(mu, __fmul_rn(sd, e));
+    const float z = __fdiv_rn(__fsub_rn(act, mu), sd);
+    z2 = __fmul_rn(z, z);
+    return act;
+}
+// entropy = sum_j(logstd_j + 0.5*log(2*pi*e)) (GRAPH:10021-10180); logstd(j) loads logstd_j
+template <class LS>
+__device__ __forceinline__ float box_entropy(LS logstd, int A) {
+    float ent = 0.f;
+    for (int j = 0; j < A; ++j) ent += logstd(j) + PPO_HALF_LOG_2PIE;
+    return ent;
+}
 
 #define PPO_TAG_ACTION 0x50504F32u    // "PPO2": action noise stream
 #define PPO_TAG_CATEG 0x43415431u     // "CAT1": uniforms of the categorical head's Gumbel-max sample
@@ -198,6 +235,50 @@ __device__ __forceinline__ void cat_dlogits(float* l, int ld, int n, int a, floa
         const float p = expf(a0) / z;
         l[j * ld] = g_nlp * (p - (j == a ? 1.f : 0.f)) + ent_w * p * ((a0 - lz) + H);
     }
+}
+// one sample's categorical train terms: neglogp(a) and entropy H of the logits, the clipped surrogate of pg_term, and the
+// logits overwritten with dL/dl_j (cat_dlogits, ent_w = ent_coef / B)
+__device__ __forceinline__ PgTerm cat_train_term(float* l, int ld, int n, int a, float adv, float oldn, float cr, float invB, float ent_w,
+                                                 float& H) {
+    float mx;
+    const float z = cat_partition(l, ld, n, mx);
+    const float nlp = logf(z) - (l[a * ld] - mx);
+    H = cat_entropy(l, ld, n, mx, z);
+    const PgTerm t = pg_term(adv, oldn, nlp, cr, invB);
+    cat_dlogits(l, ld, n, a, mx, z, H, t.g_nlp, ent_w);
+    return t;
+}
+
+// ---- gradient step: clip_by_global_norm (GRAPH:24102-25392) and TF 1.14 ApplyAdam (GRAPH:25426-31383: epsilon outside the
+// sqrt, not bias-corrected), every operation rounded as written
+// scale = clip * min(1/||g||, 1/clip), NaN when ||g|| is not finite (GRAPH:24493-24543); ss: sum of squares, gnorm = ||g||
+__device__ __forceinline__ float clip_scale(double ss, float clip_norm, float& gnorm) {
+    gnorm = (float)sqrt(ss);
+    const float inv = __fdiv_rn(1.0f, gnorm), invc = __fdiv_rn(1.0f, clip_norm);
+    float scale = __fmul_rn(clip_norm, fminf(inv, invc));
+    if (!isfinite(gnorm)) scale = __int_as_float(0x7fc00000);
+    return scale;
+}
+// step size lr * sqrt(1 - beta2^t) / (1 - beta1^t) from the beta powers before this step
+__device__ __forceinline__ float adam_alpha(float lr, float b1p, float b2p) {
+    return __fdiv_rn(__fmul_rn(lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
+}
+// moments m, v of one parameter updated in place with its clipped gradient g
+__device__ __forceinline__ void adam_moments(float g, float& m, float& v, float beta1, float beta2) {
+    m = __fadd_rn(m, __fmul_rn(__fsub_rn(g, m), __fsub_rn(1.0f, beta1)));
+    v = __fadd_rn(v, __fmul_rn(__fsub_rn(__fmul_rn(g, g), v), __fsub_rn(1.0f, beta2)));
+}
+// the parameter p after the step, from its updated moments
+__device__ __forceinline__ float adam_param(float p, float m, float v, float alpha, float eps) {
+    return __fsub_rn(p, __fdiv_rn(__fmul_rn(m, alpha), __fadd_rn(__fsqrt_rn(v), eps)));
+}
+// the step's loss row [5]: pg, vf, entropy, approxkl, clipfrac from the summed loss columns L[L_PG .. L_CLIP]
+__device__ __forceinline__ void loss_row(float* row, const float* L, float invB, float inv_world) {
+    row[0] = L[L_PG] * invB;
+    row[1] = 0.5f * (L[L_VF] * invB);
+    row[2] = L[L_ENT] * inv_world;
+    row[3] = 0.5f * (L[L_KL] * invB);
+    row[4] = L[L_CLIP] * invB;
 }
 
 __device__ __forceinline__ float warp_sum(float v) {

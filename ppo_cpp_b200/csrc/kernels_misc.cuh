@@ -855,20 +855,11 @@ __global__ void adam_kernel(const AdamArgs a) {
         }
     }
     if (threadIdx.x == 0) {
-        const double ss = s_ss[0];
-        const float gnorm = (float)sqrt(ss);  // sqrt(2 * sum L2Loss(g_i))
-        const float inv = __fdiv_rn(1.0f, gnorm), invc = __fdiv_rn(1.0f, a.clip_norm);
-        float scale = __fmul_rn(a.clip_norm, fminf(inv, invc));
-        if (!isfinite(gnorm)) scale = __int_as_float(0x7fc00000);  // GRAPH:24493-24543
-        s_scale = scale;
+        float gnorm;  // sqrt(2 * sum L2Loss(g_i))
+        s_scale = clip_scale(s_ss[0], a.clip_norm, gnorm);
         if (blockIdx.x == 0) {
             *a.gnorm_out = gnorm;
-            const float* L = a.grad + a.P;
-            a.loss_row[0] = L[L_PG] * a.invB;
-            a.loss_row[1] = 0.5f * (L[L_VF] * a.invB);
-            a.loss_row[2] = L[L_ENT] * a.inv_world;
-            a.loss_row[3] = 0.5f * (L[L_KL] * a.invB);
-            a.loss_row[4] = L[L_CLIP] * a.invB;
+            loss_row(a.loss_row, a.grad + a.P, a.invB, a.inv_world);
             a.bpow_out[0] = __fmul_rn(a.bpow_in[0], a.beta1);
             a.bpow_out[1] = __fmul_rn(a.bpow_in[1], a.beta2);
         }
@@ -876,15 +867,13 @@ __global__ void adam_kernel(const AdamArgs a) {
     __syncthreads();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.P) return;
-    const float b1p = a.bpow_in[0], b2p = a.bpow_in[1];
-    const float alpha = __fdiv_rn(__fmul_rn(lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
+    const float alpha = adam_alpha(lr, a.bpow_in[0], a.bpow_in[1]);
     const float g = __fmul_rn(a.grad[i], s_scale);
     float m = a.m[i], v = a.v[i];
-    m = __fadd_rn(m, __fmul_rn(__fsub_rn(g, m), __fsub_rn(1.0f, a.beta1)));
-    v = __fadd_rn(v, __fmul_rn(__fsub_rn(__fmul_rn(g, g), v), __fsub_rn(1.0f, a.beta2)));
+    adam_moments(g, m, v, a.beta1, a.beta2);
     a.m[i] = m;
     a.v[i] = v;
-    a.params[i] = __fsub_rn(a.params[i], __fdiv_rn(__fmul_rn(m, alpha), __fadd_rn(__fsqrt_rn(v), a.eps)));
+    a.params[i] = adam_param(a.params[i], m, v, alpha, a.eps);
 }
 
 // Fused gradient step: column-reduce the CTA slabs -> (multi-GPU: allreduce through the peer mailboxes) -> global norm
@@ -920,7 +909,7 @@ struct ReduceAdamArgs {
 // persistent epoch kernel lends an operand block that is idle during the gradient step.
 template <bool EXT = false>
 __device__ __forceinline__ void reduce_adam_device(const ReduceAdamArgs& r, int blk, int nblk, GridBarrier& bar, unsigned seq,
-                                                   float b1p, float b2p, float* loss_row, long long* prof = nullptr, unsigned sqseq = 0u,
+                                                   float b1p, float b2p, float* loss_out, long long* prof = nullptr, unsigned sqseq = 0u,
                                                    float* ext_part = nullptr) {
     __shared__ __align__(16) float part_static[EXT ? 1 : RA_MAXJ][8][64];
     float (*part)[8][64] = EXT ? reinterpret_cast<float (*)[8][64]>(ext_part) : part_static;
@@ -1061,11 +1050,8 @@ __device__ __forceinline__ void reduce_adam_device(const ReduceAdamArgs& r, int 
         // fixed-order combine: lane partials summed by a butterfly (same order in every block and on every rank)
         ss = warp_sum(ss);
         if (threadIdx.x == 0) {
-            const float gnorm = (float)sqrt(ss);
-            const float inv = __fdiv_rn(1.0f, gnorm), invc = __fdiv_rn(1.0f, a.clip_norm);
-            float scale = __fmul_rn(a.clip_norm, fminf(inv, invc));
-            if (!isfinite(gnorm)) scale = __int_as_float(0x7fc00000);
-            s_scale = scale;
+            float gnorm;
+            s_scale = clip_scale(ss, a.clip_norm, gnorm);
             if (blk == 0) *a.gnorm_out = gnorm;
         }
     }
@@ -1078,20 +1064,15 @@ __device__ __forceinline__ void reduce_adam_device(const ReduceAdamArgs& r, int 
         const float* Ls = r.grad + a.P;
         float L[5];
         for (int k = 0; k < 5; ++k) L[k] = __ldcg(Ls + k);
-        loss_row[0] = L[L_PG] * a.invB;
-        loss_row[1] = 0.5f * (L[L_VF] * a.invB);
-        loss_row[2] = L[L_ENT] * a.inv_world;
-        loss_row[3] = 0.5f * (L[L_KL] * a.invB);
-        loss_row[4] = L[L_CLIP] * a.invB;
+        loss_row(loss_out, L, a.invB, a.inv_world);
     }
     if (mine) {
-        const float alpha = __fdiv_rn(__fmul_rn(lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
+        const float alpha = adam_alpha(lr, b1p, b2p);
         const float g = __fmul_rn(gsum[0], s_scale);
-        am = __fadd_rn(am, __fmul_rn(__fsub_rn(g, am), __fsub_rn(1.0f, a.beta1)));
-        av = __fadd_rn(av, __fmul_rn(__fsub_rn(__fmul_rn(g, g), av), __fsub_rn(1.0f, a.beta2)));
+        adam_moments(g, am, av, a.beta1, a.beta2);
         a.m[c] = am;
         a.v[c] = av;
-        a.params[c] = __fsub_rn(ap, __fdiv_rn(__fmul_rn(am, alpha), __fadd_rn(__fsqrt_rn(av), a.eps)));
+        a.params[c] = adam_param(ap, am, av, alpha, a.eps);
     }
     RA_PROF();
 #undef RA_PROF
@@ -1198,11 +1179,8 @@ __global__ void __launch_bounds__(256) grad_reduce_adam_big_kernel(const ReduceA
         for (int b = threadIdx.x; b < nblk; b += 32) ss += __ldcg(r.sq_partial + b);
         ss = warp_sum(ss);
         if (threadIdx.x == 0) {
-            const float gnorm = (float)sqrt(ss);
-            const float inv = __fdiv_rn(1.0f, gnorm), invc = __fdiv_rn(1.0f, a.clip_norm);
-            float scale = __fmul_rn(a.clip_norm, fminf(inv, invc));
-            if (!isfinite(gnorm)) scale = __int_as_float(0x7fc00000);
-            s_scale = scale;
+            float gnorm;
+            s_scale = clip_scale(ss, a.clip_norm, gnorm);
             if (blk == 0) *a.gnorm_out = gnorm;
         }
     }
@@ -1211,14 +1189,10 @@ __global__ void __launch_bounds__(256) grad_reduce_adam_big_kernel(const ReduceA
         const float* Ls = r.grad + a.P;
         float L[5];
         for (int k = 0; k < 5; ++k) L[k] = __ldcg(Ls + k);
-        a.loss_row[0] = L[L_PG] * a.invB;
-        a.loss_row[1] = 0.5f * (L[L_VF] * a.invB);
-        a.loss_row[2] = L[L_ENT] * a.inv_world;
-        a.loss_row[3] = 0.5f * (L[L_KL] * a.invB);
-        a.loss_row[4] = L[L_CLIP] * a.invB;
+        loss_row(a.loss_row, L, a.invB, a.inv_world);
     }
     if (rg == 0) {  // pass C, four chunks per trip: the sixteen loads of a trip are in flight together
-        const float alpha = __fdiv_rn(__fmul_rn(lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
+        const float alpha = adam_alpha(lr, b1p, b2p);
         for (int chunk0 = blk; chunk0 < nchunks; chunk0 += 4 * nblk) {
             float gg[4], mm[4], vv[4], pp[4];
 #pragma unroll
@@ -1234,13 +1208,10 @@ __global__ void __launch_bounds__(256) grad_reduce_adam_big_kernel(const ReduceA
             for (int j = 0; j < 4; ++j) {
                 const int c = (chunk0 + j * nblk) * 64 + lane_c;
                 if (c < a.P) {
-                    const float g = __fmul_rn(gg[j], s_scale);
-                    float m = mm[j], v = vv[j];
-                    m = __fadd_rn(m, __fmul_rn(__fsub_rn(g, m), __fsub_rn(1.0f, a.beta1)));
-                    v = __fadd_rn(v, __fmul_rn(__fsub_rn(__fmul_rn(g, g), v), __fsub_rn(1.0f, a.beta2)));
-                    a.m[c] = m;
-                    a.v[c] = v;
-                    a.params[c] = __fsub_rn(pp[j], __fdiv_rn(__fmul_rn(m, alpha), __fadd_rn(__fsqrt_rn(v), a.eps)));
+                    adam_moments(__fmul_rn(gg[j], s_scale), mm[j], vv[j], a.beta1, a.beta2);
+                    a.m[c] = mm[j];
+                    a.v[c] = vv[j];
+                    a.params[c] = adam_param(pp[j], mm[j], vv[j], alpha, a.eps);
                 }
             }
         }

@@ -224,6 +224,51 @@ struct PolicyArgs {
     int mode;  // 0: step (pi + V + sample), 1: value only, 2: mean only (deterministic action)
 };
 
+__device__ __forceinline__ void store_neglogp(const PolicyArgs& a, int row, float nl) {
+    if (a.neglogp) a.neglogp[row] = nl;
+    if (a.nlp_store) a.nlp_store[row] = nl;
+}
+
+// Gaussian policy step of env `row` (mode 0) on a thread-per-row kernel: act_j = mu_j + exp(logstd_j) e_j with e_j from
+// a.eps, or from Philox stream (seed, env, *step_ctr, block j/4, PPO_TAG_ACTION), and neglogp.  logstd(j), mean(j) return
+// logstd_j and mu_j; put(j, act) stores the action.  A by reference: a runtime width is read from the kernel parameter
+// where it is used (a copy held in a register changes the generated code of the kernels); a compile-time width unrolls.
+template <class LS, class MU, class PUT>
+__device__ __forceinline__ void gauss_policy_row(const PolicyArgs& a, int row, const int& A, LS logstd, MU mean, PUT put) {
+    const uint32_t step = a.eps ? 0u : *a.step_ctr;
+    float ss = 0.f, sl = 0.f;
+#pragma unroll
+    for (int j0 = 0; j0 < A; j0 += 4) {
+        float e4[4];
+        if (!a.eps) normal4(a.seed, a.env_id0 + (uint32_t)row, step, (uint32_t)(j0 >> 2), PPO_TAG_ACTION, e4);
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const int j = j0 + q;
+            if (j < A) {
+                const float ls = logstd(j);
+                const float sd = expf(ls);  // logstd_b = mean*0 + logstd; std = exp (GRAPH:5098-5779)
+                const float e = a.eps ? a.eps[(size_t)row * A + j] : e4[q];
+                float z2;
+                put(j, gauss_sample(mean(j), sd, e, z2));
+                ss = __fadd_rn(ss, z2);
+                sl = __fadd_rn(sl, ls);
+            }
+        }
+    }
+    store_neglogp(a, row, gauss_neglogp_rn(ss, sl, A));
+}
+
+// Categorical policy step of env `row` (logits l[j * ld]): the index as fp32 in one column, sampled (mode 0; a.eps: [n][A]
+// uniforms when given) or argmax (mode 2)
+__device__ __forceinline__ void cat_policy_row(const PolicyArgs& a, int row, const float* l, int ld) {
+    const int j = a.mode == 0 ? cat_sample(l, ld, a.d.A, a.eps ? a.eps + (size_t)row * a.d.A : nullptr, a.seed, a.env_id0 + (uint32_t)row,
+                                           a.eps ? 0u : *a.step_ctr)
+                              : cat_argmax(l, ld, a.d.A);
+    if (a.action) a.action[row] = (float)j;
+    if (a.act_store) a.act_store[row] = (float)j;
+    if (a.mode == 0) store_neglogp(a, row, cat_neglogp(l, ld, a.d.A, j));
+}
+
 template <int TM>
 __host__ __device__ inline size_t policy_smem_floats(const NetDims& d) {
     return (size_t)(d.O + d.H1 + d.H2 + d.A + 1) * TM + (size_t)d.A * (TM + 1);
@@ -274,45 +319,12 @@ __global__ void __launch_bounds__(NT) policy_tile_kernel(const PolicyArgs a) {
                 if (a.value) a.value[row] = v;
                 if (a.val_store) a.val_store[row] = v;
             }
-            if (HEAD == HEAD_DISCRETE && a.mode != 1) {  // the index as fp32, one column; eps: [n][A] uniforms when given
-                const float* l = MU + m;
-                const int j = a.mode == 0 ? cat_sample(l, TM, d.A, a.eps ? a.eps + (size_t)row * d.A : nullptr, a.seed,
-                                                       a.env_id0 + (uint32_t)row, a.eps ? 0u : *a.step_ctr)
-                                          : cat_argmax(l, TM, d.A);
-                if (a.action) a.action[row] = (float)j;
-                if (a.act_store) a.act_store[row] = (float)j;
-                if (a.mode == 0) {
-                    const float nl = cat_neglogp(l, TM, d.A, j);
-                    if (a.neglogp) a.neglogp[row] = nl;
-                    if (a.nlp_store) a.nlp_store[row] = nl;
-                }
+            if (HEAD == HEAD_DISCRETE && a.mode != 1) {
+                cat_policy_row(a, row, MU + m, TM);
             } else if (a.mode == 0) {
                 const float* logstd = p + d.off[T_LOGSTD];
-                const uint32_t step = a.eps ? 0u : *a.step_ctr;
-                float ss = 0.f, sl = 0.f;
-                for (int j0 = 0; j0 < d.A; j0 += 4) {
-                    float e4[4];
-                    if (!a.eps) normal4(a.seed, a.env_id0 + (uint32_t)row, step, (uint32_t)(j0 >> 2), PPO_TAG_ACTION, e4);
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const int j = j0 + q;
-                        if (j < d.A) {
-                            const float ls = __ldg(logstd + j);
-                            const float sd = expf(ls);  // logstd_b = mean*0 + logstd; std = exp (GRAPH:5098-5779)
-                            const float e = a.eps ? a.eps[(size_t)row * d.A + j] : e4[q];
-                            const float mu = MU[j * TM + m];
-                            const float act = __fadd_rn(mu, __fmul_rn(sd, e));  // GRAPH:5992-6019
-                            const float z = __fdiv_rn(__fsub_rn(act, mu), sd);
-                            ss = __fadd_rn(ss, __fmul_rn(z, z));
-                            sl = __fadd_rn(sl, ls);
-                            Ac[j * (TM + 1) + m] = act;
-                        }
-                    }
-                }
-                // 0.5*sum(z^2) + 0.5*log(2pi)*float(A) + sum(logstd)   (GRAPH:6103-6672)
-                const float nl = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, ss), __fmul_rn(PPO_HALF_LOG_2PI, (float)d.A)), sl);
-                if (a.neglogp) a.neglogp[row] = nl;
-                if (a.nlp_store) a.nlp_store[row] = nl;
+                gauss_policy_row(a, row, d.A, [&](int j) { return __ldg(logstd + j); }, [&](int j) { return MU[j * TM + m]; },
+                                 [&](int j, float act) { Ac[j * (TM + 1) + m] = act; });
             } else if (a.mode == 2) {
                 for (int j = 0; j < d.A; ++j) Ac[j * (TM + 1) + m] = MU[j * TM + m];  // mean + 0.0 (GRAPH:6046-6076)
             }
@@ -349,6 +361,39 @@ struct TrainArgs {
     long long* prof;  // optional [2][32] phase timestamps of CTA 0 of each tower (U family, PPO_UMMA_PROF=1)
 };
 
+// This CTA's loss sums -> columns P.. of its slab (L = slab + P), the warps combined in a fixed order through s_red
+// (5 * NTH / 32 floats).  Entropy column: a categorical head's sum of H / B (x world, see UpdateScalars) over the CTA's
+// samples; a Box head's box_entropy of the pre-update logstd (logstd(j) loads logstd_j), in CTA 0 only.  A by reference as in
+// gauss_policy_row.
+template <int NTH, int HEAD, class LS>
+__device__ __forceinline__ void store_loss_columns(float* L, float l_pg, float l_vf, float l_kl, float l_cf, float l_ent, float* s_red,
+                                                   LS logstd, const int& A) {
+    const int tid = threadIdx.x;
+    constexpr int NL = HEAD == HEAD_DISCRETE ? 5 : 4;
+    float v4[NL];
+    v4[0] = l_pg; v4[1] = l_vf; v4[2] = l_kl; v4[3] = l_cf;
+    if (HEAD == HEAD_DISCRETE) v4[NL - 1] = l_ent;
+#pragma unroll
+    for (int q = 0; q < NL; ++q) v4[q] = warp_sum(v4[q]);
+    if ((tid & 31) == 0) {
+#pragma unroll
+        for (int q = 0; q < NL; ++q) s_red[(tid >> 5) * NL + q] = v4[q];
+    }
+    __syncthreads();
+    if (tid == 0) {
+        float t[NL];
+        for (int q = 0; q < NL; ++q) t[q] = 0.f;
+        for (int w = 0; w < NTH / 32; ++w)
+            for (int q = 0; q < NL; ++q) t[q] += s_red[w * NL + q];
+        L[L_PG] = t[0]; L[L_VF] = t[1]; L[L_KL] = t[2]; L[L_CLIP] = t[3];
+        float ent = 0.f;
+        if (HEAD == HEAD_DISCRETE) ent = t[NL - 1];
+        else if (blockIdx.x == 0) ent = box_entropy(logstd, A);
+        L[L_ENT] = ent;
+        L[5] = 0.f; L[6] = 0.f; L[7] = 0.f;
+    }
+}
+
 template <int TM>
 __host__ __device__ inline size_t train_smem_floats(const NetDims& d) {
     return (size_t)(d.O + 2 * d.A + 2 * d.H1 + 2 * d.H2) * TM + 5 * (size_t)TM + 64;
@@ -377,7 +422,6 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
     float* my = a.partial + (size_t)blockIdx.x * a.PS;
     const int ntiles = (a.count + TM - 1) / TM;
     const float cr = a.sc->cliprange, vr = vf_clip_range(a.vf_mode, cr, a.sc->cliprange_vf);
-    const float lo = 1.f - cr, hi = 1.f + cr;
     float l_pg = 0.f, l_vf = 0.f, l_kl = 0.f, l_cf = 0.f, l_ent = 0.f;
     bool acc = false;
 
@@ -417,22 +461,12 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
             const int m = tid;
             float* l = MU + m;
             if (m < nv) {
-                const int ai = (int)Ac[m];
-                float mx;
-                const float z = cat_partition(l, TM, d.A, mx);
-                const float nlp = logf(z) - (l[ai * TM] - mx);
-                const float H = cat_entropy(l, TM, d.A, mx, z);
-                const float adv = s_adv[m], oldn = s_oldn[m];
-                const float ratio = expf(oldn - nlp);
-                const float pg1 = -adv * ratio;
-                const float pg2 = -adv * fmaxf(fminf(ratio, hi), lo);
-                const bool take1 = pg1 >= pg2;
-                l_pg += take1 ? pg1 : pg2;
-                const float dn = nlp - oldn;
-                l_kl += dn * dn;
-                l_cf += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
+                float H;
+                const PgTerm t = cat_train_term(l, TM, d.A, (int)Ac[m], s_adv[m], s_oldn[m], cr, a.invB, a.ent_coef * a.invB, H);
+                l_pg += t.pg;
+                l_kl += t.kl;
+                l_cf += t.cf;
                 l_ent += H * (a.invB * a.sc->world);
-                cat_dlogits(l, TM, d.A, ai, mx, z, H, take1 ? (adv * ratio) * a.invB : 0.f, a.ent_coef * a.invB);
             } else {
                 for (int j = 0; j < d.A; ++j) l[j * TM] = 0.f;
             }
@@ -448,17 +482,11 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
                     ss += z * z;
                     sl += ls;
                 }
-                const float nlp = (0.5f * ss + PPO_HALF_LOG_2PI * (float)d.A) + sl;  // GRAPH:9428-9997
-                const float adv = s_adv[m], oldn = s_oldn[m];
-                const float ratio = expf(oldn - nlp);                                 // GRAPH:10423-10447
-                const float pg1 = -adv * ratio;
-                const float pg2 = -adv * fmaxf(fminf(ratio, hi), lo);                 // clip_by_value = max(min(x,hi),lo)
-                const bool take1 = pg1 >= pg2;                                        // ties -> unclipped branch (GRAPH:12609-12776)
-                l_pg += take1 ? pg1 : pg2;
-                const float dn = nlp - oldn;
-                l_kl += dn * dn;
-                l_cf += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
-                g_nlp = take1 ? (adv * ratio) * a.invB : 0.f;
+                const PgTerm t = pg_term(s_adv[m], s_oldn[m], gauss_neglogp(ss, sl, d.A), cr, a.invB);
+                l_pg += t.pg;
+                l_kl += t.kl;
+                l_cf += t.cf;
+                g_nlp = t.g_nlp;
             }
             for (int j = 0; j < d.A; ++j) {
                 const float sd = expf(__ldg(logstd + j));
@@ -512,35 +540,7 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
     }
 
     // loss sums of this CTA -> columns P.. of its slab (threads >= TM hold zeros)
-    constexpr int NL = HEAD == HEAD_DISCRETE ? 5 : 4;
-    float v4[NL];
-    v4[0] = l_pg; v4[1] = l_vf; v4[2] = l_kl; v4[3] = l_cf;
-    if (HEAD == HEAD_DISCRETE) v4[NL - 1] = l_ent;
-#pragma unroll
-    for (int q = 0; q < NL; ++q) v4[q] = warp_sum(v4[q]);
-    if ((tid & 31) == 0) {
-#pragma unroll
-        for (int q = 0; q < NL; ++q) s_red[(tid >> 5) * NL + q] = v4[q];
-    }
-    __syncthreads();
-    if (tid == 0) {
-        float t[NL];
-        for (int q = 0; q < NL; ++q) t[q] = 0.f;
-        for (int w = 0; w < NT / 32; ++w)
-            for (int q = 0; q < NL; ++q) t[q] += s_red[w * NL + q];
-        float* L = my + d.P;
-        L[L_PG] = t[0]; L[L_VF] = t[1]; L[L_KL] = t[2]; L[L_CLIP] = t[3];
-        float ent = 0.f;
-        if (HEAD == HEAD_DISCRETE) {
-            ent = t[NL - 1];  // sum of H / B (x world, see UpdateScalars) over this CTA's samples
-        } else if (blockIdx.x == 0) {
-            // entropy = sum_j(logstd_j + 0.5*log(2*pi*e)) with the pre-update weights (GRAPH:10021-10180)
-            const float* logstd = p + d.off[T_LOGSTD];
-            for (int j = 0; j < d.A; ++j) ent += __ldg(logstd + j) + PPO_HALF_LOG_2PIE;
-        }
-        L[L_ENT] = ent;
-        L[5] = 0.f; L[6] = 0.f; L[7] = 0.f;
-    }
+    store_loss_columns<NT, HEAD>(my + d.P, l_pg, l_vf, l_kl, l_cf, l_ent, s_red, [ls = p + d.off[T_LOGSTD]](int j) { return __ldg(ls + j); }, d.A);
     // loss = pg_loss - entropy*ent_coef + vf_loss*vf_coef: d(-ent_coef*entropy)/dlogstd_j = -ent_coef, added once
     // (a.ent_coef is already divided by the number of ranks whose slabs get summed)
     if (HEAD == HEAD_BOX && blockIdx.x == 0 && tid < d.A) my[d.off[T_LOGSTD] + tid] -= a.ent_coef;  // same thread wrote it in tile_rowsum

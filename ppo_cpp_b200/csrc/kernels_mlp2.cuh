@@ -262,7 +262,6 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
     float* my = a.partial + (size_t)blockIdx.x * a.PS;
     const int ntiles = (a.count + TM - 1) / TM;
     const float cr = a.sc->cliprange, vr = vf_clip_range(a.vf_mode, cr, a.sc->cliprange_vf);
-    const float lo = 1.f - cr, hi = 1.f + cr;
 
     stage_weights<NTH>(sW, a.params, d.P);
     // rows of ones behind every activation matrix (bias gradients fall out of the dW GEMM)
@@ -334,22 +333,12 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
             if (jg == 0) {
                 float* l = MU + m;
                 if (m < nv) {
-                    const int ai = (int)Ac[m];
-                    float mx;
-                    const float z = cat_partition(l, TM, d.A, mx);
-                    const float nlp = logf(z) - (l[ai * TM] - mx);
-                    const float H = cat_entropy(l, TM, d.A, mx, z);
-                    const float adv = s_adv[m], oldn = s_oldn[m];
-                    const float ratio = expf(oldn - nlp);
-                    const float pg1 = -adv * ratio;
-                    const float pg2 = -adv * fmaxf(fminf(ratio, hi), lo);
-                    const bool take1 = pg1 >= pg2;
-                    l_pg += take1 ? pg1 : pg2;
-                    const float dn = nlp - oldn;
-                    l_kl += dn * dn;
-                    l_cf += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
+                    float H;
+                    const PgTerm t = cat_train_term(l, TM, d.A, (int)Ac[m], s_adv[m], s_oldn[m], cr, a.invB, a.ent_coef * a.invB, H);
+                    l_pg += t.pg;
+                    l_kl += t.kl;
+                    l_cf += t.cf;
                     l_ent += H * (a.invB * a.sc->world);
-                    cat_dlogits(l, TM, d.A, ai, mx, z, H, take1 ? (adv * ratio) * a.invB : 0.f, a.ent_coef * a.invB);
                     float dv;
                     l_vf += value_loss_term(a.vf_mode, vr, Vs[m], s_oldv[m], s_ret[m], a.vf_coef, a.invB, dv);
                     Vs[m] = dv;
@@ -374,18 +363,12 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
                 float ss = 0.f, sl = 0.f;
                 for (int q = 0; q < JG; ++q) ss += s_red[q * TM + m];
                 for (int j = 0; j < d.A; ++j) sl += s_sd[d.A + j];
-                const float nlp = (0.5f * ss + PPO_HALF_LOG_2PI * (float)d.A) + sl;  // GRAPH:9428-9997
-                const float adv = s_adv[m], oldn = s_oldn[m];
-                const float ratio = expf(oldn - nlp);                                 // GRAPH:10423-10447
-                const float pg1 = -adv * ratio;
-                const float pg2 = -adv * fmaxf(fminf(ratio, hi), lo);                 // clip_by_value = max(min(x,hi),lo)
-                const bool take1 = pg1 >= pg2;                                        // ties -> unclipped branch
-                g_nlp = take1 ? (adv * ratio) * a.invB : 0.f;
+                const PgTerm t = pg_term(s_adv[m], s_oldn[m], gauss_neglogp(ss, sl, d.A), cr, a.invB);
+                g_nlp = t.g_nlp;
                 if (jg == 0) {
-                    l_pg += take1 ? pg1 : pg2;
-                    const float dn = nlp - oldn;
-                    l_kl += dn * dn;
-                    l_cf += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
+                    l_pg += t.pg;
+                    l_kl += t.kl;
+                    l_cf += t.cf;
                     float dv;
                     l_vf += value_loss_term(a.vf_mode, vr, Vs[m], s_oldv[m], s_ret[m], a.vf_coef, a.invB, dv);  // GRAPH:10213-10400
                     Vs[m] = dv;
@@ -425,31 +408,7 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
     }
     if (first) cp_async_wait_all();
 
-    constexpr int NL = HEAD == HEAD_DISCRETE ? 5 : 4;
-    float v4[NL];
-    v4[0] = l_pg; v4[1] = l_vf; v4[2] = l_kl; v4[3] = l_cf;
-    if (HEAD == HEAD_DISCRETE) v4[NL - 1] = l_ent;
-#pragma unroll
-    for (int q = 0; q < NL; ++q) v4[q] = warp_sum(v4[q]);
-    if ((tid & 31) == 0) {
-#pragma unroll
-        for (int q = 0; q < NL; ++q) s_red[(tid >> 5) * NL + q] = v4[q];
-    }
-    __syncthreads();
-    if (tid == 0) {
-        float t[NL];
-        for (int q = 0; q < NL; ++q) t[q] = 0.f;
-        for (int w = 0; w < NTH / 32; ++w)
-            for (int q = 0; q < NL; ++q) t[q] += s_red[w * NL + q];
-        float* Lp = my + d.P;
-        Lp[L_PG] = t[0]; Lp[L_VF] = t[1]; Lp[L_KL] = t[2]; Lp[L_CLIP] = t[3];
-        float ent = 0.f;
-        if (HEAD == HEAD_DISCRETE) ent = t[NL - 1];  // sum of H / B (x world, see UpdateScalars) over this CTA's samples
-        else if (blockIdx.x == 0)
-            for (int j = 0; j < d.A; ++j) ent += sW[d.off[T_LOGSTD] + j] + PPO_HALF_LOG_2PIE;  // GRAPH:10021-10180
-        Lp[L_ENT] = ent;
-        Lp[5] = 0.f; Lp[6] = 0.f; Lp[7] = 0.f;
-    }
+    store_loss_columns<NTH, HEAD>(my + d.P, l_pg, l_vf, l_kl, l_cf, l_ent, s_red, [ls = sW + d.off[T_LOGSTD]](int j) { return ls[j]; }, d.A);
     __syncthreads();
     // d(-ent_coef*entropy)/dlogstd_j = -ent_coef, once (a.ent_coef is pre-divided by the number of ranks)
     if (HEAD == HEAD_BOX && blockIdx.x == 0 && tid < d.A) my[d.off[T_LOGSTD] + tid] -= a.ent_coef;
@@ -506,44 +465,12 @@ __global__ void __launch_bounds__(NTH) policy_fused_kernel(const PolicyArgs a) {
                 if (a.value) a.value[row] = v;
                 if (a.val_store) a.val_store[row] = v;
             }
-            if (HEAD == HEAD_DISCRETE && a.mode != 1) {  // the index as fp32, one column; eps: [n][A] uniforms when given
-                const float* l = MU + m;
-                const int j = a.mode == 0 ? cat_sample(l, TM, d.A, a.eps ? a.eps + (size_t)row * d.A : nullptr, a.seed,
-                                                       a.env_id0 + (uint32_t)row, a.eps ? 0u : *a.step_ctr)
-                                          : cat_argmax(l, TM, d.A);
-                if (a.action) a.action[row] = (float)j;
-                if (a.act_store) a.act_store[row] = (float)j;
-                if (a.mode == 0) {
-                    const float nl = cat_neglogp(l, TM, d.A, j);
-                    if (a.neglogp) a.neglogp[row] = nl;
-                    if (a.nlp_store) a.nlp_store[row] = nl;
-                }
+            if (HEAD == HEAD_DISCRETE && a.mode != 1) {
+                cat_policy_row(a, row, MU + m, TM);
             } else if (a.mode == 0) {
                 const float* logstd = sW + d.off[T_LOGSTD];
-                const uint32_t step = a.eps ? 0u : *a.step_ctr;
-                float ss = 0.f, sl = 0.f;
-                for (int j0 = 0; j0 < d.A; j0 += 4) {
-                    float e4[4];
-                    if (!a.eps) normal4(a.seed, a.env_id0 + (uint32_t)row, step, (uint32_t)(j0 >> 2), PPO_TAG_ACTION, e4);
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const int j = j0 + q;
-                        if (j < d.A) {
-                            const float ls = logstd[j];
-                            const float sd = expf(ls);
-                            const float e = a.eps ? a.eps[(size_t)row * d.A + j] : e4[q];
-                            const float mu = MU[j * TM + m];
-                            const float act = __fadd_rn(mu, __fmul_rn(sd, e));  // GRAPH:5992-6019
-                            const float z = __fdiv_rn(__fsub_rn(act, mu), sd);
-                            ss = __fadd_rn(ss, __fmul_rn(z, z));
-                            sl = __fadd_rn(sl, ls);
-                            Ac[j * (TM + 1) + m] = act;
-                        }
-                    }
-                }
-                const float nl = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, ss), __fmul_rn(PPO_HALF_LOG_2PI, (float)d.A)), sl);
-                if (a.neglogp) a.neglogp[row] = nl;
-                if (a.nlp_store) a.nlp_store[row] = nl;
+                gauss_policy_row(a, row, d.A, [&](int j) { return logstd[j]; }, [&](int j) { return MU[j * TM + m]; },
+                                 [&](int j, float act) { Ac[j * (TM + 1) + m] = act; });
             } else if (a.mode == 2) {
                 for (int j = 0; j < d.A; ++j) Ac[j * (TM + 1) + m] = MU[j * TM + m];
             }

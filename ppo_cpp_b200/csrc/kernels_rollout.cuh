@@ -346,11 +346,10 @@ __global__ void __launch_bounds__(R_NTH) rollout_persistent_kernel(const Rollout
                     // -- Gaussian sample (GRAPH:5894-6019)
                     for (int j = lane, jj = 0; j < A; j += 32, ++jj) {
                         const float sd = jj ? sd_l[1] : sd_l[0];  // (A <= 32 + 32; asserted by the host: obs_dim == act_dim <= 32)
-                        const float mu = MU[j * TM];
-                        const float act = __fadd_rn(mu, __fmul_rn(sd, na[s * NB + j]));
-                        const float z = __fdiv_rn(__fsub_rn(act, mu), sd);
+                        float z2;
+                        const float act = gauss_sample(MU[j * TM], sd, na[s * NB + j], z2);
                         Ac[j * (TM + 1)] = act;
-                        Z2[j * TM] = __fmul_rn(z, z);
+                        Z2[j * TM] = z2;
                         a.act_store[(size_t)t * A + j] = act;
                         if (host_env) {
                             if (a.h_act_ll) ll_store(a.h_act_ll + j, __float_as_uint(act), (unsigned)t + 1u);
@@ -361,7 +360,7 @@ __global__ void __launch_bounds__(R_NTH) rollout_persistent_kernel(const Rollout
                     if (lane == 0) {  // neglogp (GRAPH:6103-6672): sequential sum in action order
                         float ss = 0.f;
                         for (int j = 0; j < A; ++j) ss = __fadd_rn(ss, Z2[j * TM]);
-                        a.nlp_store[t] = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, ss), __fmul_rn(PPO_HALF_LOG_2PI, (float)A)), sl_c);
+                        a.nlp_store[t] = gauss_neglogp_rn(ss, sl_c, A);
                         a.val_store[t] = Vs[0];
                         a.dones_store[t] = DN[0];  // done flag of the previous env step (runner.hpp:110)
                     }
@@ -603,12 +602,9 @@ __global__ void __launch_bounds__(R_NTH) rollout_persistent_kernel(const Rollout
                     for (int q = 0; q < 4; ++q) {
                         const int j = blk * 4 + q;
                         if (j < A) {
-                            const float sd = expf(logstd[j]);
-                            const float mu = MU[j * TM + m];
-                            const float act = __fadd_rn(mu, __fmul_rn(sd, e4[q]));
-                            const float z = __fdiv_rn(__fsub_rn(act, mu), sd);
-                            Ac[j * (TM + 1) + m] = act;
-                            Z2[j * TM + m] = __fmul_rn(z, z);
+                            float z2;
+                            Ac[j * (TM + 1) + m] = gauss_sample(MU[j * TM + m], expf(logstd[j]), e4[q], z2);
+                            Z2[j * TM + m] = z2;
                         }
                     }
                 }
@@ -621,7 +617,7 @@ __global__ void __launch_bounds__(R_NTH) rollout_persistent_kernel(const Rollout
                     ss = __fadd_rn(ss, Z2[j * TM + m]);
                     sl = __fadd_rn(sl, logstd[j]);
                 }
-                const float nl = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, ss), __fmul_rn(PPO_HALF_LOG_2PI, (float)A)), sl);
+                const float nl = gauss_neglogp_rn(ss, sl, A);
                 const size_t idx = (size_t)t * a.n + row;
                 for (int r = 0; r < world; ++r) {
                     rslab(a, r, a.off_nlp, 1, a.nlp_store)[idx] = nl;

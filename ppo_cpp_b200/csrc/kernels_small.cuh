@@ -154,17 +154,12 @@ __device__ __forceinline__ void small_warp_tile(const TrainArgs& a, const float*
             float g_nlp = 0.f;
             if (valid) {
                 // the clip ranges are loaded where they are used: kept live across the loop they cost the epoch kernel spills
-                const float cr = a.sc->cliprange, lo = 1.f - cr, hi = 1.f + cr;
-                const float nlp = (0.5f * ss + PPO_HALF_LOG_2PI * (float)A) + sum_ls;
-                const float ratio = expf(oldn - nlp);                          // GRAPH:10423-10447
-                const float pg1 = -adv * ratio;
-                const float pg2 = -adv * fmaxf(fminf(ratio, hi), lo);          // clip_by_value = max(min(x,hi),lo)
-                const bool take1 = pg1 >= pg2;                                 // ties -> unclipped branch
-                g_nlp = take1 ? (adv * ratio) * a.invB : 0.f;
-                l_pg += take1 ? pg1 : pg2;
-                const float dn = nlp - oldn;
-                l_kl += dn * dn;
-                l_cf += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
+                const float cr = a.sc->cliprange;
+                const PgTerm t = pg_term(adv, oldn, gauss_neglogp(ss, sum_ls, A), cr, a.invB);
+                g_nlp = t.g_nlp;
+                l_pg += t.pg;
+                l_kl += t.kl;
+                l_cf += t.cf;
                 const float vr = vf_clip_range(a.vf_mode, cr, a.sc->cliprange_vf);
                 l_vf += value_loss_term(a.vf_mode, vr, v, oldv, R, a.vf_coef, a.invB, dv);  // GRAPH:10213-10400
             }
@@ -282,8 +277,7 @@ __global__ void __launch_bounds__(NTH) train_small_kernel(const TrainArgs a) {
         float* Lp = my + D::P;
         Lp[L_PG] = t[0]; Lp[L_VF] = t[1]; Lp[L_KL] = t[2]; Lp[L_CLIP] = t[3];
         float ent = 0.f;
-        if (blockIdx.x == 0)
-            for (int j = 0; j < A; ++j) ent += sW[D::LS + j] + PPO_HALF_LOG_2PIE;  // GRAPH:10021-10180
+        if (blockIdx.x == 0) ent = box_entropy([&](int j) { return sW[D::LS + j]; }, A);
         Lp[L_ENT] = ent;
         Lp[5] = 0.f; Lp[6] = 0.f; Lp[7] = 0.f;
     }
@@ -373,31 +367,8 @@ __global__ void __launch_bounds__(NTH) policy_small_kernel(const PolicyArgs a) {
                 if (a.val_store) a.val_store[row] = v;
             }
             if (a.mode == 0) {
-                const uint32_t step = a.eps ? 0u : *a.step_ctr;
-                float ss = 0.f, sl = 0.f;
-#pragma unroll
-                for (int j0 = 0; j0 < A; j0 += 4) {
-                    float e4[4];
-                    if (!a.eps) normal4(a.seed, a.env_id0 + (uint32_t)row, step, (uint32_t)(j0 >> 2), PPO_TAG_ACTION, e4);
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const int j = j0 + q;
-                        if (j < A) {
-                            const float ls = sW[D::LS + j];
-                            const float sd = expf(ls);  // logstd_b = mean*0 + logstd; std = exp (GRAPH:5098-5779)
-                            const float e = a.eps ? a.eps[(size_t)row * A + j] : e4[q];
-                            const float act = __fadd_rn(mu[j], __fmul_rn(sd, e));  // GRAPH:5992-6019
-                            const float z = __fdiv_rn(__fsub_rn(act, mu[j]), sd);
-                            ss = __fadd_rn(ss, __fmul_rn(z, z));
-                            sl = __fadd_rn(sl, ls);
-                            sA[tid * AL + j] = act;
-                        }
-                    }
-                }
-                // 0.5*sum(z^2) + 0.5*log(2pi)*float(A) + sum(logstd)   (GRAPH:6103-6672)
-                const float nl = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, ss), __fmul_rn(PPO_HALF_LOG_2PI, (float)A)), sl);
-                if (a.neglogp) a.neglogp[row] = nl;
-                if (a.nlp_store) a.nlp_store[row] = nl;
+                gauss_policy_row(a, row, A, [&](int j) { return sW[D::LS + j]; }, [&](int j) { return mu[j]; },
+                                 [&](int j, float act) { sA[tid * AL + j] = act; });
             } else if (a.mode == 2) {
 #pragma unroll
                 for (int j = 0; j < A; ++j) sA[tid * AL + j] = mu[j];  // mean + 0.0 (GRAPH:6046-6076)
@@ -501,35 +472,25 @@ __global__ void __launch_bounds__(NTH) train_small_epoch_kernel(const TrainArgs 
         double ss = 0.0;
 #pragma unroll
         for (int w = 0; w < NTH / 32; ++w) ss += s_q[w];
-        const float gnorm = (float)sqrt(ss);
-        const float inv = __fdiv_rn(1.0f, gnorm), invc = __fdiv_rn(1.0f, ad.clip_norm);
-        float scale = __fmul_rn(ad.clip_norm, fminf(inv, invc));
-        if (!isfinite(gnorm)) scale = __int_as_float(0x7fc00000);  // GRAPH:24493-24543
+        float gnorm;
+        const float scale = clip_scale(ss, ad.clip_norm, gnorm);
         if (tid == 0) {
-            float ent = 0.f;
-            for (int j = 0; j < A; ++j) ent += sW[D::LS + j] + PPO_HALF_LOG_2PIE;  // GRAPH:10021-10180 (the parameters before this step)
-            float* lr_out = ep.loss_rows + (size_t)mb * 5;
-            lr_out[0] = lsum[0] * ad.invB;
-            lr_out[1] = 0.5f * (lsum[1] * ad.invB);
-            lr_out[2] = ent * ad.inv_world;
-            lr_out[3] = 0.5f * (lsum[2] * ad.invB);
-            lr_out[4] = lsum[3] * ad.invB;
+            const float L[5] = {lsum[0], lsum[1], box_entropy([&](int j) { return sW[D::LS + j]; }, A), lsum[2], lsum[3]};  // entropy: the parameters before this step
+            loss_row(ep.loss_rows + (size_t)mb * 5, L, ad.invB, ad.inv_world);
             *ad.gnorm_out = gnorm;
         }
         __syncthreads();  // thread 0 has read logstd before it moves
-        // ---- TF ApplyAdam (epsilon outside the sqrt), in place in shared memory
-        const float alpha = __fdiv_rn(__fmul_rn(ad.sc->lr, __fsqrt_rn(__fsub_rn(1.0f, b2p))), __fsub_rn(1.0f, b1p));
+        // ---- TF ApplyAdam, in place in shared memory
+        const float alpha = adam_alpha(ad.sc->lr, b1p, b2p);
 #pragma unroll
         for (int u = 0; u < PT; ++u) {
             const int i = tid + u * NTH;
             if (i < D::P) {
-                const float gs = __fmul_rn(g[u], scale);
                 float m = sM[i], v = sV[i];
-                m = __fadd_rn(m, __fmul_rn(__fsub_rn(gs, m), __fsub_rn(1.0f, ad.beta1)));
-                v = __fadd_rn(v, __fmul_rn(__fsub_rn(__fmul_rn(gs, gs), v), __fsub_rn(1.0f, ad.beta2)));
+                adam_moments(__fmul_rn(g[u], scale), m, v, ad.beta1, ad.beta2);
                 sM[i] = m;
                 sV[i] = v;
-                sW[i] = __fsub_rn(sW[i], __fdiv_rn(__fmul_rn(m, alpha), __fadd_rn(__fsqrt_rn(v), ad.eps)));
+                sW[i] = adam_param(sW[i], m, v, alpha, ad.eps);
             }
         }
         b1p = __fmul_rn(b1p, ad.beta1);

@@ -551,7 +551,6 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
     const uint32_t id_s16 = make_idesc(128, 16, 1, 0);    // column sums: MN-major [A_hi ; A_lo] x K-major ones
 
     const float cr = a.sc->cliprange, vr = vf_clip_range(a.vf_mode, cr, a.sc->cliprange_vf);
-    const float lo = 1.f - cr, hi = 1.f + cr;
     // the backward tensors (which carry the 1/B of the batch mean) are stored times a power of two so that they are O(1) as
     // fp16 operands (see the header); exponents are chosen per minibatch when the weights are staged
     int invB_exp;
@@ -874,17 +873,15 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
                 asm volatile("bar.sync 1, 256;" ::: "memory");
                 const float adv = f32[F32_PV + row], oldn = f32[F32_PV + TM + row];
                 if (valid) {
-                    const float nlp = (0.5f * ss + PPO_HALF_LOG_2PI * (float)A) + f32[F32_MISC + 1];
-                    const float ratio = expf(oldn - nlp);                          // GRAPH:10423-10447
-                    const float pg1 = -adv * ratio;
-                    const float pg2 = -adv * fmaxf(fminf(ratio, hi), lo);          // clip_by_value = max(min(x,hi),lo)
-                    const bool take1 = pg1 >= pg2;                                 // ties -> unclipped branch
-                    g_nlp = take1 ? ((adv * ratio) * a.invB) * S_b : 0.f;
+                    const float nlp = gauss_neglogp(ss, f32[F32_MISC + 1], A);
+                    g_nlp = pg_term(adv, oldn, nlp, cr, a.invB).g_nlp * S_b;
                     if (half == 0) {
-                        l_0 += take1 ? pg1 : pg2;
-                        const float dn = nlp - oldn;
-                        l_1 += dn * dn;
-                        l_2 += (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
+                        // the same pg_term (merged with the one above), so that its loss terms are evaluated in this branch
+                        // only: one call ahead of the branch was tried and changes this kernel's instruction mix
+                        const PgTerm t = pg_term(adv, oldn, nlp, cr, a.invB);
+                        l_0 += t.pg;
+                        l_1 += t.kl;
+                        l_2 += t.cf;
                     }
                 }
                 if (half == 0) {
@@ -1125,8 +1122,7 @@ __global__ void __launch_bounds__(NTH, 1) train_umma_kernel(const TrainArgs a, c
             if (tower == 0) {
                 put(Lp + L_PG, t[0]); put(Lp + L_KL, t[1]); put(Lp + L_CLIP, t[2]);
                 float ent = 0.f;
-                if (blockIdx.x == 0)
-                    for (int j = 0; j < A; ++j) ent += f32[F32_LS + j] + PPO_HALF_LOG_2PIE;  // GRAPH:10021-10180
+                if (blockIdx.x == 0) ent = box_entropy([&](int j) { return f32[F32_LS + j]; }, A);
                 put(Lp + L_ENT, ent);
                 put(Lp + 5, 0.f); put(Lp + 6, 0.f); put(Lp + 7, 0.f);
             } else {

@@ -393,7 +393,7 @@ __global__ void __launch_bounds__(GEMM_NTH, 1) wgemm_kernel(const GemmArgs g) {
                     if (k.tower == 0) {
                         float l_pg = 0.f, l_kl = 0.f, l_cf = 0.f;
                         if (valid) {
-                            const float cr = a.sc->cliprange, lo = 1.f - cr, hi = 1.f + cr;
+                            const float cr = a.sc->cliprange;
                             float z[A], isd[A];
                             float ss = 0.f, sl = 0.f;
 #pragma unroll
@@ -404,16 +404,11 @@ __global__ void __launch_bounds__(GEMM_NTH, 1) wgemm_kernel(const GemmArgs g) {
                                 ss += z[j] * z[j];
                                 sl += ls;
                             }
-                            const float nlp = (0.5f * ss + PPO_HALF_LOG_2PI * (float)A) + sl;
-                            const float ratio = expf(oldn - nlp);
-                            const float pg1 = -adv * ratio;
-                            const float pg2 = -adv * fmaxf(fminf(ratio, hi), lo);  // clip_by_value = max(min(x,hi),lo)
-                            const bool take1 = pg1 >= pg2;                          // ties -> unclipped branch
-                            l_pg = take1 ? pg1 : pg2;
-                            const float dn = nlp - oldn;
-                            l_kl = dn * dn;
-                            l_cf = (fabsf(ratio - 1.f) > cr) ? 1.f : 0.f;
-                            const float g_nlp = take1 ? (adv * ratio) * a.invB : 0.f;
+                            const PgTerm t = pg_term(adv, oldn, gauss_neglogp(ss, sl, A), cr, a.invB);
+                            l_pg = t.pg;
+                            l_kl = t.kl;
+                            l_cf = t.cf;
+                            const float g_nlp = t.g_nlp;
 #pragma unroll
                             for (int j = 0; j < A; ++j) {
                                 v[j] = g_nlp * (-z[j] * isd[j]);        // dL/dmu_j
@@ -801,32 +796,11 @@ __global__ void wide_policy_head_kernel(const PolicyArgs a, const WideBufs w) {
     const float* mu = w.MU + (size_t)row * 64;
     if (a.mode == 0) {
         const float* logstd = p + d.off[T_LOGSTD];
-        const uint32_t step = a.eps ? 0u : *a.step_ctr;
-        float ss = 0.f, sl = 0.f;
-        for (int j0 = 0; j0 < d.A; j0 += 4) {
-            float e4[4];
-            if (!a.eps) normal4(a.seed, a.env_id0 + (uint32_t)row, step, (uint32_t)(j0 >> 2), PPO_TAG_ACTION, e4);
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const int j = j0 + q;
-                if (j < d.A) {
-                    const float ls = __ldg(logstd + j);
-                    const float sd = expf(ls);
-                    const float e = a.eps ? a.eps[(size_t)row * d.A + j] : e4[q];
-                    const float m = mu[j] + __ldg(p + d.off[T_PI_B] + j);
-                    const float act = __fadd_rn(m, __fmul_rn(sd, e));  // GRAPH:5992-6019
-                    const float z = __fdiv_rn(__fsub_rn(act, m), sd);
-                    ss = __fadd_rn(ss, __fmul_rn(z, z));
-                    sl = __fadd_rn(sl, ls);
-                    if (a.action) a.action[(size_t)row * d.A + j] = act;
-                    if (a.act_store) a.act_store[(size_t)row * d.A + j] = act;
-                }
-            }
-        }
-        // 0.5*sum(z^2) + 0.5*log(2pi)*float(A) + sum(logstd)   (GRAPH:6103-6672)
-        const float nl = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, ss), __fmul_rn(PPO_HALF_LOG_2PI, (float)d.A)), sl);
-        if (a.neglogp) a.neglogp[row] = nl;
-        if (a.nlp_store) a.nlp_store[row] = nl;
+        gauss_policy_row(a, row, d.A, [&](int j) { return __ldg(logstd + j); }, [&](int j) { return mu[j] + __ldg(p + d.off[T_PI_B] + j); },
+                         [&](int j, float act) {
+                             if (a.action) a.action[(size_t)row * d.A + j] = act;
+                             if (a.act_store) a.act_store[(size_t)row * d.A + j] = act;
+                         });
     } else if (a.mode == 2) {
         for (int j = 0; j < d.A; ++j) {
             const float m = mu[j] + __ldg(p + d.off[T_PI_B] + j);  // mean + 0.0 (GRAPH:6046-6076)
