@@ -1,64 +1,29 @@
 """The hidden-layer activation read from the graph file (Stable-Baselines' act_fun: tf.tanh or tf.nn.relu, ppo_activation).
 
-The reference is an fp64 PyTorch autograd restatement of the PPO2 loss with torch.relu, whose gradient also masks on
-output > 0, as TensorFlow's ReluGrad does.  CPU tests: both graph readers on the writer's files and hand-edited variants, the
+The reference is test_vf_clip_and_schedules' fp64 PyTorch autograd restatement of the PPO2 loss with torch.relu, whose
+gradient also masks on output > 0, as TensorFlow's ReluGrad does.  CPU tests: both graph readers on the writer's files and hand-edited variants, the
 writer's unchanged output without activation, and the reference's tie fixture (pre-activations exactly 0).  GPU tests: every
 forward path, the persistent rollout, every train family's loss and gradients, whole updates, family selection, switching
-the activation of a live core and the host C++ CLI.  (A two-GPU ReLU update is not covered here; no real Stable-Baselines ReLU
-export is available, so the reader rule is checked against the writer's files and hand edits of them only.)"""
+the activation of a live core and the host C++ CLI (test_multi_gpu_parity.py: sharded ReLU updates).  No real Stable-Baselines
+ReLU export is available, so the reader rule is checked against the writer's files and hand edits of them only."""
 import hashlib
 import os
 import subprocess
+from functools import partial
 
 import numpy as np
 import pytest
-import torch
 
 import oracle_lib as ol
 from conftest import ROOT, load_weights, rel_err
 from ppo_cpp_b200 import meta_graph as mg
-from test_vf_clip_and_schedules import (HALF_LOG_2PI, HALF_LOG_2PIE, _layout, _tf_clip, _tf_max, rand_params,
-                                        tensor_slices, value_loss)
+from test_vf_clip_and_schedules import HALF_LOG_2PI, _layout, learner_ref, loss_grad_ref, rand_params, tensor_slices
 
 TOL = 1e-5
 ENT = 0.0007160293171182275
 
 
-# ------------------------------------------------------------------ fp64 reference (PyTorch autograd)
-def _act(name, mask):
-    if name == "tanh":
-        return torch.tanh
-    if mask == "gt":
-        return torch.relu  # d relu / dx = (relu(x) > 0), TensorFlow's ReluGrad
-    return lambda z: torch.where(z >= 0, z, torch.zeros_like(z))  # gradient on x >= 0 (a unit at exactly 0 passes it)
-
-
-def loss_grad_ref(params, obs, act, adv, ret, old_nlp, old_v, cr, activation, h1, h2, ent_coef=ENT, vf_coef=0.5, mask="gt"):
-    lay, P = _layout(h1, h2)
-    p = torch.tensor(np.asarray(params[:P], np.float64), requires_grad=True)
-    T = [p[o:o + int(np.prod(s))].reshape(s) for o, s in lay]
-    pi0w, pi0b, vf0w, vf0b, pi1w, pi1b, vf1w, vf1b, vfw, vfb, piw, pib, logstd = T
-    f = _act(activation, mask)
-    x = torch.tensor(np.asarray(obs, np.float64))
-    a = torch.tensor(np.asarray(act, np.float64))
-    adv, R, onl, ov = (torch.tensor(np.asarray(z, np.float64).ravel()) for z in (adv, ret, old_nlp, old_v))
-    mu = f(f(x @ pi0w + pi0b) @ pi1w + pi1b) @ piw + pib
-    v = (f(f(x @ vf0w + vf0b) @ vf1w + vf1b) @ vfw + vfb)[:, 0]
-    ls = logstd.reshape(-1)
-    nlp = 0.5 * (((a - mu) / torch.exp(ls)) ** 2).sum(1) + HALF_LOG_2PI * a.shape[1] + ls.sum()
-    ratio = torch.exp(onl - nlp)
-    pg = _tf_max(-adv * ratio, -adv * _tf_clip(ratio, torch.tensor(1.0 - cr, dtype=torch.float64),
-                                                torch.tensor(1.0 + cr, dtype=torch.float64))).mean()
-    vf = 0.5 * value_loss(v, ov, R, "shared", cr, 0.0).mean()
-    ent = (ls + HALF_LOG_2PIE).sum()
-    loss = pg - ent * ent_coef + vf * vf_coef
-    loss.backward()
-    with torch.no_grad():
-        kl = 0.5 * ((nlp - onl) ** 2).mean()
-        cf = ((ratio - 1.0).abs() > cr).double().mean()
-    return p.grad.numpy().copy(), np.array([pg.item(), vf.item(), ent.item(), kl.item(), cf.item()])
-
-
+# ------------------------------------------------------------------ fp64 reference (loss_grad_ref and learner_ref of test_vf_clip_and_schedules)
 def forward_ref(params, obs, activation, h1, h2):
     lay, _ = _layout(h1, h2)
     t = [params.astype(np.float64)[o:o + int(np.prod(s))].reshape(s) for o, s in lay]
@@ -123,8 +88,8 @@ def test_reference_tie_fixture_separates_gt_from_ge():
     lay, _ = _layout(4, 5)
     W0 = p[lay[0][0]:lay[0][0] + 72].reshape(18, 4).astype(np.float64)
     assert np.all((x @ W0 + p[lay[1][0]:lay[1][0] + 4])[:, 0] == 0.0)  # unit 0: pre-activation exactly 0
-    g_gt, l_gt = loss_grad_ref(p, obs, act, adv, ret, old_nlp, old_v, 0.2, "relu", 4, 5, mask="gt")
-    g_ge, l_ge = loss_grad_ref(p, obs, act, adv, ret, old_nlp, old_v, 0.2, "relu", 4, 5, mask="ge")
+    g_gt, l_gt = loss_grad_ref(p, obs, act, adv, ret, old_nlp, old_v, 0.2, activation="relu", h1=4, h2=5, mask="gt")
+    g_ge, l_ge = loss_grad_ref(p, obs, act, adv, ret, old_nlp, old_v, 0.2, activation="relu", h1=4, h2=5, mask="ge")
     assert np.array_equal(l_gt, l_ge)  # same forward pass
     sl = tensor_slices(4, 5)
     assert np.all(g_gt[sl[1]][::4] == 0.0) and np.any(g_ge[sl[1]][::4] != 0.0)  # the tied units' bias gradient
@@ -346,7 +311,7 @@ def test_loss_grad_relu_every_family_vs_fp64(monkeypatch, h, B, env, fam, fixtur
             h2v = np.maximum(x @ p[lay[4][0]:lay[4][0] + h * h].reshape(h, h) + p[lay[5][0]:lay[5][0] + h], 0)
             assert h2v.max() > 1000 and 0 < np.min(h2v[h2v > 0]) < 1e-3, (h2v.max(), np.min(h2v[h2v > 0]))
         g, l = c.loss_grad(obs, act, adv, ret, old_nlp, old_v, 0.2)
-        g64, l64 = loss_grad_ref(p, obs, act, adv, ret, old_nlp, old_v, 0.2, "relu", h, h2)
+        g64, l64 = loss_grad_ref(p, obs, act, adv, ret, old_nlp, old_v, 0.2, activation="relu", h1=h, h2=h2)
         for t in range(13):
             assert rel_err(g[sl[t]], g64[sl[t]]) < TOL, (fixture, t, rel_err(g[sl[t]], g64[sl[t]]))
         assert np.allclose(l[:4], l64[:4], rtol=TOL, atol=1e-7), (fixture, l, l64)
@@ -354,34 +319,6 @@ def test_loss_grad_relu_every_family_vs_fp64(monkeypatch, h, B, env, fam, fixtur
 
 
 # ------------------------------------------------------------------ GPU: whole updates against an fp64 learner
-def learner_ref(flat, bufs, perms, nmb, lr, cr, h1, h2, clip=0.5, b1=0.9, b2=0.999, eps=1e-5):
-    _, P = _layout(h1, h2)
-    p = flat.astype(np.float64).copy()
-    m, v = np.zeros(P), np.zeros(P)
-    b1p, b2p = b1, b2
-    nb = bufs["obs"].shape[0]
-    Bm = nb // nmb
-    rows = []
-    for perm in perms:
-        src = np.empty_like(perm)
-        src[perm] = np.arange(nb)
-        for k in range(nmb):
-            idx = src[k * Bm:(k + 1) * Bm]
-            ret, val = bufs["returns"][idx, 0], bufs["values"][idx, 0]
-            a = ret.astype(np.float64) - val
-            adv = (a - a.mean()) / (np.sqrt(((a - a.mean()) ** 2).mean()) + 1e-8)
-            g, l = loss_grad_ref(p, bufs["obs"][idx], bufs["actions"][idx], adv, ret, bufs["neglogpacs"][idx, 0], val, cr, "relu", h1, h2)
-            rows.append(l)
-            gn = np.sqrt((g * g).sum())
-            g = g * clip * min(1.0 / gn, 1.0 / clip)
-            m += (g - m) * (1 - b1)
-            v += (g * g - v) * (1 - b2)
-            p[:P] -= lr * np.sqrt(1 - b2p) / (1 - b1p) * m / (np.sqrt(v) + eps)
-            b1p *= b1
-            b2p *= b2
-    return p, np.mean(rows, axis=0)
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("h1,h2,n_envs,n_steps,nmb,epochs,fam", [(4, 5, 1, 2048, 32, 2, "small"), (64, 64, 1024, 16, 2, 2, "persistent"),
                                                                   (256, 256, 128, 32, 1, 1, "tcgen05")])
@@ -401,7 +338,7 @@ def test_train_update_relu_vs_fp64_learner(h1, h2, n_envs, n_steps, nmb, epochs,
     perms = [c.train_get_permutation(e) for e in range(epochs)]
     got = c.get_tensor("params")
     c.close()
-    p64, want = learner_ref(flat, bufs, perms, nmb, 3.9e-4, 0.2, h1, h2)
+    p64, want = learner_ref(flat, bufs, perms, nmb, 3.9e-4, 0.2, partial(loss_grad_ref, activation="relu", h1=h1, h2=h2))
     _, P = _layout(h1, h2)
     moved = np.abs(p64[:P] - flat[:P]).max()
     assert np.abs(got[:P] - p64[:P]).max() < max(5e-4, 4e-5 * epochs * nmb) * moved

@@ -6,11 +6,12 @@ TensorFlow's tie rules for the clipped surrogate and the value loss, Gumbel-max 
 CPU tests: both graph readers on the writer's files and hand edits, the layout and the checkpoint order, the index writer,
 the writer's unchanged output without action_space, and the host bandit env.  GPU tests (the F and T families, tanh and
 ReLU): policy steps with supplied uniforms and with Philox noise, loss and gradients, whole updates against an fp64 learner,
-the host-env protocol, family selection, checkpoints and the CLI.  (A two-GPU discrete update is not covered; no real
-Stable-Baselines Discrete export is available, so the reader rule is checked against the writer's files and hand edits.)"""
+the host-env protocol, family selection, checkpoints and the CLI (test_multi_gpu_parity.py: sharded discrete updates).  No
+real Stable-Baselines Discrete export is available, so the reader rule is checked against the writer's files and hand edits."""
 import hashlib
 import os
 import subprocess
+from functools import partial
 
 import numpy as np
 import pytest
@@ -19,7 +20,7 @@ import torch
 from conftest import ROOT, load_weights, rel_err
 from ppo_cpp_b200 import meta_graph as mg
 from test_abi_cpu import _parse_bundle_index
-from test_vf_clip_and_schedules import _tf_clip, _tf_max, value_loss
+from test_vf_clip_and_schedules import _tf_clip, _tf_max, learner_ref, value_loss
 
 TOL = 1e-5
 ENT = 0.01
@@ -358,34 +359,6 @@ def _replay_rollout(rng, n_envs, n_steps):
     return raw, rew, done
 
 
-def learner_ref(flat, bufs, perms, nmb, lr, cr, activation, h1, h2, clip=0.5, b1=0.9, b2=0.999, eps=1e-5):
-    _, P, _ = layout(h1, h2)
-    p = flat.astype(np.float64).copy()
-    m, v = np.zeros(P), np.zeros(P)
-    b1p, b2p = b1, b2
-    nb = bufs["obs"].shape[0]
-    Bm = nb // nmb
-    rows = []
-    for perm in perms:
-        src = np.empty_like(perm)
-        src[perm] = np.arange(nb)
-        for k in range(nmb):
-            idx = src[k * Bm:(k + 1) * Bm]
-            ret, val = bufs["returns"][idx, 0], bufs["values"][idx, 0]
-            a = ret.astype(np.float64) - val
-            adv = (a - a.mean()) / (np.sqrt(((a - a.mean()) ** 2).mean()) + 1e-8)
-            g, l = loss_grad_ref(p, bufs["obs"][idx], bufs["actions"][idx], adv, ret, bufs["neglogpacs"][idx, 0], val, cr, activation, h1, h2)
-            rows.append(l)
-            gn = np.sqrt((g * g).sum())
-            g = g * clip * min(1.0 / gn, 1.0 / clip)
-            m += (g - m) * (1 - b1)
-            v += (g * g - v) * (1 - b2)
-            p[:P] -= lr * np.sqrt(1 - b2p) / (1 - b1p) * m / (np.sqrt(v) + eps)
-            b1p *= b1
-            b2p *= b2
-    return p, np.mean(rows, axis=0)
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("activation", ["tanh", "relu"])
 @pytest.mark.parametrize("env,fam", FT)
@@ -409,7 +382,7 @@ def test_train_update_vs_fp64_learner(monkeypatch, env, fam, activation, switch)
     perms = [c.train_get_permutation(e) for e in range(epochs)]
     got = c.get_tensor("params")
     c.close()
-    p64, want = learner_ref(flat, bufs, perms, nmb, 3.9e-4, 0.2, activation, h, h)
+    p64, want = learner_ref(flat, bufs, perms, nmb, 3.9e-4, 0.2, partial(loss_grad_ref, activation=activation, h1=h, h2=h))
     _, P, _ = layout(h, h)
     moved = np.abs(p64[:P] - flat[:P]).max()
     assert np.abs(got[:P] - p64[:P]).max() < max(5e-4, 4e-5 * epochs * nmb) * moved

@@ -5,9 +5,10 @@ The reference for the losses is an independent fp64 PyTorch autograd restatement
 TensorFlow's tie rules written out (Maximum's gradient goes to its first operand on >=, clip_by_value passes it on
 -b <= x <= b; torch.maximum would split a tie 0.5 / 0.5).  CPU tests: the reference and its tie fixture, and the two graph
 readers.  GPU tests: every kernel family, whole updates, schedules replaying the captured graphs, the host C++ PPO2.
-(A two-GPU SEPARATE update is not covered here.)"""
+test_multi_gpu_parity.py runs the same learner on sharded multi-GPU updates."""
 import os
 import subprocess
+from functools import partial
 
 import numpy as np
 import pytest
@@ -38,6 +39,16 @@ def _tf_clip(x, lo, hi):
     return torch.where(t >= lo, t, lo)
 
 
+def _act(name, mask="gt"):
+    """The hidden-layer activation; ReLU's gradient masks on output > 0 (TensorFlow's ReluGrad, mask="gt") or, to show that a
+    fixture tells the two apart, on input >= 0 (mask="ge": a unit at exactly 0 passes it)."""
+    if name == "tanh":
+        return torch.tanh
+    if mask == "gt":
+        return torch.relu
+    return lambda z: torch.where(z >= 0, z, torch.zeros_like(z))
+
+
 def value_loss(v, old_v, R, mode, cr, cr_vf, tie="tf"):
     """Per-sample max(l1, l2) of Stable-Baselines' ppo2.py for ppo_vf_clip `mode`; tie="split" gives torch's own
     0.5 / 0.5 rule (used only to show that a fixture tells the two apart)."""
@@ -52,17 +63,19 @@ def value_loss(v, old_v, R, mode, cr, cr_vf, tie="tf"):
 
 
 def loss_grad_ref(params, obs, act, adv, ret, old_nlp, old_v, cr, mode="shared", cr_vf=0.0, h1=4, h2=5,
-                  ent_coef=0.0007160293171182275, vf_coef=0.5, tie="tf"):
-    """fp64 loss + gradient of the 13 trainable tensors (graph gradient order) and the five reported losses."""
-    lay, P = _layout(h1, h2)
+                  ent_coef=0.0007160293171182275, vf_coef=0.5, tie="tf", activation="tanh", mask="gt"):
+    """fp64 loss + gradient of the 13 trainable tensors (graph gradient order) and the five reported losses of a Gaussian
+    policy; the observation and action widths are those of obs and act."""
+    lay, P = _layout(h1, h2, np.shape(obs)[1], np.shape(act)[1])
     p = torch.tensor(np.asarray(params[:P], np.float64), requires_grad=True)
     T = [p[o:o + int(np.prod(s))].reshape(s) for o, s in lay]
     pi0w, pi0b, vf0w, vf0b, pi1w, pi1b, vf1w, vf1b, vfw, vfb, piw, pib, logstd = T
+    f = _act(activation, mask)
     x = torch.tensor(np.asarray(obs, np.float64))
     a = torch.tensor(np.asarray(act, np.float64))
     adv, R, onl, ov = (torch.tensor(np.asarray(z, np.float64).ravel()) for z in (adv, ret, old_nlp, old_v))
-    mu = torch.tanh(torch.tanh(x @ pi0w + pi0b) @ pi1w + pi1b) @ piw + pib
-    v = (torch.tanh(torch.tanh(x @ vf0w + vf0b) @ vf1w + vf1b) @ vfw + vfb)[:, 0]
+    mu = f(f(x @ pi0w + pi0b) @ pi1w + pi1b) @ piw + pib
+    v = (f(f(x @ vf0w + vf0b) @ vf1w + vf1b) @ vfw + vfb)[:, 0]
     ls = logstd.reshape(-1)
     nlp = 0.5 * (((a - mu) / torch.exp(ls)) ** 2).sum(1) + HALF_LOG_2PI * a.shape[1] + ls.sum()
     ratio = torch.exp(onl - nlp)
@@ -301,35 +314,42 @@ def test_separate_mode_needs_cliprange_vf():
 
 
 # ------------------------------------------------------------------ GPU: whole updates against an fp64 learner
-def learner_ref(flat, bufs, perms, nmb, lr, cr, mode, cr_vf, h1, h2, ent_coef, vf_coef=0.5, clip=0.5, b1=0.9, b2=0.999, eps=1e-5):
+def learner_ref(flat, bufs, perms, nmb, lr, cr, loss_grad, clip=0.5, b1=0.9, b2=0.999, eps=1e-5, state=None, ks=None):
     """PPO2::learn's epoch / minibatch loop (ppo2.hpp:264-335) on one rollout in fp64: per-minibatch advantage
-    normalisation, loss gradient, clip_by_global_norm and TF's ApplyAdam, on the core's own permutations."""
-    _, P = _layout(h1, h2)
+    normalisation, loss gradient, clip_by_global_norm and TF's ApplyAdam, on the core's own permutations.
+
+    loss_grad(params, obs, actions, advs, returns, old_neglogp, old_values, cliprange) -> (gradient of the trainable
+    parameters, five losses) is loss_grad_ref, or test_discrete's for a categorical head, bound to the net with
+    functools.partial.  state: the Adam moments and beta powers {"m", "v", "b1p", "b2p"} to start from (absent: zero
+    moments and powers b1, b2, a fresh core), updated in place, so that a chain of calls is a chain of updates.  ks: the
+    minibatches of each epoch to run (all of them by default; a train_minibatch call is one)."""
+    st = {} if state is None else state
     p = flat.astype(np.float64).copy()
-    m = np.zeros(P)
-    v = np.zeros(P)
-    b1p, b2p = b1, b2
+    m, v = st.get("m"), st.get("v")
+    b1p, b2p = st.get("b1p", b1), st.get("b2p", b2)
     nb = bufs["obs"].shape[0]
     Bm = nb // nmb
     rows = []
     for perm in perms:
         src = np.empty_like(perm)
         src[perm] = np.arange(nb)  # Eigen's perm * buf writes row i to slot perm[i] (ppo2.hpp:291-296)
-        for k in range(nmb):
+        for k in (range(nmb) if ks is None else ks):
             idx = src[k * Bm:(k + 1) * Bm]
             ret, val = bufs["returns"][idx, 0], bufs["values"][idx, 0]
             a = ret.astype(np.float64) - val
             adv = (a - a.mean()) / (np.sqrt(((a - a.mean()) ** 2).mean()) + 1e-8)
-            g, l = loss_grad_ref(p, bufs["obs"][idx], bufs["actions"][idx], adv, ret, bufs["neglogpacs"][idx, 0], val, cr, mode, cr_vf,
-                                 h1=h1, h2=h2, ent_coef=ent_coef, vf_coef=vf_coef)
+            g, l = loss_grad(p, bufs["obs"][idx], bufs["actions"][idx], adv, ret, bufs["neglogpacs"][idx, 0], val, cr)
             rows.append(l)
+            if m is None:
+                m, v = np.zeros_like(g), np.zeros_like(g)
             gn = np.sqrt((g * g).sum())
             g = g * clip * min(1.0 / gn, 1.0 / clip)
             m += (g - m) * (1 - b1)
             v += (g * g - v) * (1 - b2)
-            p[:P] -= lr * np.sqrt(1 - b2p) / (1 - b1p) * m / (np.sqrt(v) + eps)
+            p[:g.size] -= lr * np.sqrt(1 - b2p) / (1 - b1p) * m / (np.sqrt(v) + eps)
             b1p *= b1
             b2p *= b2
+    st.update(m=m, v=v, b1p=b1p, b2p=b2p)
     return p, np.mean(rows, axis=0)
 
 
@@ -361,7 +381,7 @@ def test_train_update_vf_vs_fp64_learner(mode, h1, h2, n_envs, n_steps, nmb, epo
     perms = [c.train_get_permutation(e) for e in range(epochs)]
     got = c.get_tensor("params")
     c.close()
-    p64, want = learner_ref(flat, bufs, perms, nmb, 3.9e-4, 0.2, mode, 0.1, h1, h2, ent)
+    p64, want = learner_ref(flat, bufs, perms, nmb, 3.9e-4, 0.2, partial(loss_grad_ref, mode=mode, cr_vf=0.1, h1=h1, h2=h2, ent_coef=ent))
     _, P = _layout(h1, h2)
     moved = np.abs(p64[:P] - flat[:P]).max()
     print(f"{mode} [{h1},{h2}] on {fam_name}: param diff / moved = {np.abs(got[:P] - p64[:P]).max() / moved:.3e}")
