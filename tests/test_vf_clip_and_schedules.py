@@ -410,25 +410,36 @@ def _schedule_run(core_mod, monkeypatch, env, h, n_envs, n_steps, nmb, epochs, m
         losses.append(c.train_update(3e-4 * frac, 0.2 * frac + 0.05, cliprange_vf=0.3 * frac))
         builds.append(c.graph_builds())
     params = c.get_tensor("params")
+    ctr, rollout = c.counters(), c.kernel_family("rollout")
     c.close()
-    return np.array(losses), params, builds
+    return np.array(losses), params, builds, ctr, rollout
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("shuffle", ["gpu", "host"])
-@pytest.mark.parametrize("h,n_envs,n_steps,nmb,epochs,mode", [(64, 256, 32, 4, 2, "separate"), (4, 8, 64, 4, 2, "none"),
-                                                              (256, 64, 32, 2, 2, "separate")])
-def test_annealed_updates_replay_graphs_and_equal_eager(monkeypatch, shuffle, h, n_envs, n_steps, nmb, epochs, mode):
+@pytest.mark.parametrize("h,n_envs,n_steps,nmb,epochs,mode,env", [
+    pytest.param(64, 256, 32, 4, 2, "separate", [], id="64-256-32-4-2-separate"),
+    pytest.param(4, 8, 64, 4, 2, "none", [], id="4-8-64-4-2-none"),
+    pytest.param(256, 64, 32, 2, 2, "separate", [], id="256-64-32-2-2-separate"),
+    # U per minibatch (train_step_device) and the per-step rollout, captured as one graph
+    pytest.param(64, 256, 32, 4, 2, "separate", ["PPO_DISABLE_PERSISTENT"], id="64-256-32-4-2-separate-PPO_DISABLE_PERSISTENT")])
+def test_annealed_updates_replay_graphs_and_equal_eager(monkeypatch, shuffle, h, n_envs, n_steps, nmb, epochs, mode, env):
     """lr, cliprange and cliprange_vf change every update: the captured graphs are replayed, not rebuilt (the graph count
-    stays at its value after the first update), and the run equals the same launches made without graphs bit for bit."""
+    stays at its value after the first update), and the run equals the same launches made without graphs bit for bit.
+    A replayed graph counts the kernels and copies it holds, so both runs report the same work."""
     from ppo_cpp_b200 import core as core_mod
-    base = ["PPO_DISABLE_GPU_SHUFFLE"] if shuffle == "host" else []
-    l_g, p_g, builds = _schedule_run(core_mod, monkeypatch, base, h, n_envs, n_steps, nmb, epochs, mode)
-    l_e, p_e, builds_e = _schedule_run(core_mod, monkeypatch, base + ["PPO_DISABLE_GRAPH"], h, n_envs, n_steps, nmb, epochs, mode)
+    base = env + (["PPO_DISABLE_GPU_SHUFFLE"] if shuffle == "host" else [])
+    l_g, p_g, builds, ctr_g, rollout = _schedule_run(core_mod, monkeypatch, base, h, n_envs, n_steps, nmb, epochs, mode)
+    l_e, p_e, builds_e, ctr_e, _ = _schedule_run(core_mod, monkeypatch, base + ["PPO_DISABLE_GRAPH"], h, n_envs, n_steps, nmb, epochs, mode)
     assert builds[0] > 0 and builds == [builds[0]] * len(builds), builds
     assert builds_e == [0] * len(builds_e)
     assert np.all(np.isfinite(l_g))
     assert np.array_equal(l_g, l_e) and np.array_equal(p_g, p_e)
+    assert ctr_g["graph_launches"] > 0 and ctr_e["graph_launches"] == 0
+    for k in ("kernel_launches", "h2d_bytes", "d2h_bytes"):
+        assert ctr_g[k] == ctr_e[k], (k, ctr_g, ctr_e)
+    # the synthetic rollout is captured as a graph only where it runs as per-step kernels
+    assert (rollout == "per-step kernels") == (h == 256 or "PPO_DISABLE_PERSISTENT" in env), rollout
 
 
 # ------------------------------------------------------------------ GPU: the host C++ PPO2 and its CLI
