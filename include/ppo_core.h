@@ -111,21 +111,42 @@ int ppo_meta_activation(const char *meta_txt_path);
  *   DISCRETE  CategoricalProbabilityDistribution over act_dim = n logits (model/pi, no logstd): an action is ONE index
  *             0 .. n-1, stored as fp32 wherever actions are passed (action width 1); it is sampled as
  *             argmax_j (l_j - log(-log(u_j))) with u uniform in [0, 1), and ppo_policy_step's eps holds those n uniforms per env.
- *             ppo_meta_parse counts 14 tensors (no logstd); checkpoints hold them in sorted-name order.
- *             The S / U / W kernel families, the persistent rollout and the synthetic env are continuous-only: a DISCRETE core
- *             runs the F or T family, and the synthetic-env entry points return PPO_ERR_UNSUPPORTED. */
-typedef enum { PPO_ACTION_BOX = 0, PPO_ACTION_DISCRETE = 1 } ppo_action_space;
-/* the ppo_action_space of a graph file: BOX with model/pi/logstd, DISCRETE without it.  When the file has PPO2's placeholder
- * loss/action_ph it must agree (float [?, n] for BOX, int32 / int64 [?] for DISCRETE), otherwise PPO_ERR_UNSUPPORTED naming the
- * node; ppo_meta_parse fails the same way. */
+ *   MULTI_DISCRETE  MultiCategoricalProbabilityDistribution: k categoricals side by side over slices of act_dim = sum(nvec)
+ *             logits (nvec[i] logits each, in order); an action is k indices (action width k, column i in 0 .. nvec[i]-1),
+ *             each sampled as DISCRETE samples its slice from the uniforms of the flat logit index, so MultiDiscrete([n]) draws
+ *             what Discrete(n) draws; neglogp and entropy are the sums over the slices.
+ *   MULTI_BINARY    BernoulliProbabilityDistribution over act_dim = n logits: an action is n columns of 0 / 1, sampled as
+ *             [u_j < sigmoid(l_j)] (eps: n uniforms per env); neglogp = sum_j sigmoid_cross_entropy_with_logits(l_j, x_j),
+ *             entropy = sum_j sigmoid_cross_entropy_with_logits(l_j, sigmoid(l_j)) with its gradient through sigmoid(l_j);
+ *             the deterministic action is round(sigmoid(l)) with ties to even (l = 0 gives 0).
+ *             An action column outside its choices (or not an integer) is PPO_ERR_INVALID in ppo_rollout_set and ppo_loss_grad.
+ *             Every head but BOX has no logstd: ppo_meta_parse counts 14 tensors; checkpoints hold them in sorted-name order.
+ *             The S / U / W kernel families, the persistent rollout and the synthetic env are continuous-only: a core with
+ *             another head runs the F or T family, and the synthetic-env entry points return PPO_ERR_UNSUPPORTED. */
+typedef enum { PPO_ACTION_BOX = 0, PPO_ACTION_DISCRETE = 1, PPO_ACTION_MULTI_DISCRETE = 2, PPO_ACTION_MULTI_BINARY = 3 } ppo_action_space;
+/* the ppo_action_space of a graph file: BOX with model/pi/logstd; without it DISCRETE, unless PPO2's placeholder loss/action_ph is
+ * int32 / int64 [?, k]: then MULTI_DISCRETE when a SplitV under model/ reads the pi head's output (the Add / BiasAdd over
+ * model/pi/b) with k size_splits summing to the pi width; without such a SplitV, MULTI_BINARY when a Sigmoid under model/ reads the
+ * pi head's output (Bernoulli's tf.sigmoid of the logits) and k is the pi width.  An int [?, k] placeholder with neither op is
+ * refused, so a Discrete graph with a rank-2 placeholder is not read as MultiBinary.  When the file has loss/action_ph it must
+ * agree (float [?, n] for BOX, int32 / int64 [?] for DISCRETE), otherwise PPO_ERR_UNSUPPORTED naming the node; ppo_meta_parse
+ * fails the same way. */
 int ppo_meta_action_space(const char *meta_txt_path);
+/* the choices per action column of a graph file's head: {n} (DISCRETE), nvec (MULTI_DISCRETE), 2s (MULTI_BINARY); returns the
+ * action width (nvec may be NULL to ask for it alone) or a negative ppo_status: PPO_ERR_INVALID for BOX or a capacity below the width */
+int ppo_meta_action_nvec(const char *meta_txt_path, int *nvec, int capacity);
 
 int ppo_core_create(const ppo_core_desc *desc, ppo_core **out); /* ppo_core_create_ex(desc, PPO_ACTION_BOX, out) */
-/* a core whose policy head is of the given ppo_action_space (fixed for the core's lifetime) */
+/* a core whose policy head is of the given ppo_action_space (fixed for the core's lifetime); MULTI_DISCRETE is PPO_ERR_INVALID
+ * here (it needs an nvec: ppo_core_create_nvec) */
 int ppo_core_create_ex(const ppo_core_desc *desc, int action_space, ppo_core **out);
+/* a MULTI_DISCRETE core with k action columns of nvec[i] >= 1 choices: sum(nvec) == desc->act_dim <= 64, k <= 64 */
+int ppo_core_create_nvec(const ppo_core_desc *desc, const int *nvec, int k, ppo_core **out);
 int ppo_core_action_space(ppo_core *core); /* the core's ppo_action_space, or a negative ppo_status */
+/* the core's choices per action column, as ppo_meta_action_nvec; returns the action width */
+int ppo_core_action_nvec(ppo_core *core, int *nvec, int capacity);
 void ppo_core_destroy(ppo_core *core);
-/* load initial weights from the graph file; its shapes and its ppo_action_space must match the core's (ppo2.hpp:90-105 reset());
+/* load initial weights from the graph file; its shapes and its ppo_action_space (and nvec) must match the core's (ppo2.hpp:90-105 reset());
  * sets the core's ppo_vf_clip and ppo_activation */
 int ppo_core_load_meta_txt(ppo_core *core, const char *meta_txt_path);
 /* the value loss of a graph-less core (default SHARED); ppo_core_load_meta_txt sets it from the graph */
@@ -146,7 +167,8 @@ int ppo_core_save_checkpoint_data(ppo_core *core, const char *prefix);
 /* the `.index` alone, for a `.data` payload held by the caller (the 15 tensors of an MLP [hidden1, hidden2] policy in ascending name
  * order, n_floats values); no device needed.  Byte-identical to TensorFlow 1.14's BundleWriter on the reference's shipped checkpoint. */
 int ppo_checkpoint_write_index(const char *prefix, int obs_dim, int act_dim, int hidden1, int hidden2, const float *data, size_t n_floats);
-/* ... for either head: PPO_ACTION_DISCRETE leaves model/pi/logstd out (14 tensors) */
+/* ... for either layout: PPO_ACTION_DISCRETE leaves model/pi/logstd out (14 tensors), the layout of every head but BOX, which
+ * ppo_core_save_checkpoint_data writes for MULTI_DISCRETE and MULTI_BINARY cores too; other values are PPO_ERR_INVALID */
 int ppo_checkpoint_write_index_ex(const char *prefix, int action_space, int obs_dim, int act_dim, int hidden1, int hidden2,
                                   const float *data, size_t n_floats);
 

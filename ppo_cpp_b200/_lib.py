@@ -18,7 +18,7 @@ HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "ppo_core.h")
 PPO_HOST, PPO_DEVICE = 0, 1
 PPO_VF_CLIP_SHARED, PPO_VF_CLIP_NONE, PPO_VF_CLIP_SEPARATE = 0, 1, 2
 PPO_ACT_TANH, PPO_ACT_RELU = 0, 1
-PPO_ACTION_BOX, PPO_ACTION_DISCRETE = 0, 1
+PPO_ACTION_BOX, PPO_ACTION_DISCRETE, PPO_ACTION_MULTI_DISCRETE, PPO_ACTION_MULTI_BINARY = 0, 1, 2, 3
 PPO_COMM_ID_BYTES = 128
 PPO_IPC_HANDLE_BYTES = 64
 ABI_VERSION = 1
@@ -81,9 +81,12 @@ def load():
         "ppo_meta_vf_clip": ([C.c_char_p], C.c_int),
         "ppo_meta_activation": ([C.c_char_p], C.c_int),
         "ppo_meta_action_space": ([C.c_char_p], C.c_int),
+        "ppo_meta_action_nvec": ([C.c_char_p, ip, C.c_int], C.c_int),
         "ppo_core_create": ([C.POINTER(CoreDesc), C.POINTER(core)], C.c_int),
         "ppo_core_create_ex": ([C.POINTER(CoreDesc), C.c_int, C.POINTER(core)], C.c_int),
+        "ppo_core_create_nvec": ([C.POINTER(CoreDesc), ip, C.c_int, C.POINTER(core)], C.c_int),
         "ppo_core_action_space": ([core], C.c_int),
+        "ppo_core_action_nvec": ([core, ip, C.c_int], C.c_int),
         "ppo_core_destroy": ([core], None),
         "ppo_core_load_meta_txt": ([core, C.c_char_p], C.c_int),
         "ppo_core_set_vf_clip": ([core, C.c_int], C.c_int),

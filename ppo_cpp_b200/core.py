@@ -22,7 +22,8 @@ VF_CLIP_NAMES = {v: k for k, v in VF_CLIP_MODES.items()}
 ACTIVATIONS = {"tanh": _lib.PPO_ACT_TANH, "relu": _lib.PPO_ACT_RELU}
 ACTIVATION_NAMES = {v: k for k, v in ACTIVATIONS.items()}
 # the policy heads of ppo_action_space, by the names write_meta_txt(action_space=...) takes
-ACTION_SPACES = {"box": _lib.PPO_ACTION_BOX, "discrete": _lib.PPO_ACTION_DISCRETE}
+ACTION_SPACES = {"box": _lib.PPO_ACTION_BOX, "discrete": _lib.PPO_ACTION_DISCRETE, "multi_discrete": _lib.PPO_ACTION_MULTI_DISCRETE,
+                 "multi_binary": _lib.PPO_ACTION_MULTI_BINARY}
 ACTION_SPACE_NAMES = {v: k for k, v in ACTION_SPACES.items()}
 BUFFER_WIDTH = {"obs": None, "returns": 1, "dones": 1, "actions": None, "values": 1, "neglogpacs": 1,
                 "true_rewards": 1, "unnormalized_rewards": 1}
@@ -90,6 +91,25 @@ def meta_action_space(path: str) -> str:
     return ACTION_SPACE_NAMES[r]
 
 
+def _nvec(fn, *args) -> list:
+    n = fn(*args, None, 0)
+    if n < 0:
+        return n
+    out = np.zeros(n, np.int32)
+    r = fn(*args, out.ctypes.data, n)
+    return r if r < 0 else [int(x) for x in out]
+
+
+def meta_action_nvec(path: str) -> list:
+    """The choices per action column of the graph file's head (read by the C parser): [n] for "discrete", nvec for "multi_discrete",
+    2s for "multi_binary"; PPOError for "box"."""
+    lib = _lib.load()
+    r = _nvec(lib.ppo_meta_action_nvec, path.encode())
+    if isinstance(r, int):
+        _check(lib, r)
+    return r
+
+
 def host_rand(seed: int, count: int) -> np.ndarray:
     lib = _lib.load()
     out = np.zeros(count, np.int32)
@@ -112,12 +132,16 @@ def comm_unique_id() -> bytes:
 
 
 class PPOCore:
-    def __init__(self, activation: str = "tanh", action_space: str = "box", **kw):
+    def __init__(self, activation: str = "tanh", action_space: str = "box", nvec=None, **kw):
         self.lib = _lib.load()
         if activation not in ACTIVATIONS:
             raise ValueError(f"activation must be one of {sorted(ACTIVATIONS)}, not {activation!r}")
         if action_space not in ACTION_SPACES:
             raise ValueError(f"action_space must be one of {sorted(ACTION_SPACES)}, not {action_space!r}")
+        if (action_space == "multi_discrete") != (nvec is not None):
+            raise ValueError("nvec goes with action_space='multi_discrete' (and only with it)")
+        if nvec is not None:
+            kw.setdefault("act_dim", int(sum(nvec)))  # the logits of the k slices
         d = CoreDesc()
         _check(self.lib, self.lib.ppo_core_desc_default(C.byref(d)))
         for k, v in kw.items():
@@ -128,11 +152,15 @@ class PPOCore:
         self._h = C.c_void_p()
         if action_space == "box":
             _check(self.lib, self.lib.ppo_core_create(C.byref(d), C.byref(self._h)))
+        elif nvec is not None:
+            nv = np.ascontiguousarray(nvec, np.int32)
+            _check(self.lib, self.lib.ppo_core_create_nvec(C.byref(d), nv.ctypes.data, nv.size, C.byref(self._h)))
         else:
             _check(self.lib, self.lib.ppo_core_create_ex(C.byref(d), ACTION_SPACES[action_space], C.byref(self._h)))
         self.O, self.A = d.obs_dim, d.act_dim
-        # floats of one stored action: the action vector (Box), or the index of a categorical head (Discrete)
-        self.AW = 1 if action_space == "discrete" else d.act_dim
+        # floats of one stored action: the action vector (Box), the index of a categorical head (Discrete), one index per slice
+        # (MultiDiscrete), one bit per logit (MultiBinary)
+        self.AW = d.act_dim if action_space == "box" else len(self.nvec)
         self.n_envs, self.n_steps = d.n_envs, d.n_steps
         self.n_batch = d.n_envs * d.n_steps
         self.n_batch_global = self.n_batch * max(1, d.world_size)
@@ -186,11 +214,20 @@ class PPOCore:
 
     @property
     def action_space(self) -> str:
-        """The core's policy head: "box" (Gaussian) or "discrete" (categorical over act_dim logits)."""
+        """The core's policy head: "box" (Gaussian), "discrete" (categorical over act_dim logits), "multi_discrete" (one categorical
+        per slice of the logits) or "multi_binary" (a Bernoulli per logit)."""
         r = self.lib.ppo_core_action_space(self._h)
         if r < 0:
             _check(self.lib, r)
         return ACTION_SPACE_NAMES[r]
+
+    @property
+    def nvec(self) -> list:
+        """The choices per action column: [act_dim] (discrete), nvec (multi_discrete), 2s (multi_binary); PPOError for a Box core."""
+        r = _nvec(self.lib.ppo_core_action_nvec, self._h)
+        if isinstance(r, int):
+            _check(self.lib, r)
+        return r
 
     def graph_builds(self) -> int:
         """CUDA graphs captured and instantiated since the core was created."""

@@ -11,18 +11,19 @@ enum TensorId {
     T_VF_W, T_VF_B, T_PI_W, T_PI_B, T_LOGSTD, T_Q_W, T_Q_B, T_COUNT
 };
 
-// Policy head (ppo_action_space in ppo_core.h): Box -> diagonal Gaussian with model/pi/logstd, Discrete(A) -> categorical over
-// A logits.  Uniform per core, a template parameter of the kernels that evaluate it.
-enum { HEAD_BOX = 0, HEAD_DISCRETE = 1 };
+// Policy head (ppo_action_space in ppo_core.h, same values): Box -> diagonal Gaussian with model/pi/logstd, Discrete(A) ->
+// categorical over A logits, MultiDiscrete(nvec) -> k categoricals over slices of the A = sum(nvec) logits, MultiBinary(A) -> A
+// Bernoullis.  Uniform per core, a template parameter of the kernels that evaluate it.
+enum { HEAD_BOX = 0, HEAD_DISCRETE = 1, HEAD_MULTI_DISCRETE = 2, HEAD_MULTI_BINARY = 3 };
 
 struct NetDims {
     int O, A, H1, H2;      // A: width of the policy output (action dimensions, or logits of a categorical head)
     int off[T_COUNT + 1];  // off[T_Q_W] = P (trainable), off[T_COUNT] = total
     int P, Pq;
-    // a categorical head has no logstd: T_LOGSTD has size 0, every other offset stays in graph gradient order
+    // only a Gaussian head has a logstd: otherwise T_LOGSTD has size 0, every other offset stays in graph gradient order
     __host__ void init(int o, int a, int h1, int h2, int head = HEAD_BOX) {
         O = o; A = a; H1 = h1; H2 = h2;
-        const int ls = head == HEAD_DISCRETE ? 0 : A;
+        const int ls = head == HEAD_BOX ? A : 0;
         const int sz[T_COUNT] = {O * H1, H1, O * H1, H1, H1 * H2, H2, H1 * H2, H2, H2, 1, H2 * A, A, ls, H2 * A, A};
         off[0] = 0;
         for (int i = 0; i < T_COUNT; ++i) off[i + 1] = off[i] + sz[i];
@@ -127,6 +128,7 @@ __device__ __forceinline__ float box_entropy(LS logstd, int A) {
 
 #define PPO_TAG_ACTION 0x50504F32u    // "PPO2": action noise stream
 #define PPO_TAG_CATEG 0x43415431u     // "CAT1": uniforms of the categorical head's Gumbel-max sample
+#define PPO_TAG_BERN 0x42455231u      // "BER1": uniforms of the Bernoulli head's sample
 #define PPO_TAG_ENVNOISE 0x454E5631u  // "ENV1": synthetic env process noise
 #define PPO_TAG_ENVRESET 0x52535431u  // "RST1": synthetic env reset state
 
@@ -246,6 +248,111 @@ __device__ __forceinline__ PgTerm cat_train_term(float* l, int ld, int n, int a,
     H = cat_entropy(l, ld, n, mx, z);
     const PgTerm t = pg_term(adv, oldn, nlp, cr, invB);
     cat_dlogits(l, ld, n, a, mx, z, H, t.g_nlp, ent_w);
+    return t;
+}
+
+// ---- MultiDiscrete head (MultiCategoricalProbabilityDistribution): k categoricals side by side over slices of the n <= 64
+// logits, given as a mask of slice starts (bit j set: a slice starts at logit j; bit 0 always set, k = popcount); an action is
+// one index per slice, within the slice.  The categorical helpers above, per slice.
+// end of the slice that starts at s0: the next start, or n
+__device__ __forceinline__ int md_slice_end(uint64_t starts, int s0, int n) {
+    const uint64_t rest = s0 >= 63 ? 0ull : starts & (~0ull << (s0 + 1));
+    return rest ? __ffsll((long long)rest) - 1 : n;
+}
+// sample: Gumbel-max per slice over the uniforms of the flat logit index (the categorical stream, so MultiDiscrete([n]) draws
+// what Discrete(n) draws); put(i, index) receives slice i's index once the slice is finished
+template <class PUT>
+__device__ __forceinline__ void md_sample(const float* l, int ld, int n, uint64_t starts, const float* u_given, uint64_t seed, uint32_t env,
+                                          uint32_t step, PUT put) {
+    float best = -__int_as_float(0x7f800000);
+    int i = 0, s0 = 0, bi = 0;
+    for (int j0 = 0; j0 < n; j0 += 4) {
+        uint4 w = make_uint4(0u, 0u, 0u, 0u);
+        if (!u_given) w = philox4x32_10(make_uint4(env, step, (uint32_t)(j0 >> 2), PPO_TAG_CATEG), make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+        const uint32_t wv[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const int j = j0 + q;
+            if (j < n) {
+                if (j > 0 && ((starts >> j) & 1ull)) {  // slice i done; ties stayed on its first index
+                    put(i++, bi - s0);
+                    s0 = bi = j;
+                    best = -__int_as_float(0x7f800000);
+                }
+                const float u = u_given ? u_given[j] : u32_to_unit(wv[q]);
+                const float g = l[j * ld] - logf(-logf(u));
+                if (g > best) { best = g; bi = j; }
+            }
+        }
+    }
+    put(i, bi - s0);
+}
+// one sample's MultiDiscrete train terms: neglogp = sum_i neglogp_i(a_i) (TF's add_n in slice order), H = sum_i H_i, the
+// clipped surrogate of pg_term, and the logits overwritten with dL/dl: slice i as cat_dlogits with its own entropy H_i.
+// act[i * ald]: slice i's index
+__device__ __forceinline__ PgTerm md_train_term(float* l, int ld, int n, uint64_t starts, const float* act, int ald, float adv, float oldn,
+                                                float cr, float invB, float ent_w, float& H) {
+    float nlp = 0.f;
+    H = 0.f;
+    for (int i = 0, s0 = 0; s0 < n; ++i) {
+        const int s1 = md_slice_end(starts, s0, n);
+        const float* s = l + s0 * ld;
+        float mx;
+        const float z = cat_partition(s, ld, s1 - s0, mx);
+        nlp += logf(z) - (s[(int)act[i * ald] * ld] - mx);
+        H += cat_entropy(s, ld, s1 - s0, mx, z);
+        s0 = s1;
+    }
+    const PgTerm t = pg_term(adv, oldn, nlp, cr, invB);
+    for (int i = 0, s0 = 0; s0 < n; ++i) {
+        const int s1 = md_slice_end(starts, s0, n);
+        float* s = l + s0 * ld;
+        float mx;
+        const float z = cat_partition(s, ld, s1 - s0, mx);
+        cat_dlogits(s, ld, s1 - s0, (int)act[i * ald], mx, z, cat_entropy(s, ld, s1 - s0, mx, z), t.g_nlp, ent_w);
+        s0 = s1;
+    }
+    return t;
+}
+
+// ---- MultiBinary head (BernoulliProbabilityDistribution) of one sample: logits l[j * ld], j < n, an action of n columns 0 / 1
+__device__ __forceinline__ float bern_sigmoid(float l) { return 1.f / (1.f + expf(-l)); }
+// TF's sigmoid_cross_entropy_with_logits: sce(l, z) = max(l, 0) - l z + log1p(exp(-|l|))
+__device__ __forceinline__ float bern_sce(float l, float z) { return fmaxf(l, 0.f) - l * z + log1pf(expf(-fabsf(l))); }
+// sample x_j = [u_j < sigmoid(l_j)], u uniform in [0, 1) from stream (seed, env, step, block j/4, PPO_TAG_BERN) or given;
+// put(j, x_j)
+template <class PUT>
+__device__ __forceinline__ void bern_sample(const float* l, int ld, int n, const float* u_given, uint64_t seed, uint32_t env, uint32_t step, PUT put) {
+    for (int j0 = 0; j0 < n; j0 += 4) {
+        uint4 w = make_uint4(0u, 0u, 0u, 0u);
+        if (!u_given) w = philox4x32_10(make_uint4(env, step, (uint32_t)(j0 >> 2), PPO_TAG_BERN), make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+        const uint32_t wv[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const int j = j0 + q;
+            if (j < n) put(j, (u_given ? u_given[j] : u32_to_unit(wv[q])) < bern_sigmoid(l[j * ld]) ? 1.f : 0.f);
+        }
+    }
+}
+// neglogp(x) = sum_j sce(l_j, x_j); x[j * xld]
+__device__ __forceinline__ float bern_neglogp(const float* l, int ld, int n, const float* x, int xld) {
+    float s = 0.f;
+    for (int j = 0; j < n; ++j) s += bern_sce(l[j * ld], x[j * xld]);
+    return s;
+}
+// one sample's MultiBinary train terms: neglogp(x), the entropy H = sum_j sce(l_j, sigmoid(l_j)), the clipped surrogate of
+// pg_term, and the logits overwritten with dL/dl_j = g_nlp (s_j - x_j) + ent_w l_j s_j (1 - s_j), s = sigmoid(l): Stable-Baselines
+// does not stop the gradient through the entropy's labels, so dH/dl = -l s (1 - s)
+__device__ __forceinline__ PgTerm bern_train_term(float* l, int ld, int n, const float* x, int xld, float adv, float oldn, float cr,
+                                                  float invB, float ent_w, float& H) {
+    const float nlp = bern_neglogp(l, ld, n, x, xld);
+    H = 0.f;
+    for (int j = 0; j < n; ++j) H += bern_sce(l[j * ld], bern_sigmoid(l[j * ld]));
+    const PgTerm t = pg_term(adv, oldn, nlp, cr, invB);
+    for (int j = 0; j < n; ++j) {
+        const float v = l[j * ld], s = bern_sigmoid(v);
+        l[j * ld] = t.g_nlp * (s - x[j * xld]) + ent_w * v * s * (1.f - s);
+    }
     return t;
 }
 

@@ -207,9 +207,11 @@ struct PolicyArgs {
     const float* params;
     const float* obs;  // [n][O] (already normalised)
     int n;
+    uint32_t md_lo;    // MultiDiscrete head: slice-start mask (md_sample), bits 0-31 here and 32-63 in md_hi, both in padding
     const float* eps;  // optional [n][A]; when NULL Philox noise for (seed, env_id0+i, *step_ctr)
     uint64_t seed;
     uint32_t env_id0;
+    uint32_t md_hi;
     const uint32_t* step_ctr;
     float* action;   // [n][A] or NULL
     float* value;    // [n] or NULL
@@ -223,6 +225,8 @@ struct PolicyArgs {
     float* dones_store;     // [n]
     int mode;  // 0: step (pi + V + sample), 1: value only, 2: mean only (deterministic action)
 };
+// the slice-start mask of a MultiDiscrete head from its two halves
+__host__ __device__ __forceinline__ uint64_t md_starts(uint32_t lo, uint32_t hi) { return ((uint64_t)hi << 32) | lo; }
 
 __device__ __forceinline__ void store_neglogp(const PolicyArgs& a, int row, float nl) {
     if (a.neglogp) a.neglogp[row] = nl;
@@ -267,6 +271,63 @@ __device__ __forceinline__ void cat_policy_row(const PolicyArgs& a, int row, con
     if (a.action) a.action[row] = (float)j;
     if (a.act_store) a.act_store[row] = (float)j;
     if (a.mode == 0) store_neglogp(a, row, cat_neglogp(l, ld, a.d.A, j));
+}
+
+// MultiDiscrete policy step: k indices in k columns, sampled per slice (mode 0, neglogp their sum) or argmax per slice (mode 2)
+__device__ __forceinline__ void md_policy_row(const PolicyArgs& a, int row, const float* l, int ld) {
+    const uint64_t starts = md_starts(a.md_lo, a.md_hi);
+    const int k = __popcll((long long)starts);
+    auto put = [&](int i, int j) {
+        if (a.action) a.action[(size_t)row * k + i] = (float)j;
+        if (a.act_store) a.act_store[(size_t)row * k + i] = (float)j;
+    };
+    if (a.mode == 0) {
+        float nlp = 0.f;
+        int s0 = 0;
+        md_sample(l, ld, a.d.A, starts, a.eps ? a.eps + (size_t)row * a.d.A : nullptr, a.seed, a.env_id0 + (uint32_t)row, a.eps ? 0u : *a.step_ctr,
+                  [&](int i, int j) {
+                      put(i, j);
+                      const int s1 = md_slice_end(starts, s0, a.d.A);
+                      nlp += cat_neglogp(l + s0 * ld, ld, s1 - s0, j);
+                      s0 = s1;
+                  });
+        store_neglogp(a, row, nlp);
+    } else {
+        for (int i = 0, s0 = 0; s0 < a.d.A; ++i) {
+            const int s1 = md_slice_end(starts, s0, a.d.A);
+            put(i, cat_argmax(l + s0 * ld, ld, s1 - s0));
+            s0 = s1;
+        }
+    }
+}
+
+// MultiBinary policy step: A columns of 0 / 1, sampled (mode 0, with neglogp) or round(sigmoid(l)) (mode 2; TF's Round is half to
+// even, so l = 0 gives 0)
+__device__ __forceinline__ void bern_policy_row(const PolicyArgs& a, int row, const float* l, int ld) {
+    const int n = a.d.A;
+    auto put = [&](int j, float x) {
+        if (a.action) a.action[(size_t)row * n + j] = x;
+        if (a.act_store) a.act_store[(size_t)row * n + j] = x;
+    };
+    if (a.mode == 0) {
+        float nlp = 0.f;
+        bern_sample(l, ld, n, a.eps ? a.eps + (size_t)row * n : nullptr, a.seed, a.env_id0 + (uint32_t)row, a.eps ? 0u : *a.step_ctr,
+                    [&](int j, float x) {
+                        put(j, x);
+                        nlp += bern_sce(l[j * ld], x);
+                    });
+        store_neglogp(a, row, nlp);
+    } else {
+        for (int j = 0; j < n; ++j) put(j, bern_sigmoid(l[j * ld]) > 0.5f ? 1.f : 0.f);
+    }
+}
+
+// the policy step of a head without logstd (modes 0 and 2), logits l[j * ld]; the actions go straight to their rows
+template <int HEAD>
+__device__ __forceinline__ void head_policy_row(const PolicyArgs& a, int row, const float* l, int ld) {
+    if constexpr (HEAD == HEAD_DISCRETE) cat_policy_row(a, row, l, ld);
+    else if constexpr (HEAD == HEAD_MULTI_DISCRETE) md_policy_row(a, row, l, ld);
+    else bern_policy_row(a, row, l, ld);
 }
 
 template <int TM>
@@ -319,8 +380,8 @@ __global__ void __launch_bounds__(NT) policy_tile_kernel(const PolicyArgs a) {
                 if (a.value) a.value[row] = v;
                 if (a.val_store) a.val_store[row] = v;
             }
-            if (HEAD == HEAD_DISCRETE && a.mode != 1) {
-                cat_policy_row(a, row, MU + m, TM);
+            if (HEAD != HEAD_BOX && a.mode != 1) {
+                head_policy_row<HEAD>(a, row, MU + m, TM);
             } else if (a.mode == 0) {
                 const float* logstd = p + d.off[T_LOGSTD];
                 gauss_policy_row(a, row, d.A, [&](int j) { return __ldg(logstd + j); }, [&](int j) { return MU[j * TM + m]; },
@@ -331,7 +392,7 @@ __global__ void __launch_bounds__(NT) policy_tile_kernel(const PolicyArgs a) {
             if (a.dones_store) a.dones_store[row] = a.dones_in[row];
         }
         __syncthreads();
-        if (HEAD == HEAD_BOX && a.mode != 1) {  // a categorical head stored its index above
+        if (HEAD == HEAD_BOX && a.mode != 1) {  // a head without logstd stored its actions above
             for (int e = tid; e < nv * d.A; e += NT) {
                 const int m = e / d.A, j = e - m * d.A;
                 const float act = Ac[j * (TM + 1) + m];
@@ -353,26 +414,47 @@ struct TrainArgs {
     const float* adv_direct;                    // already-normalised advantages per slot (ppo_loss_grad), or NULL
     int slot0, count;                           // this rank processes slots [slot0, slot0+count)
     float invB;                                 // 1 / (global minibatch size)
+    uint32_t md_lo;                             // MultiDiscrete head: slice-start mask (see PolicyArgs), in padding
     const UpdateScalars* sc;                    // cliprange, cliprange_vf of this update (device)
     int vf_mode;                                // VF_CLIP_*
     float ent_coef, vf_coef;
+    uint32_t md_hi;
     float* partial;  // [gridDim.x][PS]
     int PS;
     long long* prof;  // optional [2][32] phase timestamps of CTA 0 of each tower (U family, PPO_UMMA_PROF=1)
 };
+// the MultiDiscrete slice mask fills padding: every other field, and the parameters behind these structs, keep their offsets
+static_assert(sizeof(PolicyArgs) == 224 && sizeof(TrainArgs) == 224, "PolicyArgs / TrainArgs changed size");
+
+// floats of one stored action: the action vector (Box), the index of a categorical head, the k indices of a MultiDiscrete head,
+// the A bits of a MultiBinary head
+template <int HEAD>
+__device__ __forceinline__ int act_cols(const TrainArgs& a) {
+    return HEAD == HEAD_DISCRETE ? 1 : HEAD == HEAD_MULTI_DISCRETE ? __popcll((long long)md_starts(a.md_lo, a.md_hi)) : a.d.A;
+}
+
+// one sample's train terms of a head without logstd over n logits l[j * ld]: neglogp of the stored action (act[j * ald]) and
+// entropy H, the clipped surrogate of pg_term, and the logits overwritten with dL/dl (ent_w = ent_coef / B)
+template <int HEAD>
+__device__ __forceinline__ PgTerm head_train_term(const TrainArgs& a, float* l, int ld, int n, const float* act, int ald, float adv, float oldn,
+                                                  float cr, float invB, float ent_w, float& H) {
+    if constexpr (HEAD == HEAD_DISCRETE) return cat_train_term(l, ld, n, (int)act[0], adv, oldn, cr, invB, ent_w, H);
+    else if constexpr (HEAD == HEAD_MULTI_DISCRETE) return md_train_term(l, ld, n, md_starts(a.md_lo, a.md_hi), act, ald, adv, oldn, cr, invB, ent_w, H);
+    else return bern_train_term(l, ld, n, act, ald, adv, oldn, cr, invB, ent_w, H);
+}
 
 // This CTA's loss sums -> columns P.. of its slab (L = slab + P), the warps combined in a fixed order through s_red
-// (5 * NTH / 32 floats).  Entropy column: a categorical head's sum of H / B (x world, see UpdateScalars) over the CTA's
+// (5 * NTH / 32 floats).  Entropy column: a head without logstd: the sum of H / B (x world, see UpdateScalars) over the CTA's
 // samples; a Box head's box_entropy of the pre-update logstd (logstd(j) loads logstd_j), in CTA 0 only.  A by reference as in
 // gauss_policy_row.
 template <int NTH, int HEAD, class LS>
 __device__ __forceinline__ void store_loss_columns(float* L, float l_pg, float l_vf, float l_kl, float l_cf, float l_ent, float* s_red,
                                                    LS logstd, const int& A) {
     const int tid = threadIdx.x;
-    constexpr int NL = HEAD == HEAD_DISCRETE ? 5 : 4;
+    constexpr int NL = HEAD != HEAD_BOX ? 5 : 4;
     float v4[NL];
     v4[0] = l_pg; v4[1] = l_vf; v4[2] = l_kl; v4[3] = l_cf;
-    if (HEAD == HEAD_DISCRETE) v4[NL - 1] = l_ent;
+    if (HEAD != HEAD_BOX) v4[NL - 1] = l_ent;
 #pragma unroll
     for (int q = 0; q < NL; ++q) v4[q] = warp_sum(v4[q]);
     if ((tid & 31) == 0) {
@@ -387,7 +469,7 @@ __device__ __forceinline__ void store_loss_columns(float* L, float l_pg, float l
             for (int q = 0; q < NL; ++q) t[q] += s_red[w * NL + q];
         L[L_PG] = t[0]; L[L_VF] = t[1]; L[L_KL] = t[2]; L[L_CLIP] = t[3];
         float ent = 0.f;
-        if (HEAD == HEAD_DISCRETE) ent = t[NL - 1];
+        if (HEAD != HEAD_BOX) ent = t[NL - 1];
         else if (blockIdx.x == 0) ent = box_entropy(logstd, A);
         L[L_ENT] = ent;
         L[5] = 0.f; L[6] = 0.f; L[7] = 0.f;
@@ -447,7 +529,7 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
         }
         __syncthreads();
         tile_load_rows<TM>(a.obs, d.O, s_row, nv, Xs);
-        tile_load_rows<TM>(a.act, HEAD == HEAD_DISCRETE ? 1 : d.A, s_row, nv, Ac);
+        tile_load_rows<TM>(a.act, act_cols<HEAD>(a), s_row, nv, Ac);
         __syncthreads();
 
         // ---------------- pi tower ----------------
@@ -457,12 +539,12 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
         __syncthreads();
         tile_fwd<TM, ACT_NONE>(H2s, d.H2, p + d.off[T_PI_W], p + d.off[T_PI_B], d.A, MU);
         __syncthreads();
-        if (HEAD == HEAD_DISCRETE && tid < TM) {  // a thread per sample over the A logits; MU becomes dL/dlogits
+        if (HEAD != HEAD_BOX && tid < TM) {  // a thread per sample over the A logits; MU becomes dL/dlogits
             const int m = tid;
             float* l = MU + m;
             if (m < nv) {
                 float H;
-                const PgTerm t = cat_train_term(l, TM, d.A, (int)Ac[m], s_adv[m], s_oldn[m], cr, a.invB, a.ent_coef * a.invB, H);
+                const PgTerm t = head_train_term<HEAD>(a, l, TM, d.A, Ac + m, TM, s_adv[m], s_oldn[m], cr, a.invB, a.ent_coef * a.invB, H);
                 l_pg += t.pg;
                 l_kl += t.kl;
                 l_cf += t.cf;

@@ -301,7 +301,7 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
             const int m = e / d.O, k = e - m * d.O;
             Xs[k * TM + m] = (m < nv) ? __ldg(a.obs + (size_t)s_row[m] * d.O + k) : 0.f;
         }
-        const int AW = HEAD == HEAD_DISCRETE ? 1 : d.A;  // stored action width
+        const int AW = act_cols<HEAD>(a);  // stored action width
         for (int e = tid; e < TM * AW; e += NTH) {
             const int m = e / AW, j = e - m * AW;
             Ac[j * TM + m] = (m < nv) ? __ldg(a.act + (size_t)s_row[m] * AW + j) : 0.f;
@@ -329,12 +329,12 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
         // ---- loss stage.  Thread (m, jg) handles actions j = jg, jg + JG, ... of sample m.
         constexpr int JG = (NTH / TM) < 8 ? (NTH / TM) : 8;
         const int m = tid % TM, jg = tid / TM;
-        if (HEAD == HEAD_DISCRETE) {  // a thread per sample over the A logits; MU becomes dL/dlogits, Vs dL/dv
+        if (HEAD != HEAD_BOX) {  // a thread per sample over the A logits; MU becomes dL/dlogits, Vs dL/dv
             if (jg == 0) {
                 float* l = MU + m;
                 if (m < nv) {
                     float H;
-                    const PgTerm t = cat_train_term(l, TM, d.A, (int)Ac[m], s_adv[m], s_oldn[m], cr, a.invB, a.ent_coef * a.invB, H);
+                    const PgTerm t = head_train_term<HEAD>(a, l, TM, d.A, Ac + m, TM, s_adv[m], s_oldn[m], cr, a.invB, a.ent_coef * a.invB, H);
                     l_pg += t.pg;
                     l_kl += t.kl;
                     l_cf += t.cf;
@@ -465,8 +465,8 @@ __global__ void __launch_bounds__(NTH) policy_fused_kernel(const PolicyArgs a) {
                 if (a.value) a.value[row] = v;
                 if (a.val_store) a.val_store[row] = v;
             }
-            if (HEAD == HEAD_DISCRETE && a.mode != 1) {
-                cat_policy_row(a, row, MU + m, TM);
+            if (HEAD != HEAD_BOX && a.mode != 1) {
+                head_policy_row<HEAD>(a, row, MU + m, TM);
             } else if (a.mode == 0) {
                 const float* logstd = sW + d.off[T_LOGSTD];
                 gauss_policy_row(a, row, d.A, [&](int j) { return logstd[j]; }, [&](int j) { return MU[j * TM + m]; },
@@ -477,7 +477,7 @@ __global__ void __launch_bounds__(NTH) policy_fused_kernel(const PolicyArgs a) {
             if (a.dones_store) a.dones_store[row] = a.dones_in[row];
         }
         __syncthreads();
-        if (HEAD == HEAD_BOX && do_pi) {  // a categorical head stored its index above
+        if (HEAD == HEAD_BOX && do_pi) {  // a head without logstd stored its actions above
             for (int e = tid; e < nv * d.A; e += NTH) {
                 const int m = e / d.A, j = e - m * d.A;
                 const float act = Ac[j * (TM + 1) + m];

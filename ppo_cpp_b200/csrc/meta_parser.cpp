@@ -334,11 +334,46 @@ int classify_activation(const NodeMap& nodes, std::string& err) {
     return first_op == "Relu" ? 1 : 0;
 }
 
+// the integer values of a Const node (int_val / int64_val fields, or tensor_content of its DT_INT32 / DT_INT64 dtype)
+bool const_ints(const Msg& node, std::vector<long long>& out) {
+    const Msg* v = attr_value(node, "value");
+    const Msg* ten = v ? v->sub("tensor") : nullptr;
+    if (!ten) return false;
+    const std::string dtype = ten->str("dtype");
+    if (dtype != "DT_INT32" && dtype != "DT_INT64") return false;
+    const Field* content = ten->find("tensor_content");
+    out.clear();
+    if (content) {
+        const size_t w = dtype == "DT_INT32" ? 4 : 8;
+        if (content->scalar.size() % w) return false;
+        for (size_t i = 0; i < content->scalar.size(); i += w) {
+            if (w == 4) {
+                int32_t x;
+                std::memcpy(&x, content->scalar.data() + i, 4);
+                out.push_back(x);
+            } else {
+                int64_t x;
+                std::memcpy(&x, content->scalar.data() + i, 8);
+                out.push_back(x);
+            }
+        }
+        return true;
+    }
+    for (const auto& f : ten->fields)
+        if (f.key == "int_val" || f.key == "int64_val") out.push_back(std::atoll(f.scalar.c_str()));
+    return true;
+}
+
 // Stable-Baselines' policy head follows the action space: a Box gets DiagGaussianProbabilityDistribution (model/pi/w, model/pi/b
-// and model/pi/logstd), a Discrete(n) gets CategoricalProbabilityDistribution (n logits from model/pi/w, model/pi/b, no logstd).
-// PPO2's action placeholder loss/action_ph (pdtype.sample_placeholder([None])), when the file has it, must agree: float [?, n]
-// for Box, int32 / int64 [?] for Discrete.  Returns 0 (Box) or 1 (Discrete); -1 with err naming the node otherwise.
-int classify_action_space(const NodeMap& nodes, int n, std::string& err) {
+// and model/pi/logstd); the others have no logstd: a Discrete(n) gets CategoricalProbabilityDistribution over the n logits of
+// model/pi, a MultiDiscrete(nvec) MultiCategoricalProbabilityDistribution (tf.split of the logits by nvec, a SplitV under model/),
+// a MultiBinary(n) BernoulliProbabilityDistribution over n logits (tf.sigmoid of the logits, a Sigmoid under model/).  PPO2's
+// action placeholder loss/action_ph (pdtype.sample_placeholder([None])), when the file has it, must agree: float [?, n] for Box,
+// int32 / int64 [?] for Discrete, int32 / int64 [?, k] for the other two: a SplitV of the pi head's output (the Add / BiasAdd over
+// model/pi/b, under model/) with k size_splits summing to n makes it MultiDiscrete; without one, a Sigmoid of the pi head's output
+// under model/ and k == n make it MultiBinary.  Returns the ppo_action_space (nvec filled for MultiDiscrete); -1 with err naming
+// the node otherwise.
+int classify_action_space(const NodeMap& nodes, int n, std::vector<int>& nvec, std::string& err) {
     const bool box = nodes.count("model/pi/logstd") != 0;
     auto it = nodes.find("loss/action_ph");
     if (it == nodes.end()) return box ? 0 : 1;
@@ -346,12 +381,66 @@ int classify_action_space(const NodeMap& nodes, int n, std::string& err) {
     const std::string dtype = dt ? dt->str("type") : std::string();
     const Msg* shp = attr_value(*it->second, "shape");
     const std::vector<int> dims = shape_dims(shp ? shp->sub("shape") : nullptr);
-    const bool ok = box ? (dtype == "DT_FLOAT" && dims.size() == 2 && dims[1] == n)
-                        : ((dtype == "DT_INT32" || dtype == "DT_INT64") && dims.size() == 1);
+    const bool is_int = dtype == "DT_INT32" || dtype == "DT_INT64";
+    if (!box && is_int && dims.size() == 2) {
+        const int k = dims[1];
+        auto op_of = [&](const std::string& name) -> std::string {
+            auto f = nodes.find(name);
+            return f == nodes.end() ? std::string() : f->second->str("op");
+        };
+        auto is_pi_b = [&](const std::string& name) -> bool {  // model/pi/b or its read
+            if (name == "model/pi/b") return true;
+            auto f = nodes.find(name);
+            if (f == nodes.end() || f->second->str("op") != "Identity") return false;
+            const std::vector<std::string> in = node_inputs(*f->second);
+            return in.size() == 1 && in[0] == "model/pi/b";
+        };
+        // a node of op `op` under model/ whose first input is the pi head's output; its inputs in `si`
+        auto reads_pi_head = [&](const std::pair<const std::string, const Msg*>& kv, const char* op, std::vector<std::string>& si) -> bool {
+            if (kv.second->str("op") != op || kv.first.compare(0, 6, "model/") != 0) return false;
+            si = node_inputs(*kv.second);
+            const std::string aop = si.empty() ? std::string() : op_of(si[0]);
+            if (aop != "Add" && aop != "AddV2" && aop != "BiasAdd") return false;
+            const std::vector<std::string> ai = node_inputs(*nodes.at(si[0]));
+            return ai.size() == 2 && (is_pi_b(ai[0]) || is_pi_b(ai[1]));
+        };
+        std::vector<std::string> si;
+        for (const auto& kv : nodes) {
+            if (!reads_pi_head(kv, "SplitV", si)) continue;
+            std::vector<long long> sizes;
+            long long sum = 0;
+            bool pos = true;
+            if (si.size() < 2 || op_of(si[1]) != "Const" || !const_ints(*nodes.at(si[1]), sizes)) {
+                err = "node " + kv.first + " splits the pi head's output, but its size_splits is not an integer Const";
+                return -1;
+            }
+            for (long long v : sizes) {
+                sum += v;
+                pos = pos && v >= 1;
+            }
+            if ((int)sizes.size() != k || sum != n || !pos) {
+                err = "node " + kv.first + " splits the pi head's " + std::to_string(n) + " logits into " + std::to_string(sizes.size()) + " slices summing to " +
+                      std::to_string(sum) + "; loss/action_ph has " + std::to_string(k) + " columns (a MultiDiscrete space needs k positive slices summing to the pi width)";
+                return -1;
+            }
+            nvec.assign(sizes.begin(), sizes.end());
+            return 2;
+        }
+        for (const auto& kv : nodes) {
+            if (!reads_pi_head(kv, "Sigmoid", si)) continue;
+            if (k == n) return 3;
+            err = "node " + kv.first + " is a Bernoulli head over " + std::to_string(n) + " logits; loss/action_ph has " + std::to_string(k) + " columns";
+            return -1;
+        }
+        err = "node loss/action_ph (" + dtype + " [?, " + std::to_string(k) + "]) fits no head without model/pi/logstd: a MultiDiscrete space needs a SplitV of the pi head's "
+              "output under model/, a MultiBinary space a Sigmoid of it and k == " + std::to_string(n) + " (the pi width)";
+        return -1;
+    }
+    const bool ok = box ? (dtype == "DT_FLOAT" && dims.size() == 2 && dims[1] == n) : (is_int && dims.size() == 1);
     if (ok) return box ? 0 : 1;
     err = "node loss/action_ph (" + (dtype.empty() ? std::string("no dtype") : dtype) + ", rank " + std::to_string(dims.size()) + ") contradicts the " +
           (box ? "Gaussian head (model/pi/logstd present): a Box space needs a float [?, " + std::to_string(n) + "] placeholder"
-               : "categorical head (no model/pi/logstd): a Discrete space needs an int32 / int64 [?] placeholder");
+               : "head without model/pi/logstd: a Discrete space needs an int32 / int64 [?] placeholder, a MultiDiscrete or MultiBinary one int32 / int64 [?, k]");
     return -1;
 }
 
@@ -420,7 +509,7 @@ std::string parse_meta_txt(const std::string& path, MetaGraph& out) {
     out.hidden1 = w0[1];
     out.hidden2 = w1[1];
     out.act_dim = wp[1];
-    out.action_space = classify_action_space(nodes, out.act_dim, out.action_space_error);
+    out.action_space = classify_action_space(nodes, out.act_dim, out.nvec, out.action_space_error);
     return std::string();
 }
 

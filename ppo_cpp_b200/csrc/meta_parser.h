@@ -25,10 +25,11 @@ struct MetaGraph {
     // hidden layers per tower (activation_error says why)
     int activation = 0;
     std::string activation_error;
-    // action space of the policy head (ppo_action_space: 0 Box, a Gaussian with model/pi/logstd; 1 Discrete, a categorical
-    // without it), or -1 when loss/action_ph contradicts the head (action_space_error says why)
+    // action space of the policy head (ppo_action_space: 0 Box, a Gaussian with model/pi/logstd; without it 1 Discrete,
+    // 2 MultiDiscrete, 3 MultiBinary), or -1 when loss/action_ph contradicts the head (action_space_error says why)
     int action_space = 0;
     std::string action_space_error;
+    std::vector<int> nvec;  // MultiDiscrete: the choices per action column (size_splits of the SplitV)
     std::map<std::string, MetaTensor> tensors;  // the model/* variables with their initial values (14 without logstd)
 };
 

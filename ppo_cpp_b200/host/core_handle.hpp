@@ -9,6 +9,7 @@
 #include <memory>
 #include <stdexcept>
 #include <string>
+#include <vector>
 
 #include "../../include/ppo_core.h"
 
@@ -26,9 +27,13 @@ struct CoreDeleter {
 };
 using CorePtr = std::shared_ptr<ppo_core>;
 
-inline CorePtr make_core(const ppo_core_desc& desc, int action_space = PPO_ACTION_BOX) {
+// nvec: the choices per action column of a PPO_ACTION_MULTI_DISCRETE core (ignored otherwise)
+inline CorePtr make_core(const ppo_core_desc& desc, int action_space = PPO_ACTION_BOX, const std::vector<int>& nvec = {}) {
     ppo_core* raw = nullptr;
-    ppo_check(ppo_core_create_ex(&desc, action_space, &raw), "ppo_core_create");
+    if (action_space == PPO_ACTION_MULTI_DISCRETE)
+        ppo_check(ppo_core_create_nvec(&desc, nvec.data(), static_cast<int>(nvec.size()), &raw), "ppo_core_create");
+    else
+        ppo_check(ppo_core_create_ex(&desc, action_space, &raw), "ppo_core_create");
     return CorePtr(raw, CoreDeleter());
 }
 

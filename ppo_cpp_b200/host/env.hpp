@@ -23,6 +23,8 @@ public:
     virtual std::string get_observation_space() = 0;
     virtual int get_action_space_size() = 0;
     virtual int get_observation_space_size() = 0;
+    // a MultiDiscrete env's choices per action column (Stable-Baselines' nvec); empty for the other spaces
+    virtual std::vector<int> get_action_space_nvec() { return {}; }
     virtual int get_num_envs() { return 1; }
     virtual Mat reset() = 0;
     // returns {obs [n,O], rewards [n,1], dones [n,1]}
@@ -41,10 +43,25 @@ public:
         static const std::string s = "discrete";
         return s;
     }
+    static const std::string& SPACE_MULTI_DISCRETE() {
+        static const std::string s = "multi_discrete";
+        return s;
+    }
+    static const std::string& SPACE_MULTI_BINARY() {
+        static const std::string s = "multi_binary";
+        return s;
+    }
 };
 
 // columns of an action matrix: get_action_space_size() for a continuous env; one (the index, as a float) for a discrete env,
-// whose get_action_space_size() is the number of choices (Stable-Baselines' Discrete(n))
-inline int action_width(Env& env) { return env.get_action_space() == Env::SPACE_DISCRETE() ? 1 : env.get_action_space_size(); }
+// whose get_action_space_size() is the number of choices (Stable-Baselines' Discrete(n)); one index per column of
+// get_action_space_nvec() for a MultiDiscrete env, whose get_action_space_size() is sum(nvec) (the logits of the policy head);
+// get_action_space_size() bits (0 / 1 as floats) for a MultiBinary env
+inline int action_width(Env& env) {
+    const std::string s = env.get_action_space();
+    if (s == Env::SPACE_DISCRETE()) return 1;
+    if (s == Env::SPACE_MULTI_DISCRETE()) return static_cast<int>(env.get_action_space_nvec().size());
+    return env.get_action_space_size();
+}
 
 #endif

@@ -101,13 +101,19 @@ public:
         } else {
             d.norm_obs = 0; d.norm_reward = 0; d.training = 0;
         }
-        // a Discrete env gets a categorical head over its get_action_space_size() choices; action_space is the env's, or the
-        // sidecar's after load()
-        if (action_space != Env::SPACE_CONTINOUS() && action_space != Env::SPACE_DISCRETE())
-            throw std::runtime_error("PPO2: unsupported action space " + action_space);
+        // a Discrete env gets a categorical head over its get_action_space_size() choices, a MultiDiscrete env one categorical per
+        // column of its nvec, a MultiBinary env a Bernoulli per action bit; action_space (and nvec) are the env's, or the sidecar's
+        // after load()
+        const std::string spaces[4] = {Env::SPACE_CONTINOUS(), Env::SPACE_DISCRETE(), Env::SPACE_MULTI_DISCRETE(), Env::SPACE_MULTI_BINARY()};
+        int space = -1;  // ppo_action_space: the index into spaces
+        for (int i = 0; i < 4; ++i)
+            if (action_space == spaces[i]) space = i;
+        if (space < 0) throw std::runtime_error("PPO2: unsupported action space " + action_space);
         if (action_space != env.get_action_space())
             throw std::runtime_error("PPO2: the model's action space " + action_space + " is not the env's " + env.get_action_space());
-        const int space = action_space == Env::SPACE_DISCRETE() ? PPO_ACTION_DISCRETE : PPO_ACTION_BOX;
+        if (!loaded_nvec_.empty() && loaded_nvec_ != env.get_action_space_nvec())
+            throw std::runtime_error("PPO2: the model's MultiDiscrete nvec is not the env's");
+        const std::vector<int> nvec = env.get_action_space_nvec();
         const bool from_graph = hidden_override_[0] == 0;
         if (from_graph) {
             ppo_meta_info info;
@@ -116,8 +122,15 @@ public:
             ppo_check(graph_space < 0 ? graph_space : PPO_OK, "graph load");
             if (graph_space != space) {
                 std::cout << "the graph's policy head does not match the env's " << action_space << " action space" << std::endl;
-                throw std::runtime_error("PPO2: graph " + model_filename + " has a " + (graph_space == PPO_ACTION_DISCRETE ? "discrete" : "continuous") +
+                throw std::runtime_error("PPO2: graph " + model_filename + " has a " + (graph_space >= 0 && graph_space < 4 ? spaces[graph_space] : std::string("unknown")) +
                                          " policy head, the env a " + action_space + " action space");
+            }
+            if (space == PPO_ACTION_MULTI_DISCRETE) {
+                std::vector<int> g(64);
+                const int k = ppo_meta_action_nvec(model_filename.c_str(), g.data(), static_cast<int>(g.size()));
+                ppo_check(k < 0 ? k : PPO_OK, "graph load");
+                g.resize(k);
+                if (g != nvec) throw std::runtime_error("PPO2: graph " + model_filename + " splits its logits by another nvec than the env's");
             }
             if (info.obs_dim != d.obs_dim || info.act_dim != d.act_dim) {
                 std::cout << "graph input/output widths do not match the environment" << std::endl;
@@ -127,7 +140,7 @@ public:
         } else {
             d.hidden1 = hidden_override_[0]; d.hidden2 = hidden_override_[1];
         }
-        core_ = make_core(d, space);
+        core_ = make_core(d, space, nvec);
         if (from_graph) {
             // the graph's baked ent_coef / vf_coef / clip norm / Adam constants win over the constructor's (SURVEY §3.5)
             ppo_check(ppo_core_load_meta_txt(core_.get(), model_filename.c_str()), "graph load");
@@ -153,6 +166,7 @@ public:
         json["nminibatches"] = nminibatches; json["noptepochs"] = noptepochs; json["cliprange"] = cliprange;
         json["cliprange_vf"] = cliprange_vf; json["observation_space"] = observation_space; json["action_space"] = action_space;
         json["n_envs"] = n_envs; json["model_filename"] = model_filename;
+        if (action_space == Env::SPACE_MULTI_DISCRETE()) json["nvec"] = env.get_action_space_nvec();
         // addition over the reference: a graph-less model (reset_without_graph) has no file to recover its shape from
         if (hidden_override_[0] > 0) {
             json["hidden1"] = hidden_override_[0];
@@ -187,6 +201,7 @@ public:
         cliprange = json["cliprange"].get<float>(); cliprange_vf = json["cliprange_vf"].get<float>();
         observation_space = json["observation_space"].get<std::string>(); action_space = json["action_space"].get<std::string>();
         n_envs = json["n_envs"].get<int>();
+        loaded_nvec_ = json.contains("nvec") ? json["nvec"].get<std::vector<int>>() : std::vector<int>{};
         if (n_envs != env.get_num_envs()) {
             // the reference only stores this number; here the device buffers are sized by it, so the live env wins
             std::cout << "checkpoint was written with n_envs " << n_envs << ", environment has " << env.get_num_envs() << std::endl;
@@ -321,6 +336,7 @@ private:
     int hidden_override_[2] = {0, 0};
     uint64_t init_seed_ = 0;
     int activation_ = PPO_ACT_TANH;  // ppo_activation of the core (graph-less: chosen; otherwise the graph's)
+    std::vector<int> loaded_nvec_;   // the MultiDiscrete nvec of the sidecar read by load() (empty: none)
     CorePtr core_;
     std::unique_ptr<MlpPolicy> act_model;
 };

@@ -49,6 +49,7 @@ public:
     std::string get_action_space() override { return envs[0]->get_action_space(); }
     std::string get_observation_space() override { return envs[0]->get_observation_space(); }
     int get_action_space_size() override { return envs[0]->get_action_space_size(); }
+    std::vector<int> get_action_space_nvec() override { return envs[0]->get_action_space_nvec(); }
     int get_observation_space_size() override { return envs[0]->get_observation_space_size(); }
     int get_num_envs() override { return static_cast<int>(envs.size()); }
 

@@ -29,7 +29,8 @@ TENSOR_ORDER = [
     "model/q/w", "model/q/b",
 ]
 N_TRAINABLE_TENSORS = 13
-LOGSTD = "model/pi/logstd"  # absent with a categorical head (Discrete action space): 14 tensors, 12 trainable
+LOGSTD = "model/pi/logstd"  # absent unless the head is Gaussian (Box action space): 14 tensors, 12 trainable
+ACTION_SPACES = ("box", "discrete", "multi_discrete", "multi_binary")
 
 _TOKEN = re.compile(r'\s*(?:([A-Za-z_][A-Za-z0-9_]*)|([{}:])|("(?:[^"\\]|\\.)*")|([-+0-9.eE]+[A-Za-z]*|-?inf|nan))')
 
@@ -110,6 +111,7 @@ class MetaInfo:
     vf_clip: str = "shared"
     activation: str = "tanh"
     action_space: str = "box"
+    nvec: List[int] | None = None  # choices per action column: [n] (discrete), nvec (multi_discrete), 2s (multi_binary); None for box
     shapes: Dict[str, Tuple[int, ...]] = field(default_factory=dict)
 
     def flat_params(self, include_q: bool = True) -> np.ndarray:
@@ -262,30 +264,94 @@ def classify_activation(nodes: Dict[str, dict]) -> str:
     return "relu" if first[0] == "Relu" else "tanh"
 
 
-def classify_action_space(nodes: Dict[str, dict], n: int) -> str:
-    """The action space of Stable-Baselines' policy head: "box" (DiagGaussianProbabilityDistribution, with model/pi/logstd) or
-    "discrete" (CategoricalProbabilityDistribution over the n logits of model/pi, no logstd).  PPO2's action placeholder
-    loss/action_ph, when the graph has it, must agree: float [?, n] for "box", int32 / int64 [?] for "discrete"; otherwise
+def _const_ints(node: dict) -> List[int] | None:
+    """The integer values of a Const node (int_val / int64_val, or tensor_content of its DT_INT32 / DT_INT64 dtype), else None."""
+    v = _attr(node, "value")
+    t = v["tensor"][0] if v is not None and "tensor" in v else None
+    dtype = t["dtype"][0] if t is not None and "dtype" in t else ""
+    if dtype not in ("DT_INT32", "DT_INT64"):
+        return None
+    if "tensor_content" in t:
+        raw = t["tensor_content"][0]
+        w = 4 if dtype == "DT_INT32" else 8
+        if len(raw) % w:
+            return None
+        return [int(x) for x in np.frombuffer(raw, dtype="<i4" if w == 4 else "<i8")]
+    return [int(x) for x in t.get("int_val", []) + t.get("int64_val", [])]
+
+
+def classify_action_space(nodes: Dict[str, dict], n: int) -> Tuple[str, List[int] | None]:
+    """The action space of Stable-Baselines' policy head and, for "multi_discrete", its nvec: "box" (DiagGaussianProbabilityDistribution,
+    with model/pi/logstd); without logstd "discrete" (CategoricalProbabilityDistribution over the n logits of model/pi),
+    "multi_discrete" (MultiCategoricalProbabilityDistribution: tf.split of the logits by nvec, a SplitV under model/) or "multi_binary"
+    (BernoulliProbabilityDistribution: tf.sigmoid of the logits, a Sigmoid under model/).  PPO2's action placeholder loss/action_ph,
+    when the graph has it, must agree: float [?, n] for "box", int32 / int64 [?] for "discrete", int32 / int64 [?, k] for the other
+    two: a SplitV of the pi head's output (the Add / BiasAdd over model/pi/b, under model/) with k size_splits summing to n makes it
+    "multi_discrete"; without one, a Sigmoid of the pi head's output under model/ and k == n make it "multi_binary".  Otherwise
     ValueError naming the node.  Twin of classify_action_space in csrc/meta_parser.cpp."""
     box = LOGSTD in nodes
     ph = nodes.get("loss/action_ph")
     if ph is None:
-        return "box" if box else "discrete"
+        return ("box", None) if box else ("discrete", None)
     dt = _attr(ph, "dtype")
     dtype = dt["type"][0] if dt is not None and "type" in dt else ""
     shp = _attr(ph, "shape")
     dims = [int(d["size"][0]) for d in shp["shape"][0].get("dim", [])] if shp is not None and "shape" in shp else []
+    is_int = dtype in ("DT_INT32", "DT_INT64")
+    if not box and is_int and len(dims) == 2:
+        k = dims[1]
+
+        def op_of(name):
+            node = nodes.get(name)
+            return node["op"][0].decode() if node is not None else ""
+
+        def is_pi_b(name):  # model/pi/b or its read
+            return name == "model/pi/b" or (op_of(name) == "Identity" and _inputs(nodes[name]) == ["model/pi/b"])
+
+        def reads_pi_head(name, op):
+            if op_of(name) != op or not name.startswith("model/"):
+                return None
+            si = _inputs(nodes[name])
+            if not si or op_of(si[0]) not in ("Add", "AddV2", "BiasAdd"):
+                return None
+            ai = _inputs(nodes[si[0]])
+            return si if len(ai) == 2 and (is_pi_b(ai[0]) or is_pi_b(ai[1])) else None
+
+        for name in sorted(nodes):
+            si = reads_pi_head(name, "SplitV")
+            if si is None:
+                continue
+            sizes = _const_ints(nodes[si[1]]) if len(si) >= 2 and op_of(si[1]) == "Const" else None
+            if sizes is None:
+                raise ValueError(f"node {name} splits the pi head's output, but its size_splits is not an integer Const")
+            if len(sizes) != k or sum(sizes) != n or min(sizes) < 1:
+                raise ValueError(f"node {name} splits the pi head's {n} logits into {len(sizes)} slices summing to {sum(sizes)}; loss/action_ph has "
+                                 f"{k} columns (a MultiDiscrete space needs k positive slices summing to the pi width)")
+            return "multi_discrete", sizes
+        for name in sorted(nodes):
+            if reads_pi_head(name, "Sigmoid") is None:
+                continue
+            if k == n:
+                return "multi_binary", None
+            raise ValueError(f"node {name} is a Bernoulli head over {n} logits; loss/action_ph has {k} columns")
+        raise ValueError(f"node loss/action_ph ({dtype} [?, {k}]) fits no head without model/pi/logstd: a MultiDiscrete space needs a SplitV of "
+                         f"the pi head's output under model/, a MultiBinary space a Sigmoid of it and k == {n} (the pi width)")
     if box and dtype == "DT_FLOAT" and len(dims) == 2 and dims[1] == n:
-        return "box"
-    if not box and dtype in ("DT_INT32", "DT_INT64") and len(dims) == 1:
-        return "discrete"
+        return "box", None
+    if not box and is_int and len(dims) == 1:
+        return "discrete", None
     head = (f"Gaussian head (model/pi/logstd present): a Box space needs a float [?, {n}] placeholder" if box else
-            "categorical head (no model/pi/logstd): a Discrete space needs an int32 / int64 [?] placeholder")
+            "head without model/pi/logstd: a Discrete space needs an int32 / int64 [?] placeholder, a MultiDiscrete or MultiBinary one int32 / int64 [?, k]")
     raise ValueError(f"node loss/action_ph ({dtype or 'no dtype'}, rank {len(dims)}) contradicts the {head}")
 
 
+def action_nvec(action_space: str, n: int, nvec=None) -> List[int] | None:
+    """Choices per action column of a head over n logits: [n] (discrete), nvec (multi_discrete), 2s (multi_binary); None for box."""
+    return {"box": None, "discrete": [n], "multi_discrete": None if nvec is None else list(nvec), "multi_binary": [2] * n}[action_space]
+
+
 def meta_action_space(path: str) -> str:
-    """The action space of a graph file's policy head ("box" / "discrete"), read by this module's parser."""
+    """The action space of a graph file's policy head ("box", "discrete", "multi_discrete", "multi_binary"), read by this module's parser."""
     return parse_meta_txt(path).action_space
 
 
@@ -324,6 +390,7 @@ def parse_meta_txt(path: str) -> MetaInfo:
         return float(_tensor_value(nodes[name]).reshape(-1)[0])
 
     hidden = [shapes["model/pi_fc0/w"][1], shapes["model/pi_fc1/w"][1]]
+    space, nvec = classify_action_space(nodes, shapes["model/pi/w"][1])
     ver = ""
     try:
         ver = root["meta_info_def"][0]["tensorflow_version"][0].decode()
@@ -343,7 +410,8 @@ def parse_meta_txt(path: str) -> MetaInfo:
         tf_version=ver,
         vf_clip=classify_vf_clip(nodes),
         activation=classify_activation(nodes),
-        action_space=classify_action_space(nodes, shapes["model/pi/w"][1]),
+        action_space=space,
+        nvec=action_nvec(space, shapes["model/pi/w"][1], nvec),
         shapes=shapes,
     )
 
@@ -354,7 +422,7 @@ CKPT_ORDER = sorted(TENSOR_ORDER)
 
 
 def read_checkpoint_data(data_path: str, shapes: Dict[str, Tuple[int, ...]]) -> Dict[str, np.ndarray]:
-    """The tensors of `shapes` (15, or 14 without logstd for a categorical head) from a Saver V2 .data file."""
+    """The tensors of `shapes` (15, or 14 without logstd for a head other than Box) from a Saver V2 .data file."""
     raw = np.fromfile(data_path, dtype="<f4")
     out, off = {}, 0
     for name in CKPT_ORDER:
@@ -369,10 +437,10 @@ def read_checkpoint_data(data_path: str, shapes: Dict[str, Tuple[int, ...]]) -> 
 
 
 def param_layout(obs_dim: int, act_dim: int, h1: int, h2: int, action_space: str = "box") -> Dict[str, Tuple[int, Tuple[int, ...]]]:
-    """Offsets (in floats) of every tensor inside the flat parameter vector used by the core.  A categorical head
-    (action_space "discrete", act_dim logits) has no logstd; the other tensors keep their order."""
-    if action_space not in ("box", "discrete"):
-        raise ValueError(f"action_space must be 'box' or 'discrete', not {action_space!r}")
+    """Offsets (in floats) of every tensor inside the flat parameter vector used by the core.  Only the Gaussian head (action_space
+    "box") has a logstd; the other heads (act_dim logits) leave it out, and the other tensors keep their order."""
+    if action_space not in ACTION_SPACES:
+        raise ValueError(f"action_space must be one of {ACTION_SPACES}, not {action_space!r}")
     shp = {
         "model/pi_fc0/w": (obs_dim, h1), "model/pi_fc0/b": (h1,),
         "model/vf_fc0/w": (obs_dim, h1), "model/vf_fc0/b": (h1,),
@@ -385,7 +453,7 @@ def param_layout(obs_dim: int, act_dim: int, h1: int, h2: int, action_space: str
     }
     out, off = {}, 0
     for name in TENSOR_ORDER:
-        if name == LOGSTD and action_space == "discrete":
+        if name == LOGSTD and action_space != "box":
             continue
         out[name] = (off, shp[name])
         off += int(np.prod(shp[name]))
@@ -411,7 +479,7 @@ def _escape(b: bytes) -> str:
 
 def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 0.0, vf_coef: float = 0.5,
                    clip_norm: float = 0.5, beta1: float = 0.9, beta2: float = 0.999, adam_eps: float = 1e-5,
-                   vf_clip: str | None = None, activation: str | None = None, action_space: str | None = None) -> None:
+                   vf_clip: str | None = None, activation: str | None = None, action_space: str | None = None, nvec=None) -> None:
     """Write a minimal .meta.txt (variables + initialisers + baked constants) that both readers accept.
 
     The reference's graphs come from a Stable-Baselines/TensorFlow export script that is not part of the
@@ -423,13 +491,19 @@ def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 
     act_fun), under model/ and train_model/ as Stable-Baselines names them; without it the file has none and reads as "tanh".
     action_space = "box" | "discrete" adds PPO2's action placeholder loss/action_ph (float [?, n] / int64 [?]); "discrete" also
     leaves model/pi/logstd out (a categorical head over the n columns of model/pi/w; `tensors` need not hold logstd).  Without it
-    the file has no placeholder and a logstd, and reads as "box"."""
+    the file has no placeholder and a logstd, and reads as "box".
+    action_space = "multi_discrete" (with nvec, summing to the n columns of model/pi/w) writes an int64 [?, k] placeholder and the
+    SplitV model/split of the pi head's output by nvec; "multi_binary" an int32 [?, n] placeholder and the Sigmoid model/Sigmoid of
+    the pi head's output (the dtypes are those of Stable-Baselines' sample_dtype as far as known; the readers take either).  Both
+    leave logstd out, and write the pi head's output model/pi/add (and the read of model/pi/b) unless `activation` wrote them."""
     if vf_clip not in (None, "shared", "none", "separate"):
         raise ValueError(f"vf_clip must be None, 'shared', 'none' or 'separate', not {vf_clip!r}")
     if activation not in (None, "tanh", "relu"):
         raise ValueError(f"activation must be None, 'tanh' or 'relu', not {activation!r}")
-    if action_space not in (None, "box", "discrete"):
-        raise ValueError(f"action_space must be None, 'box' or 'discrete', not {action_space!r}")
+    if action_space not in (None,) + ACTION_SPACES:
+        raise ValueError(f"action_space must be None or one of {ACTION_SPACES}, not {action_space!r}")
+    if (action_space == "multi_discrete") != (nvec is not None):
+        raise ValueError("nvec goes with action_space='multi_discrete' (and only with it)")
     def dims(shape, ind):
         return "".join(f"{ind}dim {{\n{ind}  size: {d}\n{ind}}}\n" for d in shape)
 
@@ -451,16 +525,25 @@ def write_meta_txt(path: str, tensors: Dict[str, np.ndarray], ent_coef: float = 
 
     parts = ['meta_info_def {\n  tensorflow_version: "1.14.0"\n}\ngraph_def {\n']
     for name in TENSOR_ORDER:
-        if name == LOGSTD and action_space == "discrete":
+        if name == LOGSTD and action_space not in (None, "box"):
             continue
         arr = np.asarray(tensors[name], np.float32)
         parts.append(const_node(f"{name}/Initializer/initial_value", arr))
         parts.append(var_node(name, arr.shape))
     if action_space is not None:
         n = np.asarray(tensors["model/pi/w"]).shape[1]
-        parts.append(_action_placeholder("DT_INT64", (-1,)) if action_space == "discrete" else _action_placeholder("DT_FLOAT", (-1, n)))
+        if action_space == "multi_discrete":
+            if len(nvec) < 1 or min(nvec) < 1 or sum(nvec) != n:
+                raise ValueError(f"nvec {list(nvec)} must be positive and sum to the {n} columns of model/pi/w")
+            parts.append(_action_placeholder("DT_INT64", (-1, len(nvec))))
+        elif action_space == "multi_binary":
+            parts.append(_action_placeholder("DT_INT32", (-1, n)))
+        else:
+            parts.append(_action_placeholder("DT_INT64", (-1,)) if action_space == "discrete" else _action_placeholder("DT_FLOAT", (-1, n)))
     if activation is not None:
         parts.append(_forward_nodes(activation))
+    if action_space in ("multi_discrete", "multi_binary"):
+        parts.append(_distribution_nodes(nvec, with_head=activation is None))
     if vf_clip is not None:
         parts.append(_vf_loss_nodes(vf_clip))
     for name, val in (("loss/mul_4/y", ent_coef), ("loss/mul_5/y", vf_coef), ("loss/clip_by_global_norm/mul/x", clip_norm),
@@ -476,6 +559,23 @@ def _action_placeholder(dtype: str, shape) -> str:
     dims = "".join(f"          dim {{\n            size: {d}\n          }}\n" for d in shape)
     return (f'  node {{\n    name: "loss/action_ph"\n    op: "Placeholder"\n    attr {{\n      key: "dtype"\n      value {{\n        type: {dtype}\n      }}\n    }}\n'
             f'    attr {{\n      key: "shape"\n      value {{\n        shape {{\n{dims}        }}\n      }}\n    }}\n  }}\n')
+
+
+def _distribution_nodes(nvec, with_head: bool) -> str:
+    """The op of the head's distribution that classify_action_space reads, on the pi head's output model/pi/add: MultiDiscrete's
+    tf.split by nvec (SplitV model/split with its int32 size_splits Const), or MultiBinary's tf.sigmoid (model/Sigmoid).  With
+    with_head the pi head's output and the read of model/pi/b are written too (the forward nodes of `activation` hold them)."""
+    nodes = []
+    if with_head:
+        nodes += [_op_node("model/pi/b/read", "Identity", "model/pi/b"), _op_node("model/pi/add", "Add", "model/pi/MatMul", "model/pi/b/read")]
+    if nvec is None:
+        return "".join(nodes + [_op_node("model/Sigmoid", "Sigmoid", "model/pi/add")])
+    sizes = _escape(np.asarray(nvec, "<i4").tobytes())
+    nodes.append(f'  node {{\n    name: "model/split/size_splits"\n    op: "Const"\n    attr {{\n      key: "dtype"\n      value {{\n        type: DT_INT32\n      }}\n    }}\n'
+                 f'    attr {{\n      key: "value"\n      value {{\n        tensor {{\n          dtype: DT_INT32\n          tensor_shape {{\n'
+                 f'            dim {{\n              size: {len(nvec)}\n            }}\n          }}\n          tensor_content: "{sizes}"\n        }}\n      }}\n    }}\n  }}\n')
+    nodes += [_op_node("model/split/split_dim", "Const"), _op_node("model/split", "SplitV", "model/pi/add", "model/split/size_splits", "model/split/split_dim")]
+    return "".join(nodes)
 
 
 def _op_node(name, kind, *inputs):
