@@ -145,6 +145,26 @@ int ppo_core_create_nvec(const ppo_core_desc *desc, const int *nvec, int k, ppo_
 int ppo_core_action_space(ppo_core *core); /* the core's ppo_action_space, or a negative ppo_status */
 /* the core's choices per action column, as ppo_meta_action_nvec; returns the action width */
 int ppo_core_action_nvec(ppo_core *core, int *nvec, int capacity);
+/* Invalid-action masks (sb3-contrib's MaskableCategorical), DISCRETE and MULTI_DISCRETE cores only: ppo_core_set_action_masking on
+ * a BOX or MULTI_BINARY core is PPO_ERR_UNSUPPORTED.  Off at create; must be the same on every rank.  Turning it on allocates the
+ * "action_masks" rollout buffer (every row all allowed) and, on or off, drops the captured CUDA graphs.
+ *   A mask is const uint8_t [n][act_dim]: per row one entry per logit in logit order (act_dim for DISCRETE, sum(nvec) for
+ *   MULTI_DISCRETE), 1 allowed, 0 forbidden; any other value is PPO_ERR_INVALID, as is a categorical (the row, or a slice) that
+ *   allows nothing.  Internally a row is one 64-bit word (bit j = logit j allowed), 8 bytes per transition.
+ *   Over the allowed logits S of each categorical: the sample is argmax_{j in S} (l_j - log(-log u_j)) with the unmasked head's
+ *   uniforms (forbidden indices skipped, ties to the first index), so all-allowed draws what the unmasked head draws; neglogp =
+ *   log z_S - (l_a - m_S) with m_S = max_S l, z_S = sum_S exp(l - m_S) (summed over the slices); entropy = sum_S p (log z_S - (l - m_S));
+ *   dL/dl_j is exactly 0 for a forbidden j; the deterministic action is argmax_S l.  The value loss, clip and Adam are unchanged.
+ *   These equal sb3-contrib's results with -1e8 in the forbidden logits.
+ *   The plain entry points (ppo_policy_step, ppo_runner_reset / act / observe, ppo_rollout_set of "actions", ppo_loss_grad ...)
+ *   allow every action of the rows they touch; the _masked ones fail with PPO_ERR_INVALID while masking is off.
+ *   A mask in device memory (PPO_DEVICE) is checked on the device: its first bad row (every logit then allowed for it) is reported
+ *   as PPO_ERR_INVALID by the next ppo_runner_finish, ppo_train_update*, ppo_train_minibatch* or ppo_core_sync of the core.  With
+ *   more than one rank, ppo_train_update* and ppo_train_minibatch* first sum every rank's count of bad masks (one ncclAllReduce of
+ *   one float per call, on masking cores only), so a bad mask on one rank fails the call on every rank before any collective of it.
+ *   ppo_runner_rollout_host / _replay take no masks: PPO_ERR_UNSUPPORTED on a masking core. */
+int ppo_core_set_action_masking(ppo_core *core, int enable);
+int ppo_core_action_masking(ppo_core *core); /* 1 on, 0 off, or a negative ppo_status */
 void ppo_core_destroy(ppo_core *core);
 /* load initial weights from the graph file; its shapes and its ppo_action_space (and nvec) must match the core's (ppo2.hpp:90-105 reset());
  * sets the core's ppo_vf_clip and ppo_activation */
@@ -190,6 +210,10 @@ int ppo_policy_step(ppo_core *core, const float *obs, int n, const float *eps, f
                     float *neglogp, ppo_mem mem);
 int ppo_policy_value(ppo_core *core, const float *obs, int n, float *value, ppo_mem mem);
 int ppo_policy_mean(ppo_core *core, const float *obs, int n, float *action, ppo_mem mem); /* PPO2::eval, ppo2.hpp:225-237 */
+/* ... over the actions mask [n][act_dim] allows (see ppo_core_set_action_masking); mask lives where `mem` says */
+int ppo_policy_step_masked(ppo_core *core, const float *obs, int n, const float *eps, const uint8_t *mask, float *action, float *value,
+                           float *neglogp, ppo_mem mem);
+int ppo_policy_mean_masked(ppo_core *core, const float *obs, int n, const uint8_t *mask, float *action, ppo_mem mem);
 
 /* ---- VecNormalize (EnvNormalize, env/env_normalize.hpp:64-116) on the core's running statistics ---- */
 int ppo_vecnorm_reset(ppo_core *core, const float *raw_obs, float *obs_out, ppo_mem mem);
@@ -228,6 +252,13 @@ int ppo_runner_reset(ppo_core *core, const float *raw_obs, ppo_mem mem);
 int ppo_runner_act(ppo_core *core, int t, float *actions_out, ppo_mem mem);
 int ppo_runner_observe(ppo_core *core, int t, const float *raw_obs, const float *raw_rew, const float *done, ppo_mem mem);
 int ppo_runner_finish(ppo_core *core);
+/* ... on a masking core: the mask [n_envs][act_dim] travels with the observation it belongs to; the next ppo_runner_act samples over
+ * it and stores it at rollout row t (the mask after the last observe is that of the next rollout's step 0, as the observation is).
+ * With PPO_HOST, ppo_runner_observe_masked copies the observation, reward, done and the mask's packed words through the core's
+ * pinned staging buffer and returns without waiting for the copies (the caller's buffers may be reused at once). */
+int ppo_runner_reset_masked(ppo_core *core, const float *raw_obs, const uint8_t *mask, ppo_mem mem);
+int ppo_runner_observe_masked(ppo_core *core, int t, const float *raw_obs, const float *raw_rew, const float *done, const uint8_t *mask,
+                              ppo_mem mem);
 /* The same protocol as ONE call (the loop of Runner::run, ppo2/runner.hpp:75-129, in C): per env step the actions are
  * copied to `actions` (host, [n_envs][A]), `step` advances the host env and hands back pointers to its raw
  * observation / reward / done arrays (host, valid until the next call), which are copied to the device and
@@ -248,7 +279,9 @@ int ppo_runner_rollout_replay(ppo_core *core, const float *raw_obs, const float 
 int ppo_synth_env_reset(ppo_core *core);
 int ppo_rollout_synthetic(ppo_core *core);
 /* rollout buffers in the reference's flat layout: "obs","returns","dones","actions","values","neglogpacs",
- * "true_rewards","unnormalized_rewards" ([n_batch,18] or [n_batch]); host pointers */
+ * "true_rewards","unnormalized_rewards" ([n_batch,18] or [n_batch]); host pointers.  A masking core adds "action_masks" as fp32
+ * 0 / 1 [n_batch, act_dim]; setting it refuses a mask that forbids its row's recorded action (set the actions first: setting
+ * "actions" makes those rows' masks all allowed) */
 int ppo_rollout_get(ppo_core *core, const char *name, float *out, size_t capacity);
 int ppo_rollout_set(ppo_core *core, const char *name, const float *in, size_t count);
 
@@ -282,6 +315,11 @@ int ppo_loss_grad(ppo_core *core, const float *obs, const float *actions, const 
 int ppo_loss_grad_vf(ppo_core *core, const float *obs, const float *actions, const float *advs, const float *returns,
                      const float *old_neglogp, const float *old_values, int B, float cliprange, float cliprange_vf, float *grads,
                      float *losses);
+/* ... with masks [B][act_dim] on a masking core (host pointers): the loss over the allowed actions; a recorded action its mask
+ * forbids is PPO_ERR_INVALID.  cliprange_vf is read only in SEPARATE mode. */
+int ppo_loss_grad_masked(ppo_core *core, const float *obs, const float *actions, const uint8_t *masks, const float *advs,
+                         const float *returns, const float *old_neglogp, const float *old_values, int B, float cliprange,
+                         float cliprange_vf, float *grads, float *losses);
 /* rollout + update on the synthetic env; env-steps/s accounting is the caller's (ppo2.hpp:337-341) */
 int ppo_learn_update_synthetic(ppo_core *core, float lr, float cliprange, float *mean_losses);
 

@@ -87,6 +87,8 @@ def load():
         "ppo_core_create_nvec": ([C.POINTER(CoreDesc), ip, C.c_int, C.POINTER(core)], C.c_int),
         "ppo_core_action_space": ([core], C.c_int),
         "ppo_core_action_nvec": ([core, ip, C.c_int], C.c_int),
+        "ppo_core_set_action_masking": ([core, C.c_int], C.c_int),
+        "ppo_core_action_masking": ([core], C.c_int),
         "ppo_core_destroy": ([core], None),
         "ppo_core_load_meta_txt": ([core, C.c_char_p], C.c_int),
         "ppo_core_set_vf_clip": ([core, C.c_int], C.c_int),
@@ -108,6 +110,8 @@ def load():
         "ppo_policy_step": ([core, fp, C.c_int, fp, fp, fp, fp, C.c_int], C.c_int),
         "ppo_policy_value": ([core, fp, C.c_int, fp, C.c_int], C.c_int),
         "ppo_policy_mean": ([core, fp, C.c_int, fp, C.c_int], C.c_int),
+        "ppo_policy_step_masked": ([core, fp, C.c_int, fp, vp, fp, fp, fp, C.c_int], C.c_int),
+        "ppo_policy_mean_masked": ([core, fp, C.c_int, vp, fp, C.c_int], C.c_int),
         "ppo_vecnorm_reset": ([core, fp, fp, C.c_int], C.c_int),
         "ppo_vecnorm_step": ([core, fp, fp, fp, fp, fp, C.c_int], C.c_int),
         "ppo_vecnorm_replay": ([core, fp, fp, fp, C.c_int, fp, fp, C.c_int], C.c_int),
@@ -121,6 +125,8 @@ def load():
         "ppo_runner_act": ([core, C.c_int, fp, C.c_int], C.c_int),
         "ppo_runner_observe": ([core, C.c_int, fp, fp, fp, C.c_int], C.c_int),
         "ppo_runner_finish": ([core], C.c_int),
+        "ppo_runner_reset_masked": ([core, fp, vp, C.c_int], C.c_int),
+        "ppo_runner_observe_masked": ([core, C.c_int, fp, fp, fp, vp, C.c_int], C.c_int),
         "ppo_runner_rollout_host": ([core, C.c_void_p, C.c_void_p, fp], C.c_int),
         "ppo_runner_rollout_replay": ([core, fp, fp, fp, fp], C.c_int),
         "ppo_synth_env_reset": ([core], C.c_int),
@@ -139,6 +145,7 @@ def load():
         "ppo_advnorm": ([core, fp, fp, C.c_int, fp], C.c_int),
         "ppo_loss_grad": ([core, fp, fp, fp, fp, fp, fp, C.c_int, C.c_float, fp, fp], C.c_int),
         "ppo_loss_grad_vf": ([core, fp, fp, fp, fp, fp, fp, C.c_int, C.c_float, C.c_float, fp, fp], C.c_int),
+        "ppo_loss_grad_masked": ([core, fp, fp, vp, fp, fp, fp, fp, C.c_int, C.c_float, C.c_float, fp, fp], C.c_int),
         "ppo_learn_update_synthetic": ([core, C.c_float, C.c_float, fp], C.c_int),
         "ppo_comm_get_unique_id": ([C.c_char_p], C.c_int),
         "ppo_comm_init": ([core, C.c_char_p, C.c_int, C.c_int], C.c_int),

@@ -25,6 +25,7 @@ ACTIVATION_NAMES = {v: k for k, v in ACTIVATIONS.items()}
 ACTION_SPACES = {"box": _lib.PPO_ACTION_BOX, "discrete": _lib.PPO_ACTION_DISCRETE, "multi_discrete": _lib.PPO_ACTION_MULTI_DISCRETE,
                  "multi_binary": _lib.PPO_ACTION_MULTI_BINARY}
 ACTION_SPACE_NAMES = {v: k for k, v in ACTION_SPACES.items()}
+# the rollout buffers every core has (a masking core adds "action_masks", [n_batch, act_dim])
 BUFFER_WIDTH = {"obs": None, "returns": 1, "dones": 1, "actions": None, "values": 1, "neglogpacs": 1,
                 "true_rewards": 1, "unnormalized_rewards": 1}
 
@@ -52,6 +53,24 @@ def _addr(a):
 
 def _is_dev(a):
     return hasattr(a, "is_cuda") and a.is_cuda
+
+
+def _mask(m, n, width):
+    """An action mask (bool or 0 / 1 values, [n, width]) as the uint8 array the C ABI takes.  A mask of another shape, or with a value
+    that is not an integer 0 .. 255, is a ValueError here (the library would read past the array, or see the value rounded); the
+    other integers go through unchanged, so that the library reports them with its row and column."""
+    if m is None:
+        return None
+    a = np.asarray(m)
+    if a.shape != (n, width):
+        raise ValueError(f"an action mask has shape ({n}, {width}) (one entry per logit), not {a.shape}")
+    if a.dtype != np.uint8:
+        f = a.astype(np.float64)
+        bad = ~np.isfinite(f) | (f != np.round(f)) | (f < 0) | (f > 255)
+        if bad.any():
+            r, j = (int(x) for x in np.argwhere(bad)[0])
+            raise ValueError(f"action mask row {r}, column {j} is {a[r, j]}: a mask entry is 1 (allowed) or 0 (forbidden)")
+    return np.ascontiguousarray(a, np.uint8)
 
 
 def meta_parse(path: str):
@@ -229,6 +248,19 @@ class PPOCore:
             _check(self.lib, r)
         return r
 
+    @property
+    def action_masking(self) -> bool:
+        """Invalid-action masks on this core (Discrete / MultiDiscrete only): the *_masked calls and mask= / masks= arguments, and the
+        "action_masks" rollout buffer.  Off at creation."""
+        r = self.lib.ppo_core_action_masking(self._h)
+        if r < 0:
+            _check(self.lib, r)
+        return bool(r)
+
+    @action_masking.setter
+    def action_masking(self, on: bool):
+        _check(self.lib, self.lib.ppo_core_set_action_masking(self._h, int(bool(on))))
+
     def graph_builds(self) -> int:
         """CUDA graphs captured and instantiated since the core was created."""
         n = C.c_uint64()
@@ -272,12 +304,16 @@ class PPOCore:
         return dict(kernel_launches=c.kernel_launches, graph_launches=c.graph_launches, h2d_bytes=c.h2d_bytes, d2h_bytes=c.d2h_bytes)
 
     # ---- policy
-    def policy_step(self, obs, eps=None):
+    def policy_step(self, obs, eps=None, mask=None):
         obs = _f32(obs)
         n = obs.shape[0]
         e = None if eps is None else _f32(eps)
         act, val, nlp = np.zeros((n, self.AW), np.float32), np.zeros(n, np.float32), np.zeros(n, np.float32)
-        _check(self.lib, self.lib.ppo_policy_step(self._h, _addr(obs), n, _addr(e), _addr(act), _addr(val), _addr(nlp), PPO_HOST))
+        if mask is None:
+            _check(self.lib, self.lib.ppo_policy_step(self._h, _addr(obs), n, _addr(e), _addr(act), _addr(val), _addr(nlp), PPO_HOST))
+        else:
+            m = _mask(mask, n, self.A)
+            _check(self.lib, self.lib.ppo_policy_step_masked(self._h, _addr(obs), n, _addr(e), _addr(m), _addr(act), _addr(val), _addr(nlp), PPO_HOST))
         return act, val, nlp
 
     def policy_value(self, obs):
@@ -286,10 +322,14 @@ class PPOCore:
         _check(self.lib, self.lib.ppo_policy_value(self._h, _addr(obs), obs.shape[0], _addr(val), PPO_HOST))
         return val
 
-    def policy_mean(self, obs):
+    def policy_mean(self, obs, mask=None):
         obs = _f32(obs)
         act = np.zeros((obs.shape[0], self.AW), np.float32)
-        _check(self.lib, self.lib.ppo_policy_mean(self._h, _addr(obs), obs.shape[0], _addr(act), PPO_HOST))
+        if mask is None:
+            _check(self.lib, self.lib.ppo_policy_mean(self._h, _addr(obs), obs.shape[0], _addr(act), PPO_HOST))
+        else:
+            m = _mask(mask, obs.shape[0], self.A)
+            _check(self.lib, self.lib.ppo_policy_mean_masked(self._h, _addr(obs), obs.shape[0], _addr(m), _addr(act), PPO_HOST))
         return act
 
     # ---- VecNormalize
@@ -356,18 +396,26 @@ class PPOCore:
                                           T, N, gamma, lam, _addr(advs), _addr(returns), PPO_DEVICE))
 
     # ---- rollout
-    def runner_reset(self, raw_obs):
+    def runner_reset(self, raw_obs, mask=None):
         raw = _f32(raw_obs)
-        _check(self.lib, self.lib.ppo_runner_reset(self._h, _addr(raw), PPO_HOST))
+        if mask is None:
+            _check(self.lib, self.lib.ppo_runner_reset(self._h, _addr(raw), PPO_HOST))
+        else:
+            m = _mask(mask, self.n_envs, self.A)
+            _check(self.lib, self.lib.ppo_runner_reset_masked(self._h, _addr(raw), _addr(m), PPO_HOST))
 
     def runner_act(self, t, out: Optional[np.ndarray] = None):
         act = out if out is not None else np.zeros((self.n_envs, self.AW), np.float32)
         _check(self.lib, self.lib.ppo_runner_act(self._h, t, _addr(act), PPO_HOST))
         return act
 
-    def runner_observe(self, t, raw_obs, raw_rew, done):
+    def runner_observe(self, t, raw_obs, raw_rew, done, mask=None):
         raw, rew, dn = _f32(raw_obs), _f32(raw_rew).ravel(), _f32(done).ravel()
-        _check(self.lib, self.lib.ppo_runner_observe(self._h, t, _addr(raw), _addr(rew), _addr(dn), PPO_HOST))
+        if mask is None:
+            _check(self.lib, self.lib.ppo_runner_observe(self._h, t, _addr(raw), _addr(rew), _addr(dn), PPO_HOST))
+        else:
+            m = _mask(mask, self.n_envs, self.A)
+            _check(self.lib, self.lib.ppo_runner_observe_masked(self._h, t, _addr(raw), _addr(rew), _addr(dn), _addr(m), PPO_HOST))
 
     def runner_finish(self):
         _check(self.lib, self.lib.ppo_runner_finish(self._h))
@@ -406,7 +454,7 @@ class PPOCore:
         _check(self.lib, self.lib.ppo_rollout_synthetic(self._h))
 
     def rollout_get(self, name):
-        w = BUFFER_WIDTH[name] or (self.O if name == "obs" else self.AW)
+        w = self.A if name == "action_masks" else BUFFER_WIDTH[name] or (self.O if name == "obs" else self.AW)
         out = np.zeros((self.n_batch, w), np.float32)
         _check(self.lib, self.lib.ppo_rollout_get(self._h, name.encode(), _addr(out), out.size))
         return out
@@ -450,10 +498,16 @@ class PPOCore:
         _check(self.lib, self.lib.ppo_advnorm(self._h, _addr(r), _addr(v), r.size, _addr(out)))
         return out
 
-    def loss_grad(self, obs, actions, advs, returns, old_neglogp, old_values, cliprange, cliprange_vf=None):
+    def loss_grad(self, obs, actions, advs, returns, old_neglogp, old_values, cliprange, cliprange_vf=None, masks=None):
         o, a = _f32(obs), _f32(actions)
         ad, r, on, ov = _f32(advs).ravel(), _f32(returns).ravel(), _f32(old_neglogp).ravel(), _f32(old_values).ravel()
         grads, losses = np.zeros(self.P, np.float32), np.zeros(5, np.float32)
+        if masks is not None:
+            m = _mask(masks, o.shape[0], self.A)
+            _check(self.lib, self.lib.ppo_loss_grad_masked(self._h, _addr(o), _addr(a), _addr(m), _addr(ad), _addr(r), _addr(on), _addr(ov),
+                                                           o.shape[0], cliprange, float("nan") if cliprange_vf is None else cliprange_vf,
+                                                           _addr(grads), _addr(losses)))
+            return grads, losses
         args = (self._h, _addr(o), _addr(a), _addr(ad), _addr(r), _addr(on), _addr(ov), o.shape[0], cliprange)
         if cliprange_vf is None:
             _check(self.lib, self.lib.ppo_loss_grad(*args, _addr(grads), _addr(losses)))

@@ -176,11 +176,18 @@ __device__ __forceinline__ void normal4(uint64_t seed, uint32_t a, uint32_t b, u
 }
 
 // ---- categorical head (Stable-Baselines' CategoricalProbabilityDistribution) of one sample: logits l[j * ld], j < n
-// sample = argmax_j (l_j - log(-log(u_j))), u uniform in [0, 1) from stream (seed, env, step, block j/4, PPO_TAG_CATEG) or given;
-// u = 0 gives -inf and is never taken; ties go to the first index (TF's ArgMax)
-__device__ __forceinline__ int cat_sample(const float* l, int ld, int n, const float* u_given, uint64_t seed, uint32_t env, uint32_t step) {
+// Action masks (sb3-contrib's MaskableCategorical): m is the sample's mask word, bit j set = logit j allowed; every helper works
+// over the allowed logits S only, as if the forbidden ones were -inf.  m = ~0 (no mask) is the arithmetic of the unmasked head,
+// in the same order.  S must not be empty (the callers check the masks they are handed).
+// first allowed index of m (0 for m = ~0)
+__device__ __forceinline__ int cat_first(uint64_t m) { return __ffsll((long long)m) - 1; }
+__device__ __forceinline__ bool cat_allowed(uint64_t m, int j) { return (m >> j) & 1ull; }
+// sample = argmax_{j in S} (l_j - log(-log(u_j))), u uniform in [0, 1) from stream (seed, env, step, block j/4, PPO_TAG_CATEG) or
+// given; u = 0 gives -inf and is never taken (unless it is all S has); ties go to the first index (TF's ArgMax)
+__device__ __forceinline__ int cat_sample(const float* l, int ld, int n, const float* u_given, uint64_t seed, uint32_t env, uint32_t step,
+                                          uint64_t m = ~0ull) {
     float best = -__int_as_float(0x7f800000);
-    int bi = 0;
+    int bi = cat_first(m);
     for (int j0 = 0; j0 < n; j0 += 4) {
         uint4 w = make_uint4(0u, 0u, 0u, 0u);
         if (!u_given) w = philox4x32_10(make_uint4(env, step, (uint32_t)(j0 >> 2), PPO_TAG_CATEG), make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
@@ -188,7 +195,7 @@ __device__ __forceinline__ int cat_sample(const float* l, int ld, int n, const f
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
             const int j = j0 + q;
-            if (j < n) {
+            if (j < n && cat_allowed(m, j)) {
                 const float u = u_given ? u_given[j] : u32_to_unit(wv[q]);
                 const float g = l[j * ld] - logf(-logf(u));
                 if (g > best) { best = g; bi = j; }
@@ -197,42 +204,51 @@ __device__ __forceinline__ int cat_sample(const float* l, int ld, int n, const f
     }
     return bi;
 }
-// deterministic action: argmax_j l_j, first index on ties
-__device__ __forceinline__ int cat_argmax(const float* l, int ld, int n) {
-    int bi = 0;
-    for (int j = 1; j < n; ++j)
-        if (l[j * ld] > l[bi * ld]) bi = j;
+// deterministic action: argmax_{j in S} l_j, first index on ties
+__device__ __forceinline__ int cat_argmax(const float* l, int ld, int n, uint64_t m = ~0ull) {
+    int bi = cat_first(m);
+    for (int j = bi + 1; j < n; ++j)
+        if (cat_allowed(m, j) && l[j * ld] > l[bi * ld]) bi = j;
     return bi;
 }
-// max shift and partition: mx = max_j l_j, returns z = sum_j exp(l_j - mx)
-__device__ __forceinline__ float cat_partition(const float* l, int ld, int n, float& mx) {
-    mx = l[0];
-    for (int j = 1; j < n; ++j) mx = fmaxf(mx, l[j * ld]);
+// max shift and partition: mx = max_{j in S} l_j, returns z = sum_{j in S} exp(l_j - mx)
+__device__ __forceinline__ float cat_partition(const float* l, int ld, int n, float& mx, uint64_t m = ~0ull) {
+    const int f = cat_first(m);
+    mx = l[f * ld];
+    for (int j = f + 1; j < n; ++j)
+        if (cat_allowed(m, j)) mx = fmaxf(mx, l[j * ld]);
     float z = 0.f;
-    for (int j = 0; j < n; ++j) z += expf(l[j * ld] - mx);
+    for (int j = f; j < n; ++j)
+        if (cat_allowed(m, j)) z += expf(l[j * ld] - mx);
     return z;
 }
 // neglogp(a) = log z - (l_a - mx), as softmax_cross_entropy_with_logits_v2
-__device__ __forceinline__ float cat_neglogp(const float* l, int ld, int n, int a) {
+__device__ __forceinline__ float cat_neglogp(const float* l, int ld, int n, int a, uint64_t m = ~0ull) {
     float mx;
-    const float z = cat_partition(l, ld, n, mx);
+    const float z = cat_partition(l, ld, n, mx, m);
     return logf(z) - (l[a * ld] - mx);
 }
-// entropy H = sum_j p_j (log z - a0_j), a0 = l - mx, p = exp(a0) / z (CategoricalProbabilityDistribution.entropy)
-__device__ __forceinline__ float cat_entropy(const float* l, int ld, int n, float mx, float z) {
+// entropy H = sum_{j in S} p_j (log z - a0_j), a0 = l - mx, p = exp(a0) / z (CategoricalProbabilityDistribution.entropy; sb3-contrib's
+// where(mask, p log p, 0))
+__device__ __forceinline__ float cat_entropy(const float* l, int ld, int n, float mx, float z, uint64_t m = ~0ull) {
     const float lz = logf(z);
     float h = 0.f;
     for (int j = 0; j < n; ++j) {
+        if (!cat_allowed(m, j)) continue;
         const float a0 = l[j * ld] - mx;
         h += (expf(a0) / z) * (lz - a0);
     }
     return h;
 }
-// overwrites the logits with dL/dl_j = g_nlp (p_j - [j == a]) + ent_w p_j (log p_j + H): the pg term through neglogp (TF's
-// softmax - labels) and -ent_coef/B * dH/dl_j with ent_w = ent_coef / B
-__device__ __forceinline__ void cat_dlogits(float* l, int ld, int n, int a, float mx, float z, float H, float g_nlp, float ent_w) {
+// overwrites the logits with dL/dl_j = g_nlp (p_j - [j == a]) + ent_w p_j (log p_j + H) for j in S: the pg term through neglogp (TF's
+// softmax - labels) and -ent_coef/B * dH/dl_j with ent_w = ent_coef / B; exactly 0 for a forbidden j (torch.where blocks it)
+__device__ __forceinline__ void cat_dlogits(float* l, int ld, int n, int a, float mx, float z, float H, float g_nlp, float ent_w, uint64_t m = ~0ull) {
     const float lz = logf(z);
     for (int j = 0; j < n; ++j) {
+        if (!cat_allowed(m, j)) {
+            l[j * ld] = 0.f;
+            continue;
+        }
         const float a0 = l[j * ld] - mx;
         const float p = expf(a0) / z;
         l[j * ld] = g_nlp * (p - (j == a ? 1.f : 0.f)) + ent_w * p * ((a0 - lz) + H);
@@ -241,19 +257,20 @@ __device__ __forceinline__ void cat_dlogits(float* l, int ld, int n, int a, floa
 // one sample's categorical train terms: neglogp(a) and entropy H of the logits, the clipped surrogate of pg_term, and the
 // logits overwritten with dL/dl_j (cat_dlogits, ent_w = ent_coef / B)
 __device__ __forceinline__ PgTerm cat_train_term(float* l, int ld, int n, int a, float adv, float oldn, float cr, float invB, float ent_w,
-                                                 float& H) {
+                                                 float& H, uint64_t m = ~0ull) {
     float mx;
-    const float z = cat_partition(l, ld, n, mx);
+    const float z = cat_partition(l, ld, n, mx, m);
     const float nlp = logf(z) - (l[a * ld] - mx);
-    H = cat_entropy(l, ld, n, mx, z);
+    H = cat_entropy(l, ld, n, mx, z, m);
     const PgTerm t = pg_term(adv, oldn, nlp, cr, invB);
-    cat_dlogits(l, ld, n, a, mx, z, H, t.g_nlp, ent_w);
+    cat_dlogits(l, ld, n, a, mx, z, H, t.g_nlp, ent_w, m);
     return t;
 }
 
 // ---- MultiDiscrete head (MultiCategoricalProbabilityDistribution): k categoricals side by side over slices of the n <= 64
 // logits, given as a mask of slice starts (bit j set: a slice starts at logit j; bit 0 always set, k = popcount); an action is
-// one index per slice, within the slice.  The categorical helpers above, per slice.
+// one index per slice, within the slice.  The categorical helpers above, per slice; the action mask m is over all n logits (the
+// slice that starts at s0 sees m >> s0).
 // end of the slice that starts at s0: the next start, or n
 __device__ __forceinline__ int md_slice_end(uint64_t starts, int s0, int n) {
     const uint64_t rest = s0 >= 63 ? 0ull : starts & (~0ull << (s0 + 1));
@@ -263,9 +280,9 @@ __device__ __forceinline__ int md_slice_end(uint64_t starts, int s0, int n) {
 // what Discrete(n) draws); put(i, index) receives slice i's index once the slice is finished
 template <class PUT>
 __device__ __forceinline__ void md_sample(const float* l, int ld, int n, uint64_t starts, const float* u_given, uint64_t seed, uint32_t env,
-                                          uint32_t step, PUT put) {
+                                          uint32_t step, PUT put, uint64_t m = ~0ull) {
     float best = -__int_as_float(0x7f800000);
-    int i = 0, s0 = 0, bi = 0;
+    int i = 0, s0 = 0, bi = cat_first(m);
     for (int j0 = 0; j0 < n; j0 += 4) {
         uint4 w = make_uint4(0u, 0u, 0u, 0u);
         if (!u_given) w = philox4x32_10(make_uint4(env, step, (uint32_t)(j0 >> 2), PPO_TAG_CATEG), make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
@@ -274,14 +291,17 @@ __device__ __forceinline__ void md_sample(const float* l, int ld, int n, uint64_
         for (int q = 0; q < 4; ++q) {
             const int j = j0 + q;
             if (j < n) {
-                if (j > 0 && ((starts >> j) & 1ull)) {  // slice i done; ties stayed on its first index
+                if (j > 0 && ((starts >> j) & 1ull)) {  // slice i done; ties stayed on its first allowed index
                     put(i++, bi - s0);
-                    s0 = bi = j;
+                    s0 = j;
+                    bi = cat_first(m & (~0ull << j));
                     best = -__int_as_float(0x7f800000);
                 }
-                const float u = u_given ? u_given[j] : u32_to_unit(wv[q]);
-                const float g = l[j * ld] - logf(-logf(u));
-                if (g > best) { best = g; bi = j; }
+                if (cat_allowed(m, j)) {
+                    const float u = u_given ? u_given[j] : u32_to_unit(wv[q]);
+                    const float g = l[j * ld] - logf(-logf(u));
+                    if (g > best) { best = g; bi = j; }
+                }
             }
         }
     }
@@ -291,25 +311,27 @@ __device__ __forceinline__ void md_sample(const float* l, int ld, int n, uint64_
 // clipped surrogate of pg_term, and the logits overwritten with dL/dl: slice i as cat_dlogits with its own entropy H_i.
 // act[i * ald]: slice i's index
 __device__ __forceinline__ PgTerm md_train_term(float* l, int ld, int n, uint64_t starts, const float* act, int ald, float adv, float oldn,
-                                                float cr, float invB, float ent_w, float& H) {
+                                                float cr, float invB, float ent_w, float& H, uint64_t m = ~0ull) {
     float nlp = 0.f;
     H = 0.f;
     for (int i = 0, s0 = 0; s0 < n; ++i) {
         const int s1 = md_slice_end(starts, s0, n);
         const float* s = l + s0 * ld;
+        const uint64_t ms = m >> s0;
         float mx;
-        const float z = cat_partition(s, ld, s1 - s0, mx);
+        const float z = cat_partition(s, ld, s1 - s0, mx, ms);
         nlp += logf(z) - (s[(int)act[i * ald] * ld] - mx);
-        H += cat_entropy(s, ld, s1 - s0, mx, z);
+        H += cat_entropy(s, ld, s1 - s0, mx, z, ms);
         s0 = s1;
     }
     const PgTerm t = pg_term(adv, oldn, nlp, cr, invB);
     for (int i = 0, s0 = 0; s0 < n; ++i) {
         const int s1 = md_slice_end(starts, s0, n);
         float* s = l + s0 * ld;
+        const uint64_t ms = m >> s0;
         float mx;
-        const float z = cat_partition(s, ld, s1 - s0, mx);
-        cat_dlogits(s, ld, s1 - s0, (int)act[i * ald], mx, z, cat_entropy(s, ld, s1 - s0, mx, z), t.g_nlp, ent_w);
+        const float z = cat_partition(s, ld, s1 - s0, mx, ms);
+        cat_dlogits(s, ld, s1 - s0, (int)act[i * ald], mx, z, cat_entropy(s, ld, s1 - s0, mx, z, ms), t.g_nlp, ent_w, ms);
         s0 = s1;
     }
     return t;

@@ -569,6 +569,36 @@ __global__ void clamp_kernel(const float* __restrict__ x, size_t n, float lo, fl
 
 __global__ void bump_counter_kernel(uint32_t* c) { *c += 1u; }
 
+// Action masks in device memory: [n][A] bytes (1 allowed, 0 forbidden) -> one word per row, bit j = logit j allowed.  A row with
+// another byte value, or with a categorical (the slice that starts at each bit of `starts`) that allows nothing, is invalid: its
+// code (row << 32 | kind << 16 | column or slice << 8 | value; kind 1 = value, 2 = empty slice) goes into the sticky *err by
+// atomicMin, so the lowest bad row wins, and its word allows every logit (the kernels never see an empty categorical).
+enum { MASK_ERR_VALUE = 1, MASK_ERR_EMPTY = 2 };
+__global__ void mask_pack_kernel(const uint8_t* __restrict__ in, int n, int A, uint64_t starts, uint64_t* __restrict__ out,
+                                 unsigned long long* err) {
+    const int row = blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= n) return;
+    const uint64_t all = A >= 64 ? ~0ull : (1ull << A) - 1ull;
+    uint64_t w = 0ull;
+    unsigned long long code = ~0ull;
+    for (int j = 0; j < A; ++j) {
+        const unsigned v = in[(size_t)row * A + j];
+        if (v > 1u && code == ~0ull) code = ((unsigned long long)row << 32) | (MASK_ERR_VALUE << 16) | ((unsigned)j << 8) | v;
+        w |= (uint64_t)(v & 1u) << j;
+    }
+    for (int i = 0, s0 = 0; s0 < A && code == ~0ull; ++i) {
+        const int s1 = md_slice_end(starts, s0, A);
+        const uint64_t sl = (s1 - s0 >= 64 ? ~0ull : (1ull << (s1 - s0)) - 1ull) << s0;
+        if (!(w & sl)) code = ((unsigned long long)row << 32) | (MASK_ERR_EMPTY << 16) | ((unsigned)i << 8);
+        s0 = s1;
+    }
+    if (code != ~0ull) {
+        atomicMin(err, code);
+        w = all;
+    }
+    out[row] = w;
+}
+
 // ------------------------------------------------------------------------------------------------
 // GAE(lambda) reverse scan (Runner::set_returns, runner.hpp:159-191) over time-major [T][N] buffers.
 // One thread per (env, chunk of `chunk` steps).  A chunk that does not end at T-1 first runs `warm` extra

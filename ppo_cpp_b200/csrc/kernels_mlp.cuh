@@ -224,6 +224,10 @@ struct PolicyArgs {
     const float* dones_in;  // [n] done flag of the previous env step (runner.hpp:110)
     float* dones_store;     // [n]
     int mode;  // 0: step (pi + V + sample), 1: value only, 2: mean only (deterministic action)
+    // action masks of a Discrete / MultiDiscrete head (device_common.cuh): [n] words, bit j = logit j allowed, or NULL (all allowed);
+    // mask_store: rollout slab of step t that receives them, or NULL
+    const uint64_t* mask;
+    uint64_t* mask_store;
 };
 // the slice-start mask of a MultiDiscrete head from its two halves
 __host__ __device__ __forceinline__ uint64_t md_starts(uint32_t lo, uint32_t hi) { return ((uint64_t)hi << 32) | lo; }
@@ -262,21 +266,30 @@ __device__ __forceinline__ void gauss_policy_row(const PolicyArgs& a, int row, c
     store_neglogp(a, row, gauss_neglogp_rn(ss, sl, A));
 }
 
+// the action mask word of env `row` (all ones without masks), stored into the rollout slab when the step records one
+__device__ __forceinline__ uint64_t policy_mask_word(const PolicyArgs& a, int row) {
+    const uint64_t m = a.mask ? a.mask[row] : ~0ull;
+    if (a.mask_store) a.mask_store[row] = m;
+    return m;
+}
+
 // Categorical policy step of env `row` (logits l[j * ld]): the index as fp32 in one column, sampled (mode 0; a.eps: [n][A]
-// uniforms when given) or argmax (mode 2)
+// uniforms when given) or argmax (mode 2), over the logits the row's mask allows
 __device__ __forceinline__ void cat_policy_row(const PolicyArgs& a, int row, const float* l, int ld) {
+    const uint64_t m = policy_mask_word(a, row);
     const int j = a.mode == 0 ? cat_sample(l, ld, a.d.A, a.eps ? a.eps + (size_t)row * a.d.A : nullptr, a.seed, a.env_id0 + (uint32_t)row,
-                                           a.eps ? 0u : *a.step_ctr)
-                              : cat_argmax(l, ld, a.d.A);
+                                           a.eps ? 0u : *a.step_ctr, m)
+                              : cat_argmax(l, ld, a.d.A, m);
     if (a.action) a.action[row] = (float)j;
     if (a.act_store) a.act_store[row] = (float)j;
-    if (a.mode == 0) store_neglogp(a, row, cat_neglogp(l, ld, a.d.A, j));
+    if (a.mode == 0) store_neglogp(a, row, cat_neglogp(l, ld, a.d.A, j, m));
 }
 
 // MultiDiscrete policy step: k indices in k columns, sampled per slice (mode 0, neglogp their sum) or argmax per slice (mode 2)
 __device__ __forceinline__ void md_policy_row(const PolicyArgs& a, int row, const float* l, int ld) {
     const uint64_t starts = md_starts(a.md_lo, a.md_hi);
     const int k = __popcll((long long)starts);
+    const uint64_t m = policy_mask_word(a, row);
     auto put = [&](int i, int j) {
         if (a.action) a.action[(size_t)row * k + i] = (float)j;
         if (a.act_store) a.act_store[(size_t)row * k + i] = (float)j;
@@ -288,14 +301,15 @@ __device__ __forceinline__ void md_policy_row(const PolicyArgs& a, int row, cons
                   [&](int i, int j) {
                       put(i, j);
                       const int s1 = md_slice_end(starts, s0, a.d.A);
-                      nlp += cat_neglogp(l + s0 * ld, ld, s1 - s0, j);
+                      nlp += cat_neglogp(l + s0 * ld, ld, s1 - s0, j, m >> s0);
                       s0 = s1;
-                  });
+                  },
+                  m);
         store_neglogp(a, row, nlp);
     } else {
         for (int i = 0, s0 = 0; s0 < a.d.A; ++i) {
             const int s1 = md_slice_end(starts, s0, a.d.A);
-            put(i, cat_argmax(l + s0 * ld, ld, s1 - s0));
+            put(i, cat_argmax(l + s0 * ld, ld, s1 - s0, m >> s0));
             s0 = s1;
         }
     }
@@ -422,9 +436,10 @@ struct TrainArgs {
     float* partial;  // [gridDim.x][PS]
     int PS;
     long long* prof;  // optional [2][32] phase timestamps of CTA 0 of each tower (U family, PPO_UMMA_PROF=1)
+    const uint64_t* mask;  // action masks of a Discrete / MultiDiscrete head by physical row (as act), or NULL (all allowed)
 };
-// the MultiDiscrete slice mask fills padding: every other field, and the parameters behind these structs, keep their offsets
-static_assert(sizeof(PolicyArgs) == 224 && sizeof(TrainArgs) == 224, "PolicyArgs / TrainArgs changed size");
+// the MultiDiscrete slice mask fills padding; the action-mask pointers are appended, so every earlier field keeps its offset
+static_assert(sizeof(PolicyArgs) == 240 && sizeof(TrainArgs) == 232, "PolicyArgs / TrainArgs changed size");
 
 // floats of one stored action: the action vector (Box), the index of a categorical head, the k indices of a MultiDiscrete head,
 // the A bits of a MultiBinary head
@@ -433,13 +448,20 @@ __device__ __forceinline__ int act_cols(const TrainArgs& a) {
     return HEAD == HEAD_DISCRETE ? 1 : HEAD == HEAD_MULTI_DISCRETE ? __popcll((long long)md_starts(a.md_lo, a.md_hi)) : a.d.A;
 }
 
+// the action mask word of the sample at physical row `row` (all ones without masks; a MultiBinary head has none)
+template <int HEAD>
+__device__ __forceinline__ uint64_t train_mask_word(const TrainArgs& a, int row) {
+    if constexpr (HEAD == HEAD_DISCRETE || HEAD == HEAD_MULTI_DISCRETE) return a.mask ? a.mask[row] : ~0ull;
+    else return ~0ull;
+}
+
 // one sample's train terms of a head without logstd over n logits l[j * ld]: neglogp of the stored action (act[j * ald]) and
-// entropy H, the clipped surrogate of pg_term, and the logits overwritten with dL/dl (ent_w = ent_coef / B)
+// entropy H, the clipped surrogate of pg_term, and the logits overwritten with dL/dl (ent_w = ent_coef / B); m: the sample's mask word
 template <int HEAD>
 __device__ __forceinline__ PgTerm head_train_term(const TrainArgs& a, float* l, int ld, int n, const float* act, int ald, float adv, float oldn,
-                                                  float cr, float invB, float ent_w, float& H) {
-    if constexpr (HEAD == HEAD_DISCRETE) return cat_train_term(l, ld, n, (int)act[0], adv, oldn, cr, invB, ent_w, H);
-    else if constexpr (HEAD == HEAD_MULTI_DISCRETE) return md_train_term(l, ld, n, md_starts(a.md_lo, a.md_hi), act, ald, adv, oldn, cr, invB, ent_w, H);
+                                                  float cr, float invB, float ent_w, float& H, uint64_t m) {
+    if constexpr (HEAD == HEAD_DISCRETE) return cat_train_term(l, ld, n, (int)act[0], adv, oldn, cr, invB, ent_w, H, m);
+    else if constexpr (HEAD == HEAD_MULTI_DISCRETE) return md_train_term(l, ld, n, md_starts(a.md_lo, a.md_hi), act, ald, adv, oldn, cr, invB, ent_w, H, m);
     else return bern_train_term(l, ld, n, act, ald, adv, oldn, cr, invB, ent_w, H);
 }
 
@@ -510,11 +532,13 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         const int s0 = a.slot0 + tile * TM;
         const int nv = min(TM, a.slot0 + a.count - s0);
+        uint64_t mw = ~0ull;  // thread tid's sample: its action mask word
         if (tid < TM) {
             float adv = 0.f, r = 0.f, on = 0.f, ov = 0.f;
             int row = 0;
             if (tid < nv) {
                 row = a.gather ? a.gather[s0 + tid] : (s0 + tid);
+                mw = train_mask_word<HEAD>(a, row);
                 r = a.ret[row];
                 ov = a.val[row];
                 on = a.nlp[row];
@@ -544,7 +568,7 @@ __global__ void __launch_bounds__(NT) train_tile_kernel(const TrainArgs a) {
             float* l = MU + m;
             if (m < nv) {
                 float H;
-                const PgTerm t = head_train_term<HEAD>(a, l, TM, d.A, Ac + m, TM, s_adv[m], s_oldn[m], cr, a.invB, a.ent_coef * a.invB, H);
+                const PgTerm t = head_train_term<HEAD>(a, l, TM, d.A, Ac + m, TM, s_adv[m], s_oldn[m], cr, a.invB, a.ent_coef * a.invB, H, mw);
                 l_pg += t.pg;
                 l_kl += t.kl;
                 l_cf += t.cf;

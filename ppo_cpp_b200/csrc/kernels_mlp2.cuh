@@ -279,11 +279,13 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         const int s0 = a.slot0 + tile * TM;
         const int nv = min(TM, a.slot0 + a.count - s0);
+        uint64_t mw = ~0ull;  // thread tid's sample (the loss stage's thread for it): its action mask word
         if (tid < TM) {
             float adv = 0.f, r = 0.f, on = 0.f, ov = 0.f;
             int row = 0;
             if (tid < nv) {
                 row = a.gather ? a.gather[s0 + tid] : (s0 + tid);
+                mw = train_mask_word<HEAD>(a, row);
                 r = a.ret[row];
                 ov = a.val[row];
                 on = a.nlp[row];
@@ -334,7 +336,7 @@ __global__ void __launch_bounds__(NTH, 1) train_fused_kernel(const TrainArgs a) 
                 float* l = MU + m;
                 if (m < nv) {
                     float H;
-                    const PgTerm t = head_train_term<HEAD>(a, l, TM, d.A, Ac + m, TM, s_adv[m], s_oldn[m], cr, a.invB, a.ent_coef * a.invB, H);
+                    const PgTerm t = head_train_term<HEAD>(a, l, TM, d.A, Ac + m, TM, s_adv[m], s_oldn[m], cr, a.invB, a.ent_coef * a.invB, H, mw);
                     l_pg += t.pg;
                     l_kl += t.kl;
                     l_cf += t.cf;

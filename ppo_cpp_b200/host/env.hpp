@@ -26,6 +26,11 @@ public:
     // a MultiDiscrete env's choices per action column (Stable-Baselines' nvec); empty for the other spaces
     virtual std::vector<int> get_action_space_nvec() { return {}; }
     virtual int get_num_envs() { return 1; }
+    // invalid-action masks (sb3-contrib's action_masks()), Discrete and MultiDiscrete envs only: whether the env has them, and the
+    // mask of its current observation, [n_envs, get_action_space_size()] of 0 / 1 (1 allowed) in logit order (for MultiDiscrete the
+    // nvec slices side by side); every categorical must allow an action.  PPO2 then trains a masking core (ppo_core_set_action_masking).
+    virtual bool has_action_mask() { return false; }
+    virtual Mat get_action_mask() { return Mat(); }
     virtual Mat reset() = 0;
     // returns {obs [n,O], rewards [n,1], dones [n,1]}
     virtual std::vector<Mat> step(const Mat& actions) = 0;

@@ -5,6 +5,9 @@
 //                   1/2 [a0 == (c + 1) mod 4] + 1/2 [a1 == c mod 3].  A uniform policy earns 1/2 (1/4 + 1/3).
 //   MULTI_BINARY    MultiBinary(4): the observation is the bit pattern of a context c in 0 .. 15; the action is 4 columns of 0 / 1;
 //                   the reward is the fraction of action bits equal to c's bits.  A uniform policy earns 1/2.
+//   MASKED          Discrete(4) on the one-hot context c in 0 .. 3 with invalid-action masks: c forbids one or two actions, never the
+//                   rewarded one (c + 1) mod 4; the reward is 1 for that action and 0 otherwise.  A uniform policy over the allowed
+//                   actions earns 1/2 or 1/3.  The env counts the forbidden actions it receives (illegal_actions()).
 // A new context is drawn (splitmix64 of seed, env id and step) after every step; episodes last 16 steps.  The learned policy
 // earns up to 1 per step, so learning is visible in the mean reward.
 #ifndef PPO_B200_ENV_BANDIT_HPP
@@ -16,12 +19,19 @@
 
 class BanditEnv : public Env {
 public:
-    enum Mode { DISCRETE, MULTI_DISCRETE, MULTI_BINARY };
+    enum Mode { DISCRETE, MULTI_DISCRETE, MULTI_BINARY, MASKED };
     explicit BanditEnv(uint64_t seed = 0x1234, uint32_t env_id = 0, int n = 4, Mode mode = DISCRETE)
         : seed{seed}, env_id{env_id}, n{mode == DISCRETE ? n : 4}, mode{mode}, obs(1, this->n) { reset(); }
     std::string get_action_space() override {
-        return mode == DISCRETE ? Env::SPACE_DISCRETE() : mode == MULTI_DISCRETE ? Env::SPACE_MULTI_DISCRETE() : Env::SPACE_MULTI_BINARY();
+        return mode == DISCRETE || mode == MASKED ? Env::SPACE_DISCRETE() : mode == MULTI_DISCRETE ? Env::SPACE_MULTI_DISCRETE() : Env::SPACE_MULTI_BINARY();
     }
+    bool has_action_mask() override { return mode == MASKED; }
+    Mat get_action_mask() override {
+        Mat m(1, n);
+        for (int k = 0; k < n; ++k) m(0, k) = allowed(k) ? 1.f : 0.f;
+        return m;
+    }
+    long illegal_actions() const { return illegal; }
     std::string get_observation_space() override { return Env::SPACE_CONTINOUS(); }
     int get_action_space_size() override { return mode == MULTI_DISCRETE ? 4 + 3 : n; }
     std::vector<int> get_action_space_nvec() override { return mode == MULTI_DISCRETE ? std::vector<int>{4, 3} : std::vector<int>{}; }
@@ -32,8 +42,10 @@ public:
         return obs;
     }
     std::vector<Mat> step(const Mat& actions) override {
-        if (mode == DISCRETE) {
-            last_rew = static_cast<int>(actions(0, 0)) == (ctx + 1) % n ? 1.f : 0.f;
+        if (mode == DISCRETE || mode == MASKED) {
+            const int a = static_cast<int>(actions(0, 0));
+            if (mode == MASKED && !allowed(a)) ++illegal;
+            last_rew = a == (ctx + 1) % n ? 1.f : 0.f;
         } else if (mode == MULTI_DISCRETE) {
             last_rew = 0.5f * (static_cast<int>(actions(0, 0)) == (ctx + 1) % 4 ? 1.f : 0.f) + 0.5f * (static_cast<int>(actions(0, 1)) == ctx % 3 ? 1.f : 0.f);
         } else {
@@ -61,6 +73,8 @@ public:
     float get_time() override { return static_cast<float>(t_env); }
 
 private:
+    // MASKED: context c forbids c itself, and (c + 2) mod 4 as well in odd contexts; (c + 1) mod 4, the rewarded action, stays allowed
+    bool allowed(int a) const { return a != ctx && !((ctx & 1) && a == (ctx + 2) % n); }
     void draw() {
         uint64_t z = seed + 0x9E3779B97F4A7C15ull * (((uint64_t)env_id << 32) + (++draws));
         z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
@@ -78,6 +92,7 @@ private:
     uint32_t t_env = 0;
     uint64_t draws = 0;
     float last_rew = 0.f;
+    long illegal = 0;
 };
 
 #endif

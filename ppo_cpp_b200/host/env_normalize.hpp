@@ -23,6 +23,8 @@ public:
     std::string get_observation_space() override { return env->get_observation_space(); }
     int get_action_space_size() override { return env->get_action_space_size(); }
     std::vector<int> get_action_space_nvec() override { return env->get_action_space_nvec(); }
+    bool has_action_mask() override { return env->has_action_mask(); }
+    Mat get_action_mask() override { return env->get_action_mask(); }
     int get_observation_space_size() override { return env->get_observation_space_size(); }
     int get_num_envs() override { return env->get_num_envs(); }
 

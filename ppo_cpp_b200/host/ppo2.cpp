@@ -1,7 +1,7 @@
 // CLI with the reference's flags (ppo2.cpp:93-128) driving the B200 core.  Envs: the DART hexapod cannot be
 // built here (SURVEY §2 row 12); `--env synthetic` (default) is the host-side stand-in with the same shapes,
 // `--env mock` is the reference's EnvMock, `--env bandit` a Discrete(4) contextual bandit for the categorical head, `--env bandit_md` / `bandit_mb` its MultiDiscrete([4, 3]) /
-// MultiBinary(4) modes.  New flags: --env, --seed (commented out in the reference,
+// MultiBinary(4) modes, `--env bandit_mask` the Discrete(4) bandit with invalid-action masks.  New flags: --env, --seed (commented out in the reference,
 // ppo2.cpp:130-131), --hidden H1,H2 (graph-less orthogonal init when no --graph is given).
 #include <chrono>
 #include <cstdlib>
@@ -87,7 +87,8 @@ int main(int argc, char** argv) {
                      "  -d --dir, -g --graph --graph_path, -p --path, --id, -s --steps, -l --lr, -e --ent, -c --cr,\n"
                      "  --saves, --epochs --num_epochs, --batch_steps --n_steps, --rns, --cl, -v, -r --resume, --bullet,\n"
                      "  --duration, -j --threads, -f --fps   (as in the reference's ppo2.cpp:93-128)\n"
-                     "  --env synthetic|mock|bandit|bandit_md|bandit_mb (contextual bandits: Discrete(4), MultiDiscrete([4, 3]), MultiBinary(4)),\n"
+                     "  --env synthetic|mock|bandit|bandit_md|bandit_mb|bandit_mask (contextual bandits: Discrete(4), MultiDiscrete([4, 3]), MultiBinary(4),\n"
+                     "       Discrete(4) with invalid-action masks),\n"
                      "  --seed N, --hidden H1,H2,\n"
                      "  --cliprange_vf (-1: the graph's value loss decides; >= 0 for a graph with loss/clip_range_vf_ph),\n"
                      "  --activation tanh|relu (graph-less runs; with a graph it must name the graph's own activation)\n";
@@ -130,11 +131,17 @@ int main(int argc, char** argv) {
 
     std::unique_ptr<Env> wrapped_env;
     std::vector<std::shared_ptr<Env>> envs;
-    const bool bandit = env_kind == "bandit" || env_kind == "bandit_md" || env_kind == "bandit_mb";
-    const BanditEnv::Mode bandit_mode = env_kind == "bandit_md" ? BanditEnv::MULTI_DISCRETE : env_kind == "bandit_mb" ? BanditEnv::MULTI_BINARY : BanditEnv::DISCRETE;
+    const bool bandit = env_kind == "bandit" || env_kind == "bandit_md" || env_kind == "bandit_mb" || env_kind == "bandit_mask";
+    const BanditEnv::Mode bandit_mode = env_kind == "bandit_md" ? BanditEnv::MULTI_DISCRETE : env_kind == "bandit_mb" ? BanditEnv::MULTI_BINARY
+                                        : env_kind == "bandit_mask" ? BanditEnv::MASKED : BanditEnv::DISCRETE;
+    std::vector<const BanditEnv*> bandits;  // bandit_mask reports the forbidden actions they received
     auto make_env = [&](int i) -> std::shared_ptr<Env> {
         if (env_kind == "mock") return std::make_shared<EnvMock>(1.0);
-        if (bandit) return std::make_shared<BanditEnv>(static_cast<uint64_t>(seed_val) ^ 0x1234ull, static_cast<uint32_t>(i), 4, bandit_mode);
+        if (bandit) {
+            auto e = std::make_shared<BanditEnv>(static_cast<uint64_t>(seed_val) ^ 0x1234ull, static_cast<uint32_t>(i), 4, bandit_mode);
+            bandits.push_back(e.get());
+            return e;
+        }
         return std::make_shared<SyntheticEnv>(static_cast<uint64_t>(seed_val) ^ 0x1234ull, static_cast<uint32_t>(i));
     };
     if (threads > 1) {
@@ -143,7 +150,9 @@ int main(int argc, char** argv) {
     } else if (env_kind == "mock") {
         wrapped_env = std::make_unique<EnvMock>(1.0);
     } else if (bandit) {
-        wrapped_env = std::make_unique<BanditEnv>(static_cast<uint64_t>(seed_val) ^ 0x1234ull, 0, 4, bandit_mode);
+        auto e = std::make_unique<BanditEnv>(static_cast<uint64_t>(seed_val) ^ 0x1234ull, 0, 4, bandit_mode);
+        bandits.push_back(e.get());
+        wrapped_env = std::move(e);
     } else {
         wrapped_env = std::make_unique<SyntheticEnv>(static_cast<uint64_t>(seed_val) ^ 0x1234ull, 0);
     }
@@ -190,6 +199,11 @@ int main(int argc, char** argv) {
             if (out[2](0, 0) > .5f) break;
         }
         std::cout << "episode_reward: " << episode_reward << std::endl;
+    }
+    if (bandit_mode == BanditEnv::MASKED) {
+        long illegal = 0;
+        for (const BanditEnv* b : bandits) illegal += b->illegal_actions();
+        std::cout << "illegal_actions " << illegal << std::endl;
     }
     return 0;
 }

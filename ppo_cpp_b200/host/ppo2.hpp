@@ -150,6 +150,7 @@ public:
             ppo_check(ppo_core_set_activation(core_.get(), activation_), "activation");
         }
         ppo_check(ppo_shuffle_seed(core_.get(), shuffle_seed_), "shuffle seed");
+        if (env.has_action_mask()) ppo_check(ppo_core_set_action_masking(core_.get(), 1), "action masks");
         if (normalize) normalize->attach_core(core_);
         act_model = std::make_unique<MlpPolicy>(core_, action_width(env));
     }
@@ -227,8 +228,10 @@ public:
         std::cout << "Success load weights !! " << std::endl;
     }
 
+    // obs is the env's current observation: an env with action masks hands in its current mask with it
     Mat eval(const Mat& obs) const {
-        Mat actions = act_model->get_deterministic_action(obs);
+        const Mat mask = env.has_action_mask() ? env.get_action_mask() : Mat();
+        Mat actions = act_model->get_deterministic_action(obs, env.has_action_mask() ? &mask : nullptr);
         assert(actions.rows() == obs.rows() && actions.cols() == action_width(env));
         return actions;
     }

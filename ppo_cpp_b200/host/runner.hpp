@@ -26,7 +26,8 @@ public:
         // obs{env.reset()} (runner.hpp:48): the raw reset observation goes to the core, which applies
         // EnvNormalize::reset (statistics update + normalise + clip) on the device.
         const Mat raw = normalize ? normalize->inner().reset() : env.reset();
-        ppo_check(ppo_runner_reset(model.core().get(), raw.data(), PPO_HOST), "Runner::Runner");
+        if (env.has_action_mask()) ppo_check(ppo_runner_reset_masked(model.core().get(), raw.data(), mask_bytes().data(), PPO_HOST), "Runner::Runner");
+        else ppo_check(ppo_runner_reset(model.core().get(), raw.data(), PPO_HOST), "Runner::Runner");
     }
 
     // fetch_all = false skips the device->host export of the eight rollout buffers (PPO2::learn trains on the
@@ -40,7 +41,10 @@ public:
             const std::vector<Mat>& r = stepper.step(actions);  // env handles action clipping (runner.hpp:112)
             assert(r[0].rows() == num_envs && r[0].cols() == env.get_observation_space_size());
             assert(r[1].rows() == num_envs && r[1].cols() == 1 && r[2].rows() == num_envs && r[2].cols() == 1);
-            ppo_check(ppo_runner_observe(core, step, r[0].data(), r[1].data(), r[2].data(), PPO_HOST), "Runner::run observe");
+            if (env.has_action_mask())  // the mask of the observation the env just returned
+                ppo_check(ppo_runner_observe_masked(core, step, r[0].data(), r[1].data(), r[2].data(), mask_bytes().data(), PPO_HOST), "Runner::run observe");
+            else
+                ppo_check(ppo_runner_observe(core, step, r[0].data(), r[1].data(), r[2].data(), PPO_HOST), "Runner::run observe");
         }
         ppo_check(ppo_runner_finish(core), "Runner::run finish");  // set_returns (runner.hpp:159-191)
         MiniBatch mb{};
@@ -65,6 +69,8 @@ public:
     }
 
 private:
+    // the env's current action mask as the C ABI takes it
+    std::vector<uint8_t> mask_bytes() { return action_mask_bytes(env.get_action_mask()); }
     Env& env;
     MlpPolicy& model;
     int n_steps;

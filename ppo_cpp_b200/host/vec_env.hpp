@@ -50,6 +50,13 @@ public:
     std::string get_observation_space() override { return envs[0]->get_observation_space(); }
     int get_action_space_size() override { return envs[0]->get_action_space_size(); }
     std::vector<int> get_action_space_nvec() override { return envs[0]->get_action_space_nvec(); }
+    bool has_action_mask() override { return envs[0]->has_action_mask(); }
+    // row i: sub-env i's mask (read between steps, when no worker touches the envs)
+    Mat get_action_mask() override {
+        Mat result = Mat::Zero(get_num_envs(), get_action_space_size());
+        for (size_t i = 0; i < envs.size(); ++i) result.set_row(static_cast<int>(i), envs[i]->get_action_mask());
+        return result;
+    }
     int get_observation_space_size() override { return envs[0]->get_observation_space_size(); }
     int get_num_envs() override { return static_cast<int>(envs.size()); }
 
